@@ -253,6 +253,47 @@ LGMI_API int lgmi_batch_device_ptrs(lgmi_batch_t* b, void** d_planes, void** d_s
  * 16 B per emitted record, 12 B per site.                                     */
 LGMI_API int lgmi_batch_algorithmic_bytes(lgmi_batch_t* b, uint64_t* bytes);
 
+/* ----- split units: one deep unit over several batches / devices ----------- *
+ * A unit whose pair work is too large for one device is cut into pieces by    *
+ * rows of its pair grid.  The piece of rows [a, b) of a unit of S sites is    *
+ * the SUFFIX unit of sites [a, S) (plane_off + 3*a*W, n_sites S - a,          *
+ * site_off + a: no re-encoding) with row limit b - a: only its pairs (i, j)   *
+ * with i < b - a are evaluated, and they are a prefix of the suffix's pair    *
+ * order.  The pieces' records, in row order, with i and j shifted by a, are   *
+ * the whole unit's records.                                                   *
+ *                                                                             *
+ * lgmi_batch_create with a row limit per unit: row_limit[k] == 0 is an        *
+ * ordinary unit (exactly as lgmi_batch_create); otherwise unit k is a piece   *
+ * and row_limit[k] is a multiple of 128 or n_sites (else LGMI_ERR_ARG).  A    *
+ * piece keeps the MI of its pairs in pair order in the batch (NaN: no MI),    *
+ * its site_mean / site_cnt entries stay NaN / 0, and n_candidates and         *
+ * n_evaluated count its own pairs.                                            */
+LGMI_API int lgmi_batch_create_rows(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units,
+                                    const uint32_t* row_limit, uint64_t plane_words, uint64_t n_sites,
+                                    lgmi_batch_t** out);
+/* async H2D of word_end - word_begin plane words from `planes` (host memory  *
+ * holding just those words) to the batch's plane words [word_begin,           *
+ * word_end), and of all site_flags (n_sites bytes)                            */
+LGMI_API int lgmi_batch_upload_rows(lgmi_batch_t* b, const uint32_t* planes, uint64_t word_begin, uint64_t word_end,
+                                    const uint8_t* site_flags);
+/* device-to-device copy of n_words plane words of another batch (possibly on  *
+ * another device) into this one, queued on dst's stream behind everything     *
+ * src's stream has queued at the time of the call (its upload).  Peer access  *
+ * is enabled where the devices allow it; the copy works without.             */
+LGMI_API int lgmi_batch_copy_planes(lgmi_batch_t* dst, uint64_t dst_word, const lgmi_batch_t* src, uint64_t src_word,
+                                    uint64_t n_words);
+/* The per-site means and counts of a split unit of n_sites sites: n_pieces    *
+ * pieces in row order, piece p being unit unit_in_batch[p] of batches[p],     *
+ * each already run (on any device).  Their MI slices are gathered back to     *
+ * back on ctx's device and the per-site pass of an unsplit run is applied to  *
+ * the result: the same bits as lgmi_batch_create + run of the whole unit      *
+ * (mutual_information.py:48-60).  site_flags: the unit's n_sites flag bytes.  *
+ * LGMI_ERR_STATE if a piece has not been run, LGMI_ERR_ARG if the pieces do   *
+ * not make up the unit.                                                       */
+LGMI_API int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site_flags, uint32_t n_pieces,
+                              lgmi_batch_t* const* batches, const uint32_t* unit_in_batch, double* mean_out,
+                              uint32_t* cnt_out);
+
 /* ----- pipelined step over HOST buffers ------------------------------------ *
  * Same result as upload + run + download of one batch (mismatch.py:387-404    *
  * for every unit), but the units are cut into n_chunks consecutive groups of  *

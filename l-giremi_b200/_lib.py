@@ -44,6 +44,7 @@ EXPORTS = (
     "lgmi_set_small_path", "lgmi_set_tile_path", "lgmi_set_dense_path",
     "lgmi_batch_create", "lgmi_batch_destroy", "lgmi_batch_upload", "lgmi_batch_run",
     "lgmi_batch_download", "lgmi_batch_sync", "lgmi_batch_device_ptrs",
+    "lgmi_batch_create_rows", "lgmi_batch_upload_rows", "lgmi_batch_copy_planes", "lgmi_split_means",
     "lgmi_batch_algorithmic_bytes", "lgmi_pipeline_create", "lgmi_pipeline_step", "lgmi_pipeline_step_packed",
     "lgmi_pipeline_begin", "lgmi_pipeline_begin_packed", "lgmi_pipeline_collect", "lgmi_pipeline_finish",
     "lgmi_pipeline_destroy",
@@ -119,6 +120,10 @@ def load():
         "lgmi_batch_sync": (i32, [vp, C.POINTER(Result)]),
         "lgmi_batch_device_ptrs": (i32, [vp, pvp, pvp, pvp, pvp]),
         "lgmi_batch_algorithmic_bytes": (i32, [vp, C.POINTER(u64)]),
+        "lgmi_batch_create_rows": (i32, [vp, vp, u32, vp, u64, u64, pvp]),
+        "lgmi_batch_upload_rows": (i32, [vp, vp, u64, u64, vp]),
+        "lgmi_batch_copy_planes": (i32, [vp, u64, vp, u64, u64]),
+        "lgmi_split_means": (i32, [vp, u32, vp, u32, vp, vp, vp, vp]),
         "lgmi_pipeline_create": (i32, [vp, vp, u32, u64, u64, u32, pvp]),
         "lgmi_pipeline_step": (i32, [vp, vp, vp, i32, u32, C.POINTER(Result)]),
         "lgmi_pipeline_step_packed": (i32, [vp, vp, vp, i32, u32, C.POINTER(Result)]),

@@ -211,14 +211,24 @@ class StepResult:
 
 
 class Batch:
-    """Device-side batch: create once, then upload / run / download repeatedly."""
+    """Device-side batch: create once, then upload / run / download repeatedly.
 
-    def __init__(self, ctx: Context, pb: PlaneBatch):
+    row_limit (one entry per unit, or None): a unit with a non-zero entry is a piece of a split unit -- the suffix
+    of sites [a, S) of a unit, of which only the pairs (i, j) with i < row_limit are evaluated and emitted
+    (lgmi_batch_create_rows).  Its site_mean / site_cnt entries stay NaN / 0: split_means gives them."""
+
+    def __init__(self, ctx: Context, pb: PlaneBatch, row_limit=None):
         self.ctx, self.pb = ctx, pb
         self._lib = ctx._lib
         h = C.c_void_p()
-        check(self._lib.lgmi_batch_create(ctx.handle, ptr(pb.units), pb.n_units, pb.planes.size,
-                                          pb.n_sites, C.byref(h)), ctx.handle)
+        if row_limit is None:
+            check(self._lib.lgmi_batch_create(ctx.handle, ptr(pb.units), pb.n_units, pb.planes.size,
+                                              pb.n_sites, C.byref(h)), ctx.handle)
+        else:
+            self.row_limit = np.ascontiguousarray(row_limit, dtype=np.uint32)
+            assert self.row_limit.size == pb.n_units
+            check(self._lib.lgmi_batch_create_rows(ctx.handle, ptr(pb.units), pb.n_units, ptr(self.row_limit),
+                                                   pb.planes.size, pb.n_sites, C.byref(h)), ctx.handle)
         self.handle = h
 
     def upload(self, planes=None, site_flags=None):
@@ -228,6 +238,23 @@ class Batch:
         assert site_flags.dtype == np.uint8 and site_flags.size == self.pb.n_sites
         self._keep = (planes, site_flags)
         check(self._lib.lgmi_batch_upload(self.handle, ptr(planes), ptr(site_flags)), self.ctx.handle)
+
+    def upload_rows(self, word_begin, words, site_flags=None):
+        """Uploads the host words `words` to the plane words [word_begin, word_begin + len(words)) of the batch,
+        and every flag byte; the rest of the planes comes from elsewhere, e.g. copy_planes_from.  The host arrays
+        must stay untouched until the next sync."""
+        words = np.ascontiguousarray(words, dtype=np.uint32)
+        site_flags = self.pb.site_flags if site_flags is None else site_flags
+        assert site_flags.dtype == np.uint8 and site_flags.size == self.pb.n_sites
+        self._keep_rows = getattr(self, "_keep_rows", []) + [words, site_flags]
+        check(self._lib.lgmi_batch_upload_rows(self.handle, ptr(words), int(word_begin), int(word_begin) + words.size,
+                                               ptr(site_flags)), self.ctx.handle)
+
+    def copy_planes_from(self, dst_word, src: "Batch", src_word, n_words):
+        """Device-to-device copy of n_words plane words of `src` (any device) to dst_word of this batch, behind
+        whatever src's stream has queued (lgmi_batch_copy_planes)."""
+        check(self._lib.lgmi_batch_copy_planes(self.handle, int(dst_word), src.handle, int(src_word), int(n_words)),
+              self.ctx.handle)
 
     def run(self, min_common, mode=MODE_ALL_PAIRS):
         check(self._lib.lgmi_batch_run(self.handle, int(min_common), int(mode)), self.ctx.handle)
@@ -378,6 +405,20 @@ def stream_steps(pipes, inputs, min_common, mode=MODE_HET_ONLY, copy=True, packe
         res = pipes[j % depth].finish(copy=copy)
         del held[j]
         yield j, res
+
+
+def split_means(ctx: Context, site_flags, pieces):
+    """Per-site mean MI and row count of a split unit (lgmi_split_means): `pieces` = [(Batch, unit index in it)]
+    in row order, each already run; `site_flags` the unit's flag bytes.  The same bits as an unsplit run."""
+    flags = np.ascontiguousarray(site_flags, dtype=np.uint8)
+    n = flags.size
+    handles = (C.c_void_p * len(pieces))(*[b.handle.value for b, _k in pieces])
+    units = np.array([k for _b, k in pieces], dtype=np.uint32)
+    mean = np.empty(n, dtype=np.float64)
+    cnt = np.empty(n, dtype=np.uint32)
+    check(ctx._lib.lgmi_split_means(ctx.handle, n, ptr(flags), len(pieces), C.cast(handles, C.c_void_p), ptr(units),
+                                    ptr(mean), ptr(cnt)), ctx.handle)
+    return mean, cnt
 
 
 PIPELINE_MIN_CANDIDATES = 2_000_000   # below this one submit is as fast as a pipelined one

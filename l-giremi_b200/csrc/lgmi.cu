@@ -154,6 +154,7 @@ struct DenseTileList {
 };
 struct DensePlan {
   uint32_t unit = 0, S = 0, W = 0, S_pad = 0, k_blocks = 0;
+  uint32_t rows = 0;          // pairs (i, j) with i < rows are read: S, or the row limit of a piece
   uint32_t oth_cap = 0;       // listed "other" reads per site (four-block form)
   bool four = false;          // the four-block form may be chosen (else the run is told "nine" up front)
   DenseTileList list4, list9; // P, M x P, M  /  C, P, M x C, P, M
@@ -250,15 +251,37 @@ struct lgmi_batch {
   // candidates with a het_snp partner (what SKIP_NONHET evaluates); known once host flags have been seen
   uint64_t n_het_candidates = 0;
   bool het_known = false;
+  // lgmi_batch_create_rows: per unit its row limit (0: an ordinary unit) and first dense slot; empty otherwise
+  std::vector<uint32_t> h_row_limit;
+  std::vector<uint64_t> h_dense_off;
+  cudaEvent_t copy_ev = nullptr;  // lgmi_batch_copy_planes from this batch: what its stream has queued so far
 };
 
-// candidate pairs next to a het_snp site, from the host copy of the flag bytes
-static uint64_t het_candidates(const std::vector<lgmi_unit_desc>& units, const uint8_t* site_flags) {
+// pairs (i, j), i < j < S, with i < rows: the first rows rows of the pair order (lg_row_off(rows, S))
+static uint64_t piece_pairs(uint32_t rows, uint32_t S) { return rows ? lg_row_off(rows, S) : 0ull; }
+
+// candidate pairs next to a het_snp site, from the host copy of the flag bytes (a piece: its own pairs only)
+static uint64_t het_candidates(const std::vector<lgmi_unit_desc>& units, const std::vector<uint32_t>& row_limit,
+                               const uint8_t* site_flags) {
   uint64_t tot = 0;
-  for (const lgmi_unit_desc& u : units) {
+  for (size_t k = 0; k < units.size(); ++k) {
+    const lgmi_unit_desc& u = units[k];
+    const uint8_t* f = site_flags + u.site_off;
+    auto het = [&](uint32_t s) { return (f[s] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP; };
+    const uint32_t rows = row_limit.empty() ? 0u : row_limit[k];
+    if (rows) {
+      // pairs of the piece minus those whose sites are both non-het: walk the rows from the last, counting the
+      // non-het sites after each
+      uint64_t o_after = 0, both = 0;
+      for (uint32_t s = u.n_sites; s-- > 0;) {
+        if (s < rows && !het(s)) both += o_after;
+        o_after += het(s) ? 0u : 1u;
+      }
+      tot += piece_pairs(rows, u.n_sites) - both;
+      continue;
+    }
     uint64_t h = 0;
-    for (uint32_t s = 0; s < u.n_sites; ++s)
-      h += (site_flags[u.site_off + s] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP ? 1u : 0u;
+    for (uint32_t s = 0; s < u.n_sites; ++s) h += het(s) ? 1u : 0u;
     const uint64_t S = u.n_sites, o = S - h;
     tot += (S >= 2 ? S * (S - 1) / 2 : 0) - (o >= 2 ? o * (o - 1) / 2 : 0);
   }
@@ -519,6 +542,7 @@ extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
   ctx->dev_pool.release(b->d_oth_cnt);
   ctx->dev_pool.release(b->d_oth_list);
   ctx->dev_pool.release(b->d_unit_mode);
+  if (b->copy_ev) cudaEventDestroy(b->copy_ev);
   if (b->side_stream) cudaStreamDestroy(b->side_stream);
   for (cudaEvent_t e : b->side_ev)
     if (e) cudaEventDestroy(e);
@@ -543,8 +567,11 @@ extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
   delete b;
 }
 
-extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units,
-                                 uint64_t plane_words, uint64_t n_sites, lgmi_batch_t** out) {
+// lgmi_batch_create, and with row_limit (non-NULL) lgmi_batch_create_rows: a unit k with row_limit[k] != 0 is a
+// piece of a split unit -- only its pairs (i, j) with i < row_limit[k] are evaluated and emitted, always through a
+// dense MI slot (the slices of the pieces make up the whole unit's, lgmi_split_means), and it has no per-site means
+static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units, const uint32_t* row_limit,
+                        uint64_t plane_words, uint64_t n_sites, lgmi_batch_t** out) {
   if (!ctx || !out || (!units && n_units)) return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_create: NULL argument");
   *out = nullptr;
   CU(ctx, cudaSetDevice(ctx->device));
@@ -555,6 +582,10 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
   b->plane_words = plane_words;
   b->n_sites = n_sites;
   b->h_units.assign(units, units + n_units);
+  if (row_limit) {
+    b->h_row_limit.assign(row_limit, row_limit + n_units);
+    b->h_dense_off.assign(n_units, ~0ull);
+  }
 
   std::vector<DevUnit> du(n_units);
   std::vector<FastItem> fast_items, pre_items;
@@ -582,6 +613,14 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
                   "unit %u: inconsistent descriptor (S=%u R=%u W=%u plane_off=%llu site_off=%u)", k,
                   u.n_sites, u.n_reads, u.row_words, (unsigned long long)u.plane_off, u.site_off);
     }
+    const uint32_t limit = row_limit ? row_limit[k] : 0u;
+    const bool piece = limit != 0u;
+    if (piece && (limit > u.n_sites || (limit % 128u && limit != u.n_sites))) {
+      delete b;
+      return fail(ctx, LGMI_ERR_ARG, "unit %u: row limit %u is neither a multiple of 128 below S nor S = %u", k, limit,
+                  u.n_sites);
+    }
+    const uint32_t rows = piece ? limit : u.n_sites;  // row blocks at or past it hold no pair of the unit
     const size_t first_gram_tile = gram_tiles.size();  // this unit's k_tile_gram work items start here
     DevUnit& d = du[k];
     d.plane_off = u.plane_off;
@@ -590,7 +629,7 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
     d.W = u.row_words;
     d.site_off = u.site_off;
     d.first_item = (uint32_t)b->h_items.size();
-    const uint64_t np = u.n_sites >= 2 ? (uint64_t)u.n_sites * (u.n_sites - 1) / 2 : 0;
+    const uint64_t np = piece ? piece_pairs(limit, u.n_sites) : u.n_sites >= 2 ? (uint64_t)u.n_sites * (u.n_sites - 1) / 2 : 0;
     b->n_candidates += np;
     b->max_reads = std::max(b->max_reads, u.n_reads);
     const uint32_t nit = np ? (uint32_t)((np + kPairsMax - 1) / kPairsMax) : 1u;
@@ -606,6 +645,7 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
       pl.S = u.n_sites;
       pl.W = u.row_words;
       pl.S_pad = (u.n_sites + (uint32_t)kDenseBN - 1u) / (uint32_t)kDenseBN * (uint32_t)kDenseBN;
+      pl.rows = rows;
       pl.k_blocks = u.row_words * 32u / (uint32_t)kDenseBK;  // W is a multiple of 4: whole 128-read blocks
       pl.plane_off = u.plane_off;
       pl.gram_off = gram_words;
@@ -617,7 +657,7 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
         for (uint32_t a = g0; a < 3; ++a)
           for (uint32_t bb = g0; bb < 3; ++bb)
             for (uint32_t J = 0; J < pl.S_pad / (uint32_t)kDenseBN; ++J)
-              for (uint32_t I = 0; I < pl.S_pad / (uint32_t)kDenseBM; ++I) {
+              for (uint32_t I = 0; I < (rows + (uint32_t)kDenseBM - 1u) / (uint32_t)kDenseBM; ++I) {
                 // some pair i < j inside the tile, both real sites
                 const uint32_t i_min = I * (uint32_t)kDenseBM;
                 const uint32_t j_max = std::min(J * (uint32_t)kDenseBN + (uint32_t)kDenseBN, pl.S) - 1u;
@@ -661,18 +701,18 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
       d.gram_off = pl.gram_off;
       d.S_pad = pl.S_pad;
       b->dense_plans.push_back(pl);
-    } else if (np && !(nit == 1 && u.n_sites <= (uint32_t)kFastMaxS && u.n_reads <= (uint32_t)kFastMaxR)) {
+    } else if (np && (piece || !(nit == 1 && u.n_sites <= (uint32_t)kFastMaxS && u.n_reads <= (uint32_t)kFastMaxR))) {
       // tiled popcount path: MI of every pair precomputed by k_tile_mi into the dense scratch
       // (or, by default, counted on the tensor cores by k_tile_gram and finished by k_tile_finish)
       const bool gram = ctx->tile_path && u.n_reads >= 1u && u.n_reads <= kTgMaxReads;
       d.tiled = gram ? 2 : 1;
-      if (nit == 1) {
+      if (nit == 1 && !piece) {
         d.dense_off = dense;
         dense += np;
       }
       if (gram) {
         any_gram_tiled = true;
-        const uint32_t nI = (u.n_sites + (uint32_t)kTgSitesI - 1u) / (uint32_t)kTgSitesI;
+        const uint32_t nI = (rows + (uint32_t)kTgSitesI - 1u) / (uint32_t)kTgSitesI;
         const uint32_t nJ = (u.n_sites + (uint32_t)kTgSitesJ - 1u) / (uint32_t)kTgSitesJ;
         for (uint32_t I = 0; I < nI; ++I)
           for (uint32_t J = 0; J < nJ; ++J) {
@@ -684,25 +724,27 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
           }
       } else {
         const uint32_t nb = (u.n_sites + (uint32_t)kTileSites - 1u) / (uint32_t)kTileSites;
-        for (uint32_t I = 0; I < nb; ++I)
+        for (uint32_t I = 0; I < (rows + (uint32_t)kTileSites - 1u) / (uint32_t)kTileSites; ++I)
           for (uint32_t J = I; J < nb; ++J) {
             tile_items.push_back(TileItem{k, (uint16_t)I, (uint16_t)J});
             tile_words.push_back(u.row_words);
           }
       }
     }
-    if (nit > 1) {
+    if (nit > 1 || piece) {
       d.dense_off = dense;
       dense += np;
-      for (uint32_t s0 = 0; s0 < u.n_sites; s0 += (uint32_t)kMeanSites) mean_items.push_back(MeanItem{k, s0});
+      if (!piece)  // (a piece's means would be partial: lgmi_split_means computes them over all pieces)
+        for (uint32_t s0 = 0; s0 < u.n_sites; s0 += (uint32_t)kMeanSites) mean_items.push_back(MeanItem{k, s0});
     }
+    if (piece) b->h_dense_off[k] = d.dense_off;
     for (size_t t = first_gram_tile; t < gram_tiles.size(); ++t) gram_tiles[t].dense_off = d.dense_off;  // known now
     for (uint32_t t = 0; t < nit; ++t) {
       Item it;
       it.unit = k;
       it.pair_begin = t * (uint32_t)kPairsMax;
       it.pair_cnt = (uint32_t)std::min<uint64_t>(kPairsMax, np - (uint64_t)t * kPairsMax);
-      it.flags = (t == 0 ? ITEM_FIRST : 0u) | (nit == 1 ? ITEM_SINGLE : 0u) | (d.tiled ? ITEM_TILED : 0u) |
+      it.flags = (t == 0 ? ITEM_FIRST : 0u) | (nit == 1 && !piece ? ITEM_SINGLE : 0u) | (d.tiled ? ITEM_TILED : 0u) |
                  (d.tiled == 2 ? ITEM_TILED_GRAM : 0u) | (d.gram_off != kNoGram ? ITEM_GRAM : 0u);
       if (d.tiled || d.gram_off != kNoGram) ++b->n_tiled_work_items;  // (not k_pairs_generic<0>'s)
       if (d.tiled) {
@@ -712,7 +754,8 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
         td.S = u.n_sites, td.site_off = u.site_off, td.dense_off = d.dense_off;
         tiled_desc.push_back(td);
       }
-      if (nit == 1 && np >= 1 && d.gram_off == kNoGram && u.n_sites <= (uint32_t)kFastMaxS && u.n_reads <= (uint32_t)kFastMaxR) {
+      if (!piece && nit == 1 && np >= 1 && d.gram_off == kNoGram && u.n_sites <= (uint32_t)kFastMaxS &&
+          u.n_reads <= (uint32_t)kFastMaxR) {
         it.flags |= ITEM_FAST;  // (a unit sent to the tensor-core path by a lowered threshold is not also k_pairs_fast's)
         FastItem f;
         f.plane_off = u.plane_off;
@@ -881,6 +924,19 @@ extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint3
   return LGMI_OK;
 }
 
+extern "C" int lgmi_batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units,
+                                 uint64_t plane_words, uint64_t n_sites, lgmi_batch_t** out) {
+  return batch_create(ctx, units, n_units, nullptr, plane_words, n_sites, out);
+}
+
+extern "C" int lgmi_batch_create_rows(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units,
+                                      const uint32_t* row_limit, uint64_t plane_words, uint64_t n_sites,
+                                      lgmi_batch_t** out) {
+  if (!row_limit && n_units) return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_create_rows: row_limit is NULL");
+  static const uint32_t none = 0u;
+  return batch_create(ctx, units, n_units, n_units ? row_limit : &none, plane_words, n_sites, out);
+}
+
 extern "C" int lgmi_batch_upload(lgmi_batch_t* b, const uint32_t* planes, const uint8_t* site_flags) {
   if (!b) return LGMI_ERR_ARG;
   lgmi_ctx* ctx = b->ctx;
@@ -891,9 +947,60 @@ extern "C" int lgmi_batch_upload(lgmi_batch_t* b, const uint32_t* planes, const 
     CU(ctx, cudaMemcpyAsync(b->d_planes, planes, b->plane_words * sizeof(uint32_t), cudaMemcpyHostToDevice, bstream(b)));
   if (b->n_sites)
     CU(ctx, cudaMemcpyAsync(b->d_flags, site_flags, b->n_sites, cudaMemcpyHostToDevice, bstream(b)));
-  b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, site_flags) : 0;
+  b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags) : 0;
   b->het_known = true;
   b->uploaded = true;
+  return LGMI_OK;
+}
+
+extern "C" int lgmi_batch_upload_rows(lgmi_batch_t* b, const uint32_t* planes, uint64_t word_begin, uint64_t word_end,
+                                      const uint8_t* site_flags) {
+  if (!b) return LGMI_ERR_ARG;
+  lgmi_ctx* ctx = b->ctx;
+  if (word_begin > word_end || word_end > b->plane_words)
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_upload_rows: words [%llu, %llu) outside the %llu plane words",
+                (unsigned long long)word_begin, (unsigned long long)word_end, (unsigned long long)b->plane_words);
+  if ((!planes && word_end > word_begin) || (!site_flags && b->n_sites))
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_upload_rows: NULL input");
+  CU(ctx, cudaSetDevice(ctx->device));
+  if (word_end > word_begin)
+    CU(ctx, cudaMemcpyAsync(b->d_planes + word_begin, planes, (word_end - word_begin) * sizeof(uint32_t),
+                            cudaMemcpyHostToDevice, bstream(b)));
+  if (b->n_sites)
+    CU(ctx, cudaMemcpyAsync(b->d_flags, site_flags, b->n_sites, cudaMemcpyHostToDevice, bstream(b)));
+  b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags) : 0;
+  b->het_known = true;
+  b->uploaded = true;
+  return LGMI_OK;
+}
+
+extern "C" int lgmi_batch_copy_planes(lgmi_batch_t* dst, uint64_t dst_word, const lgmi_batch_t* src, uint64_t src_word,
+                                      uint64_t n_words) {
+  if (!dst || !src) return LGMI_ERR_ARG;
+  lgmi_ctx* ctx = dst->ctx;
+  if (dst_word > dst->plane_words || n_words > dst->plane_words - dst_word || src_word > src->plane_words ||
+      n_words > src->plane_words - src_word)
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_copy_planes: %llu words from %llu to %llu out of range",
+                (unsigned long long)n_words, (unsigned long long)src_word, (unsigned long long)dst_word);
+  if (!n_words) return LGMI_OK;
+  lgmi_batch* s = const_cast<lgmi_batch*>(src);
+  const int sdev = s->ctx->device, ddev = ctx->device;
+  // the copy follows everything src's stream has queued so far (its upload)
+  CU(ctx, cudaSetDevice(sdev));
+  if (!s->copy_ev) CU(ctx, cudaEventCreateWithFlags(&s->copy_ev, cudaEventDisableTiming));
+  CU(ctx, cudaEventRecord(s->copy_ev, bstream(s)));
+  CU(ctx, cudaSetDevice(ddev));
+  if (sdev != ddev) {
+    // direct peer copies where the devices allow them; without peer access the runtime stages through the host
+    int can = 0;
+    if (cudaDeviceCanAccessPeer(&can, ddev, sdev) == cudaSuccess && can &&
+        cudaDeviceEnablePeerAccess(sdev, 0) != cudaSuccess)
+      cudaGetLastError();  // (cudaErrorPeerAccessAlreadyEnabled, or no peer access: the copy works either way)
+  }
+  CU(ctx, cudaStreamWaitEvent(bstream(dst), s->copy_ev, 0));
+  CU(ctx, cudaMemcpyPeerAsync(dst->d_planes + dst_word, ddev, s->d_planes + src_word, sdev, n_words * sizeof(uint32_t),
+                              bstream(dst)));
+  dst->uploaded = true;
   return LGMI_OK;
 }
 
@@ -1040,7 +1147,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       // longer pays for lists and transposes it does not use: 2.01 -> 1.65 ms.)
       CU(ctx, cudaEventRecord(b->fix_fork, bstream(b)));
       CU(ctx, cudaStreamWaitEvent(b->fix_stream, b->fix_fork, 0));
-      k_other_fix<<<pl.S, kFixThreads, 0, b->fix_stream>>>(b->d_xt, K_pad, pl.S, pl.S_pad, b->d_oth_cnt, b->d_oth_list, pl.oth_cap,
+      k_other_fix<<<pl.S, kFixThreads, 0, b->fix_stream>>>(b->d_xt, K_pad, pl.S, pl.S_pad, pl.rows, b->d_oth_cnt, b->d_oth_list, pl.oth_cap,
                                                         b->d_gram + pl.gram_off, mode);
       ++ctx->launches;
       CU(ctx, cudaEventRecord(b->fix_join, b->fix_stream));
@@ -1361,6 +1468,80 @@ extern "C" int lgmi_batch_algorithmic_bytes(lgmi_batch_t* b, uint64_t* bytes) {
   return LGMI_OK;
 }
 
+// --------------------------------------------------------------------------- split units
+// The dense MI slices of a unit's pieces, back to back, are the whole unit's dense MI array (the pieces' pairs are
+// consecutive ranges of its pair order); k_site_mean_dense over that array is the unsplit run's per-site pass.
+extern "C" int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site_flags, uint32_t n_pieces,
+                                lgmi_batch_t* const* batches, const uint32_t* unit_in_batch, double* mean_out,
+                                uint32_t* cnt_out) {
+  if (!ctx || !batches || !unit_in_batch || !n_pieces || (n_sites && (!site_flags || !mean_out || !cnt_out)))
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: NULL argument");
+  const uint32_t S = n_sites;
+  std::vector<uint64_t> slice(n_pieces);
+  uint64_t row = 0, total = 0;  // piece p: the suffix [row, S) with its row limit
+  for (uint32_t p = 0; p < n_pieces; ++p) {
+    lgmi_batch* b = batches[p];
+    if (!b) return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: piece %u is NULL", p);
+    const uint32_t k = unit_in_batch[p];
+    if (k >= b->n_units || b->h_row_limit.empty() || !b->h_row_limit[k])
+      return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: piece %u is not a unit with a row limit", p);
+    if (!b->ran) return fail(ctx, LGMI_ERR_STATE, "lgmi_split_means: piece %u has not been run", p);
+    const uint32_t Sp = b->h_units[k].n_sites, rows = b->h_row_limit[k];
+    if (row >= S || (uint64_t)Sp != S - row)
+      return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: piece %u (%u sites) is not the suffix of sites [%llu, %u)", p, Sp,
+                  (unsigned long long)row, S);
+    slice[p] = piece_pairs(rows, Sp);
+    total += slice[p];
+    row += rows;
+  }
+  const uint64_t np = (uint64_t)S * (S - (S ? 1u : 0u)) / 2;
+  if (row != S || total != np)
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: the pieces cover %llu of %llu rows (%llu of %llu pairs)",
+                (unsigned long long)row, (unsigned long long)S, (unsigned long long)total, (unsigned long long)np);
+  if (!S) return LGMI_OK;
+  // scratch: dense [np] | mean [S] | cnt [S] | flags [S] | unit | mean items
+  auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  const uint32_t n_items = (S + (uint32_t)kMeanSites - 1u) / (uint32_t)kMeanSites;
+  const size_t o_mean = up16(np * sizeof(double)), o_cnt = o_mean + up16((size_t)S * sizeof(double));
+  const size_t o_flags = o_cnt + up16((size_t)S * sizeof(uint32_t)), o_unit = o_flags + up16(S);
+  const size_t o_items = o_unit + up16(sizeof(DevUnit)), bytes = o_items + n_items * sizeof(MeanItem);
+  for (uint32_t p = 0; p < n_pieces; ++p) {  // the pieces' kernels have finished (they may run on other devices)
+    CU(ctx, cudaSetDevice(batches[p]->ctx->device));
+    CU(ctx, cudaStreamSynchronize(bstream(batches[p])));
+  }
+  CU(ctx, cudaSetDevice(ctx->device));
+  int rc = ensure_scratch(ctx, bytes);
+  if (rc) return rc;
+  char* scratch = static_cast<char*>(ctx->d_scratch);
+  uint64_t at = 0;
+  for (uint32_t p = 0; p < n_pieces; ++p) {
+    const lgmi_batch* b = batches[p];
+    if (slice[p])
+      CU(ctx, cudaMemcpyPeerAsync(scratch + at * sizeof(double), ctx->device, b->d_dense + b->h_dense_off[unit_in_batch[p]],
+                                  b->ctx->device, slice[p] * sizeof(double), ctx->stream));
+    at += slice[p];
+  }
+  DevUnit u{};
+  u.S = S;
+  u.dense_off = 0;
+  u.gram_off = kNoGram;
+  std::vector<MeanItem> items(n_items);
+  for (uint32_t t = 0; t < n_items; ++t) items[t] = MeanItem{0u, t * (uint32_t)kMeanSites};
+  CU(ctx, cudaMemcpyAsync(scratch + o_flags, site_flags, S, cudaMemcpyHostToDevice, ctx->stream));
+  CU(ctx, cudaMemcpyAsync(scratch + o_unit, &u, sizeof u, cudaMemcpyHostToDevice, ctx->stream));
+  CU(ctx, cudaMemcpyAsync(scratch + o_items, items.data(), n_items * sizeof(MeanItem), cudaMemcpyHostToDevice, ctx->stream));
+  k_site_mean_dense<<<n_items, kMeanThreads, 0, ctx->stream>>>(
+      reinterpret_cast<const DevUnit*>(scratch + o_unit), reinterpret_cast<const MeanItem*>(scratch + o_items),
+      reinterpret_cast<const uint8_t*>(scratch + o_flags), reinterpret_cast<const double*>(scratch),
+      reinterpret_cast<double*>(scratch + o_mean), reinterpret_cast<uint32_t*>(scratch + o_cnt));
+  ++ctx->launches;
+  CU(ctx, cudaGetLastError());
+  CU(ctx, cudaMemcpyAsync(mean_out, scratch + o_mean, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(ctx, cudaMemcpyAsync(cnt_out, scratch + o_cnt, (size_t)S * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(ctx, cudaStreamSynchronize(ctx->stream));
+  return LGMI_OK;
+}
+
 // --------------------------------------------------------------------------- pipelined step
 // The batch cut into consecutive groups of units, each a batch of its own on its own
 // stream: H2D of group k+1, kernels of group k and D2H of group k-1 overlap (two copy
@@ -1600,7 +1781,7 @@ static int pipeline_begin(lgmi_pipeline* p, const uint32_t* planes, bool packed,
     }
     b->uploaded = true;
     if (mode & LGMI_MODE_SKIP_NONHET) {
-      b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, site_flags + c.site0) : 0;
+      b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags + c.site0) : 0;
       b->het_known = true;
     }
     if (!rc) rc = lgmi_batch_run(b, min_common, mode);

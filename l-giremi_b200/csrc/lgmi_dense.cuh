@@ -200,14 +200,16 @@ __global__ void __launch_bounds__(256) k_dense_x(const uint32_t* __restrict__ pl
 // by a carry-save tree into three words (ones, twos, fours), added into packed 4-bit counters (two such groups),
 // those into packed bytes (252 reads), those into shared memory.  Written where gram_table reads them: slot
 // 0 / 1 / 2 of pair (s, t), t > s, = reads "other" at s and other / minor / major at t; slot 3 / 6 of pair
-// (t, s), t < s, = reads minor / major at t and "other" at s.
+// (t, s), t < s, = reads minor / major at t and "other" at s.  rows: the row limit of a piece of a split unit
+// (S otherwise, a multiple of 128 below S): only pairs with a first site below it are read, so a site at or past
+// it counts its partners below the limit and nothing else.
 constexpr int kFixThreads = 384;  // 12 warps = 3 labels x 2 word halves x 2 read halves
 constexpr uint32_t kFixStride = 65u;  // words of shared memory per partner bit: (bit, word) and (word, bit) walks both hit 32 banks
 
 __device__ __forceinline__ uint32_t fix_spread(uint32_t x, uint32_t q) { return (x >> q) & 0x11111111u; }
 
 __global__ void __launch_bounds__(kFixThreads, 3) k_other_fix(const uint32_t* __restrict__ xt, uint64_t K_pad, uint32_t S,
-                                                           uint32_t S_pad, const uint32_t* __restrict__ cnt,
+                                                           uint32_t S_pad, uint32_t rows, const uint32_t* __restrict__ cnt,
                                                            const uint32_t* __restrict__ list, uint32_t cap,
                                                            uint32_t* __restrict__ gram, const uint32_t* __restrict__ mode) {
   if (*mode) return;
@@ -215,15 +217,16 @@ __global__ void __launch_bounds__(kFixThreads, 3) k_other_fix(const uint32_t* __
   const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
   const uint32_t label = warp % 3u, half = (warp / 3u) & 1u, parity = warp / 6u;
   const uint32_t s = blockIdx.x, Sw = S_pad >> 5;
+  const uint32_t Sw_s = s < rows ? Sw : rows >> 5;  // words of the partners this site needs
   const uint32_t n = min(cnt[s], cap);
   const uint32_t* __restrict__ mine = list + (size_t)s * cap;
   const size_t plane = (size_t)S_pad * S_pad;
   const uint32_t n_mine = n > parity ? (n - parity + 1u) / 2u : 0u;  // this warp's listed reads: k = parity + 2 m
-  for (uint32_t w0 = 0; w0 < Sw; w0 += 64u) {
+  for (uint32_t w0 = 0; w0 < Sw_s; w0 += 64u) {
     for (uint32_t e = tid; e < 3u * 32u * kFixStride; e += kFixThreads) (&acc[0][0])[e] = 0u;
     __syncthreads();
     const uint32_t wl = half * 32u + lane, word = w0 + wl;
-    const bool valid = word < Sw;
+    const bool valid = word < Sw_s;
     const uint32_t* __restrict__ col = xt + (size_t)label * K_pad * Sw + (valid ? word : 0u);  // (an invalid lane's sums go nowhere)
     uint32_t nb[4] = {0u, 0u, 0u, 0u}, by[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
     auto bytes_to_smem = [&]() {
@@ -282,7 +285,7 @@ __global__ void __launch_bounds__(kFixThreads, 3) k_other_fix(const uint32_t* __
     __syncthreads();
     for (uint32_t tl = tid; tl < 2048u; tl += kFixThreads) {
       const uint32_t t = w0 * 32u + tl;
-      if (t >= S) break;
+      if (t >= S || (s >= rows && t >= rows)) break;
       const uint32_t at = (tl & 31u) * kFixStride + (tl >> 5);
       if (t > s) {
         uint32_t* out = gram + (size_t)s * S_pad + t;

@@ -7,8 +7,11 @@ owns the devices: it partitions the (footprint, strand) units of all chunks by p
 pair-count cost (longest-processing-time bin packing, lgmi_partition_lpt), submits one shard per
 GPU from a thread pool (the C-ABI calls release the GIL; a handle is used by one thread at a time),
 and merges the results back into the reference's row order.  Units are independent:
-no collective, no peer traffic.  `shard.py` is the same thing for one PROCESS per GPU
-(torch.distributed launches: bench.py --gpus N)."""
+no collective.  A unit whose cost alone exceeds a device's share is split by rows of its pair
+grid into pieces on several devices (split_plan); its planes cross the host link once, in
+row ranges, and each piece fetches the rows it also needs from the other pieces' devices.
+`shard.py` is the same thing for one PROCESS per GPU (torch.distributed launches:
+bench.py --gpus N); it does not split units."""
 from __future__ import annotations
 
 from concurrent.futures import ThreadPoolExecutor
@@ -22,7 +25,8 @@ from .encode import PlaneBatch
 
 class MergedResult:
     """Results of several shards put back in global unit order: the fields of api.StepResult
-    that callers read (records, site_mean, site_cnt, unit_rec_off, counts)."""
+    that callers read (records, site_mean, site_cnt, unit_rec_off, counts).  split_units maps each
+    unit that was split to its pieces [(device index, first row, end row)] in row order."""
 
     def __init__(self, records, site_mean, site_cnt, unit_rec_off, n_candidates, counts=None, shard_ms=None,
                  shard_units=None):
@@ -30,6 +34,7 @@ class MergedResult:
         self.unit_rec_off, self.n_candidates, self.counts = unit_rec_off, n_candidates, counts
         self.n_records = len(records)
         self.shard_ms, self.shard_units = shard_ms, shard_units
+        self.split_units = {}
 
     def unit_records(self, unit):
         return self.records[int(self.unit_rec_off[unit]):int(self.unit_rec_off[unit + 1])]
@@ -40,15 +45,34 @@ class MergedResult:
         return self.counts[int(self.unit_rec_off[unit]):int(self.unit_rec_off[unit + 1])]
 
 
-def merge_shards(units, n_sites, parts) -> MergedResult:
+def merge_shards(units, n_sites, parts, split=()) -> MergedResult:
     """`parts` = [(global unit indices ascending, records, site_mean, site_cnt, unit_rec_off, counts | None)]
-    per shard, each in its own local order -> one result in global order.  Pure index bookkeeping."""
+    per shard, each in its own local order -> one result in global order.  `split` = [(global unit,
+    [(first row, records, counts | None)] of its pieces in row order, site_mean, site_cnt)] for the units
+    that were split: a piece's i and j count from its first row.  Pure index bookkeeping."""
     n_units = len(units)
     site_mean = np.full(n_sites, np.nan)
     site_cnt = np.zeros(n_sites, dtype=np.uint32)
     per_unit = np.zeros(n_units, dtype=np.int64)
     site_off = units['site_off'].astype(np.int64)
     n_s = units['n_sites'].astype(np.int64)
+    # a split unit: its pieces' rows back to back, i and j shifted to the unit's own site numbers
+    joined = []
+    for unit, pieces, mean, cnt in split:
+        rec = np.concatenate([np.asarray(r) for _a, r, _c in pieces]) if pieces else np.empty(0, PAIR_REC)
+        if len(rec):
+            shift = np.concatenate([np.full(len(r), a, dtype=np.int64) for a, r, _c in pieces])
+            rec['i'] = (rec['i'].astype(np.int64) + shift).astype(np.uint16)
+            rec['j'] = (rec['j'].astype(np.int64) + shift).astype(np.uint16)
+        cnts = None
+        if any(c is not None for _a, _r, c in pieces):
+            cnts = np.concatenate([np.asarray(c).reshape(-1, 9) for _a, r, c in pieces]) \
+                if len(rec) else np.zeros((0, 9), dtype=np.uint32)
+        per_unit[unit] = len(rec)
+        a, n = int(site_off[unit]), int(n_s[unit])
+        site_mean[a:a + n] = mean
+        site_cnt[a:a + n] = cnt
+        joined.append((int(unit), rec, cnts))
     for index, _rec, mean, cnt, off, _counts in parts:
         index = np.asarray(index, dtype=np.int64)
         per_unit[index] = np.diff(np.asarray(off).astype(np.int64))
@@ -62,8 +86,14 @@ def merge_shards(units, n_sites, parts) -> MergedResult:
     unit_rec_off[1:] = np.cumsum(per_unit)
     total = int(unit_rec_off[-1])
     records = np.empty(total, dtype=PAIR_REC)
-    want_counts = any(p[5] is not None for p in parts)
+    want_counts = any(p[5] is not None for p in parts) or any(c is not None for _u, _r, c in joined)
     counts = np.empty((total, 9), dtype=np.uint32) if want_counts else None
+    for unit, rec, cnts in joined:
+        a = int(unit_rec_off[unit])
+        records[a:a + len(rec)] = rec
+        records['unit'][a:a + len(rec)] = unit
+        if counts is not None and cnts is not None:
+            counts[a:a + len(rec)] = cnts
     for index, rec, _mean, _cnt, off, cnts in parts:
         index = np.asarray(index, dtype=np.int64)
         if not len(index):
@@ -79,6 +109,80 @@ def merge_shards(units, n_sites, parts) -> MergedResult:
         if counts is not None and cnts is not None and len(dst):
             counts[dst] = cnts
     return MergedResult(records, site_mean, site_cnt, unit_rec_off, int((n_s * (n_s - 1) // 2).sum()), counts)
+
+
+SPLIT_ROWS = 128   # piece boundaries fall on multiples of this many rows (lgmi_batch_create_rows)
+
+
+def _rows_pairs(S, rows):
+    """Pairs (i, j), i < j < S, with i < rows, for an array of row counts."""
+    rows = np.asarray(rows, dtype=np.int64)
+    return rows * S - rows * (rows + 1) // 2
+
+
+def split_rows(S, m):
+    """Row boundaries 0 = b_0 < ... < b_m = S of m pieces of a unit of S sites, at multiples of SPLIT_ROWS, with the
+    largest piece's pair count as small as that granularity allows (the slowest device sets the time)."""
+    S = int(S)
+    ends = np.minimum(np.arange(1, -(-S // SPLIT_ROWS) + 1, dtype=np.int64) * SPLIT_ROWS, S)
+    blocks = np.diff(np.concatenate(([0], _rows_pairs(S, ends))))    # pairs of each 128-row block
+    nb = len(blocks)
+    m = max(1, min(int(m), nb))
+
+    def cut(cap):   # greedy: each piece takes blocks while it stays within cap, leaving one block per later piece
+        bounds, t = [0], 0
+        for p in range(m - 1):
+            acc, t = blocks[t], t + 1
+            while t < nb - (m - 1 - p) and acc + blocks[t] <= cap:
+                acc, t = acc + blocks[t], t + 1
+            bounds.append(int(ends[t - 1]))
+        return bounds + [S], int(blocks[t:].sum())
+
+    lo, hi = int(blocks.max()), int(blocks.sum())     # the smallest cap for which the last piece fits too
+    while lo < hi:
+        mid = (lo + hi) // 2
+        if cut(mid)[1] <= mid:
+            hi = mid
+        else:
+            lo = mid + 1
+    return cut(lo)[0]
+
+
+def split_plan(units, n_dev):
+    """Which units to split, and how, for n_dev devices: {unit: row boundaries}.  A unit of more than
+    SPLIT_ROWS sites whose cost (api.unit_costs) exceeds total / n_dev is cut into
+    min(n_dev, ceil(cost * n_dev / total), ceil(S / SPLIT_ROWS)) pieces of about equal pair counts."""
+    if n_dev < 2 or not len(units):
+        return {}
+    cost = api.unit_costs(units).astype(np.float64)
+    total = cost.sum()
+    S = units['n_sites'].astype(np.int64)
+    out = {}
+    for u in np.flatnonzero((S > SPLIT_ROWS) & (cost * n_dev > total)):
+        m = min(n_dev, int(np.ceil(cost[u] * n_dev / total)), int(-(-S[u] // SPLIT_ROWS)))
+        if m >= 2:
+            out[int(u)] = split_rows(S[u], m)
+    return out
+
+
+def plan_pieces(units, n_dev):
+    """LPT partition of the ordinary units and of the pieces of the split units together.  Returns
+    (shards, pieces, splits): shards[k] the ascending ordinary units of device k, pieces[k] its pieces as
+    (unit, first row, end row), splits the split_plan."""
+    splits = split_plan(units, n_dev)
+    whole = np.array([u for u in range(len(units)) if u not in splits], dtype=np.int64)
+    items = [(int(u), 0, 0) for u in whole]
+    cost = [api.unit_costs(units[whole])] if len(whole) else []
+    chunk = 64
+    for u, b in splits.items():
+        S, R = int(units['n_sites'][u]), int(units['n_reads'][u])
+        for a, e in zip(b[:-1], b[1:]):
+            items.append((u, a, e))
+            cost.append(np.array([(_rows_pairs(S, e) - _rows_pairs(S, a)) * ((R + chunk - 1) // chunk)], np.uint64))
+    bin_of, _load = api.partition_lpt(np.concatenate(cost) if cost else np.zeros(0, np.uint64), n_dev)
+    shards = [whole[bin_of[:len(whole)] == k] for k in range(n_dev)]
+    pieces = [[items[t] for t in range(len(whole), len(items)) if bin_of[t] == k] for k in range(n_dev)]
+    return shards, pieces, splits
 
 
 class DevicePool:
@@ -105,31 +209,112 @@ class DevicePool:
         self.contexts = []
 
     def plan(self, pb: PlaneBatch):
-        """[ascending global unit indices of each device's shard] by LPT on S(S-1)/2 * ceil(R/64)."""
-        bin_of, _load = api.partition_lpt(api.unit_costs(pb.units), len(self.devices))
-        return [np.flatnonzero(bin_of == k) for k in range(len(self.devices))]
+        """[ascending global unit indices of each device's shard] by LPT on S(S-1)/2 * ceil(R/64), when no unit is
+        split (split_plan); otherwise (shards, pieces, splits) of plan_pieces."""
+        shards, pieces, splits = plan_pieces(pb.units, len(self.devices))
+        return (shards, pieces, splits) if splits else shards
 
     def run(self, pb: PlaneBatch, min_common_reads=5, mode=api.MODE_HET_ONLY):
         """The MI step of `pb` over all devices; same result as api.mi_step_batched on one."""
-        if len(self.devices) == 1 or pb.n_units < 2 * len(self.devices):
+        n_dev = len(self.devices)
+        shards, pieces, splits = plan_pieces(pb.units, n_dev)
+        self.last_piece_ms, self.last_split_means_ms = [None] * n_dev, None   # (what the last run measured)
+        if not splits and (n_dev == 1 or pb.n_units < 2 * n_dev):
             return api.mi_step_batched(pb, min_common_reads, mode, ctx=self.contexts[0])
-        shards = self.plan(pb)
+        import time
+        batches = self._piece_batches(pb, pieces) if splits else [None] * n_dev
 
         def work(k):
-            index = shards[k]
-            if not len(index):
-                return None
-            import time
+            index, b = shards[k], batches[k]
             t0 = time.perf_counter()
-            res = api.mi_step_batched(pb.subset(index), min_common_reads, mode, ctx=self.contexts[k])
-            return (index, res.records, res.site_mean, res.site_cnt, res.unit_rec_off, res.counts,
-                    1e3 * (time.perf_counter() - t0))
+            res = None
+            if b is not None:
+                b.run(min_common_reads, mode)
+            if len(index):
+                res = api.mi_step_batched(pb.subset(index), min_common_reads, mode, ctx=self.contexts[k])
+            if b is not None:
+                b.result = b.download(copy=True)
+                self.last_piece_ms[k] = b.result.kernel_ms
+            return res, 1e3 * (time.perf_counter() - t0)
 
-        done = [r for r in self._threads.map(work, range(len(self.devices))) if r is not None]
-        merged = merge_shards(pb.units, pb.n_sites, [r[:6] for r in done])
-        merged.shard_ms = [r[6] for r in done]
-        merged.shard_units = [len(r[0]) for r in done]
+        try:
+            done = list(self._threads.map(work, range(n_dev)))
+            parts = [(shards[k], r.records, r.site_mean, r.site_cnt, r.unit_rec_off, r.counts)
+                     for k, (r, _ms) in enumerate(done) if r is not None]
+            split, where = [], {}
+            t0 = time.perf_counter()
+            for u, bounds in splits.items():
+                # (device, position in its piece batch) of every piece of u, in row order
+                loc = sorted((a, k, q) for k in range(n_dev) for q, (v, a, _e) in enumerate(pieces[k]) if v == u)
+                owner = self.contexts[loc[0][1]]
+                S, off = int(pb.units['n_sites'][u]), int(pb.units['site_off'][u])
+                mean, cnt = api.split_means(owner, pb.site_flags[off:off + S], [(batches[k], q) for _a, k, q in loc])
+                recs = []
+                for a, k, q in loc:
+                    res = batches[k].result
+                    recs.append((a, res.unit_records(q), res.unit_counts(q) if res.counts is not None else None))
+                split.append((u, recs, mean, cnt))
+                where[u] = [(k, a, a + int(batches[k].row_limit[q])) for a, k, q in loc]
+            self.last_split_means_ms = 1e3 * (time.perf_counter() - t0)
+        finally:
+            for b in batches:
+                if b is not None:
+                    b.close()
+        merged = merge_shards(pb.units, pb.n_sites, parts, split)
+        merged.split_units = where
+        merged.shard_ms = [ms for _r, ms in done]
+        # units per device; a split unit counts on the device of its first piece, which computes its means
+        owned = [len(shards[k]) for k in range(n_dev)]
+        for u, w in where.items():
+            owned[w[0][0]] += 1
+        merged.shard_units = owned
         return merged
+
+    def _piece_batches(self, pb, pieces):
+        """One batch of pieces per device (None where there is none), planes in place: each piece's own rows
+        uploaded from the host, the rows after them copied from the devices of the later pieces of its unit."""
+        n_dev = len(self.devices)
+        batches = [None] * n_dev
+        rows_at = {}   # (unit, first row) -> (device, first plane word of the piece there, end row)
+        for k in range(n_dev):
+            if not pieces[k]:
+                continue
+            desc = np.zeros(len(pieces[k]), dtype=pb.units.dtype)
+            flags = []
+            word = site = 0
+            for q, (u, a, e) in enumerate(pieces[k]):
+                g = pb.units[u]
+                S, W = int(g['n_sites']), int(g['row_words'])
+                desc[q] = (word, S - a, int(g['n_reads']), W, site)    # the suffix unit of sites [a, S)
+                flags.append(pb.site_flags[int(g['site_off']) + a:int(g['site_off']) + S])
+                rows_at[(u, a)] = (k, word, e)
+                word += 3 * (S - a) * W
+                site += S - a
+            # (np.empty: the batch only reads the planes' size; their words come from upload_rows / copies)
+            sub = PlaneBatch(desc, np.empty(word, dtype=np.uint32), np.concatenate(flags))
+            batches[k] = api.Batch(self.contexts[k], sub, row_limit=[e - a for _u, a, e in pieces[k]])
+        try:
+            def upload(k):   # the host link once: every piece uploads its own rows, one thread per device
+                for q, (u, a, e) in enumerate(pieces[k]):
+                    W, base = int(pb.units['row_words'][u]), int(pb.units['plane_off'][u])
+                    batches[k].upload_rows(int(batches[k].pb.units['plane_off'][q]),
+                                           pb.planes[base + 3 * a * W:base + 3 * e * W])
+            list(self._threads.map(upload, [k for k in range(n_dev) if pieces[k]]))
+            # then, from this thread, each piece's rows after its own from the pieces that uploaded them: a copy
+            # waits on an event recorded behind the upload already queued on the source's stream
+            for k in range(n_dev):
+                for q, (u, a, e) in enumerate(pieces[k]):
+                    W = int(pb.units['row_words'][u])
+                    dst0 = int(batches[k].pb.units['plane_off'][q])
+                    for (v, c), (ks, src0, ce) in rows_at.items():
+                        if v == u and c >= e:
+                            batches[k].copy_planes_from(dst0 + 3 * (c - a) * W, batches[ks], src0, 3 * (ce - c) * W)
+        except BaseException:
+            for b in batches:
+                if b is not None:
+                    b.close()
+            raise
+        return batches
 
 
 _pool = None
