@@ -213,21 +213,15 @@ LGMI_API int lgmi_set_dense_threshold(lgmi_t* ctx, uint32_t min_sites, uint32_t 
  * either way; applies to batches created afterwards.  Environment                  *
  * LGMI_DENSE_PATH=4/9 sets the default.                                            */
 LGMI_API int lgmi_set_dense_path(lgmi_t* ctx, int blocks);
-/* Small units (<= 60 sites, <= 256 reads) have their counts built by          *
- * AND+popcount (0, default) or as one small int8 Gram matrix per unit on the  *
- * tensor cores (tensor_cores != 0: k_small_gram + k_pairs_pre).  Same         *
- * integers either way; applies to batches created afterwards.  Environment    *
- * LGMI_SMALL_PATH=0/1 sets the default.                                       */
-LGMI_API int lgmi_set_small_path(lgmi_t* ctx, int tensor_cores);
 /* Mid-depth units (more than 64 sites or 256 reads, below the dense threshold)   *
  * have their counts built on the tensor cores in one batched launch              *
- * (tensor_cores = 2, default: the warp-specialised k_tile_gram_ws expands the    *
+ * (tensor_cores != 0, default: the warp-specialised k_tile_gram_ws expands the   *
  * bit-planes in the kernel, one tcgen05 int8 MMA per label row block, then       *
- * k_tile_finish; 1: the same tiles by the single-role k_tile_gram) or by tiled   *
- * AND+popcount (0: k_tile_mi; units deeper than 65 535 reads always).  Same      *
- * integers and the same MI bits every way (mutual_information.py:15-41); applies *
- * to batches created afterwards.  Environment LGMI_TILE_PATH=0/1/2 sets the      *
- * default.                                                                       */
+ * k_tile_finish) or by tiled AND+popcount (0: k_tile_mi; units deeper than       *
+ * 65 535 reads always).  Same integers and the same MI bits either way           *
+ * (mutual_information.py:15-41); applies to batches created afterwards.          *
+ * Environment LGMI_TILE_PATH=0 selects the popcount form, any other value the    *
+ * tensor cores.                                                                  */
 LGMI_API int lgmi_set_tile_path(lgmi_t* ctx, int tensor_cores);
 
 /* ----- batched MI step: replaces the per-unit loop                           *

@@ -41,7 +41,7 @@ DENSE_DEFAULT = (48, 8192)    # lgmi_set_dense_threshold defaults: (min_sites, m
 EXPORTS = (
     "lgmi_version", "lgmi_create", "lgmi_destroy", "lgmi_last_error", "lgmi_set_stream",
     "lgmi_pinned_alloc", "lgmi_pinned_free", "lgmi_launch_count", "lgmi_set_dense_threshold",
-    "lgmi_set_small_path", "lgmi_set_tile_path", "lgmi_set_dense_path",
+    "lgmi_set_tile_path", "lgmi_set_dense_path",
     "lgmi_batch_create", "lgmi_batch_destroy", "lgmi_batch_upload", "lgmi_batch_run",
     "lgmi_batch_download", "lgmi_batch_sync", "lgmi_batch_device_ptrs",
     "lgmi_batch_create_rows", "lgmi_batch_upload_rows", "lgmi_batch_copy_planes", "lgmi_split_means",
@@ -109,7 +109,6 @@ def load():
         "lgmi_pinned_free": (i32, [vp, vp]),
         "lgmi_launch_count": (u64, [vp]),
         "lgmi_set_dense_threshold": (i32, [vp, u32, u32]),
-        "lgmi_set_small_path": (i32, [vp, i32]),
         "lgmi_set_tile_path": (i32, [vp, i32]),
         "lgmi_set_dense_path": (i32, [vp, i32]),
         "lgmi_batch_create": (i32, [vp, vp, u32, u64, u64, pvp]),

@@ -55,18 +55,14 @@ class Context:
         """Units at least this large take the int8 tensor-core path (batches created afterwards)."""
         check(self._lib.lgmi_set_dense_threshold(self.handle, int(min_sites), int(min_reads)), self.handle)
 
-    def set_small_path(self, tensor_cores):
-        """Small units counted by popcount (False, default) or on the tensor cores (True)."""
-        check(self._lib.lgmi_set_small_path(self.handle, 1 if tensor_cores else 0), self.handle)
-
     def set_dense_path(self, blocks):
         """Deep units: 4 = four Gram blocks + "other" cells from the listed reads while those are rare (decided on
         the device per unit and run; default), 9 = always nine blocks (lgmi_set_dense_path)."""
         check(self._lib.lgmi_set_dense_path(self.handle, int(blocks)), self.handle)
 
     def set_tile_path(self, tensor_cores):
-        """Mid-depth units counted on the tensor cores (True / 1, default: k_tile_gram; 2: the warp-specialised
-        k_tile_gram_ws) or by tiled popcount (False / 0)."""
+        """Mid-depth units counted on the tensor cores (True / non-zero, default: k_tile_gram_ws + k_tile_finish)
+        or by tiled popcount (False / 0: k_tile_mi)."""
         check(self._lib.lgmi_set_tile_path(self.handle, int(tensor_cores)), self.handle)
 
     @property

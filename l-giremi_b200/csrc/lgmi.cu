@@ -123,12 +123,9 @@ struct lgmi_ctx {
   // persistent launch shape of k_pairs
   int num_sms = 0;
   int pairs_ctas_per_sm = 0;
-  int pre_ctas_per_sm = 0;
   int dense_path = 4;  // deep units: 4 = four Gram blocks + sparse "other" cells where the "other" reads are rare (decided on
                        // the device per unit and run), 9 = always nine blocks
-  int small_path = 0;  // 0: popcount (k_pairs_fast, default: faster, see DESIGN.md); 1: counted on the tensor cores
-  int tile_path = 2;   // mid-depth units: 0 popcount (k_tile_mi), 1 tensor cores (k_tile_gram),
-                       // 2 tensor cores, warp-specialised (k_tile_gram_ws, default)
+  int tile_path = 1;   // mid-depth units: 0 popcount (k_tile_mi), else tensor cores (k_tile_gram_ws, default)
   // tensor-core path: units at least this large build their tables with k_gram_i8
   uint32_t dense_min_sites = 48, dense_min_reads = 8192;
   void* encode_tiled = nullptr;  // cuTensorMapEncodeTiled, resolved through the runtime (no libcuda link)
@@ -210,18 +207,12 @@ struct lgmi_batch {
   cudaEvent_t fix_fork = nullptr, fix_join = nullptr;  // joined before the tables are read)
   DenseTile* d_tiles = nullptr;
   uint64_t dense_macs = 0;      // multiply-accumulates the tile lists amount to
-  // small units counted on the tensor cores
-  FastItem* d_pre_items = nullptr;
-  uint32_t n_pre = 0;
-  unsigned long long* d_val = nullptr;  // packed counts, 8 bytes per candidate pair of those units
   // tiled popcount path
   TileItem* d_tile_items = nullptr;
   uint32_t n_tile_items = 0;
-  TgTile* d_gram_tiles = nullptr;      // k_tile_gram's work items (128 x 48 site blocks)
+  TgTile* d_gram_tiles = nullptr;      // k_tile_gram_ws's work items (128 x 48 site blocks)
   uint32_t n_gram_tiles = 0;
-  int gram_kernel = 1;                 // 1 k_tile_gram, 2 k_tile_gram_ws (the context's tile path when the batch was made)
   uint2* d_tile_cnt = nullptr;         // its output: 24 bytes of counts per pair slot
-  uint32_t* d_tile_next = nullptr;     // its work counter
   uint32_t n_tiled_work_items = 0;     // work items (Item) of the tiled and of the deep units: k_pairs_generic<1>'s and <2>'s
   TiledDesc* d_tiled_desc = nullptr;   // k_pairs_generic<1>'s items, one self-contained record each
   uint32_t n_tiled_desc = 0;
@@ -384,24 +375,11 @@ extern "C" int lgmi_create(int device, lgmi_t** out) {
     lgmi_destroy(ctx);
     return rc;
   }
-  if (cudaFuncSetAttribute(k_small_gram, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(SgSmem) + 1024)) !=
-          cudaSuccess ||
-      cudaFuncSetAttribute(k_pairs_pre, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PreSmem)) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->pre_ctas_per_sm, k_pairs_pre, kFastThreads, sizeof(PreSmem)) !=
-          cudaSuccess ||
-      ctx->pre_ctas_per_sm < 1) {
-    int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: small-unit tensor path cannot be resident (%s)",
-                  cudaGetErrorString(cudaGetLastError()));
-    lgmi_destroy(ctx);
-    return rc;
-  }
-  if (const char* e = getenv("LGMI_SMALL_PATH")) ctx->small_path = atoi(e) ? 1 : 0;
   if (const char* e = getenv("LGMI_DENSE_PATH")) ctx->dense_path = atoi(e) == 9 ? 9 : 4;
-  if (const char* e = getenv("LGMI_TILE_PATH")) ctx->tile_path = std::min(2, std::max(0, atoi(e)));
+  if (const char* e = getenv("LGMI_TILE_PATH")) ctx->tile_path = atoi(e) ? 1 : 0;
   if (const char* e = getenv("LGMI_GRAPHS")) ctx->pipeline_graphs = atoi(e) ? 1 : 0;
-  if (cudaFuncSetAttribute(k_tile_gram, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTgSmemBytes) != cudaSuccess ||
-      cudaFuncSetAttribute(k_tile_gram_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTwSmemBytes) != cudaSuccess) {
-    int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: k_tile_gram cannot be resident (%s)",
+  if (cudaFuncSetAttribute(k_tile_gram_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTwSmemBytes) != cudaSuccess) {
+    int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: k_tile_gram_ws cannot be resident (%s)",
                   cudaGetErrorString(cudaGetLastError()));
     lgmi_destroy(ctx);
     return rc;
@@ -478,12 +456,6 @@ extern "C" int lgmi_pinned_free(lgmi_t* ctx, void* ptr) {
 
 extern "C" uint64_t lgmi_launch_count(const lgmi_t* ctx) { return ctx ? ctx->launches : 0; }
 
-extern "C" int lgmi_set_small_path(lgmi_t* ctx, int tensor_cores) {
-  if (!ctx) return LGMI_ERR_ARG;
-  ctx->small_path = tensor_cores ? 1 : 0;
-  return LGMI_OK;
-}
-
 extern "C" int lgmi_set_dense_path(lgmi_t* ctx, int blocks) {
   if (!ctx) return LGMI_ERR_ARG;
   if (blocks != 4 && blocks != 9) return fail(ctx, LGMI_ERR_ARG, "lgmi_set_dense_path: blocks must be 4 or 9");
@@ -493,7 +465,7 @@ extern "C" int lgmi_set_dense_path(lgmi_t* ctx, int blocks) {
 
 extern "C" int lgmi_set_tile_path(lgmi_t* ctx, int tensor_cores) {
   if (!ctx) return LGMI_ERR_ARG;
-  ctx->tile_path = tensor_cores < 0 ? 0 : (tensor_cores > 2 ? 2 : tensor_cores);
+  ctx->tile_path = tensor_cores ? 1 : 0;
   return LGMI_OK;
 }
 
@@ -554,10 +526,7 @@ extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
   ctx->dev_pool.release(b->d_gram_tiles);
   ctx->dev_pool.release(b->d_tiled_desc);
   ctx->dev_pool.release(b->d_tile_cnt);
-  ctx->dev_pool.release(b->d_tile_next);
   ctx->dev_pool.release(b->d_tile_counts);
-  ctx->dev_pool.release(b->d_pre_items);
-  ctx->dev_pool.release(b->d_val);
   ctx->host_pool.release(b->h_header);
   ctx->host_pool.release(b->h_records);
   ctx->host_pool.release(b->h_counts);
@@ -588,8 +557,7 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
   }
 
   std::vector<DevUnit> du(n_units);
-  std::vector<FastItem> fast_items, pre_items;
-  uint64_t val_slots = 0;
+  std::vector<FastItem> fast_items;
   std::vector<MeanItem> mean_items;
   std::vector<DenseTile> dense_tiles;
   std::vector<TileItem> tile_items;
@@ -621,7 +589,7 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
                   u.n_sites);
     }
     const uint32_t rows = piece ? limit : u.n_sites;  // row blocks at or past it hold no pair of the unit
-    const size_t first_gram_tile = gram_tiles.size();  // this unit's k_tile_gram work items start here
+    const size_t first_gram_tile = gram_tiles.size();  // this unit's k_tile_gram_ws work items start here
     DevUnit& d = du[k];
     d.plane_off = u.plane_off;
     d.S = u.n_sites;
@@ -703,7 +671,7 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
       b->dense_plans.push_back(pl);
     } else if (np && (piece || !(nit == 1 && u.n_sites <= (uint32_t)kFastMaxS && u.n_reads <= (uint32_t)kFastMaxR))) {
       // tiled popcount path: MI of every pair precomputed by k_tile_mi into the dense scratch
-      // (or, by default, counted on the tensor cores by k_tile_gram and finished by k_tile_finish)
+      // (or, by default, counted on the tensor cores by k_tile_gram_ws and finished by k_tile_finish)
       const bool gram = ctx->tile_path && u.n_reads >= 1u && u.n_reads <= kTgMaxReads;
       d.tiled = gram ? 2 : 1;
       if (nit == 1 && !piece) {
@@ -766,14 +734,7 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
         f.R = (uint16_t)u.n_reads;
         f.W = u.row_words;
         f.pad = 0;
-        if (ctx->small_path && u.n_sites <= (uint32_t)kSgMaxS && val_slots + np + 1 < 0xffffffffull) {
-          it.flags |= ITEM_PRE;
-          f.pad = (uint32_t)val_slots;          // first slot of the unit's packed counts (even: 16-byte aligned)
-          val_slots += (np + 1) & ~1ull;
-          pre_items.push_back(f);
-        } else {
-          fast_items.push_back(f);
-        }
+        fast_items.push_back(f);
       }
       b->h_items.push_back(it);
     }
@@ -796,11 +757,9 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
   });
   b->n_tile_items = (uint32_t)tile_items.size();
   b->n_gram_tiles = (uint32_t)gram_tiles.size();
-  b->gram_kernel = ctx->tile_path == 2 ? 2 : 1;
 
   b->n_items = (uint32_t)b->h_items.size();
   b->n_fast = (uint32_t)fast_items.size();
-  b->n_pre = (uint32_t)pre_items.size();
   b->n_mean_items = (uint32_t)mean_items.size();
   b->n_dense = dense;
 
@@ -816,7 +775,7 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
   } while (0)
 
   for (cudaEvent_t& e : b->ev) BCU(cudaEventCreate(&e));
-  if ((b->n_fast || b->n_pre) && (!b->dense_plans.empty() || b->n_tile_items || b->n_gram_tiles)) {
+  if (b->n_fast && (!b->dense_plans.empty() || b->n_tile_items || b->n_gram_tiles)) {
     BCU(cudaStreamCreateWithFlags(&b->side_stream, cudaStreamNonBlocking));
     for (cudaEvent_t& e : b->side_ev) BCU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   }
@@ -840,18 +799,11 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
   BCU(pool_malloc(ctx, &b->d_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
   BCU(pool_malloc(ctx, &b->d_dense, std::max<uint64_t>(1, dense) * sizeof(double)));
   BCU(pool_malloc(ctx, &b->d_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
-  if (!pre_items.empty()) {
-    BCU(pool_malloc(ctx, &b->d_pre_items, pre_items.size() * sizeof(FastItem)));
-    BCU(cudaMemcpyAsync(b->d_pre_items, pre_items.data(), pre_items.size() * sizeof(FastItem), cudaMemcpyHostToDevice,
-                        bstream(b)));
-    BCU(pool_malloc(ctx, &b->d_val, val_slots * sizeof(unsigned long long)));
-  }
   if (!tile_items.empty()) {
     BCU(pool_malloc(ctx, &b->d_tile_items, tile_items.size() * sizeof(TileItem)));
     BCU(cudaMemcpyAsync(b->d_tile_items, tile_items.data(), tile_items.size() * sizeof(TileItem), cudaMemcpyHostToDevice,
                         bstream(b)));
   }
-  BCU(pool_malloc(ctx, &b->d_tile_next, sizeof(uint32_t)));
   if (!gram_tiles.empty()) {
     BCU(pool_malloc(ctx, &b->d_gram_tiles, gram_tiles.size() * sizeof(TgTile)));
     BCU(cudaMemcpyAsync(b->d_gram_tiles, gram_tiles.data(), gram_tiles.size() * sizeof(TgTile), cudaMemcpyHostToDevice,
@@ -1113,9 +1065,8 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     k_run_init<<<(unsigned)((n + 255) / 256), 256, 0, bstream(b)>>>(b->d_header, b->own_stream ? b->h_header : nullptr,
                                                                   b->d_unit_rec_off, b->n_units + 1,
                                                                   b->d_item_dense, b->n_items, b->d_n_generic,
-                                                                  b->n_items - b->n_fast - b->n_pre - b->n_tiled_work_items, b->d_site_mean,
-                                                                  b->d_site_cnt,
-                                                                  b->n_sites, b->d_tile_next);
+                                                                  b->n_items - b->n_fast - b->n_tiled_work_items, b->d_site_mean,
+                                                                  b->d_site_cnt, b->n_sites);
     ++ctx->launches;
   }
   if (timing) CU(ctx, cudaEventRecord(b->ev[4], bstream(b)));
@@ -1201,32 +1152,12 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     T.tiles = b->d_gram_tiles;
     T.n_tiles = b->n_gram_tiles;
     T.cnt = b->d_tile_cnt;
-    T.next = b->d_tile_next;
     T.error = reinterpret_cast<uint32_t*>(&b->d_header->pad);
     const unsigned ggrid = (unsigned)std::min<uint32_t>(b->n_gram_tiles, (uint32_t)ctx->num_sms);
-    if (b->gram_kernel == 2) k_tile_gram_ws<<<ggrid, kTwThreads, kTwSmemBytes, bstream(b)>>>(T);
-    else k_tile_gram<<<ggrid, kTgThreads, kTgSmemBytes, bstream(b)>>>(T);
+    k_tile_gram_ws<<<ggrid, kTwThreads, kTwSmemBytes, bstream(b)>>>(T);
     ++ctx->launches;
     const unsigned fgrid = (unsigned)std::min<uint64_t>(b->n_items, (uint64_t)ctx->num_sms * 8u);
     k_tile_finish<<<fgrid, kThreads, 0, bstream(b)>>>(P, b->d_tile_cnt);
-    ++ctx->launches;
-  }
-  if (b->n_pre) {
-    // small units: counts of every pair on the tensor cores -> packed values + emitted pairs per unit
-    SgParams G;
-    G.items = b->d_pre_items;
-    G.n_items = b->n_pre;
-    G.planes = b->d_planes;
-    G.site_flags = b->d_flags;
-    G.min_common = min_common;
-    G.mode = mode;
-    G.val = b->d_val;
-    G.item_cnt = b->d_item_cnt;
-    G.item_dense = b->d_item_dense;
-    G.n_generic = b->d_n_generic;
-    G.error = reinterpret_cast<uint32_t*>(&b->d_header->pad);
-    const unsigned grid = (unsigned)std::min<uint64_t>(b->n_pre, (uint64_t)ctx->num_sms * 2u);
-    k_small_gram<<<grid, kSgThreads, sizeof(SgSmem) + 1024, small>>>(G);
     ++ctx->launches;
   }
   if (b->n_fast) {
@@ -1251,7 +1182,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
   }
   if (b->n_items) {
     // K0 of everything else + scan: every item's place in the ordered output
-    if (b->n_items > b->n_fast + b->n_pre) {
+    if (b->n_items > b->n_fast) {
       const unsigned cgrid = (unsigned)std::min<uint64_t>(b->n_items, (uint64_t)ctx->num_sms * 8u);
       k_count<<<cgrid, kThreads, 0, bstream(b)>>>(P);
       ++ctx->launches;
@@ -1268,7 +1199,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     CU(ctx, cudaEventRecord(b->side_ev[2], bstream(b)));
     CU(ctx, cudaStreamWaitEvent(small, b->side_ev[2], 0));
   }
-  if (b->n_fast || b->n_pre) {
+  if (b->n_fast) {
     FastParams F;
     F.items = b->d_fast_items;
     F.n_items = b->n_fast;
@@ -1289,25 +1220,13 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     F.site_cnt = b->d_site_cnt;
     F.unit_rec_off = b->d_unit_rec_off;
     F.unit_base = b->unit_base;
-    if (b->n_pre) {
-      PreParams Q;
-      Q.F = F;
-      Q.F.items = b->d_pre_items;
-      Q.F.n_items = b->n_pre;
-      Q.val = b->d_val;
-      const unsigned grid = (unsigned)std::min<uint64_t>(b->n_pre, (uint64_t)ctx->num_sms * ctx->pre_ctas_per_sm);
-      k_pairs_pre<<<grid, kFastThreads, sizeof(PreSmem), small>>>(Q);
-      ++ctx->launches;
-    }
-    if (b->n_fast) {
-      // persistent CTAs: a whole number of CTAs per SM, never more than there are items
-      const unsigned grid = (unsigned)std::min<uint64_t>(b->n_fast, (uint64_t)ctx->num_sms * ctx->pairs_ctas_per_sm);
-      if ((mode & (LGMI_MODE_HET_ONLY | LGMI_MODE_SKIP_NONHET)) == (LGMI_MODE_HET_ONLY | LGMI_MODE_SKIP_NONHET))
-        k_pairs_fast_het<<<grid, kFastThreads, sizeof(FastSmem), small>>>(F);
-      else
-        k_pairs_fast<<<grid, kFastThreads, sizeof(FastSmem), small>>>(F);
-      ++ctx->launches;
-    }
+    // persistent CTAs: a whole number of CTAs per SM, never more than there are items
+    const unsigned grid = (unsigned)std::min<uint64_t>(b->n_fast, (uint64_t)ctx->num_sms * ctx->pairs_ctas_per_sm);
+    if ((mode & (LGMI_MODE_HET_ONLY | LGMI_MODE_SKIP_NONHET)) == (LGMI_MODE_HET_ONLY | LGMI_MODE_SKIP_NONHET))
+      k_pairs_fast_het<<<grid, kFastThreads, sizeof(FastSmem), small>>>(F);
+    else
+      k_pairs_fast<<<grid, kFastThreads, sizeof(FastSmem), small>>>(F);
+    ++ctx->launches;
   }
   if (timing) CU(ctx, cudaEventRecord(b->ev[3], bstream(b)));
   if (forked) CU(ctx, cudaEventRecord(b->side_ev[3], small));
@@ -1384,7 +1303,7 @@ static int fill_scalars(lgmi_batch* b, lgmi_result* out) {
   out->n_dense_units = (uint32_t)b->dense_plans.size();
   out->dense_macs = b->dense_macs;
   if (b->h_header->pad)
-    return fail(ctx, LGMI_ERR_CUDA, "k_gram_i8 / k_tile_gram: a pipeline barrier timed out (tensor-core path)");
+    return fail(ctx, LGMI_ERR_CUDA, "k_gram_i8 / k_tile_gram_ws: a pipeline barrier timed out (tensor-core path)");
   return LGMI_OK;
 }
 

@@ -20,7 +20,6 @@
 #include "lgmi_math.cuh"
 #include "lgmi_fast_kernel.cuh"
 #include "lgmi_dense.cuh"
-#include "lgmi_small.cuh"
 
 namespace lgmi {
 
@@ -34,13 +33,13 @@ struct DevUnit {
   uint32_t S, R, W, site_off;
   uint32_t first_item, n_items;
   uint32_t S_pad;
-  uint32_t tiled;      // MI of every pair is precomputed into the dense scratch: 1 by k_tile_mi, 2 by k_tile_gram + k_tile_finish
+  uint32_t tiled;      // MI of every pair is precomputed into the dense scratch: 1 by k_tile_mi, 2 by k_tile_gram_ws + k_tile_finish
 };
 constexpr uint64_t kNoGram = ~0ull;
 
 enum : uint32_t {
-  ITEM_FIRST = 1u, ITEM_SINGLE = 2u, ITEM_FAST = 4u, ITEM_PRE = 8u /* counted by k_small_gram */,
-  ITEM_TILED = 16u /* MI precomputed by k_tile_mi or k_tile_gram + k_tile_finish */,
+  ITEM_FIRST = 1u, ITEM_SINGLE = 2u, ITEM_FAST = 4u,
+  ITEM_TILED = 16u /* MI precomputed by k_tile_mi or k_tile_gram_ws + k_tile_finish */,
   ITEM_TILED_GRAM = 32u /* ... by the latter, which also counts the item's emitted pairs */,
   ITEM_GRAM = 64u /* deep unit: tables from the count matrices of the tensor-core path (k_pairs_generic<2>) */
 };
@@ -767,7 +766,7 @@ __global__ void __launch_bounds__(kThreads) k_count(const RunParams P) {
   const bool skip_nonhet = het_only && (P.mode & LGMI_MODE_SKIP_NONHET) != 0u;
   for (uint32_t item_idx = blockIdx.x; item_idx < P.n_items; item_idx += gridDim.x) {
     const Item it = P.items[item_idx];
-    if (it.flags & (ITEM_PRE | ITEM_FAST | ITEM_TILED_GRAM)) continue;  // counted by k_small_gram / k_count_fast / k_tile_finish
+    if (it.flags & (ITEM_FAST | ITEM_TILED_GRAM)) continue;  // counted by k_count_fast / k_tile_finish
     const DevUnit u = P.units[it.unit];
     const uint8_t* __restrict__ flags = P.site_flags + u.site_off;
     uint32_t mine = 0;
@@ -1016,14 +1015,12 @@ __global__ void __launch_bounds__(256) k_split_records(const Header* __restrict_
 __global__ void k_run_init(Header* __restrict__ header, Header* __restrict__ host_header,
                            unsigned long long* __restrict__ unit_rec_off, uint32_t n_off,
                            uint8_t* __restrict__ item_dense, uint32_t n_items, uint32_t* __restrict__ n_generic,
-                           uint32_t n_generic0, double* __restrict__ mean, uint32_t* __restrict__ cnt, uint64_t n_sites,
-                           uint32_t* __restrict__ tile_next) {
+                           uint32_t n_generic0, double* __restrict__ mean, uint32_t* __restrict__ cnt, uint64_t n_sites) {
   const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (k == 0) {
     header->n_records = 0ull;
     header->pad = 0ull;
     *n_generic = n_generic0;
-    *tile_next = 0u;  // k_tile_gram's work counter
     if (host_header) {  // pinned host memory (unified addressing): the pipelined step reads the count from there
       host_header->n_records = 0ull;
       host_header->pad = 0ull;

@@ -2,7 +2,7 @@
 // 64 sites or 256 reads) and too shallow for k_gram_i8's one-GEMM-per-unit form, counted
 // on the tensor cores in ONE batched launch over all of them.
 //
-//   k_tile_gram   work item = (unit, block I of 128 sites, block J of 48 sites) with some pair
+//   k_tile_gram_ws work item = (unit, block I of 128 sites, block J of 48 sites) with some pair
 //                 i < j.  Per 128-read k-block the CTA expands the unit's bit-planes IN THE
 //                 KERNEL (no indicator matrix in HBM, no TMA) straight into the K-major
 //                 128-byte-swizzled shared-memory layout tcgen05 reads:
@@ -12,10 +12,10 @@
 //                 tcgen05.mma.cta_group::1.kind::i8 M=128 N=144 -- one per label a, each into
 //                 its own 144 TMEM columns.  A TMEM lane is then a SITE: the thread that owns
 //                 lane i reads the nine cells of pair (i, j) from its own lane
-//                 (D_a[i][48 b + j]) without a shuffle.  Two smem stages: the expansion of
-//                 k-block k+1 overlaps the MMAs of k-block k (mbarrier per stage, bounded waits).
-//                 Readout: 8 warps = 4 lane quarters x 2 column halves, tcgen05.ld 32x32b.x8,
-//                 nine u16 counts + flag bits per pair (24 B) into a scratch in pair order.
+//                 (D_a[i][48 b + j]) without a shuffle.  Expansion, MMAs and readout run in
+//                 their own warps over two smem stages (mbarriers, bounded waits); the readout
+//                 (tcgen05.ld 32x32b.x8) writes nine u16 counts + flag bits per pair (24 B)
+//                 into a scratch in pair order.
 //   k_tile_finish one thread per pair: min-common filter + fp64 MI from the nine counts ->
 //                 the unit's dense MI scratch (NaN: dropped / not evaluated) and the number of
 //                 emitted pairs per work item (what k_count does for the other paths).
@@ -37,7 +37,6 @@ constexpr int kTgSitesI = 128;                        // sites per row block: on
 constexpr int kTgSitesJ = 48;                         // partner sites per column block
 constexpr int kTgSites = kTgSitesI + kTgSitesJ;       // plane rows a tile reads per k-block
 constexpr int kTgN = 3 * kTgSitesJ;                   // 144 columns per accumulator (label-major)
-constexpr int kTgThreads = 384;                       // 12 warps: readout = 4 lane quarters x 3 groups of 16 partners
 constexpr uint32_t kTgATile = 128u * 128u;            // one label tile of A: 128 rows x 128 reads, 16 KB
 constexpr uint32_t kTgABytes = 3u * kTgATile;         // 48 KB
 constexpr uint32_t kTgBBytes = (uint32_t)kTgN * 128u; // 18 KB
@@ -45,12 +44,7 @@ constexpr uint32_t kTgStageBytes = kTgABytes + kTgBBytes;
 constexpr int kTgStages = 2;                          // expanded operand stages
 constexpr int kTgAhead = 2;                           // k-blocks of raw planes requested ahead (cp.async)
 constexpr int kTgRawStages = kTgAhead + 1;
-constexpr uint32_t kTgRawBytes = (uint32_t)kTgSites * 3u * 16u;  // [site][plane M, m, C][4 words] = 8448 B
-constexpr int kTgRing = 8;                            // ring of tile ids.  The request cursor can be kTgAhead + 1 tiles past the
-constexpr int kTgRingAhead = kTgAhead + 3;            // tile being computed; ids are fetched one tile earlier than that, so
-                                                      // that a whole step (two barriers) lies between write and first read
 constexpr uint32_t kTgLutBytes = 256u * 8u;           // 8 bits -> 8 bytes
-constexpr uint32_t kTgSmemBytes = kTgStages * kTgStageBytes + kTgRawStages * kTgRawBytes + kTgLutBytes + 1024u /*align*/ + 256u /*barriers*/;
 constexpr uint32_t kTgTmemCols = 512;                 // 3 x 144 used
 constexpr uint32_t kTgMaxReads = 65535;               // counts are stored as u16
 
@@ -65,13 +59,18 @@ __device__ __forceinline__ void tmem_load_x8(uint32_t taddr, uint32_t (&r)[8]) {
                : "memory");
 }
 // 8 bits -> 8 bytes of 0/1 from a 256-entry shared-memory table (2 KB): two look-ups replace the sixteen
-// shift / multiply / mask operations of spread16
+// shift / multiply / mask operations of four spread4 calls
 __device__ __forceinline__ void tg_lut_init(uint2* __restrict__ lut, uint32_t tid, uint32_t n_threads) {
   for (uint32_t k = tid; k < 256u; k += n_threads) lut[k] = make_uint2(spread4(k & 15u), spread4(k >> 4));
 }
 __device__ __forceinline__ uint4 tg_spread16(const uint2* __restrict__ lut, uint32_t bits) {
   const uint2 lo = lut[bits & 0xffu], hi = lut[(bits >> 8) & 0xffu];
   return make_uint4(lo.x, lo.y, hi.x, hi.y);
+}
+
+__device__ __forceinline__ void tg_store(uint8_t* __restrict__ Xkb, uint32_t row, uint32_t chunk, uint4 v) {
+  // K-major SWIZZLE_128B: 8-row groups of 1024 B, 16-byte chunk index XOR row-in-group
+  *reinterpret_cast<uint4*>(Xkb + (row >> 3) * 1024u + (row & 7u) * 128u + ((chunk ^ (row & 7u)) << 4)) = v;
 }
 
 // tcgen05.wait::ld with the loaded registers as in/out operands: nothing that reads them can be
@@ -99,7 +98,6 @@ struct TileGramParams {
   const TgTile* tiles;
   uint32_t n_tiles;
   uint2* cnt;              // three 8-byte words per pair slot (DevUnit::dense_off + pair index)
-  uint32_t* next;          // work counter (zeroed by k_run_init)
   uint32_t* error;
 };
 
@@ -155,187 +153,10 @@ __device__ __forceinline__ void tg_readout(const TileGramParams& P, uint32_t tme
   }
 }
 
-// position in this CTA's stream of (tile, k-block) steps; `seq` counts the CTA's tiles, the tile id comes from the ring
-struct TgCursor {
-  uint32_t seq, kb, nkb;        // nkb == 0: past the end
-  uint32_t i0, j0, S, W, site_off;
-  const uint32_t* planes;       // the unit's first word
-  uint64_t dense_off;
-  __device__ __forceinline__ bool valid() const { return nkb != 0u; }
-  __device__ __forceinline__ void load(const TileGramParams& P, const uint32_t* ring) {
-    const uint32_t t = ring[seq % (uint32_t)kTgRing];
-    nkb = 0u;
-    kb = 0u;
-    if (t >= P.n_tiles) return;
-    const uint4 a = __ldg(reinterpret_cast<const uint4*>(P.tiles + t)), b = __ldg(reinterpret_cast<const uint4*>(P.tiles + t) + 1);
-    planes = P.planes + (((unsigned long long)a.y << 32) | a.x);
-    dense_off = ((unsigned long long)a.w << 32) | a.z;
-    S = b.x;
-    W = b.y;
-    site_off = b.z;
-    i0 = (b.w & 0xffffu) * (uint32_t)kTgSitesI;
-    j0 = (b.w >> 16) * (uint32_t)kTgSitesJ;
-    nkb = W >> 2;  // whole k-blocks of 128 reads (W is a multiple of 4; pad bits are zero)
-  }
-  __device__ __forceinline__ void advance(const TileGramParams& P, const uint32_t* ring) {
-    if (!valid()) return;
-    if (++kb < nkb) return;
-    ++seq;
-    load(P, ring);
-  }
-};
-
-// request the raw plane words of one k-block of a tile: 16 bytes per (site, plane); absent sites are skipped
-__device__ __forceinline__ void tg_request(uint8_t* __restrict__ raw, const TgCursor& c) {
-  if (!c.valid()) return;
-#pragma unroll
-  for (uint32_t e = threadIdx.x; e < (uint32_t)kTgSites * 3u; e += kTgThreads) {
-    const uint32_t sl = e / 3u, plane = e - 3u * sl;
-    const uint32_t s = (sl < (uint32_t)kTgSitesI) ? c.i0 + sl : c.j0 + (sl - (uint32_t)kTgSitesI);
-    if (s < c.S) cp_async16(raw + (size_t)e * 16u, c.planes + ((size_t)s * 3u + plane) * c.W + c.kb * 4u, true);
-  }
-}
-
-// one k-block (128 reads) of the tile's operands from the staged raw words: thread item = (site, 32-read word)
-// -> the three label rows' 2 x 16 bytes each, straight into the swizzled K-major layout.  Rows of absent sites
-// (>= S) are left as they are: their products land in accumulator rows / columns nobody reads.
-__device__ __forceinline__ void tg_expand(uint8_t* __restrict__ stage, const uint8_t* __restrict__ raw, const TgCursor& c,
-                                          const uint2* __restrict__ lut) {
-  constexpr uint32_t kItemsA = (uint32_t)kTgSitesI * 4u, kItems = (uint32_t)kTgSites * 4u;
-#pragma unroll
-  for (uint32_t e = threadIdx.x; e < kItems; e += kTgThreads) {
-    const bool is_a = e < kItemsA;
-    const uint32_t sl_all = e >> 2, w = e & 3u;               // site row of the raw stage
-    const uint32_t sl = is_a ? sl_all : sl_all - (uint32_t)kTgSitesI;
-    const uint32_t s = (is_a ? c.i0 : c.j0) + sl;
-    if (s >= c.S) continue;
-    const uint32_t* __restrict__ src = reinterpret_cast<const uint32_t*>(raw) + sl_all * 12u + w;
-    const uint32_t M = src[0], m = src[4], C = src[8];
-    const uint32_t L2 = M & C, L1 = m & C & ~M, L0 = C & ~M & ~m;
-    uint8_t* t0 = is_a ? stage : stage + kTgABytes;                 // label "other"
-    uint8_t* t1 = is_a ? stage + kTgATile : t0;                     // minor
-    uint8_t* t2 = is_a ? stage + 2u * kTgATile : t0;                // major
-    const uint32_t r0 = sl, r1 = is_a ? sl : (uint32_t)kTgSitesJ + sl, r2 = is_a ? sl : 2u * (uint32_t)kTgSitesJ + sl;
-    sg_store(t0, r0, 2u * w, tg_spread16(lut, L0));
-    sg_store(t0, r0, 2u * w + 1u, tg_spread16(lut, L0 >> 16));
-    sg_store(t1, r1, 2u * w, tg_spread16(lut, L1));
-    sg_store(t1, r1, 2u * w + 1u, tg_spread16(lut, L1 >> 16));
-    sg_store(t2, r2, 2u * w, tg_spread16(lut, L2));
-    sg_store(t2, r2, 2u * w + 1u, tg_spread16(lut, L2 >> 16));
-  }
-}
-
-__global__ void __launch_bounds__(kTgThreads, 1) k_tile_gram(const TileGramParams P) {
-  extern __shared__ uint8_t tg_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tg_raw) + 1023u) & ~uintptr_t(1023));
-  uint8_t* raw0 = smem + kTgStages * kTgStageBytes;
-  uint2* lut = reinterpret_cast<uint2*>(raw0 + kTgRawStages * kTgRawBytes);
-  uint64_t* mma_done = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(lut) + kTgLutBytes);  // [stages]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(mma_done + kTgStages);
-  uint32_t* ring = tmem_slot + 1;                                                       // [kTgRing] tile ids
-  const uint32_t tid = threadIdx.x, warp = tid >> 5;
-
-  if (tid == 0) {
-    for (int s = 0; s < kTgStages; ++s) mbar_init(&mma_done[s], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    for (int q = 0; q < kTgRingAhead; ++q) ring[q] = atomicAdd(P.next, 1u);  // this CTA's first tiles
-  }
-  tg_lut_init(lut, tid, kTgThreads);
-  __syncwarp();
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(kTgTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t idesc = umma_idesc_u8(128u, (uint32_t)kTgN);
-  const bool skip_nonhet = (P.mode & LGMI_MODE_HET_ONLY) && (P.mode & LGMI_MODE_SKIP_NONHET);
-
-  // every commit on a stage's barrier is waited for exactly once, in order (parity per stage)
-  // (bit s of each word: no runtime-indexed arrays, which would live in local memory)
-  uint32_t parity = 0u, pending = 0u, stage = 0u;
-  auto wait_stage = [&](uint32_t s) {
-    if ((pending >> s) & 1u) {
-      mbar_wait(&mma_done[s], (parity >> s) & 1u, P.error);
-      parity ^= 1u << s;
-      pending &= ~(1u << s);
-    }
-  };
-
-  // two cursors over the CTA's (tile, k-block) steps: `cur` is computed, `pre` runs kTgAhead steps ahead and only
-  // requests raw plane words (cp.async), across tile boundaries
-  TgCursor cur, pre;
-  cur.seq = 0u;
-  cur.load(P, ring);
-  pre = cur;
-#pragma unroll
-  for (int d = 0; d < kTgAhead; ++d) {
-    tg_request(raw0 + (uint32_t)d * kTgRawBytes, pre);
-    cp_async_commit();
-    pre.advance(P, ring);
-  }
-
-  for (uint32_t step = 0; cur.valid(); ++step) {
-    tg_request(raw0 + ((step + (uint32_t)kTgAhead) % (uint32_t)kTgRawStages) * kTgRawBytes, pre);
-    cp_async_commit();            // (possibly empty: exactly one group per step)
-    pre.advance(P, ring);
-    cp_async_wait<kTgAhead>();    // this thread's part of step `step` has landed
-    wait_stage(stage);            // the MMAs that read this operand stage two steps ago
-    __syncthreads();              // ... everybody's part
-    uint8_t* st = smem + stage * kTgStageBytes;
-    tg_expand(st, raw0 + (step % (uint32_t)kTgRawStages) * kTgRawBytes, cur, lut);
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> visible to the tensor core
-    __syncthreads();              // (also: the raw stage is consumed; it is requested again next step)
-    if (tid == 0) {
-      tc_fence_after();
-      const uint32_t sa = smem_u32(st), sb = sa + kTgABytes;
-      const uint64_t db = umma_desc_sw128(sb);
-#pragma unroll
-      for (uint32_t k = 0; k < 4; ++k) {  // K = 32 reads per instruction: +32 B on both operands
-#pragma unroll
-        for (uint32_t a = 0; a < 3; ++a)
-          umma_i8(tmem_base + a * (uint32_t)kTgN, umma_desc_sw128(sa + a * kTgATile) + 2ull * k, db + 2ull * k, idesc,
-                  (cur.kb | k) != 0u);
-      }
-      umma_commit(&mma_done[stage]);
-    }
-    pending |= 1u << stage;
-    stage ^= 1u;
-
-    if (cur.kb + 1u == cur.nkb) {
-      // ---- the tile's MMAs are all issued: wait for them (commits complete in issue order), then read out
-      wait_stage(stage);  // older commit first
-      wait_stage(stage ^ 1u);
-      tc_fence_after();
-      // lane = site i; this warp's lane quarter and its 16 partner columns
-      tg_readout(P, tmem_base, warp & 3u, (warp >> 2) * 16u, 2u, cur.i0, cur.j0, cur.S, cur.site_off, cur.dense_off, skip_nonhet);
-      tc_fence_before();
-      __syncthreads();  // accumulators read: TMEM may be overwritten by the next tile's first MMA
-      tc_fence_after();
-      // one more tile id into the ring (a slot whose previous tile finished long ago); its first reader is the
-      // request cursor at the end of the NEXT tile's first step at the earliest (see kTgRingAhead)
-      if (tid == 0) ring[(cur.seq + (uint32_t)kTgRingAhead) % (uint32_t)kTgRing] = atomicAdd(P.next, 1u);
-    }
-    cur.advance(P, ring);
-  }
-  cp_async_wait<0>();
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTgTmemCols) : "memory");
-  }
-}
-
 // ---------------------------------------------------------------------------
-// k_tile_gram_ws: the same tiles, warp-specialised.  k_tile_gram above runs its phases one after the other
-// in every warp (request, expand, barrier, one thread issues the MMAs while the others wait at the next
-// barrier, ... , wait for the MMAs, read out); with tiles of three or four k-blocks the SM is idle most
-// of the time.  Here three groups of warps run their own loops over the CTA's tiles (static stride:
+// k_tile_gram_ws, warp-specialised: with tiles of three or four k-blocks, a CTA whose warps all ran the phases
+// one after the other (request, expand, barrier, MMAs, wait, read out) would leave the SM idle most of the
+// time.  Here three groups of warps run their own loops over the CTA's tiles (static stride:
 // tile = blockIdx.x + n * gridDim.x, deepest first) and meet only through mbarriers:
 //   warps 0-7   expanders   each thread requests ITS OWN raw plane words by cp.async (4 bytes per
 //                           (site, plane, word): what it reads back is what it asked for, so no
@@ -422,12 +243,12 @@ __device__ __forceinline__ void tw_expand(uint8_t* __restrict__ stage, const uin
     uint8_t* t1 = is_a ? stage + kTgATile : t0;
     uint8_t* t2 = is_a ? stage + 2u * kTgATile : t0;
     const uint32_t r0 = sl, r1 = is_a ? sl : (uint32_t)kTgSitesJ + sl, r2 = is_a ? sl : 2u * (uint32_t)kTgSitesJ + sl;
-    sg_store(t0, r0, 2u * w, tg_spread16(lut, L0));
-    sg_store(t0, r0, 2u * w + 1u, tg_spread16(lut, L0 >> 16));
-    sg_store(t1, r1, 2u * w, tg_spread16(lut, L1));
-    sg_store(t1, r1, 2u * w + 1u, tg_spread16(lut, L1 >> 16));
-    sg_store(t2, r2, 2u * w, tg_spread16(lut, L2));
-    sg_store(t2, r2, 2u * w + 1u, tg_spread16(lut, L2 >> 16));
+    tg_store(t0, r0, 2u * w, tg_spread16(lut, L0));
+    tg_store(t0, r0, 2u * w + 1u, tg_spread16(lut, L0 >> 16));
+    tg_store(t1, r1, 2u * w, tg_spread16(lut, L1));
+    tg_store(t1, r1, 2u * w + 1u, tg_spread16(lut, L1 >> 16));
+    tg_store(t2, r2, 2u * w, tg_spread16(lut, L2));
+    tg_store(t2, r2, 2u * w + 1u, tg_spread16(lut, L2 >> 16));
   }
 }
 
@@ -555,7 +376,7 @@ __global__ void __launch_bounds__(kTwThreads, 1) k_tile_gram_ws(const TileGramPa
 }
 
 // ---------------------------------------------------------------------------
-// MI of the pairs k_tile_gram counted: one CTA per work item (<= 2048 consecutive pairs of a unit).
+// MI of the pairs k_tile_gram_ws counted: one CTA per work item (<= 2048 consecutive pairs of a unit).
 // Pass 1 (one thread per pair): min-common filter, emitted-pair count of the item (what k_count computes for
 // the other paths), NaN into the dense MI scratch for the pairs without MI, and the others listed as "2x2"
 // (no "other" label among the common reads) or "3x3".  Pass 2: the branch-free fp64 epilogues of lgmi_fast.cuh

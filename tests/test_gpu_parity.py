@@ -256,10 +256,9 @@ def test_many_sites_multi_item_unit(lg, gpu_ctx):
 
 
 def test_mid_units_popcount_and_tensor_paths_agree(lg, gpu_ctx):
-    """Mid-depth units (more than 64 sites or 256 reads): k_tile_gram + k_tile_finish (tcgen05, path 1), its
-    warp-specialised form k_tile_gram_ws (path 2, the default) and k_tile_mi (popcount, path 0) must give the same records,
-    tables and means bit for bit, and all match the oracle.  Shapes straddle the 128-site row blocks, the 48-site
-    column blocks and the 128-read k-blocks."""
+    """Mid-depth units (more than 64 sites or 256 reads): k_tile_gram_ws + k_tile_finish (tcgen05, the default) and
+    k_tile_mi (popcount, path 0) must give the same records, tables and means bit for bit, and both match the oracle.
+    Shapes straddle the 128-site row blocks, the 48-site column blocks and the 128-read k-blocks."""
     rng = np.random.default_rng(20261031)
     shapes = [(65, 40), (48, 257), (49, 300), (129, 129), (97, 1000), (2, 700), (3, 4097), (257, 70), (200, 385),
               (145, 128), (64, 9000)]
@@ -268,18 +267,17 @@ def test_mid_units_popcount_and_tensor_paths_agree(lg, gpu_ctx):
     pb = lg.pack_units(eus)
     out = {}
     try:
-        for path in (1, 2, 0):
+        for path in (2, 0):
             gpu_ctx.set_tile_path(path)
             full = check_batch(lg, gpu_ctx, eus, 6, min_exact=0.9)
             het = lg.mi_step_batched(pb, 9, lg.MODE_HET_ONLY | lg.MODE_SKIP_NONHET | lg.MODE_EMIT_COUNTS, ctx=gpu_ctx)
             out[path] = (full, het)
     finally:
         gpu_ctx.set_tile_path(2)                                # (the default)
-    for path in (1, 2):
-        for a, b in zip(out[path], out[0]):
-            assert np.array_equal(a.records, b.records) and np.array_equal(a.counts, b.counts)
-            assert np.array_equal(a.site_mean, b.site_mean, equal_nan=True) and np.array_equal(a.site_cnt, b.site_cnt)
-            assert np.array_equal(a.unit_rec_off, b.unit_rec_off)
+    for a, b in zip(out[2], out[0]):
+        assert np.array_equal(a.records, b.records) and np.array_equal(a.counts, b.counts)
+        assert np.array_equal(a.site_mean, b.site_mean, equal_nan=True) and np.array_equal(a.site_cnt, b.site_cnt)
+        assert np.array_equal(a.unit_rec_off, b.unit_rec_off)
 
 
 # --------------------------------------------------------------------------- tensor-core path (K3)
@@ -437,49 +435,28 @@ def test_cfg3_full_size_dense_equals_popcount_and_oracle(lg, gpu_ctx):
     assert_mi_close(rec['mi'][at], mi, 0.9)
 
 
-def test_small_units_popcount_and_tensor_paths_agree(lg, gpu_ctx):
-    """Small units (<= 60 sites, <= 256 reads) counted by k_pairs_fast's AND+popcount (default) and
-    by k_small_gram (int8 Gram matrix per unit): same records, 3x3 tables and means bit
-    for bit, both against the oracle; sizes around every block boundary of the tensor layout
-    (10 sites per 32-lane group, 40 per M block, 128 reads per k-block)."""
+def test_small_units_block_boundaries(lg, gpu_ctx):
+    """Small units (<= 64 sites, <= 256 reads: k_count_fast + k_pairs_fast) from 2 to 64 sites and 6 to 256
+    reads, on both sides of 128 reads (one or two k-blocks of plane words), plus fuzz units: records, 3x3
+    tables and means against the oracle at min_common 1, 6 and 20."""
     rng = np.random.default_rng(41)
     shapes = [(2, 6), (3, 40), (9, 128), (10, 129), (11, 200), (20, 256), (30, 31), (31, 255), (39, 100), (40, 128),
               (41, 129), (50, 200), (59, 256), (60, 200), (61, 200), (64, 256)]
     eus = [_synth_unit(rng, S, R, float(rng.uniform(0.3, 0.95))) for S, R in shapes]
     eus += [lg.encode_mismatches(random_mismatches(rng)) for _ in range(60)]
     eus = [e for e in eus if not e.bad_sites]
-    mode = lg.MODE_ALL_PAIRS | lg.MODE_EMIT_COUNTS
-    try:
-        gpu_ctx.set_small_path(False)
-        popc = check_batch(lg, gpu_ctx, eus, 6)
-        gpu_ctx.set_small_path(True)
-        tens = check_batch(lg, gpu_ctx, eus, 6)
-        for mc in (1, 20):
-            gpu_ctx.set_small_path(False)
-            a = lg.mi_step_batched(lg.pack_units(eus), mc, mode, ctx=gpu_ctx)
-            gpu_ctx.set_small_path(True)
-            b = lg.mi_step_batched(lg.pack_units(eus), mc, mode, ctx=gpu_ctx)
-            assert np.array_equal(a.records, b.records) and np.array_equal(a.counts, b.counts)
-            assert np.array_equal(a.site_mean, b.site_mean, equal_nan=True)
-    finally:
-        gpu_ctx.set_small_path(False)
-    assert np.array_equal(popc.records, tens.records) and np.array_equal(popc.counts, tens.counts)
-    assert np.array_equal(popc.site_mean, tens.site_mean, equal_nan=True)
+    for mc in (1, 6, 20):
+        check_batch(lg, gpu_ctx, eus, mc)
 
 
 def test_small_units_many_others_fall_back(lg, gpu_ctx):
     """More than 7 'other' reads in a cell does not fit the packed form: the unit is flagged and
-    the generic kernel takes it, on either small-unit path."""
+    the generic kernel takes it."""
     rng = np.random.default_rng(42)
     lab = rng.choice(np.array([0, 1, 2, 255], np.uint8), size=(12, 150), p=[0.3, 0.3, 0.3, 0.1])
     eu = enc.EncodedUnit(list(range(12)), ['het_snp', 'mismatch'] * 6, lab)
     ok = _synth_unit(rng, 20, 100, 0.6)
-    for tensor in (True, False):
-        gpu_ctx.set_small_path(tensor)
-        try:
-            check_batch(lg, gpu_ctx, [ok, eu, ok], 6)
-        finally:
-            gpu_ctx.set_small_path(False)
+    check_batch(lg, gpu_ctx, [ok, eu, ok], 6)
 
 
 # --------------------------------------------------------------------------- pipelined step
@@ -689,7 +666,7 @@ def test_cfg4_full_size_properties_and_oracle_sample(lg, gpu_ctx):
     S, R = pb.units['n_sites'].astype(np.int64), pb.units['n_reads'].astype(np.int64)
     out = {}
     try:
-        for path in (1, 2, 0):
+        for path in (2, 0):
             gpu_ctx.set_tile_path(path)
             b = lg.Batch(gpu_ctx, pb)
             b.upload()
@@ -702,11 +679,10 @@ def test_cfg4_full_size_properties_and_oracle_sample(lg, gpu_ctx):
             b.close()
     finally:
         gpu_ctx.set_tile_path(2)                                # (the default)
-    res = out[1]
-    for path in (2, 0):                      # many tiles per CTA here: the tile-to-tile hand-over of both tensor-core forms
-        assert np.array_equal(res.records, out[path].records)
-        assert np.array_equal(res.site_mean, out[path].site_mean, equal_nan=True)
-        assert np.array_equal(res.site_cnt, out[path].site_cnt)
+    res = out[2]                             # many tiles per CTA here: the tile-to-tile hand-over of k_tile_gram_ws
+    assert np.array_equal(res.records, out[0].records)
+    assert np.array_equal(res.site_mean, out[0].site_mean, equal_nan=True)
+    assert np.array_equal(res.site_cnt, out[0].site_cnt)
     _order_and_mean_properties(pb, res)
     rng = np.random.default_rng(2)
     small = np.flatnonzero((S <= 64) & (R <= 256) & (S >= 2))

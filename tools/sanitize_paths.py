@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Small run through every kernel path (small popcount, small tensor, tiled, deep tensor,
-generic fallback, pipeline, ecdf) for compute-sanitizer memcheck.  No timing, no assertions
-beyond agreement of the two small-unit paths."""
+"""Small run through every kernel path (small popcount, tiled, deep tensor, generic fallback,
+pipeline, ecdf) for compute-sanitizer memcheck.  No timing, no assertions beyond agreement of
+the paths."""
 import importlib
 import os
 import sys
@@ -32,14 +32,9 @@ lab = rng.choice(np.array([0, 1, 2, 255], np.uint8), size=(12, 150), p=[0.3, 0.3
 eus.append(enc.EncodedUnit(list(range(12)), ['het_snp', 'mismatch'] * 6, lab))
 pb = lg.pack_units(eus)
 mode = lg.MODE_ALL_PAIRS | lg.MODE_EMIT_COUNTS
-out = {}
-for tensor in (False, True):
-    ctx.set_small_path(tensor)
-    out[tensor] = lg.mi_step_batched(pb, 6, mode, ctx=ctx, n_chunks=1)
-    for m in (lg.MODE_HET_ONLY, lg.MODE_HET_ONLY | lg.MODE_SKIP_NONHET):
-        lg.mi_step_batched(pb, 3, m, ctx=ctx, n_chunks=1)
-assert np.array_equal(out[False].records, out[True].records) and np.array_equal(out[False].counts, out[True].counts)
-ctx.set_small_path(False)
+out = lg.mi_step_batched(pb, 6, mode, ctx=ctx, n_chunks=1)
+for m in (lg.MODE_HET_ONLY, lg.MODE_HET_ONLY | lg.MODE_SKIP_NONHET):
+    lg.mi_step_batched(pb, 3, m, ctx=ctx, n_chunks=1)
 ctx.set_dense_threshold(2, 1)                     # everything with a pair through k_expand_planes + k_gram_i8
 d = lg.mi_step_batched(pb, 6, mode, ctx=ctx, n_chunks=1)
 assert d.n_dense_units >= 10
@@ -48,16 +43,16 @@ r = p.step(6, mode | lg.MODE_SPLIT_RECORDS, packed=True)
 assert r.n_dense_units == d.n_dense_units and np.array_equal(r.records, d.records) and np.array_equal(r.counts, d.counts)
 p.close()
 ctx.set_dense_threshold(*lg.DENSE_DEFAULT)
-assert np.array_equal(d.records, out[False].records) and np.array_equal(d.counts, out[False].counts)
+assert np.array_equal(d.records, out.records) and np.array_equal(d.counts, out.counts)
 for chunks in (2, 5, 40):
     p = lg.Pipeline(ctx, pb, chunks)
     r = p.step(6, mode)
-    assert np.array_equal(r.records, out[False].records)
+    assert np.array_equal(r.records, out.records)
     p.close()
 empty = lg.pack_units([])
 assert lg.mi_step_batched(empty, 6, mode, ctx=ctx).n_records == 0
 p = lg.Pipeline(ctx, empty, 3)
 assert p.step(6, lg.MODE_HET_ONLY).n_records == 0
 p.close()
-mip, call = lg.mip_and_calls(out[False].site_mean, pb.site_flags & 3, 0.05, ctx=ctx)
-print("sanitize run ok:", out[False].n_records, "records,", ctx.launch_count, "launches")
+mip, call = lg.mip_and_calls(out.site_mean, pb.site_flags & 3, 0.05, ctx=ctx)
+print("sanitize run ok:", out.n_records, "records,", ctx.launch_count, "launches")

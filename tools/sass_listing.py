@@ -3,7 +3,7 @@
 (cuobjdump -sass l-giremi_b200/liblgmi.so), one instruction per line without the encodings,
 preceded by a mnemonic histogram and the tensor-core / TMA / async-copy mnemonics found.
 
-    python tools/sass_listing.py [kernel ...]      # default: k_gram_i8 k_tile_gram k_tile_finish k_pairs_fast"""
+    python tools/sass_listing.py [kernel ...]      # default: k_gram_i8 k_tile_gram_ws k_tile_finish k_pairs_fast"""
 import collections
 import os
 import re
@@ -12,7 +12,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "l-giremi_b200", "liblgmi.so")
-DEFAULT = ["k_gram_i8", "k_tile_gram", "k_tile_finish", "k_pairs_fast"]
+DEFAULT = ["k_gram_i8", "k_tile_gram_ws", "k_tile_finish", "k_pairs_fast"]
 ASYNC = ("UTC", "LDTM", "STTM", "UTMA", "LDGSTS", "SYNCS", "UBLKCP")
 
 
