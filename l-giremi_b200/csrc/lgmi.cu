@@ -16,6 +16,7 @@
 #include <new>
 #include <queue>
 #include <map>
+#include <memory>
 #include <string>
 #include <unordered_map>
 #include <vector>
@@ -25,6 +26,7 @@
 
 #include "../../include/lgmi.h"
 #include "lgmi_kernels.cuh"
+#include "lgmi_plan.h"
 
 extern "C" void lgmi_build_lntab(double* hi_lo_pairs, uint64_t k_begin, uint64_t k_end);
 
@@ -143,22 +145,6 @@ static cudaError_t pool_host_alloc(lgmi_ctx* ctx, T** out, size_t bytes) {
   return ctx->host_pool.alloc(reinterpret_cast<void**>(out), bytes);
 }
 
-// one unit of the tensor-core path
-struct DenseTileList {
-  uint64_t off = 0, macs = 0;
-  uint32_t n = 0;
-  uint32_t n_whole = 0;  // the first n_whole work items are whole tiles; the rest share tiles (last wave, split in K)
-};
-struct DensePlan {
-  uint32_t unit = 0, S = 0, W = 0, S_pad = 0, k_blocks = 0;
-  uint32_t rows = 0;          // pairs (i, j) with i < rows are read: S, or the row limit of a piece
-  uint32_t oth_cap = 0;       // listed "other" reads per site (four-block form)
-  bool four = false;          // the four-block form may be chosen (else the run is told "nine" up front)
-  DenseTileList list4, list9; // P, M x P, M  /  C, P, M x C, P, M
-  uint64_t plane_off = 0, gram_off = 0;
-  CUtensorMap tmap;
-};
-
 struct lgmi_batch {
   lgmi_ctx* ctx = nullptr;
   cudaStream_t own_stream = nullptr;  // pipeline chunks run on their own stream; otherwise the context's
@@ -168,7 +154,6 @@ struct lgmi_batch {
   uint64_t plane_words = 0, n_sites = 0, n_candidates = 0, n_dense = 0;
   uint32_t max_reads = 0;
   std::vector<lgmi_unit_desc> h_units;
-  std::vector<Item> h_items;
   // device
   DevUnit* d_units = nullptr;
   Item* d_items = nullptr;
@@ -194,6 +179,7 @@ struct lgmi_batch {
   unsigned long long* d_unit_rec_off = nullptr;
   // tensor-core path
   std::vector<DensePlan> dense_plans;
+  std::vector<CUtensorMap> tmaps;  // per deep unit, parallel to dense_plans: its X for k_gram_i8's TMA loads
   uint8_t* d_x = nullptr;       // indicator matrix of the unit being contracted (reused unit after unit)
   uint32_t* d_gram = nullptr;   // nine count matrices per dense unit
   uint32_t* d_xt = nullptr;     // four-block form: transposed label planes of the unit being contracted
@@ -217,7 +203,6 @@ struct lgmi_batch {
   TiledDesc* d_tiled_desc = nullptr;   // k_pairs_generic<1>'s items, one self-contained record each
   uint32_t n_tiled_desc = 0;
   uint32_t* d_tile_counts = nullptr;  // EMIT_COUNTS only, allocated on first use
-  uint64_t n_tiled_slots = 0;
   // host (pinned) mirrors
   Header* h_header = nullptr;
   lgmi_pair_rec* h_records = nullptr;
@@ -247,37 +232,6 @@ struct lgmi_batch {
   std::vector<uint64_t> h_dense_off;
   cudaEvent_t copy_ev = nullptr;  // lgmi_batch_copy_planes from this batch: what its stream has queued so far
 };
-
-// pairs (i, j), i < j < S, with i < rows: the first rows rows of the pair order (lg_row_off(rows, S))
-static uint64_t piece_pairs(uint32_t rows, uint32_t S) { return rows ? lg_row_off(rows, S) : 0ull; }
-
-// candidate pairs next to a het_snp site, from the host copy of the flag bytes (a piece: its own pairs only)
-static uint64_t het_candidates(const std::vector<lgmi_unit_desc>& units, const std::vector<uint32_t>& row_limit,
-                               const uint8_t* site_flags) {
-  uint64_t tot = 0;
-  for (size_t k = 0; k < units.size(); ++k) {
-    const lgmi_unit_desc& u = units[k];
-    const uint8_t* f = site_flags + u.site_off;
-    auto het = [&](uint32_t s) { return (f[s] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP; };
-    const uint32_t rows = row_limit.empty() ? 0u : row_limit[k];
-    if (rows) {
-      // pairs of the piece minus those whose sites are both non-het: walk the rows from the last, counting the
-      // non-het sites after each
-      uint64_t o_after = 0, both = 0;
-      for (uint32_t s = u.n_sites; s-- > 0;) {
-        if (s < rows && !het(s)) both += o_after;
-        o_after += het(s) ? 0u : 1u;
-      }
-      tot += piece_pairs(rows, u.n_sites) - both;
-      continue;
-    }
-    uint64_t h = 0;
-    for (uint32_t s = 0; s < u.n_sites; ++s) h += het(s) ? 1u : 0u;
-    const uint64_t S = u.n_sites, o = S - h;
-    tot += (S >= 2 ? S * (S - 1) / 2 : 0) - (o >= 2 ? o * (o - 1) / 2 : 0);
-  }
-  return tot;
-}
 
 // --------------------------------------------------------------------------- helpers
 static inline cudaStream_t bstream(const lgmi_batch* b) { return b->own_stream ? b->own_stream : b->ctx->stream; }
@@ -536,15 +490,22 @@ extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
   delete b;
 }
 
-// lgmi_batch_create, and with row_limit (non-NULL) lgmi_batch_create_rows: a unit k with row_limit[k] != 0 is a
-// piece of a split unit -- only its pairs (i, j) with i < row_limit[k] are evaluated and emitted, always through a
-// dense MI slot (the slices of the pieces make up the whole unit's, lgmi_split_means), and it has no per-site means
+// lgmi_batch_create, and with row_limit (non-NULL) lgmi_batch_create_rows (a unit k with row_limit[k] != 0 is a piece
+// of a split unit, plan_batch): the batch's plan, then its buffers and tables on the device and the tensor maps of
+// its deep units.  Nothing is allocated for a batch whose plan fails.
 static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units, const uint32_t* row_limit,
                         uint64_t plane_words, uint64_t n_sites, lgmi_batch_t** out) {
   if (!ctx || !out || (!units && n_units)) return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_create: NULL argument");
   *out = nullptr;
   CU(ctx, cudaSetDevice(ctx->device));
-  lgmi_batch* b = new (std::nothrow) lgmi_batch();
+  const PlanConfig cfg{(uint32_t)ctx->num_sms, ctx->dense_path, ctx->tile_path, ctx->dense_min_sites, ctx->dense_min_reads};
+  BatchPlan plan;
+  std::string err;
+  if (const int rc = plan_batch(units, n_units, row_limit, plane_words, n_sites, cfg, &plan, &err))
+    return fail(ctx, rc, "%s", err.c_str());
+
+  // every failure from here on releases what the batch holds so far
+  std::unique_ptr<lgmi_batch, void (*)(lgmi_batch*)> b(new (std::nothrow) lgmi_batch(), lgmi_batch_destroy);
   if (!b) return fail(ctx, LGMI_ERR_NOMEM, "lgmi_batch_create: out of host memory");
   b->ctx = ctx;
   b->n_units = n_units;
@@ -553,326 +514,100 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
   b->h_units.assign(units, units + n_units);
   if (row_limit) {
     b->h_row_limit.assign(row_limit, row_limit + n_units);
-    b->h_dense_off.assign(n_units, ~0ull);
+    b->h_dense_off.resize(n_units);
+    for (uint32_t k = 0; k < n_units; ++k) b->h_dense_off[k] = plan.units[k].dense_off;
   }
-
-  std::vector<DevUnit> du(n_units);
-  std::vector<FastItem> fast_items;
-  std::vector<MeanItem> mean_items;
-  std::vector<DenseTile> dense_tiles;
-  std::vector<TileItem> tile_items;
-  std::vector<TiledDesc> tiled_desc;  // k_pairs_generic<1>'s items
-  std::vector<TgTile> gram_tiles;
-  std::vector<uint32_t> tile_words, gram_words_of;  // W of each tile's unit (launch order: longest first)
-  bool any_gram_tiled = false;
-  uint64_t dense = 0, gram_words = 0, x_bytes = 0, xt_words = 0, oth_words = 0;
-  uint32_t oth_sites = 0;
-  for (uint32_t k = 0; k < n_units; ++k) {
-    const lgmi_unit_desc& u = units[k];
-    if (u.n_sites > 65535u) {
-      delete b;
-      return fail(ctx, LGMI_ERR_UNSUPPORTED, "unit %u: %u sites > 65535", k, u.n_sites);
-    }
-    if (u.row_words != 4u * ((u.n_reads + 127u) / 128u) || (u.plane_off & 3ull) ||
-        u.plane_off + 3ull * u.n_sites * u.row_words > plane_words ||
-        (uint64_t)u.site_off + u.n_sites > n_sites) {
-      delete b;
-      return fail(ctx, LGMI_ERR_ARG,
-                  "unit %u: inconsistent descriptor (S=%u R=%u W=%u plane_off=%llu site_off=%u)", k,
-                  u.n_sites, u.n_reads, u.row_words, (unsigned long long)u.plane_off, u.site_off);
-    }
-    const uint32_t limit = row_limit ? row_limit[k] : 0u;
-    const bool piece = limit != 0u;
-    if (piece && (limit > u.n_sites || (limit % 128u && limit != u.n_sites))) {
-      delete b;
-      return fail(ctx, LGMI_ERR_ARG, "unit %u: row limit %u is neither a multiple of 128 below S nor S = %u", k, limit,
-                  u.n_sites);
-    }
-    const uint32_t rows = piece ? limit : u.n_sites;  // row blocks at or past it hold no pair of the unit
-    const size_t first_gram_tile = gram_tiles.size();  // this unit's k_tile_gram_ws work items start here
-    DevUnit& d = du[k];
-    d.plane_off = u.plane_off;
-    d.S = u.n_sites;
-    d.R = u.n_reads;
-    d.W = u.row_words;
-    d.site_off = u.site_off;
-    d.first_item = (uint32_t)b->h_items.size();
-    const uint64_t np = piece ? piece_pairs(limit, u.n_sites) : u.n_sites >= 2 ? (uint64_t)u.n_sites * (u.n_sites - 1) / 2 : 0;
-    b->n_candidates += np;
-    b->max_reads = std::max(b->max_reads, u.n_reads);
-    const uint32_t nit = np ? (uint32_t)((np + kPairsMax - 1) / kPairsMax) : 1u;
-    d.n_items = nit;
-    d.dense_off = ~0ull;
-    d.gram_off = kNoGram;
-    d.S_pad = 0;
-    d.tiled = 0;
-    if (np && u.n_sites >= ctx->dense_min_sites && u.n_reads >= ctx->dense_min_reads) {
-      // tensor-core path: the unit's nine count matrices come from k_gram_i8
-      DensePlan pl;
-      pl.unit = k;
-      pl.S = u.n_sites;
-      pl.W = u.row_words;
-      pl.S_pad = (u.n_sites + (uint32_t)kDenseBN - 1u) / (uint32_t)kDenseBN * (uint32_t)kDenseBN;
-      pl.rows = rows;
-      pl.k_blocks = u.row_words * 32u / (uint32_t)kDenseBK;  // W is a multiple of 4: whole 128-read blocks
-      pl.plane_off = u.plane_off;
-      pl.gram_off = gram_words;
-      // (k_other_fix addresses a label's transposed plane with 32-bit word offsets)
-      pl.four = ctx->dense_path == 4 && (uint64_t)pl.k_blocks * kDenseBK * (pl.S_pad / 32u) < (1ull << 32);
-      pl.oth_cap = std::max<uint32_t>(kDenseOthMin, u.n_reads / kDenseOthDiv);
-      auto build_list = [&](DenseTileList& L, uint32_t g0) {  // row groups g0 .. 2 of X against each other
-        L.off = dense_tiles.size();
-        for (uint32_t a = g0; a < 3; ++a)
-          for (uint32_t bb = g0; bb < 3; ++bb)
-            for (uint32_t J = 0; J < pl.S_pad / (uint32_t)kDenseBN; ++J)
-              for (uint32_t I = 0; I < (rows + (uint32_t)kDenseBM - 1u) / (uint32_t)kDenseBM; ++I) {
-                // some pair i < j inside the tile, both real sites
-                const uint32_t i_min = I * (uint32_t)kDenseBM;
-                const uint32_t j_max = std::min(J * (uint32_t)kDenseBN + (uint32_t)kDenseBN, pl.S) - 1u;
-                if (J * (uint32_t)kDenseBN >= pl.S || i_min >= j_max) continue;
-                dense_tiles.push_back(DenseTile{(uint8_t)a, (uint8_t)bb, (uint16_t)I, (uint16_t)J, 0, 0u, pl.k_blocks});
-              }
-        // one CTA per SM walks the list with stride #SMs: a last, partly filled wave leaves SMs idle for a whole
-        // tile time, so its tiles are cut along K into as many parts as fill it (added atomically into zeroed tiles)
-        const uint32_t n = (uint32_t)(dense_tiles.size() - L.off), grid = (uint32_t)ctx->num_sms;
-        const uint32_t rem = n % grid;
-        uint32_t parts = rem ? std::min<uint32_t>(8u, grid / rem) : 1u;
-        while (parts > 1u && pl.k_blocks < 8u * parts) --parts;  // at least 8 k-blocks (1 024 reads) per part
-        L.n_whole = n;
-        if (parts >= 2u) {
-          L.n_whole = n - rem;
-          std::vector<DenseTile> tail(dense_tiles.end() - rem, dense_tiles.end());
-          dense_tiles.resize(dense_tiles.size() - rem);
-          for (uint32_t q = 0; q < parts; ++q)
-            for (DenseTile t : tail) {
-              t.kb0 = (uint32_t)((uint64_t)pl.k_blocks * q / parts);
-              t.kb1 = (uint32_t)((uint64_t)pl.k_blocks * (q + 1) / parts);
-              t.partial = 1;
-              dense_tiles.push_back(t);
-            }
-        }
-        L.n = (uint32_t)(dense_tiles.size() - L.off);
-        for (uint32_t t = 0; t < L.n; ++t) {
-          const DenseTile& dt = dense_tiles[L.off + t];
-          L.macs += (uint64_t)kDenseBM * kDenseBN * (dt.kb1 - dt.kb0) * kDenseBK;
-        }
-      };
-      if (pl.four) build_list(pl.list4, 1u);
-      build_list(pl.list9, 0u);
-      if (pl.four) {
-        xt_words = std::max<uint64_t>(xt_words, 3ull * pl.k_blocks * kDenseBK * (pl.S_pad / 32u));
-        oth_words = std::max<uint64_t>(oth_words, (uint64_t)pl.S * pl.oth_cap);
-        oth_sites = std::max<uint32_t>(oth_sites, pl.S);
-      }
-      gram_words += 9ull * pl.S_pad * pl.S_pad;
-      x_bytes = std::max<uint64_t>(x_bytes, 3ull * pl.S_pad * pl.k_blocks * kDenseBK);
-      d.gram_off = pl.gram_off;
-      d.S_pad = pl.S_pad;
-      b->dense_plans.push_back(pl);
-    } else if (np && (piece || !(nit == 1 && u.n_sites <= (uint32_t)kFastMaxS && u.n_reads <= (uint32_t)kFastMaxR))) {
-      // tiled popcount path: MI of every pair precomputed by k_tile_mi into the dense scratch
-      // (or, by default, counted on the tensor cores by k_tile_gram_ws and finished by k_tile_finish)
-      const bool gram = ctx->tile_path && u.n_reads >= 1u && u.n_reads <= kTgMaxReads;
-      d.tiled = gram ? 2 : 1;
-      if (nit == 1 && !piece) {
-        d.dense_off = dense;
-        dense += np;
-      }
-      if (gram) {
-        any_gram_tiled = true;
-        const uint32_t nI = (rows + (uint32_t)kTgSitesI - 1u) / (uint32_t)kTgSitesI;
-        const uint32_t nJ = (u.n_sites + (uint32_t)kTgSitesJ - 1u) / (uint32_t)kTgSitesJ;
-        for (uint32_t I = 0; I < nI; ++I)
-          for (uint32_t J = 0; J < nJ; ++J) {
-            // some pair i < j with i in row block I and j in column block J
-            const uint32_t j_max = std::min((J + 1u) * (uint32_t)kTgSitesJ, u.n_sites) - 1u;
-            if (I * (uint32_t)kTgSitesI >= j_max) continue;
-            gram_tiles.push_back(TgTile{u.plane_off, 0ull /* set below */, u.n_sites, u.row_words, u.site_off, (uint16_t)I, (uint16_t)J});
-            gram_words_of.push_back(u.row_words);
-          }
-      } else {
-        const uint32_t nb = (u.n_sites + (uint32_t)kTileSites - 1u) / (uint32_t)kTileSites;
-        for (uint32_t I = 0; I < (rows + (uint32_t)kTileSites - 1u) / (uint32_t)kTileSites; ++I)
-          for (uint32_t J = I; J < nb; ++J) {
-            tile_items.push_back(TileItem{k, (uint16_t)I, (uint16_t)J});
-            tile_words.push_back(u.row_words);
-          }
-      }
-    }
-    if (nit > 1 || piece) {
-      d.dense_off = dense;
-      dense += np;
-      if (!piece)  // (a piece's means would be partial: lgmi_split_means computes them over all pieces)
-        for (uint32_t s0 = 0; s0 < u.n_sites; s0 += (uint32_t)kMeanSites) mean_items.push_back(MeanItem{k, s0});
-    }
-    if (piece) b->h_dense_off[k] = d.dense_off;
-    for (size_t t = first_gram_tile; t < gram_tiles.size(); ++t) gram_tiles[t].dense_off = d.dense_off;  // known now
-    for (uint32_t t = 0; t < nit; ++t) {
-      Item it;
-      it.unit = k;
-      it.pair_begin = t * (uint32_t)kPairsMax;
-      it.pair_cnt = (uint32_t)std::min<uint64_t>(kPairsMax, np - (uint64_t)t * kPairsMax);
-      it.flags = (t == 0 ? ITEM_FIRST : 0u) | (nit == 1 && !piece ? ITEM_SINGLE : 0u) | (d.tiled ? ITEM_TILED : 0u) |
-                 (d.tiled == 2 ? ITEM_TILED_GRAM : 0u) | (d.gram_off != kNoGram ? ITEM_GRAM : 0u);
-      if (d.tiled || d.gram_off != kNoGram) ++b->n_tiled_work_items;  // (not k_pairs_generic<0>'s)
-      if (d.tiled) {
-        TiledDesc td{};
-        td.item_idx = (uint32_t)b->h_items.size();
-        td.unit = k, td.pair_begin = it.pair_begin, td.pair_cnt = it.pair_cnt, td.flags = it.flags;
-        td.S = u.n_sites, td.site_off = u.site_off, td.dense_off = d.dense_off;
-        tiled_desc.push_back(td);
-      }
-      if (!piece && nit == 1 && np >= 1 && d.gram_off == kNoGram && u.n_sites <= (uint32_t)kFastMaxS &&
-          u.n_reads <= (uint32_t)kFastMaxR) {
-        it.flags |= ITEM_FAST;  // (a unit sent to the tensor-core path by a lowered threshold is not also k_pairs_fast's)
-        FastItem f;
-        f.plane_off = u.plane_off;
-        f.site_off = u.site_off;
-        f.unit = k;
-        f.item = (uint32_t)b->h_items.size();
-        f.S = (uint16_t)u.n_sites;
-        f.R = (uint16_t)u.n_reads;
-        f.W = u.row_words;
-        f.pad = 0;
-        fast_items.push_back(f);
-      }
-      b->h_items.push_back(it);
-    }
-  }
-  auto deepest_first = [](auto& items, const std::vector<uint32_t>& words) {
-    // the deepest tiles first: CTAs are handed out in order, so the long ones do not end up in the tail
-    std::vector<uint32_t> order(items.size());
-    for (uint32_t t = 0; t < order.size(); ++t) order[t] = t;
-    std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return words[x] > words[y]; });
-    typename std::remove_reference<decltype(items)>::type sorted(items.size());
-    for (uint32_t t = 0; t < order.size(); ++t) sorted[t] = items[order[t]];
-    items.swap(sorted);
+  b->n_items = (uint32_t)plan.items.size();
+  b->n_fast = (uint32_t)plan.fast_items.size();
+  b->n_mean_items = (uint32_t)plan.mean_items.size();
+  b->n_tile_items = (uint32_t)plan.tile_items.size();
+  b->n_gram_tiles = (uint32_t)plan.gram_tiles.size();
+  b->n_tiled_desc = (uint32_t)plan.tiled_desc.size();
+  b->n_tiled_work_items = plan.n_tiled_work_items;
+  b->n_dense = plan.n_dense;
+  b->n_candidates = plan.n_candidates;
+  b->max_reads = plan.max_reads;
+  b->dense_plans = std::move(plan.dense_plans);
+  const cudaStream_t st = bstream(b.get());
+  // a table of the plan on the device: at least min_n entries, the plan's uploaded
+  auto upload = [&](auto** dst, const auto& v, size_t min_n) {
+    const size_t sz = sizeof(v[0]);
+    cudaError_t e = pool_malloc(ctx, dst, std::max(min_n, v.size()) * sz);
+    if (e == cudaSuccess && !v.empty()) e = cudaMemcpyAsync(*dst, v.data(), v.size() * sz, cudaMemcpyHostToDevice, st);
+    return e;
   };
-  deepest_first(tile_items, tile_words);
-  deepest_first(gram_tiles, gram_words_of);
-  // per-site sums: a CTA's time grows with its unit's number of sites (one serial chain of S steps per site), so the
-  // CTAs of the largest units go first and the short ones fill the tail
-  std::stable_sort(mean_items.begin(), mean_items.end(), [&](const MeanItem& x, const MeanItem& y) {
-    return units[x.unit].n_sites > units[y.unit].n_sites;
-  });
-  b->n_tile_items = (uint32_t)tile_items.size();
-  b->n_gram_tiles = (uint32_t)gram_tiles.size();
 
-  b->n_items = (uint32_t)b->h_items.size();
-  b->n_fast = (uint32_t)fast_items.size();
-  b->n_mean_items = (uint32_t)mean_items.size();
-  b->n_dense = dense;
-
-#define BCU(call)                                                                    \
-  do {                                                                               \
-    cudaError_t e__ = (call);                                                        \
-    if (e__ != cudaSuccess) {                                                        \
-      int rc__ = fail(ctx, (e__ == cudaErrorMemoryAllocation) ? LGMI_ERR_NOMEM : LGMI_ERR_CUDA, \
-                      "%s failed: %s", #call, cudaGetErrorString(e__));              \
-      lgmi_batch_destroy(b);                                                         \
-      return rc__;                                                                   \
-    }                                                                                \
-  } while (0)
-
-  for (cudaEvent_t& e : b->ev) BCU(cudaEventCreate(&e));
+  for (cudaEvent_t& e : b->ev) CU(ctx, cudaEventCreate(&e));
   if (b->n_fast && (!b->dense_plans.empty() || b->n_tile_items || b->n_gram_tiles)) {
-    BCU(cudaStreamCreateWithFlags(&b->side_stream, cudaStreamNonBlocking));
-    for (cudaEvent_t& e : b->side_ev) BCU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    CU(ctx, cudaStreamCreateWithFlags(&b->side_stream, cudaStreamNonBlocking));
+    for (cudaEvent_t& e : b->side_ev) CU(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   }
-  BCU(pool_malloc(ctx, &b->d_units, std::max<size_t>(1, n_units) * sizeof(DevUnit)));
-  BCU(pool_malloc(ctx, &b->d_items, std::max<size_t>(1, b->n_items) * sizeof(Item)));
-  BCU(pool_malloc(ctx, &b->d_fast_items, std::max<size_t>(1, fast_items.size()) * sizeof(FastItem)));
-  BCU(pool_malloc(ctx, &b->d_fast_empty, std::max<size_t>(1, fast_items.size())));
-  BCU(pool_malloc(ctx, &b->d_item_dense, std::max<size_t>(1, b->n_items)));
-  BCU(pool_malloc(ctx, &b->d_n_generic, sizeof(uint32_t)));
-  BCU(pool_malloc(ctx, &b->d_mean_items, std::max<size_t>(1, mean_items.size()) * sizeof(MeanItem)));
-  BCU(pool_malloc(ctx, &b->d_planes, std::max<uint64_t>(4, plane_words) * sizeof(uint32_t)));
-  BCU(pool_malloc(ctx, &b->d_flags, std::max<uint64_t>(1, n_sites)));
-  BCU(pool_malloc(ctx, &b->d_item_cnt, ((size_t)b->n_items + 1) * sizeof(unsigned long long)));
-  BCU(pool_malloc(ctx, &b->d_item_off, ((size_t)b->n_items + 1) * sizeof(unsigned long long)));
-  BCU(cub::DeviceScan::ExclusiveSum(nullptr, b->scan_tmp_bytes, b->d_item_cnt, b->d_item_off, (int)b->n_items + 1,
-                                    bstream(b)));
-  BCU(pool_malloc(ctx, &b->d_scan_tmp, std::max<size_t>(b->scan_tmp_bytes, 16)));
-  BCU(cudaMemsetAsync(b->d_item_cnt, 0, ((size_t)b->n_items + 1) * sizeof(unsigned long long), bstream(b)));
-  BCU(pool_malloc(ctx, &b->d_header, sizeof(Header)));
-  BCU(pool_malloc(ctx, &b->d_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
-  BCU(pool_malloc(ctx, &b->d_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
-  BCU(pool_malloc(ctx, &b->d_dense, std::max<uint64_t>(1, dense) * sizeof(double)));
-  BCU(pool_malloc(ctx, &b->d_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
-  if (!tile_items.empty()) {
-    BCU(pool_malloc(ctx, &b->d_tile_items, tile_items.size() * sizeof(TileItem)));
-    BCU(cudaMemcpyAsync(b->d_tile_items, tile_items.data(), tile_items.size() * sizeof(TileItem), cudaMemcpyHostToDevice,
-                        bstream(b)));
+  CU(ctx, upload(&b->d_units, plan.units, 1));
+  CU(ctx, upload(&b->d_items, plan.items, 1));
+  CU(ctx, upload(&b->d_fast_items, plan.fast_items, 1));
+  CU(ctx, pool_malloc(ctx, &b->d_fast_empty, std::max<size_t>(1, b->n_fast)));
+  CU(ctx, pool_malloc(ctx, &b->d_item_dense, std::max<size_t>(1, b->n_items)));
+  CU(ctx, pool_malloc(ctx, &b->d_n_generic, sizeof(uint32_t)));
+  CU(ctx, upload(&b->d_mean_items, plan.mean_items, 1));
+  CU(ctx, pool_malloc(ctx, &b->d_planes, std::max<uint64_t>(4, plane_words) * sizeof(uint32_t)));
+  CU(ctx, pool_malloc(ctx, &b->d_flags, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, pool_malloc(ctx, &b->d_item_cnt, ((size_t)b->n_items + 1) * sizeof(unsigned long long)));
+  CU(ctx, pool_malloc(ctx, &b->d_item_off, ((size_t)b->n_items + 1) * sizeof(unsigned long long)));
+  CU(ctx, cub::DeviceScan::ExclusiveSum(nullptr, b->scan_tmp_bytes, b->d_item_cnt, b->d_item_off, (int)b->n_items + 1, st));
+  CU(ctx, pool_malloc(ctx, &b->d_scan_tmp, std::max<size_t>(b->scan_tmp_bytes, 16)));
+  CU(ctx, cudaMemsetAsync(b->d_item_cnt, 0, ((size_t)b->n_items + 1) * sizeof(unsigned long long), st));
+  CU(ctx, pool_malloc(ctx, &b->d_header, sizeof(Header)));
+  CU(ctx, pool_malloc(ctx, &b->d_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
+  CU(ctx, pool_malloc(ctx, &b->d_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
+  CU(ctx, pool_malloc(ctx, &b->d_dense, std::max<uint64_t>(1, plan.n_dense) * sizeof(double)));
+  CU(ctx, pool_malloc(ctx, &b->d_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
+  if (b->n_tile_items) CU(ctx, upload(&b->d_tile_items, plan.tile_items, 0));
+  if (b->n_gram_tiles) {
+    CU(ctx, upload(&b->d_gram_tiles, plan.gram_tiles, 0));
+    CU(ctx, pool_malloc(ctx, &b->d_tile_cnt, std::max<uint64_t>(1, plan.n_dense) * 3ull * sizeof(uint2)));
   }
-  if (!gram_tiles.empty()) {
-    BCU(pool_malloc(ctx, &b->d_gram_tiles, gram_tiles.size() * sizeof(TgTile)));
-    BCU(cudaMemcpyAsync(b->d_gram_tiles, gram_tiles.data(), gram_tiles.size() * sizeof(TgTile), cudaMemcpyHostToDevice,
-                        bstream(b)));
-  }
-  b->n_tiled_desc = (uint32_t)tiled_desc.size();
-  if (!tiled_desc.empty()) {
-    BCU(pool_malloc(ctx, &b->d_tiled_desc, tiled_desc.size() * sizeof(TiledDesc)));
-    BCU(cudaMemcpyAsync(b->d_tiled_desc, tiled_desc.data(), tiled_desc.size() * sizeof(TiledDesc), cudaMemcpyHostToDevice,
-                        bstream(b)));
-  }
-  if (any_gram_tiled) BCU(pool_malloc(ctx, &b->d_tile_cnt, std::max<uint64_t>(1, dense) * 3ull * sizeof(uint2)));
+  if (b->n_tiled_desc) CU(ctx, upload(&b->d_tiled_desc, plan.tiled_desc, 0));
   if (!b->dense_plans.empty()) {
-    BCU(pool_malloc(ctx, &b->d_x, x_bytes));
-    BCU(cudaMemsetAsync(b->d_x, 0, x_bytes, bstream(b)));  // rows of the site padding stay zero
-    BCU(pool_malloc(ctx, &b->d_gram, gram_words * sizeof(uint32_t)));
-    BCU(pool_malloc(ctx, &b->d_unit_mode, (size_t)n_units * sizeof(uint32_t)));
-    if (xt_words) {
-      BCU(pool_malloc(ctx, &b->d_xt, xt_words * sizeof(uint32_t)));
-      BCU(pool_malloc(ctx, &b->d_oth_list, oth_words * sizeof(uint32_t)));
-      BCU(pool_malloc(ctx, &b->d_oth_cnt, (size_t)oth_sites * sizeof(uint32_t)));
-      BCU(cudaStreamCreateWithFlags(&b->fix_stream, cudaStreamNonBlocking));
-      BCU(cudaEventCreateWithFlags(&b->fix_fork, cudaEventDisableTiming));
-      BCU(cudaEventCreateWithFlags(&b->fix_join, cudaEventDisableTiming));
+    CU(ctx, pool_malloc(ctx, &b->d_x, plan.x_bytes));
+    CU(ctx, cudaMemsetAsync(b->d_x, 0, plan.x_bytes, st));  // rows of the site padding stay zero
+    CU(ctx, pool_malloc(ctx, &b->d_gram, plan.gram_words * sizeof(uint32_t)));
+    CU(ctx, pool_malloc(ctx, &b->d_unit_mode, (size_t)n_units * sizeof(uint32_t)));
+    if (plan.xt_words) {
+      CU(ctx, pool_malloc(ctx, &b->d_xt, plan.xt_words * sizeof(uint32_t)));
+      CU(ctx, pool_malloc(ctx, &b->d_oth_list, plan.oth_words * sizeof(uint32_t)));
+      CU(ctx, pool_malloc(ctx, &b->d_oth_cnt, (size_t)plan.oth_sites * sizeof(uint32_t)));
+      CU(ctx, cudaStreamCreateWithFlags(&b->fix_stream, cudaStreamNonBlocking));
+      CU(ctx, cudaEventCreateWithFlags(&b->fix_fork, cudaEventDisableTiming));
+      CU(ctx, cudaEventCreateWithFlags(&b->fix_join, cudaEventDisableTiming));
     }
-    BCU(pool_malloc(ctx, &b->d_tiles, dense_tiles.size() * sizeof(DenseTile)));
-    BCU(cudaMemcpyAsync(b->d_tiles, dense_tiles.data(), dense_tiles.size() * sizeof(DenseTile), cudaMemcpyHostToDevice,
-                        bstream(b)));
+    CU(ctx, upload(&b->d_tiles, plan.dense_tiles, 0));
     typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
     EncodeTiled encode = reinterpret_cast<EncodeTiled>(ctx->encode_tiled);
-    for (DensePlan& pl : b->dense_plans) {
+    b->tmaps.resize(b->dense_plans.size());
+    for (size_t d = 0; d < b->dense_plans.size(); ++d) {
+      const DensePlan& pl = b->dense_plans[d];
       // X of this unit: [3 * S_pad rows][K_pad bytes], K contiguous; box = 128 rows x 128 bytes, 128B swizzle
       const cuuint64_t dims[2] = {(cuuint64_t)pl.k_blocks * kDenseBK, 3ull * pl.S_pad};
       const cuuint64_t strides[1] = {(cuuint64_t)pl.k_blocks * kDenseBK};
       const cuuint32_t box[2] = {(cuuint32_t)kDenseBK, 128u};
       const cuuint32_t estr[2] = {1u, 1u};
-      const CUresult r = encode(&pl.tmap, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, b->d_x, dims, strides, box, estr,
+      const CUresult r = encode(&b->tmaps[d], CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, b->d_x, dims, strides, box, estr,
                                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        int rc__ = fail(ctx, LGMI_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for unit %u", (int)r, pl.unit);
-        lgmi_batch_destroy(b);
-        return rc__;
-      }
+      if (r != CUDA_SUCCESS) return fail(ctx, LGMI_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for unit %u", (int)r, pl.unit);
     }
   }
   b->rec_cap = std::max<uint64_t>(1, b->n_candidates);
-  BCU(pool_malloc(ctx, &b->d_records, b->rec_cap * sizeof(lgmi_pair_rec)));
-  BCU(pool_host_alloc(ctx, &b->h_header, sizeof(Header)));
-  BCU(pool_host_alloc(ctx, &b->h_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
-  BCU(pool_host_alloc(ctx, &b->h_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
-  BCU(pool_host_alloc(ctx, &b->h_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
-  if (n_units) BCU(cudaMemcpyAsync(b->d_units, du.data(), n_units * sizeof(DevUnit), cudaMemcpyHostToDevice, bstream(b)));
-  if (b->n_items) BCU(cudaMemcpyAsync(b->d_items, b->h_items.data(), b->n_items * sizeof(Item), cudaMemcpyHostToDevice, bstream(b)));
-  if (!fast_items.empty())
-    BCU(cudaMemcpyAsync(b->d_fast_items, fast_items.data(), fast_items.size() * sizeof(FastItem), cudaMemcpyHostToDevice,
-                        bstream(b)));
-  if (!mean_items.empty())
-    BCU(cudaMemcpyAsync(b->d_mean_items, mean_items.data(), mean_items.size() * sizeof(MeanItem), cudaMemcpyHostToDevice, bstream(b)));
-  BCU(cudaStreamSynchronize(bstream(b)));  // the host vectors above go out of scope
-#undef BCU
-  int rc = ensure_lntab(ctx, std::max<uint32_t>(b->max_reads, 1u));
-  if (rc) {
-    lgmi_batch_destroy(b);
-    return rc;
-  }
-  *out = b;
+  CU(ctx, pool_malloc(ctx, &b->d_records, b->rec_cap * sizeof(lgmi_pair_rec)));
+  CU(ctx, pool_host_alloc(ctx, &b->h_header, sizeof(Header)));
+  CU(ctx, pool_host_alloc(ctx, &b->h_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
+  CU(ctx, pool_host_alloc(ctx, &b->h_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
+  CU(ctx, pool_host_alloc(ctx, &b->h_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
+  CU(ctx, cudaStreamSynchronize(st));  // the plan's tables go out of scope
+  if (const int rc = ensure_lntab(ctx, std::max<uint32_t>(b->max_reads, 1u))) return rc;
+  *out = b.release();
   return LGMI_OK;
 }
 
@@ -1130,7 +865,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
                                                                      mode, (uint32_t)form);
         ++ctx->launches;
       }
-      k_gram_i8<<<ggrid, kDenseThreads, kDenseSmemBytes, bstream(b)>>>(pl.tmap, D);
+      k_gram_i8<<<ggrid, kDenseThreads, kDenseSmemBytes, bstream(b)>>>(b->tmaps[&pl - b->dense_plans.data()], D);
       ++ctx->launches;
     }
     if (last && timing) CU(ctx, cudaEventRecord(b->ev[7], bstream(b)));

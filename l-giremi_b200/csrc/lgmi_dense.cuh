@@ -37,25 +37,15 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "lgmi_plan.h"  // the tile shape kDenseBM x kDenseBN x kDenseBK and DenseTile
+
 namespace lgmi {
 
-constexpr int kDenseBM = 128;      // tile rows   (sites i of plane a)
-constexpr int kDenseBN = 256;      // tile columns (sites j of plane b)
-constexpr int kDenseBK = 128;      // bytes of K per stage == one 128B swizzle row
 constexpr int kDenseStages = 4;
 constexpr int kDenseThreads = 256;
 constexpr uint32_t kDenseStageBytes = (kDenseBM + kDenseBN) * kDenseBK;  // 48 KB
 constexpr uint32_t kDenseSmemBytes = kDenseStages * kDenseStageBytes + 1024 /*align*/ + 256 /*barriers*/;
 constexpr uint32_t kDenseTmemCols = 256;
-
-struct DenseTile {
-  uint8_t a, b;       // row groups of X (0 covered, 1 major or minor, 2 major)
-  uint16_t I, J;      // site blocks: rows [128 I, +128), columns [256 J, +256)
-  uint16_t partial;   // 1: the tile's K range is shared by several items (last wave): results are added atomically
-                      //    into a zeroed tile
-  uint32_t kb0, kb1;  // k-blocks [kb0, kb1) of this work item (32 bits: a unit may have millions of reads)
-};
-static_assert(sizeof(DenseTile) == 16, "DenseTile layout");
 
 struct DenseParams {
   const DenseTile* tiles;
@@ -71,9 +61,6 @@ struct DenseParams {
 // ------------------------------------------------------------------ expansion
 // 4 bits -> 4 bytes of 0/1
 __device__ __forceinline__ uint32_t spread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; }
-
-constexpr uint32_t kDenseOthDiv = 64u;   // a site lists up to max(256, R / 64) reads with label "other"
-constexpr uint32_t kDenseOthMin = 256u;
 
 // 32 x 32 bit transpose across a warp: lane p ends up with bit q = bit p of lane q's word
 __device__ __forceinline__ uint32_t transpose32(uint32_t x, uint32_t lane) {

@@ -30,13 +30,12 @@
 #include <stdint.h>
 
 #include "lgmi_math.cuh"
+#include "lgmi_plan.h"  // kFastMaxS, kFastMaxR and FastItem
 
 namespace lgmi {
 
 constexpr int kFastThreads = 256;
 constexpr int kFastWarps = kFastThreads / 32;
-constexpr int kFastMaxS = 64;        // sites per unit on the fast path
-constexpr int kFastMaxR = 256;       // reads per unit on the fast path
 constexpr int kFastMaxPairs = 2048;  // >= 64*63/2 = 2016, whole 32-pair chunks
 constexpr int kFastChunks = kFastMaxPairs / 32;
 constexpr int kRowStride = 28;       // words per landed site row: M[8] | P[8] | C[8] | pad[4]
@@ -67,17 +66,6 @@ struct GlobalTab {
     return r;
   }
   __device__ __forceinline__ double inv_at(uint32_t k) const { return k ? __drcp_rn((double)k) : 0.0; }
-};
-
-// one work item of the fast kernel == one whole unit
-struct __align__(16) FastItem {
-  unsigned long long plane_off;  // words
-  uint32_t site_off;
-  uint32_t unit;
-  uint32_t item;                 // index into item_off / item_cnt
-  uint16_t S, R;
-  uint32_t W;                    // row words of the input planes (4 or 8)
-  uint32_t pad;
 };
 
 struct FastSmem {

@@ -1,11 +1,15 @@
 // lgmi_kernels.cuh -- sm_100a kernels of the MI step.
 //
-//   k_pairs            K1+K2: per-pair AND+popcount contingency counts over the
-//                      common reads, fused fp64 MI epilogue, min-common filter,
-//                      het filter, ORDERED compaction of the surviving pairs
-//                      (single pass, decoupled look-back across CTAs) and, for
-//                      units that fit one CTA, the per-site mean MI.
-//   k_site_mean_dense  per-site mean MI for units spanning several CTAs.
+//   k_count, k_count_fast  K0: emitted pairs per work item; an exclusive scan of
+//                      these fixes every item's place in the ordered output.
+//   k_pairs_generic    K1+K2: per-pair contingency counts over the common reads
+//                      (AND+popcount, or read from what k_tile_mi, k_tile_gram_ws
+//                      or k_gram_i8 computed), fp64 MI, min-common and het
+//                      filters, emission at the item's offset and, for units of
+//                      one item, the per-site mean MI.  The small units take
+//                      k_pairs_fast (lgmi_fast_kernel.cuh).
+//   k_tile_mi          counts + MI of the mid-depth units per 16 x 16 site block.
+//   k_site_mean_dense  per-site mean MI for units spanning several items.
 //   k_site_mean_csr    mean of caller-supplied rows (drop-in for
 //                      mean_mismatch_pair_mutual_info).
 //   k_ecdf_*           K4: het-SNP mean collection, searchsorted-left, mip, call.
@@ -18,48 +22,13 @@
 
 #include "../../include/lgmi.h"
 #include "lgmi_math.cuh"
+#include "lgmi_plan.h"
 #include "lgmi_fast_kernel.cuh"
 #include "lgmi_dense.cuh"
 
 namespace lgmi {
 
-constexpr int kThreads = 256;   // CTA size of k_pairs
-constexpr int kPairsMax = 2048; // pairs per work item (>= 64*63/2: a 64-site unit is one item)
-
-struct DevUnit {
-  uint64_t plane_off;  // words
-  uint64_t dense_off;  // first slot in the dense MI scratch (multi-item units), else ~0
-  uint64_t gram_off;   // first word of the unit's nine count matrices (tensor-core path), else ~0
-  uint32_t S, R, W, site_off;
-  uint32_t first_item, n_items;
-  uint32_t S_pad;
-  uint32_t tiled;      // MI of every pair is precomputed into the dense scratch: 1 by k_tile_mi, 2 by k_tile_gram_ws + k_tile_finish
-};
-constexpr uint64_t kNoGram = ~0ull;
-
-enum : uint32_t {
-  ITEM_FIRST = 1u, ITEM_SINGLE = 2u, ITEM_FAST = 4u,
-  ITEM_TILED = 16u /* MI precomputed by k_tile_mi or k_tile_gram_ws + k_tile_finish */,
-  ITEM_TILED_GRAM = 32u /* ... by the latter, which also counts the item's emitted pairs */,
-  ITEM_GRAM = 64u /* deep unit: tables from the count matrices of the tensor-core path (k_pairs_generic<2>) */
-};
-
-struct Item {
-  uint32_t unit;
-  uint32_t pair_begin;
-  uint32_t pair_cnt;
-  uint32_t flags;
-};
-
-// Everything k_pairs_generic<1> needs of a work item of a mid-depth (tiled) unit, in one 48-byte record built on
-// the host: the kernel requests the next record (cp.async) while it works on the current item, instead of the
-// chain items[] -> units[] at the head of every item.
-struct __align__(16) TiledDesc {
-  uint32_t item_idx, unit, pair_begin, pair_cnt;
-  uint32_t flags, S, site_off, pad;
-  uint64_t dense_off, pad2;
-};
-static_assert(sizeof(TiledDesc) == 48, "three 16-byte copies per record");
+constexpr int kThreads = 256;   // CTA size of k_pairs_generic, k_count, k_count_fast, k_tile_mi and k_tile_finish
 
 struct Header {
   unsigned long long n_records;
@@ -481,14 +450,8 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
 // pair's MI (NaN: dropped by min-common / not evaluated) to the unit's dense
 // scratch in pair order.  k_count / k_pairs_generic then only compact and order
 // what is already there.
-constexpr int kTileSites = 16;   // sites per block
 constexpr int kTileKC = 32;      // words of each plane per staged chunk
 constexpr int kTileStride = 36;  // words per staged row: 16-byte aligned; 8 consecutive rows cover all 32 banks
-
-struct TileItem {
-  uint32_t unit;
-  uint16_t I, J;  // site blocks of 16 sites, I <= J
-};
 
 // running bit-sliced count of one AND+popcount set
 struct CsaAcc {
@@ -819,13 +782,8 @@ __global__ void __launch_bounds__(kThreads) k_count(const RunParams P) {
 // side by side, one site per lane, partners ascending.  The order of the additions is part of
 // the result (mutual_information.py:56-58 is a left-to-right float sum), so each site's sum is
 // serial; the 32 sites of a block are not.
-constexpr int kMeanSites = 32;    // sites per CTA (= lanes of the consuming warp)
 constexpr int kMeanThreads = 256;
 constexpr int kMeanBufs = 5;      // tile buffers: one being summed, one being masked, three in flight
-struct MeanItem {
-  uint32_t unit;
-  uint32_t site_begin;
-};
 __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src, bool copy) {
   const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem_dst);
   const int n = copy ? 8 : 0;  // src-size 0: the 8 destination bytes are zero-filled

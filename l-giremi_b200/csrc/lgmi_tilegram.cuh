@@ -19,7 +19,7 @@
 //   k_tile_finish one thread per pair: min-common filter + fp64 MI from the nine counts ->
 //                 the unit's dense MI scratch (NaN: dropped / not evaluated) and the number of
 //                 emitted pairs per work item (what k_count does for the other paths).
-// k_pairs_generic<true> / k_site_mean_dense then order, emit and average as for k_tile_mi,
+// k_pairs_generic<1> / k_site_mean_dense then order, emit and average as for k_tile_mi,
 // which stays as the popcount form of this path (lgmi_set_tile_path(ctx, 0); units deeper
 // than 65 535 reads, whose counts do not fit 16 bits, always take it).
 //
@@ -29,12 +29,11 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-// (included at the end of lgmi_kernels.cuh: DevUnit, Item, TileItem, RunParams, LnGlobal are defined there)
+// (included at the end of lgmi_kernels.cuh: RunParams and LnGlobal are defined there; the tile shape
+// kTgSitesI x kTgSitesJ, kTgMaxReads and TgTile in lgmi_plan.h)
 
 namespace lgmi {
 
-constexpr int kTgSitesI = 128;                        // sites per row block: one per TMEM lane
-constexpr int kTgSitesJ = 48;                         // partner sites per column block
 constexpr int kTgSites = kTgSitesI + kTgSitesJ;       // plane rows a tile reads per k-block
 constexpr int kTgN = 3 * kTgSitesJ;                   // 144 columns per accumulator (label-major)
 constexpr uint32_t kTgATile = 128u * 128u;            // one label tile of A: 128 rows x 128 reads, 16 KB
@@ -46,7 +45,6 @@ constexpr int kTgAhead = 2;                           // k-blocks of raw planes 
 constexpr int kTgRawStages = kTgAhead + 1;
 constexpr uint32_t kTgLutBytes = 256u * 8u;           // 8 bits -> 8 bytes
 constexpr uint32_t kTgTmemCols = 512;                 // 3 x 144 used
-constexpr uint32_t kTgMaxReads = 65535;               // counts are stored as u16
 
 // flag bits of a pair's 24-byte count record
 constexpr uint32_t kTgNotEvaluated = 1u;  // SKIP_NONHET and no het_snp partner
@@ -81,15 +79,6 @@ __device__ __forceinline__ void tmem_wait_x8(uint32_t (&r)[8]) {
                :
                : "memory");
 }
-
-// one work item, self-contained (built on the host: no dependent look-up of the unit table in the kernel)
-struct __align__(16) TgTile {
-  unsigned long long plane_off;  // first word of the unit's planes
-  unsigned long long dense_off;  // first pair slot of the unit
-  uint32_t S, W, site_off;
-  uint16_t I, J;                 // row block of 128 sites, column block of 48 sites
-};
-static_assert(sizeof(TgTile) == 32, "TgTile layout");
 
 struct TileGramParams {
   const uint32_t* planes;

@@ -289,7 +289,7 @@ def _synth_unit(rng, S, R, cov):
 
 @pytest.fixture()
 def dense_everything(lg, gpu_ctx):
-    """Every unit with a pair goes through k_expand_planes + k_gram_i8."""
+    """Every unit with a pair goes through k_dense_x + k_gram_i8."""
     gpu_ctx.set_dense_threshold(2, 1)
     yield gpu_ctx
     gpu_ctx.set_dense_threshold(*lg.DENSE_DEFAULT)

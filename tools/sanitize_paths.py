@@ -35,7 +35,7 @@ mode = lg.MODE_ALL_PAIRS | lg.MODE_EMIT_COUNTS
 out = lg.mi_step_batched(pb, 6, mode, ctx=ctx, n_chunks=1)
 for m in (lg.MODE_HET_ONLY, lg.MODE_HET_ONLY | lg.MODE_SKIP_NONHET):
     lg.mi_step_batched(pb, 3, m, ctx=ctx, n_chunks=1)
-ctx.set_dense_threshold(2, 1)                     # everything with a pair through k_expand_planes + k_gram_i8
+ctx.set_dense_threshold(2, 1)                     # everything with a pair through k_dense_x + k_gram_i8
 d = lg.mi_step_batched(pb, 6, mode, ctx=ctx, n_chunks=1)
 assert d.n_dense_units >= 10
 p = lg.Pipeline(ctx, pb, 3)                       # ... also inside the groups of a pipelined step, packed input
