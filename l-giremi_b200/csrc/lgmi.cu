@@ -1201,6 +1201,29 @@ extern "C" int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* si
 // stream: H2D of group k+1, kernels of group k and D2H of group k-1 overlap (two copy
 // engines + the SMs).  Outputs are merged into one set of pinned host arrays in the
 // reference's row order, identical to upload + run + download of the whole batch.
+
+// the input and output form of a step, decoded from its mode once (pipeline_begin)
+struct StepForm {
+  bool split = false;        // MI and (i, j) in arrays of their own (LGMI_MODE_SPLIT_RECORDS or COMPACT_OUTPUT)
+  bool compact = false;      // LGMI_MODE_COMPACT_OUTPUT: split rows with 2-byte (i, j) where possible, no site_cnt
+  bool ij16 = false;         // ... and possible: no unit has more than 256 sites
+  bool tight = false;        // LGMI_MODE_TIGHT_INPUT
+  bool want_counts = false;  // LGMI_MODE_EMIT_COUNTS
+  uint32_t run_mode = 0;     // the mode without the bits that are a matter of the copies, not of the kernels
+  size_t ij_bytes() const { return ij16 ? sizeof(uint16_t) : sizeof(uint32_t); }
+};
+
+static StepForm step_form(uint32_t mode, uint32_t max_sites) {
+  StepForm f;
+  f.compact = (mode & LGMI_MODE_COMPACT_OUTPUT) != 0u;
+  f.split = (mode & LGMI_MODE_SPLIT_RECORDS) != 0u || f.compact;
+  f.ij16 = f.compact && max_sites <= 256u;
+  f.tight = (mode & LGMI_MODE_TIGHT_INPUT) != 0u;
+  f.want_counts = (mode & LGMI_MODE_EMIT_COUNTS) != 0u;
+  f.run_mode = mode & ~(LGMI_MODE_SPLIT_RECORDS | LGMI_MODE_COMPACT_OUTPUT | LGMI_MODE_TIGHT_INPUT);
+  return f;
+}
+
 struct lgmi_pipeline {
   lgmi_ctx* ctx = nullptr;
   uint32_t n_units = 0;
@@ -1231,14 +1254,13 @@ struct lgmi_pipeline {
   uint32_t* h_rec_ij = nullptr;   // (2-byte entries under LGMI_MODE_COMPACT_OUTPUT when every unit has <= 256 sites)
   uint64_t h_rec_ij_cap = 0;
   uint32_t max_sites = 0;
-  std::vector<uint64_t> tight_off;  // per unit: first word in the tight two-plane input
   double* h_site_mean = nullptr;
   uint32_t* h_site_cnt = nullptr;
   unsigned long long* h_unit_rec_off = nullptr;
   // a step between lgmi_pipeline_begin* and lgmi_pipeline_finish
   bool in_flight = false;   // begun, not finished
   bool collected = false;   // ... and its downloads queued (lgmi_pipeline_collect)
-  uint32_t pend_mode = 0;
+  StepForm form;
   uint64_t pend_rows = 0;
 };
 
@@ -1278,101 +1300,46 @@ extern "C" int lgmi_pipeline_create(lgmi_t* ctx, const lgmi_unit_desc* units, ui
                                     uint64_t n_sites, uint32_t n_chunks, lgmi_pipeline_t** out) {
   if (!ctx || !out || (!units && n_units)) return fail(ctx, LGMI_ERR_ARG, "lgmi_pipeline_create: NULL argument");
   *out = nullptr;
-  if (n_chunks == 0) return fail(ctx, LGMI_ERR_ARG, "lgmi_pipeline_create: n_chunks must be >= 1");
+  PipelinePlan plan;
+  std::string err;
+  if (const int rc = plan_pipeline(units, n_units, n_chunks, &plan, &err)) return fail(ctx, rc, "%s", err.c_str());
   CU(ctx, cudaSetDevice(ctx->device));
-  // groups are slices of the input buffers: units must be laid out back to back, in order
-  uint64_t total = 0;
-  for (uint32_t k = 0; k < n_units; ++k) {
-    const lgmi_unit_desc& u = units[k];
-    const uint64_t want_plane = k ? units[k - 1].plane_off + 3ull * units[k - 1].n_sites * units[k - 1].row_words : u.plane_off;
-    const uint64_t want_site = k ? (uint64_t)units[k - 1].site_off + units[k - 1].n_sites : u.site_off;
-    if (u.plane_off != want_plane || u.site_off != want_site)
-      return fail(ctx, LGMI_ERR_UNSUPPORTED, "lgmi_pipeline_create: unit %u is not laid out right after unit %u", k, k - 1);
-    total += u.n_sites >= 2 ? (uint64_t)u.n_sites * (u.n_sites - 1) / 2 : 0;
-  }
-  lgmi_pipeline* p = new (std::nothrow) lgmi_pipeline();
+
+  // every failure from here on releases what the pipeline holds so far
+  std::unique_ptr<lgmi_pipeline, void (*)(lgmi_pipeline*)> p(new (std::nothrow) lgmi_pipeline(), lgmi_pipeline_destroy);
   if (!p) return fail(ctx, LGMI_ERR_NOMEM, "lgmi_pipeline_create: out of host memory");
   p->ctx = ctx;
   p->n_units = n_units;
   p->plane_words = plane_words;
   p->n_sites = n_sites;
-  p->n_candidates = total;
-#define PCU(call)                                                                              \
-  do {                                                                                         \
-    cudaError_t e__ = (call);                                                                  \
-    if (e__ != cudaSuccess) {                                                                  \
-      int rc__ = fail(ctx, (e__ == cudaErrorMemoryAllocation) ? LGMI_ERR_NOMEM : LGMI_ERR_CUDA, \
-                      "%s failed: %s", #call, cudaGetErrorString(e__));                        \
-      lgmi_pipeline_destroy(p);                                                                \
-      return rc__;                                                                             \
-    }                                                                                          \
-  } while (0)
-  // the tight two-plane form (LGMI_MODE_TIGHT_INPUT): rows of ceil(R/32) words, units back to back
-  p->tight_off.resize((size_t)n_units + 1);
-  {
-    uint64_t off = 0;
-    for (uint32_t k = 0; k < n_units; ++k) {
-      p->tight_off[k] = off;
-      off += 2ull * units[k].n_sites * ((units[k].n_reads + 31u) / 32u);
-      p->max_sites = std::max(p->max_sites, units[k].n_sites);
+  p->n_candidates = plan.n_candidates;
+  p->max_sites = plan.max_sites;
+  for (const GroupPlan& g : plan.groups) {
+    p->chunks.emplace_back();
+    lgmi_pipeline::Chunk& c = p->chunks.back();
+    if (const int rc = lgmi_batch_create(ctx, g.units.data(), g.n_units, g.plane_words, g.n_sites, &c.b)) return rc;
+    c.b->unit_base = g.unit0;  // records carry the unit's index in the whole batch
+    c.unit0 = g.unit0;
+    c.n_units = g.n_units;
+    c.plane0 = g.plane0;
+    c.site0 = g.site0;
+    c.tight0 = g.tight0;
+    c.tight_words = g.tight_words;
+    if (g.n_units) {
+      const size_t bytes = g.tight_off.size() * sizeof(unsigned long long);
+      CU(ctx, pool_malloc(ctx, &c.d_tight_off, bytes));
+      CU(ctx, cudaMemcpy(c.d_tight_off, g.tight_off.data(), bytes, cudaMemcpyHostToDevice));
     }
-    p->tight_off[n_units] = off;
+    CU(ctx, cudaStreamCreateWithFlags(&c.b->own_stream, cudaStreamNonBlocking));
+    CU(ctx, cudaEventCreateWithFlags(&c.done, cudaEventDisableTiming));
+    CU(ctx, cudaEventCreateWithFlags(&c.landed, cudaEventDisableTiming));
   }
-  // equal shares of the work: candidate pairs plus a term for the bytes to move
-  std::vector<uint64_t> cost(n_units);
-  uint64_t cost_total = 0;
-  for (uint32_t k = 0; k < n_units; ++k) {
-    const lgmi_unit_desc& u = units[k];
-    cost[k] = (u.n_sites >= 2 ? (uint64_t)u.n_sites * (u.n_sites - 1) / 2 : 0) + (uint64_t)u.n_sites * u.row_words / 4 + 1;
-    cost_total += cost[k];
-  }
-  n_chunks = std::min<uint32_t>(n_chunks, std::max<uint32_t>(1, n_units));
-  uint32_t k = 0;
-  uint64_t done_cost = 0;
-  for (uint32_t c = 0; c < n_chunks && (k < n_units || c == 0); ++c) {
-    lgmi_pipeline::Chunk ch;
-    ch.unit0 = k;
-    const uint64_t target = cost_total * (c + 1) / n_chunks;
-    while (k < n_units && (done_cost < target || c + 1 == n_chunks)) done_cost += cost[k++];
-    ch.n_units = k - ch.unit0;
-    if (ch.n_units == 0 && n_units) continue;  // one unit outweighs a whole share
-    ch.plane0 = ch.n_units ? units[ch.unit0].plane_off : 0;
-    ch.site0 = ch.n_units ? units[ch.unit0].site_off : 0;
-    std::vector<lgmi_unit_desc> local(units + ch.unit0, units + k);
-    uint64_t pw = 0, ns = 0;
-    for (lgmi_unit_desc& u : local) {
-      u.plane_off -= ch.plane0;
-      u.site_off -= (uint32_t)ch.site0;
-      pw = u.plane_off + 3ull * u.n_sites * u.row_words;
-      ns = (uint64_t)u.site_off + u.n_sites;
-    }
-    int rc = lgmi_batch_create(ctx, local.data(), ch.n_units, pw, ns, &ch.b);
-    if (rc) {
-      lgmi_pipeline_destroy(p);
-      return rc;
-    }
-    p->chunks.push_back(ch);
-    lgmi_pipeline::Chunk& ref = p->chunks.back();
-    ref.b->unit_base = ref.unit0;  // records carry the unit's index in the whole batch
-    ref.tight0 = p->tight_off[ref.unit0];
-    ref.tight_words = p->tight_off[ref.unit0 + ref.n_units] - ref.tight0;
-    if (ref.n_units) {
-      std::vector<unsigned long long> rel(ref.n_units);
-      for (uint32_t q = 0; q < ref.n_units; ++q) rel[q] = p->tight_off[ref.unit0 + q] - ref.tight0;
-      PCU(pool_malloc(ctx, &ref.d_tight_off, rel.size() * sizeof(unsigned long long)));
-      PCU(cudaMemcpy(ref.d_tight_off, rel.data(), rel.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice));
-    }
-    PCU(cudaStreamCreateWithFlags(&ref.b->own_stream, cudaStreamNonBlocking));
-    PCU(cudaEventCreateWithFlags(&ref.done, cudaEventDisableTiming));
-    PCU(cudaEventCreateWithFlags(&ref.landed, cudaEventDisableTiming));
-  }
-  PCU(cudaStreamCreateWithFlags(&p->h2d, cudaStreamNonBlocking));
-  PCU(cudaStreamCreateWithFlags(&p->d2h, cudaStreamNonBlocking));
-  PCU(pool_host_alloc(ctx, &p->h_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
-  PCU(pool_host_alloc(ctx, &p->h_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
-  PCU(pool_host_alloc(ctx, &p->h_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
-#undef PCU
-  *out = p;
+  CU(ctx, cudaStreamCreateWithFlags(&p->h2d, cudaStreamNonBlocking));
+  CU(ctx, cudaStreamCreateWithFlags(&p->d2h, cudaStreamNonBlocking));
+  CU(ctx, pool_host_alloc(ctx, &p->h_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
+  CU(ctx, pool_host_alloc(ctx, &p->h_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
+  CU(ctx, pool_host_alloc(ctx, &p->h_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
+  *out = p.release();
   return LGMI_OK;
 }
 
@@ -1402,25 +1369,20 @@ static int pipeline_begin(lgmi_pipeline* p, const uint32_t* planes, bool packed,
   if ((!planes && p->plane_words) || (!site_flags && p->n_sites))
     return fail(ctx, LGMI_ERR_ARG, "lgmi_pipeline_step: NULL input");
   CU(ctx, cudaSetDevice(ctx->device));
-  const bool compact = (mode & LGMI_MODE_COMPACT_OUTPUT) != 0u;  // split rows with 2-byte (i, j) where possible, no site_cnt
-  const bool split = (mode & LGMI_MODE_SPLIT_RECORDS) != 0u || compact;
-  const bool ij16 = compact && p->max_sites <= 256u;
-  const bool tight = (mode & LGMI_MODE_TIGHT_INPUT) != 0u;
-  if (tight && !packed) return fail(ctx, LGMI_ERR_ARG, "LGMI_MODE_TIGHT_INPUT is a form of the two-plane input (lgmi_pipeline_step_packed)");
-  p->pend_mode = mode;
-  mode &= ~(LGMI_MODE_SPLIT_RECORDS | LGMI_MODE_COMPACT_OUTPUT | LGMI_MODE_TIGHT_INPUT);  // a matter of the copies, not of the kernels
+  const StepForm f = step_form(mode, p->max_sites);
+  if (f.tight && !packed) return fail(ctx, LGMI_ERR_ARG, "LGMI_MODE_TIGHT_INPUT is a form of the two-plane input (lgmi_pipeline_step_packed)");
+  p->form = f;
   for (lgmi_pipeline::Chunk& c : p->chunks) {
     lgmi_batch* b = c.b;
     cudaStream_t st = b->own_stream;
-    int rc = LGMI_OK;
     // input on the upload stream, in group order; the group's own stream picks up when it has landed
     if (b->n_sites) CU(ctx, cudaMemcpyAsync(b->d_flags, site_flags + c.site0, b->n_sites, cudaMemcpyHostToDevice, p->h2d));
     const uint64_t words2 = b->plane_words / 3u * 2u;           // staging sized for the padded form: either fits
-    const uint64_t words_in = tight ? c.tight_words : words2;
+    const uint64_t words_in = f.tight ? c.tight_words : words2;
     if (packed) {  // two planes per site over PCIe, expanded on the device
       if (!c.d_packed && words2) CU(ctx, pool_malloc(ctx, &c.d_packed, words2 * sizeof(uint32_t)));
       if (words_in)
-        CU(ctx, cudaMemcpyAsync(c.d_packed, planes + (tight ? c.tight0 : c.plane0 / 3u * 2u), words_in * sizeof(uint32_t),
+        CU(ctx, cudaMemcpyAsync(c.d_packed, planes + (f.tight ? c.tight0 : c.plane0 / 3u * 2u), words_in * sizeof(uint32_t),
                                 cudaMemcpyHostToDevice, p->h2d));
     } else if (b->plane_words) {
       CU(ctx, cudaMemcpyAsync(b->d_planes, planes + c.plane0, b->plane_words * sizeof(uint32_t), cudaMemcpyHostToDevice,
@@ -1430,23 +1392,22 @@ static int pipeline_begin(lgmi_pipeline* p, const uint32_t* planes, bool packed,
     CU(ctx, cudaStreamWaitEvent(st, c.landed, 0));
     if (packed && words2) {
       k_unpack2<<<std::min<uint32_t>(b->n_units, (uint32_t)ctx->num_sms * 16u), 256, 0, st>>>(
-          b->d_units, b->n_units, c.d_packed, b->d_planes, tight ? c.d_tight_off : nullptr);
+          b->d_units, b->n_units, c.d_packed, b->d_planes, f.tight ? c.d_tight_off : nullptr);
       ++ctx->launches;
     }
     b->uploaded = true;
-    if (mode & LGMI_MODE_SKIP_NONHET) {
+    if (f.run_mode & LGMI_MODE_SKIP_NONHET) {
       b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags + c.site0) : 0;
       b->het_known = true;
     }
-    if (!rc) rc = lgmi_batch_run(b, min_common, mode);
-    if (rc) return rc;
-    if (split) {
+    if (const int rc = lgmi_batch_run(b, min_common, f.run_mode)) return rc;
+    if (f.split) {
       if (!c.d_rec_mi) {
         CU(ctx, pool_malloc(ctx, &c.d_rec_mi, b->rec_cap * sizeof(double)));
         CU(ctx, pool_malloc(ctx, &c.d_rec_ij, b->rec_cap * sizeof(uint32_t)));
       }
       k_split_records<<<(unsigned)ctx->num_sms * 8u, 256, 0, st>>>(b->d_header, b->d_records, c.d_rec_mi, c.d_rec_ij,
-                                                                   ij16 ? reinterpret_cast<uint16_t*>(c.d_rec_ij) : nullptr);
+                                                                   f.ij16 ? reinterpret_cast<uint16_t*>(c.d_rec_ij) : nullptr);
       ++ctx->launches;
     }
     CU(ctx, cudaEventRecord(c.done, st));  // the group's record count is in its (host-resident) header by then
@@ -1463,12 +1424,8 @@ static int pipeline_collect(lgmi_pipeline* p) {
   if (!p->in_flight) return fail(ctx, LGMI_ERR_STATE, "lgmi_pipeline_collect / finish: no step has been begun");
   if (p->collected) return LGMI_OK;
   CU(ctx, cudaSetDevice(ctx->device));
-  const uint32_t mode = p->pend_mode;
-  const bool want_counts = (mode & LGMI_MODE_EMIT_COUNTS) != 0u;
-  const bool compact = (mode & LGMI_MODE_COMPACT_OUTPUT) != 0u;
-  const bool split = (mode & LGMI_MODE_SPLIT_RECORDS) != 0u || compact;
-  const bool ij16 = compact && p->max_sites <= 256u;
-  const size_t ij_bytes = ij16 ? sizeof(uint16_t) : sizeof(uint32_t);
+  const StepForm& f = p->form;
+  const size_t ij_bytes = f.ij_bytes();
   static const bool debug = getenv("LGMI_PIPE_DEBUG") != nullptr;
   const auto t_begin = std::chrono::steady_clock::now();
   auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
@@ -1481,31 +1438,31 @@ static int pipeline_collect(lgmi_pipeline* p) {
     const uint64_t nrec = b->h_header->n_records;
     if (nrec > b->rec_cap) return fail(ctx, LGMI_ERR_STATE, "record count %llu exceeds capacity", (unsigned long long)nrec);
     int rc = LGMI_OK;
-    if (split) {
+    if (f.split) {
       rc = grow_pinned(p, p->h_rec_mi, p->h_rec_mi_cap, base + nrec, base, sizeof(double));
       if (!rc) rc = grow_pinned(p, p->h_rec_ij, p->h_rec_ij_cap, base + nrec, base, sizeof(uint32_t));
     } else {
       rc = grow_pinned(p, p->h_records, p->h_rec_cap, base + nrec, base, sizeof(lgmi_pair_rec));
     }
-    if (!rc && want_counts) rc = grow_pinned(p, p->h_counts, p->h_counts_cap, base + nrec, base, 9 * sizeof(uint32_t));
+    if (!rc && f.want_counts) rc = grow_pinned(p, p->h_counts, p->h_counts_cap, base + nrec, base, 9 * sizeof(uint32_t));
     if (rc) return rc;
     cudaStream_t st = p->d2h;  // the group is complete (event above): nothing here waits on a kernel
     if (nrec) {
-      if (split) {
+      if (f.split) {
         CU(ctx, cudaMemcpyAsync(p->h_rec_mi + base, c.d_rec_mi, nrec * sizeof(double), cudaMemcpyDeviceToHost, st));
         CU(ctx, cudaMemcpyAsync(reinterpret_cast<char*>(p->h_rec_ij) + base * ij_bytes, c.d_rec_ij, nrec * ij_bytes,
                                 cudaMemcpyDeviceToHost, st));
       } else {
         CU(ctx, cudaMemcpyAsync(p->h_records + base, b->d_records, nrec * sizeof(lgmi_pair_rec), cudaMemcpyDeviceToHost, st));
       }
-      if (want_counts)
+      if (f.want_counts)
         CU(ctx, cudaMemcpyAsync(p->h_counts + base * 9ull, b->d_counts, nrec * 9ull * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     }
     CU(ctx, cudaMemcpyAsync(b->h_unit_rec_off, b->d_unit_rec_off, ((size_t)b->n_units + 1) * sizeof(unsigned long long),
                             cudaMemcpyDeviceToHost, st));
     if (b->n_sites) {
       CU(ctx, cudaMemcpyAsync(p->h_site_mean + c.site0, b->d_site_mean, b->n_sites * sizeof(double), cudaMemcpyDeviceToHost, st));
-      if (!compact)
+      if (!f.compact)
         CU(ctx, cudaMemcpyAsync(p->h_site_cnt + c.site0, b->d_site_cnt, b->n_sites * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     }
     c.base = base;
@@ -1534,11 +1491,7 @@ static int pipeline_finish(lgmi_pipeline* p, lgmi_result* out) {
     return rc_collect;
   }
   p->in_flight = p->collected = false;
-  const uint32_t mode = p->pend_mode;
-  const bool want_counts = (mode & LGMI_MODE_EMIT_COUNTS) != 0u;
-  const bool compact = (mode & LGMI_MODE_COMPACT_OUTPUT) != 0u;
-  const bool split = (mode & LGMI_MODE_SPLIT_RECORDS) != 0u || compact;
-  const size_t ij_bytes = (compact && p->max_sites <= 256u) ? sizeof(uint16_t) : sizeof(uint32_t);
+  const StepForm& f = p->form;
   const uint64_t base = p->pend_rows;
   CU(ctx, cudaStreamSynchronize(p->d2h));
   for (lgmi_pipeline::Chunk& c : p->chunks) {
@@ -1549,14 +1502,14 @@ static int pipeline_finish(lgmi_pipeline* p, lgmi_result* out) {
   out->n_candidates = p->n_candidates;
   out->n_evaluated = 0;
   out->n_records = base;
-  out->records = split ? nullptr : p->h_records;
-  out->rec_mi = split ? p->h_rec_mi : nullptr;
-  out->rec_ij = split ? p->h_rec_ij : nullptr;
-  out->rec_ij_bytes = split ? (uint32_t)ij_bytes : 0u;
-  out->counts = want_counts ? p->h_counts : nullptr;
+  out->records = f.split ? nullptr : p->h_records;
+  out->rec_mi = f.split ? p->h_rec_mi : nullptr;
+  out->rec_ij = f.split ? p->h_rec_ij : nullptr;
+  out->rec_ij_bytes = f.split ? (uint32_t)f.ij_bytes() : 0u;
+  out->counts = f.want_counts ? p->h_counts : nullptr;
   out->n_sites = p->n_sites;
   out->site_mean = p->h_site_mean;
-  out->site_cnt = compact ? nullptr : p->h_site_cnt;
+  out->site_cnt = f.compact ? nullptr : p->h_site_cnt;
   out->unit_rec_off = reinterpret_cast<const uint64_t*>(p->h_unit_rec_off);
   for (lgmi_pipeline::Chunk& c : p->chunks) {
     lgmi_result r;

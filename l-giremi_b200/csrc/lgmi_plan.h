@@ -1,6 +1,7 @@
 // lgmi_plan.h -- the host-side plan of a batch: which kernel path each unit takes and the work tables the
-// kernels read.  Plain C++17 (no CUDA types or calls): lgmi.cu uploads what plan_batch() builds, and the CPU
-// tests (tests/csrc/plan_host.cpp) check the same tables without a device.
+// kernels read; and the groups of a pipelined step.  Plain C++17 (no CUDA types or calls): lgmi.cu uploads what
+// plan_batch() builds and sets up the groups plan_pipeline() cuts, and the CPU tests (tests/csrc/plan_host.cpp)
+// check the same plans without a device.
 #pragma once
 #include <stdint.h>
 
@@ -385,6 +386,78 @@ inline int plan_batch(const lgmi_unit_desc* units, uint32_t n_units, const uint3
   std::stable_sort(P.mean_items.begin(), P.mean_items.end(), [&](const MeanItem& x, const MeanItem& y) {
     return units[x.unit].n_sites > units[y.unit].n_sites;
   });
+  return LGMI_OK;
+}
+
+// ------------------------------------------------------------------ the plan of a pipelined step
+// one group: a batch of its own over the units [unit0, unit0 + n_units) of the whole batch
+struct GroupPlan {
+  uint32_t unit0 = 0, n_units = 0;
+  uint64_t plane0 = 0, site0 = 0;             // the group's first plane word and site in the whole batch
+  uint64_t tight0 = 0, tight_words = 0;       // its slice of the tight two-plane input (LGMI_MODE_TIGHT_INPUT)
+  std::vector<lgmi_unit_desc> units;          // its descriptors, rebased to plane0 / site0
+  uint64_t plane_words = 0, n_sites = 0;      // ... and the sizes of its batch
+  std::vector<unsigned long long> tight_off;  // first word of each unit in the tight input, relative to tight0
+};
+
+struct PipelinePlan {
+  std::vector<GroupPlan> groups;
+  uint64_t n_candidates = 0;
+  uint32_t max_sites = 0;
+};
+
+// The groups of a pipelined step: the units cut into at most n_chunks consecutive groups of about equal cost.  A
+// group's input is a slice of the whole batch's, so the units must lie back to back, in order.  Returns LGMI_OK, or
+// LGMI_ERR_ARG / LGMI_ERR_UNSUPPORTED with *err set.
+inline int plan_pipeline(const lgmi_unit_desc* units, uint32_t n_units, uint32_t n_chunks, PipelinePlan* plan,
+                         std::string* err) {
+  PipelinePlan& P = *plan;
+  P = PipelinePlan();
+  if (n_chunks == 0) return plan_error(err, LGMI_ERR_ARG, "lgmi_pipeline_create: n_chunks must be >= 1");
+  std::vector<uint64_t> tight_off((size_t)n_units + 1, 0), cost(n_units);
+  uint64_t cost_total = 0;
+  for (uint32_t k = 0; k < n_units; ++k) {
+    const lgmi_unit_desc& u = units[k];
+    const uint64_t want_plane = k ? units[k - 1].plane_off + 3ull * units[k - 1].n_sites * units[k - 1].row_words : u.plane_off;
+    const uint64_t want_site = k ? (uint64_t)units[k - 1].site_off + units[k - 1].n_sites : u.site_off;
+    if (u.plane_off != want_plane || u.site_off != want_site)
+      return plan_error(err, LGMI_ERR_UNSUPPORTED, "lgmi_pipeline_create: unit %u is not laid out right after unit %u",
+                        k, k - 1);
+    const uint64_t np = unit_pairs(u.n_sites, 0u);
+    P.n_candidates += np;
+    P.max_sites = std::max(P.max_sites, u.n_sites);
+    // the tight two-plane form: rows of ceil(R/32) words, units back to back
+    tight_off[k + 1] = tight_off[k] + 2ull * u.n_sites * ((u.n_reads + 31u) / 32u);
+    // equal shares of the work: candidate pairs plus a term for the bytes to move
+    cost[k] = np + (uint64_t)u.n_sites * u.row_words / 4 + 1;
+    cost_total += cost[k];
+  }
+  n_chunks = std::min<uint32_t>(n_chunks, std::max<uint32_t>(1, n_units));
+  uint32_t k = 0;
+  uint64_t done_cost = 0;
+  for (uint32_t c = 0; c < n_chunks && (k < n_units || c == 0); ++c) {
+    const uint32_t unit0 = k;
+    const uint64_t target = cost_total * (c + 1) / n_chunks;
+    while (k < n_units && (done_cost < target || c + 1 == n_chunks)) done_cost += cost[k++];
+    if (k == unit0 && n_units) continue;  // one unit outweighs a whole share
+    GroupPlan g;
+    g.unit0 = unit0;
+    g.n_units = k - unit0;
+    g.plane0 = g.n_units ? units[unit0].plane_off : 0;
+    g.site0 = g.n_units ? units[unit0].site_off : 0;
+    g.tight0 = tight_off[unit0];
+    g.tight_words = tight_off[k] - g.tight0;
+    g.units.assign(units + unit0, units + k);
+    for (uint32_t q = 0; q < g.n_units; ++q) {
+      lgmi_unit_desc& u = g.units[q];
+      u.plane_off -= g.plane0;
+      u.site_off -= (uint32_t)g.site0;
+      g.plane_words = u.plane_off + 3ull * u.n_sites * u.row_words;
+      g.n_sites = (uint64_t)u.site_off + u.n_sites;
+      g.tight_off.push_back(tight_off[unit0 + q] - g.tight0);
+    }
+    P.groups.push_back(std::move(g));
+  }
   return LGMI_OK;
 }
 

@@ -1,6 +1,6 @@
 // Host build of l-giremi_b200/csrc/lgmi_plan.h for the CPU tests of the batch plan (tests/test_plan_host.py):
-// the same plan_batch() lgmi_batch_create runs, its tables copied out for ctypes.  Test infrastructure; not part of
-// the product library.
+// the same plan_batch() lgmi_batch_create runs and plan_pipeline() lgmi_pipeline_create runs, their tables copied
+// out for ctypes.  Test infrastructure; not part of the product library.
 #include <cstdint>
 #include <cstring>
 #include "../../l-giremi_b200/csrc/lgmi_plan.h"
@@ -85,5 +85,36 @@ uint64_t p_het_candidates(const lgmi_unit_desc* units, uint32_t n_units, const u
   std::vector<uint32_t> rl;
   if (row_limit) rl.assign(row_limit, row_limit + n_units);
   return het_candidates(u, rl, site_flags);
+}
+
+// the plan of a pipelined step: a handle, or NULL with *rc and err[0 .. err_cap) set
+void* p_pipeline(const lgmi_unit_desc* units, uint32_t n_units, uint32_t n_chunks, int* rc, char* err,
+                 uint32_t err_cap) {
+  PipelinePlan* p = new PipelinePlan();
+  std::string msg;
+  *rc = plan_pipeline(units, n_units, n_chunks, p, &msg);
+  if (*rc == LGMI_OK) return p;
+  snprintf(err, err_cap, "%s", msg.c_str());
+  delete p;
+  return nullptr;
+}
+void p_pipeline_free(void* h) { delete static_cast<PipelinePlan*>(h); }
+
+// n_candidates, max_sites.  Returns the number of groups.
+uint64_t p_pipeline_sizes(void* h, uint64_t* out) {
+  const PipelinePlan& p = *static_cast<PipelinePlan*>(h);
+  out[0] = p.n_candidates;
+  out[1] = p.max_sites;
+  return p.groups.size();
+}
+
+// group g: 8 words unit0, n_units, plane0, site0, tight0, tight_words, plane_words, n_sites; its rebased descriptors
+// and relative tight offsets (n_units of each) are copied to units / tight_off unless NULL
+void p_group(void* h, uint32_t g, uint64_t* out, void* units, void* tight_off) {
+  const GroupPlan& q = static_cast<PipelinePlan*>(h)->groups[g];
+  const uint64_t v[8] = {q.unit0, q.n_units, q.plane0, q.site0, q.tight0, q.tight_words, q.plane_words, q.n_sites};
+  memcpy(out, v, sizeof v);
+  copy_out(q.units, units);
+  copy_out(q.tight_off, tight_off);
 }
 }

@@ -1,5 +1,6 @@
 """The batch plan (csrc/lgmi_plan.h) built for the host: which kernel path each unit takes and the work tables
-lgmi_batch_create uploads, each checked against a computation of its own here.  No device needed."""
+lgmi_batch_create uploads, and the groups lgmi_pipeline_create sets up, each checked against a computation of its
+own here.  No device needed."""
 import ctypes
 import os
 import subprocess
@@ -70,6 +71,14 @@ def plan_host():
     lib.p_route.argtypes = [vp, u32, vp]
     lib.p_het_candidates.restype = u64
     lib.p_het_candidates.argtypes = [vp, u32, vp, vp]
+    lib.p_pipeline.restype = vp
+    lib.p_pipeline.argtypes = [vp, u32, u32, vp, ctypes.c_char_p, u32]
+    lib.p_pipeline_free.restype = None
+    lib.p_pipeline_free.argtypes = [vp]
+    lib.p_pipeline_sizes.restype = u64
+    lib.p_pipeline_sizes.argtypes = [vp, vp]
+    lib.p_group.restype = None
+    lib.p_group.argtypes = [vp, u32, vp, vp, vp]
     for t, dt in enumerate(DTYPES):
         assert lib.p_table_elem(t) == dt.itemsize, TABLES[t]
     return lib
@@ -395,3 +404,165 @@ def test_errors(plan_host):
     for limit in (100, 257, 301):
         assert err([(300, 100)], [limit]) == (
             LGMI_ERR_ARG, "unit 0: row limit %d is neither a multiple of 128 below S nor S = 300" % limit)
+
+
+# --------------------------------------------------------------------------- the groups of a pipelined step
+GROUP_FIELDS = ["unit0", "n_units", "plane0", "site0", "tight0", "tight_words", "plane_words", "n_sites"]
+
+
+def pipeline_plan(lib, units, n_chunks):
+    """(groups, n_candidates, max_sites) of plan_pipeline; each group a dict with its rebased descriptors and
+    relative tight offsets (raises on a planning error)."""
+    units = np.ascontiguousarray(units, UNIT_DESC)
+    rc, err = ctypes.c_int(0), ctypes.create_string_buffer(512)
+    h = lib.p_pipeline(units.ctypes.data, len(units), n_chunks, ctypes.byref(rc), err, 512)
+    if not h:
+        raise ValueError(rc.value, err.value.decode())
+    try:
+        sizes = np.zeros(2, np.uint64)
+        groups = []
+        for g in range(lib.p_pipeline_sizes(h, sizes.ctypes.data)):
+            v = np.zeros(len(GROUP_FIELDS), np.uint64)
+            lib.p_group(h, g, v.ctypes.data, None, None)
+            grp = {k: int(x) for k, x in zip(GROUP_FIELDS, v)}
+            grp["units"] = np.zeros(grp["n_units"], UNIT_DESC)
+            grp["tight_off"] = np.zeros(grp["n_units"], np.uint64)
+            lib.p_group(h, g, v.ctypes.data, grp["units"].ctypes.data, grp["tight_off"].ctypes.data)
+            groups.append(grp)
+        return groups, int(sizes[0]), int(sizes[1])
+    finally:
+        lib.p_pipeline_free(h)
+
+
+def equal_cost_cut(units, n_chunks, clamp=True):
+    """(unit0, n_units) of each group: group c ends at the first unit boundary where the running cost (candidate pairs
+    + S * W / 4 + 1 per unit) reaches c + 1 shares of the total, the last group at the end; empty groups are dropped,
+    except the one group of a batch without units.  clamp: at most one group per unit."""
+    n = len(units)
+    cost = [pairs(int(u["n_sites"])) + int(u["n_sites"]) * int(u["row_words"]) // 4 + 1 for u in units]
+    prefix = np.concatenate(([0], np.cumsum(cost, dtype=np.int64)))
+    total = int(prefix[-1])
+    shares = min(n_chunks, max(1, n)) if clamp else n_chunks
+    ends = [n if c + 1 == shares else int(np.searchsorted(prefix, total * (c + 1) // shares)) for c in range(shares)]
+    bounds = [0] + ends
+    return [(a, b - a) for a, b in zip(bounds, bounds[1:]) if b > a] or [(0, 0)]
+
+
+def tight_layout(units):
+    """First word of each unit in the tight two-plane input (rows of ceil(R/32) words, units back to back), and the
+    end."""
+    S, R = units["n_sites"].astype(np.int64), units["n_reads"].astype(np.int64)
+    return np.concatenate(([0], np.cumsum(2 * S * ((R + 31) // 32))))
+
+
+def check_pipeline(lib, units, n_chunks):
+    """plan_pipeline against equal_cost_cut, the descriptors rebased by hand and tight_layout; returns the groups."""
+    groups, n_candidates, max_sites = pipeline_plan(lib, units, n_chunks)
+    assert [(g["unit0"], g["n_units"]) for g in groups] == equal_cost_cut(units, n_chunks)
+    assert 1 <= len(groups) <= min(n_chunks, max(1, len(units)))
+    # contiguous, in order, covering [0, n_units)
+    assert groups[0]["unit0"] == 0 and groups[-1]["unit0"] + groups[-1]["n_units"] == len(units)
+    assert all(a["unit0"] + a["n_units"] == b["unit0"] for a, b in zip(groups, groups[1:]))
+    tight = tight_layout(units)
+    for g in groups:
+        mine = units[g["unit0"]:g["unit0"] + g["n_units"]]
+        S, W = mine["n_sites"].astype(np.int64), mine["row_words"].astype(np.int64)
+        assert g["plane0"] == (int(mine[0]["plane_off"]) if len(mine) else 0)
+        assert g["site0"] == (int(mine[0]["site_off"]) if len(mine) else 0)
+        want = mine.copy()
+        want["plane_off"] -= g["plane0"]
+        want["site_off"] -= g["site0"]
+        assert g["units"].tobytes() == want.tobytes()
+        assert g["plane_words"] == int((3 * S * W).sum()) and g["n_sites"] == int(S.sum())
+        assert g["tight0"] == tight[g["unit0"]]
+        assert g["tight_words"] == tight[g["unit0"] + g["n_units"]] - g["tight0"]
+        assert g["tight_off"].tolist() == (tight[g["unit0"]:g["unit0"] + g["n_units"]] - g["tight0"]).tolist()
+    assert n_candidates == sum(pairs(int(S)) for S in units["n_sites"])
+    assert max_sites == max((int(S) for S in units["n_sites"]), default=0)
+    return groups
+
+
+@pytest.mark.parametrize("n_chunks", [1, 2, 5, 64])
+def test_pipeline_groups_heavy_tail(plan_host, lg, n_chunks):
+    """The 90-unit heavy tail of the GPU pipeline test: the equal-cost cut, and the relative tight offsets pick each
+    unit's rows out of PlaneBatch.packed2(tight=True) (the padded two-plane rows without their padding)."""
+    import importlib
+    synth = importlib.import_module("l-giremi_b200.synth")
+    pb, _ = synth.make_heavy_tail(20261024, 90, s_max=200, r_max=3000)
+    groups = check_pipeline(plan_host, pb.units, n_chunks)
+    assert len(groups) == n_chunks or n_chunks == 64
+    padded, tight = pb.packed2(), pb.packed2(tight=True)
+    assert groups[-1]["tight0"] + groups[-1]["tight_words"] == tight.size
+    for g in groups:
+        for q, u in enumerate(g["units"]):
+            k = g["unit0"] + q
+            S, W, wt = int(u["n_sites"]), int(u["row_words"]), (int(u["n_reads"]) + 31) // 32
+            rows = tight[g["tight0"] + int(g["tight_off"][q]):][:2 * S * wt].reshape(S, 2, wt)
+            want = padded[int(pb.units["plane_off"][k]) // 3 * 2:][:2 * S * W].reshape(S, 2, W)[:, :, :wt]
+            assert np.array_equal(rows, want)
+
+
+def test_pipeline_groups_uniform(plan_host):
+    """A cfg2-like table (20 000 units of 50 sites x 200 reads) in 4 groups of 5 000 units."""
+    units, pw, ns = descs([(50, 200)] * 20000)
+    groups = check_pipeline(plan_host, units, 4)
+    assert [g["n_units"] for g in groups] == [5000] * 4
+    assert sum(g["plane_words"] for g in groups) == pw and sum(g["n_sites"] for g in groups) == ns
+
+
+def test_pipeline_groups_edge_cases(plan_host):
+    """More groups asked for than units, a unit that outweighs whole shares, no units at all, one unit."""
+    # at most one group per unit: cut into 64 shares instead of 3, these units would make three groups, not two
+    units, _, _ = descs([(2, 10), (4, 10), (2, 10)])
+    assert equal_cost_cut(units, 64, clamp=False) == [(0, 1), (1, 1), (2, 1)]
+    assert [(g["unit0"], g["n_units"]) for g in check_pipeline(plan_host, units, 64)] == [(0, 2), (2, 1)]
+    # a dominant unit covers the shares of several groups: those groups are skipped, not left empty
+    units, _, _ = descs([(10, 10)] * 3 + [(2000, 100)] + [(10, 10)] * 3)
+    groups = check_pipeline(plan_host, units, 4)
+    assert [(g["unit0"], g["n_units"]) for g in groups] == [(0, 4), (4, 3)]
+    # no units: one empty group
+    units, _, _ = descs([])
+    for n_chunks in (1, 4):
+        groups = check_pipeline(plan_host, units, n_chunks)
+        assert len(groups) == 1 and groups[0]["n_units"] == 0 and groups[0]["plane_words"] == groups[0]["n_sites"] == 0
+    # one unit, and units without pairs
+    for shapes in ([(300, 5000)], [(0, 0), (1, 7), (0, 0)]):
+        units, _, _ = descs(shapes)
+        assert len(check_pipeline(plan_host, units, 8)) == len(shapes)
+
+
+def test_pipeline_groups_random(plan_host):
+    """Random tables, with units without pairs among them, at random group counts."""
+    rng = np.random.default_rng(11)
+    for _ in range(40):
+        n = int(rng.integers(0, 60))
+        shapes = [(int(rng.choice([0, 1, 2, int(rng.integers(2, 400))])), int(rng.integers(0, 5000))) for _ in range(n)]
+        units, _, _ = descs(shapes)
+        check_pipeline(plan_host, units, int(rng.integers(1, 80)))
+
+
+def test_pipeline_errors(plan_host):
+    """No groups, and units that are not back to back: the error code and message of lgmi_pipeline_create, naming
+    the first unit out of place."""
+    def err(units, n_chunks):
+        with pytest.raises(ValueError) as e:
+            pipeline_plan(plan_host, units, n_chunks)
+        return e.value.args
+
+    units, _, _ = descs([(5, 40)] * 4)
+    assert err(units, 0) == (LGMI_ERR_ARG, "lgmi_pipeline_create: n_chunks must be >= 1")
+    assert err(units[::-1], 2) == (LGMI_ERR_UNSUPPORTED, "lgmi_pipeline_create: unit 1 is not laid out right after unit 0")
+    gap = units.copy()
+    gap["plane_off"][2:] += 4
+    assert err(gap, 2) == (LGMI_ERR_UNSUPPORTED, "lgmi_pipeline_create: unit 2 is not laid out right after unit 1")
+    sites = units.copy()
+    sites["site_off"][3] += 1
+    gap["site_off"][3] += 1
+    assert err(sites, 1) == (LGMI_ERR_UNSUPPORTED, "lgmi_pipeline_create: unit 3 is not laid out right after unit 2")
+    assert err(gap, 1) == (LGMI_ERR_UNSUPPORTED, "lgmi_pipeline_create: unit 2 is not laid out right after unit 1")
+    # the first unit may start anywhere
+    start = units.copy()
+    start["plane_off"] += 8
+    start["site_off"] += 3
+    groups = check_pipeline(plan_host, start, 2)
+    assert groups[0]["plane0"] == 8 and groups[0]["site0"] == 3
