@@ -15,10 +15,8 @@
 #include <cstring>
 #include <new>
 #include <queue>
-#include <map>
 #include <memory>
 #include <string>
-#include <unordered_map>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -27,6 +25,7 @@
 #include "../../include/lgmi.h"
 #include "lgmi_kernels.cuh"
 #include "lgmi_plan.h"
+#include "lgmi_pool.h"
 
 extern "C" void lgmi_build_lntab(double* hi_lo_pairs, uint64_t k_begin, uint64_t k_end);
 
@@ -34,94 +33,69 @@ using namespace lgmi;
 
 static thread_local std::string g_create_error;
 
-// Size-bucketed cache of device and pinned-host blocks owned by a context.  Batches and pipelines are created and
-// destroyed per submit by the drop-in seam (one chunk of footprints = one submit); cudaMalloc / cudaHostAlloc /
-// cudaFree cost tens of microseconds to milliseconds each and cudaFree synchronises the device, so their buffers
-// are recycled instead.  A block is only returned to the cache after the owning batch's stream has been
-// synchronised (lgmi_batch_destroy), i.e. nothing in flight can still touch it.
-struct MemPool {
-  std::multimap<size_t, void*> free_blocks;
-  std::unordered_map<void*, size_t> live;
-  size_t cached_bytes = 0, cap_bytes = 0;
-  uint64_t hits = 0, misses = 0;
-  bool host = false;
-  static size_t bucket(size_t n) {  // sixteenth-of-an-octave steps: at most 1/8 over-allocation
-    if (n <= 4096) return 4096;
-    size_t p = 1;
-    while (p < n) p <<= 1;
-    const size_t step = p >> 4;
-    return (n + step - 1) / step * step;
-  }
-  cudaError_t raw_alloc(void** out, size_t sz) {
-    return host ? cudaHostAlloc(out, sz, cudaHostAllocDefault) : cudaMalloc(out, sz);
-  }
-  void raw_free(void* p) {
-    if (host) cudaFreeHost(p); else cudaFree(p);
-  }
-  void trim() {
-    for (auto& kv : free_blocks) raw_free(kv.second);
-    free_blocks.clear();
-    cached_bytes = 0;
-  }
-  cudaError_t alloc(void** out, size_t bytes) {
-    const size_t sz = bucket(bytes ? bytes : 1);
-    auto it = free_blocks.lower_bound(sz);
-    if (it != free_blocks.end() && it->first <= sz + sz / 4) {
-      *out = it->second;
-      live[*out] = it->first;
-      cached_bytes -= it->first;
-      free_blocks.erase(it);
-      ++hits;
-      return cudaSuccess;
-    }
-    ++misses;
-    cudaError_t e = raw_alloc(out, sz);
-    if (e == cudaErrorMemoryAllocation) {  // give the cache back and try once more
-      cudaGetLastError();
-      trim();
-      e = raw_alloc(out, sz);
-    }
-    if (e == cudaSuccess) live[*out] = sz;
-    return e;
-  }
-  void release(void* p) {
-    if (!p) return;
-    auto it = live.find(p);
-    if (it == live.end()) {  // not ours (never happens): hand it to the runtime
-      raw_free(p);
-      return;
-    }
-    const size_t sz = it->second;
-    live.erase(it);
-    if (cached_bytes + sz > cap_bytes) {
-      raw_free(p);
-      return;
-    }
-    free_blocks.emplace(sz, p);
-    cached_bytes += sz;
-  }
-  void destroy() {
-    trim();
-    for (auto& kv : live) raw_free(kv.first);
-    live.clear();
-  }
+// Owners of CUDA handles and of the context's plain cudaMalloc blocks: the deleter is the runtime's destroy call.
+template <auto Destroy>
+struct CudaDeleter {
+  template <class P>
+  void operator()(P p) const { Destroy(p); }
 };
+using Stream = std::unique_ptr<CUstream_st, CudaDeleter<cudaStreamDestroy>>;
+using Event = std::unique_ptr<CUevent_st, CudaDeleter<cudaEventDestroy>>;
+using GraphExec = std::unique_ptr<CUgraphExec_st, CudaDeleter<cudaGraphExecDestroy>>;
+template <class T>
+using DevPtr = std::unique_ptr<T, CudaDeleter<cudaFree>>;
+
+static cudaError_t create(Stream& s) {
+  cudaStream_t h = nullptr;
+  const cudaError_t e = cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking);
+  s.reset(h);
+  return e;
+}
+static cudaError_t create(Event& ev, unsigned flags) {
+  cudaEvent_t h = nullptr;
+  const cudaError_t e = cudaEventCreateWithFlags(&h, flags);
+  ev.reset(h);
+  return e;
+}
+// the block held before is freed first
+template <class T>
+static cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) {
+  p.reset();
+  T* h = nullptr;
+  const cudaError_t e = cudaMalloc(&h, bytes);
+  p.reset(h);
+  return e;
+}
+
+// The raw allocations behind the context's pools.  An exhausted device or host returns cudaErrorMemoryAllocation,
+// which CU reports as LGMI_ERR_NOMEM; the runtime also keeps it as the thread's last error, cleared here so that a
+// later cudaGetLastError() check does not report it again.
+static int no_sticky_oom(cudaError_t e) {
+  if (e == cudaErrorMemoryAllocation) cudaGetLastError();
+  return e;
+}
+static const RawAllocator kDeviceBlocks{[](void** out, size_t n) { return no_sticky_oom(cudaMalloc(out, n)); },
+                                        [](void* p) { cudaFree(p); }, cudaErrorMemoryAllocation};
+static const RawAllocator kPinnedBlocks{
+    [](void** out, size_t n) { return no_sticky_oom(cudaHostAlloc(out, n, cudaHostAllocDefault)); },
+    [](void* p) { cudaFreeHost(p); }, cudaErrorMemoryAllocation};
 
 struct lgmi_ctx {
+  ~lgmi_ctx();
   int device = 0;
-  cudaStream_t own_stream = nullptr;
+  Stream own_stream;  // (declared first: destroyed after everything below)
   cudaStream_t stream = nullptr;
   std::string err;
   uint64_t launches = 0;
   // ln table
-  lg_dd* d_lntab = nullptr;
+  DevPtr<lg_dd> d_lntab;
   uint64_t ln_cap = 0;  // entries 0..ln_cap-1 valid
   // one-shot submit state
   lgmi_batch* oneshot = nullptr;
   // scratch for ecdf / csr
-  void* d_scratch = nullptr;
+  DevPtr<char> d_scratch;
   size_t scratch_cap = 0;
-  uint16_t* d_ij_tab = nullptr;  // triangular pair tables for S <= 64 (lg_ij_tab_off)
+  DevPtr<uint16_t> d_ij_tab;  // triangular pair tables for S <= 64 (lg_ij_tab_off)
   // persistent launch shape of k_pairs
   int num_sms = 0;
   int pairs_ctas_per_sm = 0;
@@ -131,94 +105,85 @@ struct lgmi_ctx {
   // tensor-core path: units at least this large build their tables with k_gram_i8
   uint32_t dense_min_sites = 48, dense_min_reads = 8192;
   void* encode_tiled = nullptr;  // cuTensorMapEncodeTiled, resolved through the runtime (no libcuda link)
-  MemPool dev_pool, host_pool;   // recycled buffers of batches / pipelines
+  MemPool dev_pool{kDeviceBlocks}, host_pool{kPinnedBlocks};  // recycled buffers of batches / pipelines
   uint64_t lntab_gen = 0;        // bumped when the ln table moves: captured graphs hold its address
   int pipeline_graphs = 1;       // groups of a pipelined step replay their launch chain as a CUDA graph (LGMI_GRAPHS=0: off)
 };
 
-template <class T>
-static cudaError_t pool_malloc(lgmi_ctx* ctx, T** out, size_t bytes) {
-  return ctx->dev_pool.alloc(reinterpret_cast<void**>(out), bytes);
-}
-template <class T>
-static cudaError_t pool_host_alloc(lgmi_ctx* ctx, T** out, size_t bytes) {
-  return ctx->host_pool.alloc(reinterpret_cast<void**>(out), bytes);
-}
-
 struct lgmi_batch {
-  lgmi_ctx* ctx = nullptr;
-  cudaStream_t own_stream = nullptr;  // pipeline chunks run on their own stream; otherwise the context's
+  explicit lgmi_batch(lgmi_ctx* c) : ctx(c) {}
+  ~lgmi_batch();
+  lgmi_ctx* const ctx;
+  Stream own_stream;                  // pipeline chunks run on their own stream; otherwise the context's
   uint32_t unit_base = 0;             // added to the unit field of every record (pipeline chunks)
-  cudaEvent_t ev[8] = {};             // 0-1 whole run, 2-3 k_pairs_fast, 4-5 tensor-core path, 6-7 last k_gram_i8
+  Event ev[8];                        // 0-1 whole run, 2-3 k_pairs_fast, 4-5 tensor-core path, 6-7 last k_gram_i8
   uint32_t n_units = 0, n_items = 0, n_mean_items = 0, n_fast = 0;
   uint64_t plane_words = 0, n_sites = 0, n_candidates = 0, n_dense = 0;
   uint32_t max_reads = 0;
   std::vector<lgmi_unit_desc> h_units;
   // device
-  DevUnit* d_units = nullptr;
-  Item* d_items = nullptr;
-  FastItem* d_fast_items = nullptr;
-  uint8_t* d_fast_empty = nullptr;           // per fast item: the pre-pass counted no emitted pair
-  uint8_t* d_item_dense = nullptr;
-  uint32_t* d_n_generic = nullptr;
-  MeanItem* d_mean_items = nullptr;     // 32-site blocks of the multi-item units
-  uint32_t* d_planes = nullptr;
-  uint8_t* d_flags = nullptr;
-  unsigned long long* d_item_cnt = nullptr;  // n_items + 1 (last stays 0)
-  unsigned long long* d_item_off = nullptr;  // n_items + 1
-  void* d_scan_tmp = nullptr;
+  PoolBuf<DevUnit> d_units;
+  PoolBuf<Item> d_items;
+  PoolBuf<FastItem> d_fast_items;
+  PoolBuf<uint8_t> d_fast_empty;           // per fast item: the pre-pass counted no emitted pair
+  PoolBuf<uint8_t> d_item_dense;
+  PoolBuf<uint32_t> d_n_generic;
+  PoolBuf<MeanItem> d_mean_items;     // 32-site blocks of the multi-item units
+  PoolBuf<uint32_t> d_planes;
+  PoolBuf<uint8_t> d_flags;
+  PoolBuf<unsigned long long> d_item_cnt;  // n_items + 1 (last stays 0)
+  PoolBuf<unsigned long long> d_item_off;  // n_items + 1
+  PoolBuf<char> d_scan_tmp;
   size_t scan_tmp_bytes = 0;
-  Header* d_header = nullptr;
-  lgmi_pair_rec* d_records = nullptr;
+  PoolBuf<Header> d_header;
+  PoolBuf<lgmi_pair_rec> d_records;
   uint64_t rec_cap = 0;
-  uint32_t* d_counts = nullptr;
-  uint64_t counts_cap = 0;
-  double* d_site_mean = nullptr;
-  uint32_t* d_site_cnt = nullptr;
-  double* d_dense = nullptr;
-  unsigned long long* d_unit_rec_off = nullptr;
+  PoolBuf<uint32_t> d_counts;  // EMIT_COUNTS only, 9 per record slot, allocated on first use
+  PoolBuf<double> d_site_mean;
+  PoolBuf<uint32_t> d_site_cnt;
+  PoolBuf<double> d_dense;
+  PoolBuf<unsigned long long> d_unit_rec_off;
   // tensor-core path
   std::vector<DensePlan> dense_plans;
   std::vector<CUtensorMap> tmaps;  // per deep unit, parallel to dense_plans: its X for k_gram_i8's TMA loads
-  uint8_t* d_x = nullptr;       // indicator matrix of the unit being contracted (reused unit after unit)
-  uint32_t* d_gram = nullptr;   // nine count matrices per dense unit
-  uint32_t* d_xt = nullptr;     // four-block form: transposed label planes of the unit being contracted
-  uint32_t* d_oth_cnt = nullptr, *d_oth_list = nullptr;  // ... and its listed "other" reads per site
-  uint32_t* d_unit_mode = nullptr;  // per unit: the form of this run (0 four blocks, else nine)
+  PoolBuf<uint8_t> d_x;       // indicator matrix of the unit being contracted (reused unit after unit)
+  PoolBuf<uint32_t> d_gram;   // nine count matrices per dense unit
+  PoolBuf<uint32_t> d_xt;     // four-block form: transposed label planes of the unit being contracted
+  PoolBuf<uint32_t> d_oth_cnt, d_oth_list;  // ... and its listed "other" reads per site
+  PoolBuf<uint32_t> d_unit_mode;  // per unit: the form of this run (0 four blocks, else nine)
   // graph replays / pipeline groups: the small units' kernels (k_count_fast before the scan, k_pairs_fast after it) run on
   // a second stream beside the kernels of the larger units (forked and joined by events inside the captured chain)
-  cudaStream_t side_stream = nullptr;
-  cudaEvent_t side_ev[4] = {};
-  cudaStream_t fix_stream = nullptr;             // k_other_fix runs beside k_dense_x (forked after k_dense_prep,
-  cudaEvent_t fix_fork = nullptr, fix_join = nullptr;  // joined before the tables are read)
-  DenseTile* d_tiles = nullptr;
+  Stream side_stream;
+  Event side_ev[4];
+  Stream fix_stream;           // k_other_fix runs beside k_dense_x (forked after k_dense_prep,
+  Event fix_fork, fix_join;    // joined before the tables are read)
+  PoolBuf<DenseTile> d_tiles;
   uint64_t dense_macs = 0;      // multiply-accumulates the tile lists amount to
   // tiled popcount path
-  TileItem* d_tile_items = nullptr;
+  PoolBuf<TileItem> d_tile_items;
   uint32_t n_tile_items = 0;
-  TgTile* d_gram_tiles = nullptr;      // k_tile_gram_ws's work items (128 x 48 site blocks)
+  PoolBuf<TgTile> d_gram_tiles;      // k_tile_gram_ws's work items (128 x 48 site blocks)
   uint32_t n_gram_tiles = 0;
-  uint2* d_tile_cnt = nullptr;         // its output: 24 bytes of counts per pair slot
+  PoolBuf<uint2> d_tile_cnt;         // its output: 24 bytes of counts per pair slot
   uint32_t n_tiled_work_items = 0;     // work items (Item) of the tiled and of the deep units: k_pairs_generic<1>'s and <2>'s
-  TiledDesc* d_tiled_desc = nullptr;   // k_pairs_generic<1>'s items, one self-contained record each
+  PoolBuf<TiledDesc> d_tiled_desc;   // k_pairs_generic<1>'s items, one self-contained record each
   uint32_t n_tiled_desc = 0;
-  uint32_t* d_tile_counts = nullptr;  // EMIT_COUNTS only, allocated on first use
+  PoolBuf<uint32_t> d_tile_counts;  // EMIT_COUNTS only, allocated on first use
   // host (pinned) mirrors
-  Header* h_header = nullptr;
-  lgmi_pair_rec* h_records = nullptr;
-  uint64_t h_rec_cap = 0;
-  uint32_t* h_counts = nullptr;
-  uint64_t h_counts_cap = 0;
-  double* h_site_mean = nullptr;
-  uint32_t* h_site_cnt = nullptr;
-  unsigned long long* h_unit_rec_off = nullptr;
-  // launch chains captured as CUDA graphs, one per (min_common, mode)
+  PoolBuf<Header> h_header;
+  PoolBuf<lgmi_pair_rec> h_records;
+  PoolBuf<uint32_t> h_counts;
+  PoolBuf<double> h_site_mean;
+  PoolBuf<uint32_t> h_site_cnt;
+  PoolBuf<unsigned long long> h_unit_rec_off;
+  // launch chains captured as CUDA graphs, one per (min_common, mode).  A graph holds the addresses it was captured
+  // with: declared after the buffers, so destroyed before them.
   struct Graph {
     int min_common;
     uint32_t mode;
     uint64_t lntab_gen;
     uint64_t launches;  // kernels in the chain
-    cudaGraphExec_t exec;
+    GraphExec exec;
   };
   std::vector<Graph> graphs;
   // run state
@@ -230,11 +195,11 @@ struct lgmi_batch {
   // lgmi_batch_create_rows: per unit its row limit (0: an ordinary unit) and first dense slot; empty otherwise
   std::vector<uint32_t> h_row_limit;
   std::vector<uint64_t> h_dense_off;
-  cudaEvent_t copy_ev = nullptr;  // lgmi_batch_copy_planes from this batch: what its stream has queued so far
+  Event copy_ev;  // lgmi_batch_copy_planes from this batch: what its stream has queued so far
 };
 
 // --------------------------------------------------------------------------- helpers
-static inline cudaStream_t bstream(const lgmi_batch* b) { return b->own_stream ? b->own_stream : b->ctx->stream; }
+static inline cudaStream_t bstream(const lgmi_batch* b) { return b->own_stream ? b->own_stream.get() : b->ctx->stream; }
 
 static int fail(lgmi_ctx* ctx, int code, const char* fmt, ...) {
   char buf[512];
@@ -248,7 +213,7 @@ static int fail(lgmi_ctx* ctx, int code, const char* fmt, ...) {
 
 #define CU(ctx, call)                                                                      \
   do {                                                                                     \
-    cudaError_t e__ = (call);                                                              \
+    const cudaError_t e__ = static_cast<cudaError_t>(call);                                \
     if (e__ != cudaSuccess)                                                                \
       return fail((ctx), (e__ == cudaErrorMemoryAllocation) ? LGMI_ERR_NOMEM : LGMI_ERR_CUDA, \
                   "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e__), __FILE__, __LINE__); \
@@ -261,11 +226,9 @@ static int ensure_lntab(lgmi_ctx* ctx, uint64_t k_max) {
   std::vector<double> host(2 * cap);
   lgmi_build_lntab(host.data(), 0, cap);
   CU(ctx, cudaStreamSynchronize(ctx->stream));
-  if (ctx->d_lntab) CU(ctx, cudaFree(ctx->d_lntab));
-  ctx->d_lntab = nullptr;
   ctx->ln_cap = 0;
-  CU(ctx, cudaMalloc(&ctx->d_lntab, cap * sizeof(lg_dd)));
-  CU(ctx, cudaMemcpy(ctx->d_lntab, host.data(), cap * sizeof(lg_dd), cudaMemcpyHostToDevice));
+  CU(ctx, dev_alloc(ctx->d_lntab, cap * sizeof(lg_dd)));
+  CU(ctx, cudaMemcpy(ctx->d_lntab.get(), host.data(), cap * sizeof(lg_dd), cudaMemcpyHostToDevice));
   ctx->ln_cap = cap;
   ++ctx->lntab_gen;
   return LGMI_OK;
@@ -274,11 +237,9 @@ static int ensure_lntab(lgmi_ctx* ctx, uint64_t k_max) {
 static int ensure_scratch(lgmi_ctx* ctx, size_t bytes) {
   if (bytes <= ctx->scratch_cap) return LGMI_OK;
   CU(ctx, cudaStreamSynchronize(ctx->stream));
-  if (ctx->d_scratch) CU(ctx, cudaFree(ctx->d_scratch));
-  ctx->d_scratch = nullptr;
   ctx->scratch_cap = 0;
   size_t cap = std::max<size_t>(bytes, 1 << 20);
-  CU(ctx, cudaMalloc(&ctx->d_scratch, cap));
+  CU(ctx, dev_alloc(ctx->d_scratch, cap));
   ctx->scratch_cap = cap;
   return LGMI_OK;
 }
@@ -302,18 +263,14 @@ extern "C" int lgmi_create(int device, lgmi_t** out) {
     return fail(nullptr, LGMI_ERR_NODEVICE,
                 "lgmi_create: device %d is sm_%d%d; this build contains sm_100a code only", device,
                 prop.major, prop.minor);
-  lgmi_ctx* ctx = new (std::nothrow) lgmi_ctx();
+  // every failure from here on releases what the context holds so far
+  std::unique_ptr<lgmi_ctx> ctx(new (std::nothrow) lgmi_ctx());
   if (!ctx) return fail(nullptr, LGMI_ERR_NOMEM, "lgmi_create: out of host memory");
   ctx->device = device;
-  if (cudaSetDevice(device) != cudaSuccess ||
-      cudaStreamCreateWithFlags(&ctx->own_stream, cudaStreamNonBlocking) != cudaSuccess) {
-    int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: %s", cudaGetErrorString(cudaGetLastError()));
-    delete ctx;
-    return rc;
-  }
-  ctx->stream = ctx->own_stream;
+  if (cudaSetDevice(device) != cudaSuccess || create(ctx->own_stream) != cudaSuccess)
+    return fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: %s", cudaGetErrorString(cudaGetLastError()));
+  ctx->stream = ctx->own_stream.get();
   ctx->num_sms = prop.multiProcessorCount;
-  ctx->host_pool.host = true;
   ctx->dev_pool.cap_bytes = 16ull << 30;   // cached (idle) bytes kept at most; LGMI_POOL_MB overrides both
   ctx->host_pool.cap_bytes = 4ull << 30;
   if (const char* e = getenv("LGMI_POOL_MB")) ctx->dev_pool.cap_bytes = ctx->host_pool.cap_bytes = (size_t)atoll(e) << 20;
@@ -323,32 +280,23 @@ extern "C" int lgmi_create(int device, lgmi_t** out) {
           cudaSuccess ||
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->pairs_ctas_per_sm, k_pairs_fast, kFastThreads,
                                                     sizeof(FastSmem)) != cudaSuccess ||
-      ctx->pairs_ctas_per_sm < 1) {
-    int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: k_pairs_fast cannot be resident (%s)",
-                  cudaGetErrorString(cudaGetLastError()));
-    lgmi_destroy(ctx);
-    return rc;
-  }
+      ctx->pairs_ctas_per_sm < 1)
+    return fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: k_pairs_fast cannot be resident (%s)",
+                cudaGetErrorString(cudaGetLastError()));
   if (const char* e = getenv("LGMI_DENSE_PATH")) ctx->dense_path = atoi(e) == 9 ? 9 : 4;
   if (const char* e = getenv("LGMI_TILE_PATH")) ctx->tile_path = atoi(e) ? 1 : 0;
   if (const char* e = getenv("LGMI_GRAPHS")) ctx->pipeline_graphs = atoi(e) ? 1 : 0;
-  if (cudaFuncSetAttribute(k_tile_gram_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTwSmemBytes) != cudaSuccess) {
-    int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: k_tile_gram_ws cannot be resident (%s)",
-                  cudaGetErrorString(cudaGetLastError()));
-    lgmi_destroy(ctx);
-    return rc;
-  }
+  if (cudaFuncSetAttribute(k_tile_gram_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTwSmemBytes) != cudaSuccess)
+    return fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: k_tile_gram_ws cannot be resident (%s)",
+                cudaGetErrorString(cudaGetLastError()));
   {
     cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ctx->encode_tiled, cudaEnableDefault, &q) != cudaSuccess ||
         q != cudaDriverEntryPointSuccess || !ctx->encode_tiled ||
         cudaFuncSetAttribute(k_gram_i8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDenseSmemBytes) !=
-            cudaSuccess) {
-      int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: tensor-core path unavailable (%s)",
-                    cudaGetErrorString(cudaGetLastError()));
-      lgmi_destroy(ctx);
-      return rc;
-    }
+            cudaSuccess)
+      return fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: tensor-core path unavailable (%s)",
+                  cudaGetErrorString(cudaGetLastError()));
   }
   {
     std::vector<uint16_t> tab(kIjTabEntries);
@@ -357,31 +305,24 @@ extern "C" int lgmi_create(int device, lgmi_t** out) {
       for (uint32_t i = 0; i + 1 < S; ++i)
         for (uint32_t j = i + 1; j < S; ++j) tab[p++] = (uint16_t)(i * 64u + j);
     }
-    if (cudaMalloc(&ctx->d_ij_tab, tab.size() * sizeof(uint16_t)) != cudaSuccess ||
-        cudaMemcpy(ctx->d_ij_tab, tab.data(), tab.size() * sizeof(uint16_t), cudaMemcpyHostToDevice) != cudaSuccess) {
-      int rc = fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: pair table upload failed (%s)",
-                    cudaGetErrorString(cudaGetLastError()));
-      lgmi_destroy(ctx);
-      return rc;
-    }
+    if (dev_alloc(ctx->d_ij_tab, tab.size() * sizeof(uint16_t)) != cudaSuccess ||
+        cudaMemcpy(ctx->d_ij_tab.get(), tab.data(), tab.size() * sizeof(uint16_t), cudaMemcpyHostToDevice) != cudaSuccess)
+      return fail(nullptr, LGMI_ERR_CUDA, "lgmi_create: pair table upload failed (%s)",
+                  cudaGetErrorString(cudaGetLastError()));
   }
-  *out = ctx;
+  *out = ctx.release();
   return LGMI_OK;
 }
 
-extern "C" void lgmi_destroy(lgmi_t* ctx) {
-  if (!ctx) return;
-  cudaSetDevice(ctx->device);
-  if (ctx->oneshot) lgmi_batch_destroy(ctx->oneshot);
-  cudaStreamSynchronize(ctx->stream);
-  if (ctx->d_lntab) cudaFree(ctx->d_lntab);
-  if (ctx->d_scratch) cudaFree(ctx->d_scratch);
-  if (ctx->d_ij_tab) cudaFree(ctx->d_ij_tab);
-  ctx->dev_pool.destroy();
-  ctx->host_pool.destroy();
-  if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
-  delete ctx;
+// Runtime calls act on the current device, and DevicePool threads hold contexts on different GPUs: every destructor
+// that releases device resources selects its context's device first.
+lgmi_ctx::~lgmi_ctx() {
+  cudaSetDevice(device);
+  delete oneshot;  // its blocks go back to the pools below
+  if (stream) cudaStreamSynchronize(stream);
 }
+
+extern "C" void lgmi_destroy(lgmi_t* ctx) { delete ctx; }
 
 extern "C" const char* lgmi_last_error(const lgmi_t* ctx) {
   return ctx ? ctx->err.c_str() : g_create_error.c_str();
@@ -391,7 +332,7 @@ extern "C" int lgmi_set_stream(lgmi_t* ctx, void* cuda_stream) {
   if (!ctx) return LGMI_ERR_ARG;
   CU(ctx, cudaSetDevice(ctx->device));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
-  ctx->stream = cuda_stream ? reinterpret_cast<cudaStream_t>(cuda_stream) : ctx->own_stream;
+  ctx->stream = cuda_stream ? reinterpret_cast<cudaStream_t>(cuda_stream) : ctx->own_stream.get();
   return LGMI_OK;
 }
 
@@ -432,61 +373,14 @@ extern "C" int lgmi_set_dense_threshold(lgmi_t* ctx, uint32_t min_sites, uint32_
 }
 
 // --------------------------------------------------------------------------- batch
+lgmi_batch::~lgmi_batch() {
+  cudaSetDevice(ctx->device);
+  cudaStreamSynchronize(bstream(this));  // nothing in flight touches a block when it goes back to the cache
+}
+
 extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
   if (!b) return;
-  lgmi_ctx* ctx = b->ctx;  // (always set: a batch is born with its context)
-  if (b->ctx) {
-    cudaSetDevice(b->ctx->device);
-    cudaStreamSynchronize(bstream(b));
-    if (b->ctx->oneshot == b) b->ctx->oneshot = nullptr;
-  }
-  for (cudaEvent_t e : b->ev)
-    if (e) cudaEventDestroy(e);
-  for (lgmi_batch::Graph& g : b->graphs) cudaGraphExecDestroy(g.exec);
-  ctx->dev_pool.release(b->d_units);
-  ctx->dev_pool.release(b->d_items);
-  ctx->dev_pool.release(b->d_fast_items);
-  ctx->dev_pool.release(b->d_fast_empty);
-  ctx->dev_pool.release(b->d_item_dense);
-  ctx->dev_pool.release(b->d_n_generic);
-  ctx->dev_pool.release(b->d_mean_items);
-  ctx->dev_pool.release(b->d_planes);
-  ctx->dev_pool.release(b->d_flags);
-  ctx->dev_pool.release(b->d_item_cnt);
-  ctx->dev_pool.release(b->d_item_off);
-  ctx->dev_pool.release(b->d_scan_tmp);
-  ctx->dev_pool.release(b->d_header);
-  ctx->dev_pool.release(b->d_records);
-  ctx->dev_pool.release(b->d_counts);
-  ctx->dev_pool.release(b->d_site_mean);
-  ctx->dev_pool.release(b->d_site_cnt);
-  ctx->dev_pool.release(b->d_dense);
-  ctx->dev_pool.release(b->d_unit_rec_off);
-  ctx->dev_pool.release(b->d_x);
-  ctx->dev_pool.release(b->d_gram);
-  ctx->dev_pool.release(b->d_xt);
-  ctx->dev_pool.release(b->d_oth_cnt);
-  ctx->dev_pool.release(b->d_oth_list);
-  ctx->dev_pool.release(b->d_unit_mode);
-  if (b->copy_ev) cudaEventDestroy(b->copy_ev);
-  if (b->side_stream) cudaStreamDestroy(b->side_stream);
-  for (cudaEvent_t e : b->side_ev)
-    if (e) cudaEventDestroy(e);
-  if (b->fix_stream) cudaStreamDestroy(b->fix_stream);
-  if (b->fix_fork) cudaEventDestroy(b->fix_fork);
-  if (b->fix_join) cudaEventDestroy(b->fix_join);
-  ctx->dev_pool.release(b->d_tiles);
-  ctx->dev_pool.release(b->d_tile_items);
-  ctx->dev_pool.release(b->d_gram_tiles);
-  ctx->dev_pool.release(b->d_tiled_desc);
-  ctx->dev_pool.release(b->d_tile_cnt);
-  ctx->dev_pool.release(b->d_tile_counts);
-  ctx->host_pool.release(b->h_header);
-  ctx->host_pool.release(b->h_records);
-  ctx->host_pool.release(b->h_counts);
-  ctx->host_pool.release(b->h_site_mean);
-  ctx->host_pool.release(b->h_site_cnt);
-  ctx->host_pool.release(b->h_unit_rec_off);
+  if (b->ctx->oneshot == b) b->ctx->oneshot = nullptr;
   delete b;
 }
 
@@ -505,9 +399,8 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
     return fail(ctx, rc, "%s", err.c_str());
 
   // every failure from here on releases what the batch holds so far
-  std::unique_ptr<lgmi_batch, void (*)(lgmi_batch*)> b(new (std::nothrow) lgmi_batch(), lgmi_batch_destroy);
+  std::unique_ptr<lgmi_batch> b(new (std::nothrow) lgmi_batch(ctx));
   if (!b) return fail(ctx, LGMI_ERR_NOMEM, "lgmi_batch_create: out of host memory");
-  b->ctx = ctx;
   b->n_units = n_units;
   b->plane_words = plane_words;
   b->n_sites = n_sites;
@@ -530,57 +423,58 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
   b->dense_plans = std::move(plan.dense_plans);
   const cudaStream_t st = bstream(b.get());
   // a table of the plan on the device: at least min_n entries, the plan's uploaded
-  auto upload = [&](auto** dst, const auto& v, size_t min_n) {
-    const size_t sz = sizeof(v[0]);
-    cudaError_t e = pool_malloc(ctx, dst, std::max(min_n, v.size()) * sz);
-    if (e == cudaSuccess && !v.empty()) e = cudaMemcpyAsync(*dst, v.data(), v.size() * sz, cudaMemcpyHostToDevice, st);
+  auto upload = [&](auto& dst, const auto& v, size_t min_n) {
+    auto e = static_cast<cudaError_t>(dst.alloc(ctx->dev_pool, std::max(min_n, v.size())));
+    if (e == cudaSuccess && !v.empty())
+      e = cudaMemcpyAsync(dst, v.data(), v.size() * sizeof(v[0]), cudaMemcpyHostToDevice, st);
     return e;
   };
 
-  for (cudaEvent_t& e : b->ev) CU(ctx, cudaEventCreate(&e));
+  for (Event& e : b->ev) CU(ctx, create(e, cudaEventDefault));
   if (b->n_fast && (!b->dense_plans.empty() || b->n_tile_items || b->n_gram_tiles)) {
-    CU(ctx, cudaStreamCreateWithFlags(&b->side_stream, cudaStreamNonBlocking));
-    for (cudaEvent_t& e : b->side_ev) CU(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    CU(ctx, create(b->side_stream));
+    for (Event& e : b->side_ev) CU(ctx, create(e, cudaEventDisableTiming));
   }
-  CU(ctx, upload(&b->d_units, plan.units, 1));
-  CU(ctx, upload(&b->d_items, plan.items, 1));
-  CU(ctx, upload(&b->d_fast_items, plan.fast_items, 1));
-  CU(ctx, pool_malloc(ctx, &b->d_fast_empty, std::max<size_t>(1, b->n_fast)));
-  CU(ctx, pool_malloc(ctx, &b->d_item_dense, std::max<size_t>(1, b->n_items)));
-  CU(ctx, pool_malloc(ctx, &b->d_n_generic, sizeof(uint32_t)));
-  CU(ctx, upload(&b->d_mean_items, plan.mean_items, 1));
-  CU(ctx, pool_malloc(ctx, &b->d_planes, std::max<uint64_t>(4, plane_words) * sizeof(uint32_t)));
-  CU(ctx, pool_malloc(ctx, &b->d_flags, std::max<uint64_t>(1, n_sites)));
-  CU(ctx, pool_malloc(ctx, &b->d_item_cnt, ((size_t)b->n_items + 1) * sizeof(unsigned long long)));
-  CU(ctx, pool_malloc(ctx, &b->d_item_off, ((size_t)b->n_items + 1) * sizeof(unsigned long long)));
-  CU(ctx, cub::DeviceScan::ExclusiveSum(nullptr, b->scan_tmp_bytes, b->d_item_cnt, b->d_item_off, (int)b->n_items + 1, st));
-  CU(ctx, pool_malloc(ctx, &b->d_scan_tmp, std::max<size_t>(b->scan_tmp_bytes, 16)));
+  CU(ctx, upload(b->d_units, plan.units, 1));
+  CU(ctx, upload(b->d_items, plan.items, 1));
+  CU(ctx, upload(b->d_fast_items, plan.fast_items, 1));
+  CU(ctx, b->d_fast_empty.alloc(ctx->dev_pool, std::max<size_t>(1, b->n_fast)));
+  CU(ctx, b->d_item_dense.alloc(ctx->dev_pool, std::max<size_t>(1, b->n_items)));
+  CU(ctx, b->d_n_generic.alloc(ctx->dev_pool, 1));
+  CU(ctx, upload(b->d_mean_items, plan.mean_items, 1));
+  CU(ctx, b->d_planes.alloc(ctx->dev_pool, std::max<uint64_t>(4, plane_words)));
+  CU(ctx, b->d_flags.alloc(ctx->dev_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, b->d_item_cnt.alloc(ctx->dev_pool, (size_t)b->n_items + 1));
+  CU(ctx, b->d_item_off.alloc(ctx->dev_pool, (size_t)b->n_items + 1));
+  CU(ctx, cub::DeviceScan::ExclusiveSum(nullptr, b->scan_tmp_bytes, b->d_item_cnt.get(), b->d_item_off.get(),
+                                        (int)b->n_items + 1, st));
+  CU(ctx, b->d_scan_tmp.alloc(ctx->dev_pool, std::max<size_t>(b->scan_tmp_bytes, 16)));
   CU(ctx, cudaMemsetAsync(b->d_item_cnt, 0, ((size_t)b->n_items + 1) * sizeof(unsigned long long), st));
-  CU(ctx, pool_malloc(ctx, &b->d_header, sizeof(Header)));
-  CU(ctx, pool_malloc(ctx, &b->d_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
-  CU(ctx, pool_malloc(ctx, &b->d_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
-  CU(ctx, pool_malloc(ctx, &b->d_dense, std::max<uint64_t>(1, plan.n_dense) * sizeof(double)));
-  CU(ctx, pool_malloc(ctx, &b->d_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
-  if (b->n_tile_items) CU(ctx, upload(&b->d_tile_items, plan.tile_items, 0));
+  CU(ctx, b->d_header.alloc(ctx->dev_pool, 1));
+  CU(ctx, b->d_site_mean.alloc(ctx->dev_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, b->d_site_cnt.alloc(ctx->dev_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, b->d_dense.alloc(ctx->dev_pool, std::max<uint64_t>(1, plan.n_dense)));
+  CU(ctx, b->d_unit_rec_off.alloc(ctx->dev_pool, (size_t)n_units + 1));
+  if (b->n_tile_items) CU(ctx, upload(b->d_tile_items, plan.tile_items, 0));
   if (b->n_gram_tiles) {
-    CU(ctx, upload(&b->d_gram_tiles, plan.gram_tiles, 0));
-    CU(ctx, pool_malloc(ctx, &b->d_tile_cnt, std::max<uint64_t>(1, plan.n_dense) * 3ull * sizeof(uint2)));
+    CU(ctx, upload(b->d_gram_tiles, plan.gram_tiles, 0));
+    CU(ctx, b->d_tile_cnt.alloc(ctx->dev_pool, std::max<uint64_t>(1, plan.n_dense) * 3ull));
   }
-  if (b->n_tiled_desc) CU(ctx, upload(&b->d_tiled_desc, plan.tiled_desc, 0));
+  if (b->n_tiled_desc) CU(ctx, upload(b->d_tiled_desc, plan.tiled_desc, 0));
   if (!b->dense_plans.empty()) {
-    CU(ctx, pool_malloc(ctx, &b->d_x, plan.x_bytes));
+    CU(ctx, b->d_x.alloc(ctx->dev_pool, plan.x_bytes));
     CU(ctx, cudaMemsetAsync(b->d_x, 0, plan.x_bytes, st));  // rows of the site padding stay zero
-    CU(ctx, pool_malloc(ctx, &b->d_gram, plan.gram_words * sizeof(uint32_t)));
-    CU(ctx, pool_malloc(ctx, &b->d_unit_mode, (size_t)n_units * sizeof(uint32_t)));
+    CU(ctx, b->d_gram.alloc(ctx->dev_pool, plan.gram_words));
+    CU(ctx, b->d_unit_mode.alloc(ctx->dev_pool, n_units));
     if (plan.xt_words) {
-      CU(ctx, pool_malloc(ctx, &b->d_xt, plan.xt_words * sizeof(uint32_t)));
-      CU(ctx, pool_malloc(ctx, &b->d_oth_list, plan.oth_words * sizeof(uint32_t)));
-      CU(ctx, pool_malloc(ctx, &b->d_oth_cnt, (size_t)plan.oth_sites * sizeof(uint32_t)));
-      CU(ctx, cudaStreamCreateWithFlags(&b->fix_stream, cudaStreamNonBlocking));
-      CU(ctx, cudaEventCreateWithFlags(&b->fix_fork, cudaEventDisableTiming));
-      CU(ctx, cudaEventCreateWithFlags(&b->fix_join, cudaEventDisableTiming));
+      CU(ctx, b->d_xt.alloc(ctx->dev_pool, plan.xt_words));
+      CU(ctx, b->d_oth_list.alloc(ctx->dev_pool, plan.oth_words));
+      CU(ctx, b->d_oth_cnt.alloc(ctx->dev_pool, plan.oth_sites));
+      CU(ctx, create(b->fix_stream));
+      CU(ctx, create(b->fix_fork, cudaEventDisableTiming));
+      CU(ctx, create(b->fix_join, cudaEventDisableTiming));
     }
-    CU(ctx, upload(&b->d_tiles, plan.dense_tiles, 0));
+    CU(ctx, upload(b->d_tiles, plan.dense_tiles, 0));
     typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -600,11 +494,11 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
     }
   }
   b->rec_cap = std::max<uint64_t>(1, b->n_candidates);
-  CU(ctx, pool_malloc(ctx, &b->d_records, b->rec_cap * sizeof(lgmi_pair_rec)));
-  CU(ctx, pool_host_alloc(ctx, &b->h_header, sizeof(Header)));
-  CU(ctx, pool_host_alloc(ctx, &b->h_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
-  CU(ctx, pool_host_alloc(ctx, &b->h_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
-  CU(ctx, pool_host_alloc(ctx, &b->h_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
+  CU(ctx, b->d_records.alloc(ctx->dev_pool, b->rec_cap));
+  CU(ctx, b->h_header.alloc(ctx->host_pool, 1));
+  CU(ctx, b->h_site_mean.alloc(ctx->host_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, b->h_site_cnt.alloc(ctx->host_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, b->h_unit_rec_off.alloc(ctx->host_pool, (size_t)n_units + 1));
   CU(ctx, cudaStreamSynchronize(st));  // the plan's tables go out of scope
   if (const int rc = ensure_lntab(ctx, std::max<uint32_t>(b->max_reads, 1u))) return rc;
   *out = b.release();
@@ -674,8 +568,8 @@ extern "C" int lgmi_batch_copy_planes(lgmi_batch_t* dst, uint64_t dst_word, cons
   const int sdev = s->ctx->device, ddev = ctx->device;
   // the copy follows everything src's stream has queued so far (its upload)
   CU(ctx, cudaSetDevice(sdev));
-  if (!s->copy_ev) CU(ctx, cudaEventCreateWithFlags(&s->copy_ev, cudaEventDisableTiming));
-  CU(ctx, cudaEventRecord(s->copy_ev, bstream(s)));
+  if (!s->copy_ev) CU(ctx, create(s->copy_ev, cudaEventDisableTiming));
+  CU(ctx, cudaEventRecord(s->copy_ev.get(), bstream(s)));
   CU(ctx, cudaSetDevice(ddev));
   if (sdev != ddev) {
     // direct peer copies where the devices allow them; without peer access the runtime stages through the host
@@ -684,16 +578,11 @@ extern "C" int lgmi_batch_copy_planes(lgmi_batch_t* dst, uint64_t dst_word, cons
         cudaDeviceEnablePeerAccess(sdev, 0) != cudaSuccess)
       cudaGetLastError();  // (cudaErrorPeerAccessAlreadyEnabled, or no peer access: the copy works either way)
   }
-  CU(ctx, cudaStreamWaitEvent(bstream(dst), s->copy_ev, 0));
+  CU(ctx, cudaStreamWaitEvent(bstream(dst), s->copy_ev.get(), 0));
   CU(ctx, cudaMemcpyPeerAsync(dst->d_planes + dst_word, ddev, s->d_planes + src_word, sdev, n_words * sizeof(uint32_t),
                               bstream(dst)));
   dst->uploaded = true;
   return LGMI_OK;
-}
-
-static void drop_graphs(lgmi_batch* b) {
-  for (lgmi_batch::Graph& g : b->graphs) cudaGraphExecDestroy(g.exec);
-  b->graphs.clear();
 }
 
 static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing);
@@ -709,26 +598,22 @@ extern "C" int lgmi_batch_run(lgmi_batch_t* b, int min_common, uint32_t mode) {
   const bool as_graph = (mode & LGMI_MODE_GRAPH) != 0u || (b->own_stream != nullptr && ctx->pipeline_graphs);
   mode &= ~LGMI_MODE_GRAPH;
   // buffers the chain needs exist before anything is launched or captured
-  if ((mode & LGMI_MODE_EMIT_COUNTS) && b->counts_cap < b->rec_cap) {
+  if ((mode & LGMI_MODE_EMIT_COUNTS) && b->d_counts.size() < b->rec_cap * 9ull) {
     CU(ctx, cudaStreamSynchronize(bstream(b)));
-    if (b->d_counts) ctx->dev_pool.release(b->d_counts);
-    b->d_counts = nullptr;
-    b->counts_cap = 0;
-    drop_graphs(b);
-    CU(ctx, pool_malloc(ctx, &b->d_counts, b->rec_cap * 9ull * sizeof(uint32_t)));
-    b->counts_cap = b->rec_cap;
+    b->graphs.clear();  // they hold the addresses they were captured with
+    CU(ctx, b->d_counts.alloc(ctx->dev_pool, b->rec_cap * 9ull));
   }
   if ((mode & LGMI_MODE_EMIT_COUNTS) && (b->n_tile_items || b->n_gram_tiles) && !b->d_tile_counts) {
     CU(ctx, cudaStreamSynchronize(bstream(b)));
-    drop_graphs(b);
-    CU(ctx, pool_malloc(ctx, &b->d_tile_counts, std::max<uint64_t>(1, b->n_dense) * 9ull * sizeof(uint32_t)));
+    b->graphs.clear();
+    CU(ctx, b->d_tile_counts.alloc(ctx->dev_pool, std::max<uint64_t>(1, b->n_dense) * 9ull));
   }
   if (!as_graph) return run_chain(b, min_common, mode, b->own_stream == nullptr);
   lgmi_batch::Graph* hit = nullptr;
   for (lgmi_batch::Graph& g : b->graphs)
     if (g.min_common == min_common && g.mode == mode) hit = &g;
   if (hit && hit->lntab_gen != ctx->lntab_gen) {  // the ln table has moved since the capture
-    drop_graphs(b);
+    b->graphs.clear();
     hit = nullptr;
   }
   if (!hit) {
@@ -749,10 +634,10 @@ extern "C" int lgmi_batch_run(lgmi_batch_t* b, int min_common, uint32_t mode) {
     const cudaError_t ei = cudaGraphInstantiate(&exec, graph, 0);
     cudaGraphDestroy(graph);
     if (ei != cudaSuccess) return fail(ctx, LGMI_ERR_CUDA, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ei));
-    b->graphs.push_back(lgmi_batch::Graph{min_common, mode, ctx->lntab_gen, n_launch, exec});
+    b->graphs.push_back(lgmi_batch::Graph{min_common, mode, ctx->lntab_gen, n_launch, GraphExec(exec)});
     hit = &b->graphs.back();
   }
-  CU(ctx, cudaGraphLaunch(hit->exec, bstream(b)));
+  CU(ctx, cudaGraphLaunch(hit->exec.get(), bstream(b)));
   ctx->launches += hit->launches;
   b->ran = true;
   b->last_mode = mode;
@@ -772,7 +657,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
   P.n_units = b->n_units;
   P.planes = b->d_planes;
   P.site_flags = b->d_flags;
-  P.lntab = ctx->d_lntab;
+  P.lntab = ctx->d_lntab.get();
   P.ln_cap = (uint32_t)std::min<uint64_t>(ctx->ln_cap, 0xffffffffull);
   P.min_common = min_common;
   P.mode = mode;
@@ -793,25 +678,25 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
   P.tile_counts = b->d_tile_counts;
 
   // (pipeline groups and graph replays skip the per-kernel events)
-  if (timing) CU(ctx, cudaEventRecord(b->ev[0], bstream(b)));
+  if (timing) CU(ctx, cudaEventRecord(b->ev[0].get(), bstream(b)));
   {
     // one launch resets the run state: header, offsets, flags, NaN means (sites of pair-less units keep them)
     const uint64_t n = std::max<uint64_t>(std::max<uint64_t>(b->n_sites, b->n_items), (uint64_t)b->n_units + 1);
-    k_run_init<<<(unsigned)((n + 255) / 256), 256, 0, bstream(b)>>>(b->d_header, b->own_stream ? b->h_header : nullptr,
+    k_run_init<<<(unsigned)((n + 255) / 256), 256, 0, bstream(b)>>>(b->d_header, b->own_stream ? b->h_header.get() : nullptr,
                                                                   b->d_unit_rec_off, b->n_units + 1,
                                                                   b->d_item_dense, b->n_items, b->d_n_generic,
                                                                   b->n_items - b->n_fast - b->n_tiled_work_items, b->d_site_mean,
                                                                   b->d_site_cnt, b->n_sites);
     ++ctx->launches;
   }
-  if (timing) CU(ctx, cudaEventRecord(b->ev[4], bstream(b)));
+  if (timing) CU(ctx, cudaEventRecord(b->ev[4].get(), bstream(b)));
   // untimed runs (graph captures, pipeline groups) of mixed batches: the small units' kernels on the side stream
   static const bool fork_ok = !(getenv("LGMI_FORK") && atoi(getenv("LGMI_FORK")) == 0);  // LGMI_FORK=0: one stream
   const bool forked = !timing && b->side_stream != nullptr && fork_ok;
-  cudaStream_t small = forked ? b->side_stream : bstream(b);
+  cudaStream_t small = forked ? b->side_stream.get() : bstream(b);
   if (forked) {
-    CU(ctx, cudaEventRecord(b->side_ev[0], bstream(b)));
-    CU(ctx, cudaStreamWaitEvent(small, b->side_ev[0], 0));
+    CU(ctx, cudaEventRecord(b->side_ev[0].get(), bstream(b)));
+    CU(ctx, cudaStreamWaitEvent(small, b->side_ev[0].get(), 0));
   }
   if (!b->dense_plans.empty())  // every dense unit starts a run in the four-block form
     CU(ctx, cudaMemsetAsync(b->d_unit_mode, 0, (size_t)b->n_units * sizeof(uint32_t), bstream(b)));
@@ -831,12 +716,12 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       // k_dense_x mostly runs after it and the step costs what one fused pass cost; capping it at two CTAs per SM,
       // or k_dense_x first on a smaller grid, was slower -- tools/experiments/README.md.  The nine-block form no
       // longer pays for lists and transposes it does not use: 2.01 -> 1.65 ms.)
-      CU(ctx, cudaEventRecord(b->fix_fork, bstream(b)));
-      CU(ctx, cudaStreamWaitEvent(b->fix_stream, b->fix_fork, 0));
-      k_other_fix<<<pl.S, kFixThreads, 0, b->fix_stream>>>(b->d_xt, K_pad, pl.S, pl.S_pad, pl.rows, b->d_oth_cnt, b->d_oth_list, pl.oth_cap,
-                                                        b->d_gram + pl.gram_off, mode);
+      CU(ctx, cudaEventRecord(b->fix_fork.get(), bstream(b)));
+      CU(ctx, cudaStreamWaitEvent(b->fix_stream.get(), b->fix_fork.get(), 0));
+      k_other_fix<<<pl.S, kFixThreads, 0, b->fix_stream.get()>>>(b->d_xt, K_pad, pl.S, pl.S_pad, pl.rows, b->d_oth_cnt,
+                                                              b->d_oth_list, pl.oth_cap, b->d_gram + pl.gram_off, mode);
       ++ctx->launches;
-      CU(ctx, cudaEventRecord(b->fix_join, b->fix_stream));
+      CU(ctx, cudaEventRecord(b->fix_join.get(), b->fix_stream.get()));
     } else {
       CU(ctx, cudaMemsetAsync(mode, 1, sizeof(uint32_t), bstream(b)));  // (any non-zero value: nine blocks)
     }
@@ -847,7 +732,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       ++ctx->launches;
     }
     const bool last = &pl == &b->dense_plans.back();
-    if (last && timing) CU(ctx, cudaEventRecord(b->ev[6], bstream(b)));
+    if (last && timing) CU(ctx, cudaEventRecord(b->ev[6].get(), bstream(b)));
     for (int form = pl.four ? 0 : 1; form < 2; ++form) {  // the launch of the form the unit is not in returns at once
       const DenseTileList& L = form ? pl.list9 : pl.list4;
       DenseParams D;
@@ -868,10 +753,10 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       k_gram_i8<<<ggrid, kDenseThreads, kDenseSmemBytes, bstream(b)>>>(b->tmaps[&pl - b->dense_plans.data()], D);
       ++ctx->launches;
     }
-    if (last && timing) CU(ctx, cudaEventRecord(b->ev[7], bstream(b)));
-    if (pl.four) CU(ctx, cudaStreamWaitEvent(bstream(b), b->fix_join, 0));
+    if (last && timing) CU(ctx, cudaEventRecord(b->ev[7].get(), bstream(b)));
+    if (pl.four) CU(ctx, cudaStreamWaitEvent(bstream(b), b->fix_join.get(), 0));
   }
-  if (timing) CU(ctx, cudaEventRecord(b->ev[5], bstream(b)));
+  if (timing) CU(ctx, cudaEventRecord(b->ev[5].get(), bstream(b)));
   if (b->n_tile_items) {
     // K1 + K2 of the medium units: counts + MI per 16 x 16 block of site pairs
     const unsigned tgrid = (unsigned)std::min<uint64_t>(b->n_tile_items, (uint64_t)ctx->num_sms * 3u);
@@ -902,7 +787,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     C.n_items = b->n_fast;
     C.planes = b->d_planes;
     C.site_flags = b->d_flags;
-    C.ij_tab = ctx->d_ij_tab;
+    C.ij_tab = ctx->d_ij_tab.get();
     C.min_common = min_common;
     C.mode = mode;
     C.item_cnt = b->d_item_cnt;
@@ -912,8 +797,8 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     ++ctx->launches;
   }
   if (forked) {  // the scan needs every item's count
-    CU(ctx, cudaEventRecord(b->side_ev[1], small));
-    CU(ctx, cudaStreamWaitEvent(bstream(b), b->side_ev[1], 0));
+    CU(ctx, cudaEventRecord(b->side_ev[1].get(), small));
+    CU(ctx, cudaStreamWaitEvent(bstream(b), b->side_ev[1].get(), 0));
   }
   if (b->n_items) {
     // K0 of everything else + scan: every item's place in the ordered output
@@ -922,17 +807,17 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       k_count<<<cgrid, kThreads, 0, bstream(b)>>>(P);
       ++ctx->launches;
     }
-    CU(ctx, cub::DeviceScan::ExclusiveSum(b->d_scan_tmp, b->scan_tmp_bytes, b->d_item_cnt, b->d_item_off,
+    CU(ctx, cub::DeviceScan::ExclusiveSum(b->d_scan_tmp.get(), b->scan_tmp_bytes, b->d_item_cnt.get(), b->d_item_off.get(),
                                           (int)b->n_items + 1, bstream(b)));
     ++ctx->launches;
     k_scan_finish<<<1, 32, 0, bstream(b)>>>(b->d_item_off + b->n_items, b->d_header,
-                                            b->own_stream ? b->h_header : nullptr, b->d_unit_rec_off + b->n_units);
+                                            b->own_stream ? b->h_header.get() : nullptr, b->d_unit_rec_off + b->n_units);
     ++ctx->launches;
   }
-  if (timing) CU(ctx, cudaEventRecord(b->ev[2], bstream(b)));
+  if (timing) CU(ctx, cudaEventRecord(b->ev[2].get(), bstream(b)));
   if (forked) {
-    CU(ctx, cudaEventRecord(b->side_ev[2], bstream(b)));
-    CU(ctx, cudaStreamWaitEvent(small, b->side_ev[2], 0));
+    CU(ctx, cudaEventRecord(b->side_ev[2].get(), bstream(b)));
+    CU(ctx, cudaStreamWaitEvent(small, b->side_ev[2].get(), 0));
   }
   if (b->n_fast) {
     FastParams F;
@@ -940,9 +825,9 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     F.n_items = b->n_fast;
     F.planes = b->d_planes;
     F.site_flags = b->d_flags;
-    F.lntab = ctx->d_lntab;
+    F.lntab = ctx->d_lntab.get();
     F.ln_cap = P.ln_cap;
-    F.ij_tab = ctx->d_ij_tab;
+    F.ij_tab = ctx->d_ij_tab.get();
     F.min_common = min_common;
     F.mode = mode;
     F.item_off = b->d_item_off;
@@ -963,8 +848,8 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       k_pairs_fast<<<grid, kFastThreads, sizeof(FastSmem), small>>>(F);
     ++ctx->launches;
   }
-  if (timing) CU(ctx, cudaEventRecord(b->ev[3], bstream(b)));
-  if (forked) CU(ctx, cudaEventRecord(b->side_ev[3], small));
+  if (timing) CU(ctx, cudaEventRecord(b->ev[3].get(), bstream(b)));
+  if (forked) CU(ctx, cudaEventRecord(b->side_ev[3].get(), small));
   if (b->n_items) {
     // everything the small-unit kernel does not take
     if (b->n_tiled_desc) {  // ordering + emission of what k_tile_mi / k_tile_finish computed
@@ -982,7 +867,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
                                                                        b->d_site_mean, b->d_site_cnt);
     ++ctx->launches;
   }
-  if (forked) CU(ctx, cudaStreamWaitEvent(bstream(b), b->side_ev[3], 0));
+  if (forked) CU(ctx, cudaStreamWaitEvent(bstream(b), b->side_ev[3].get(), 0));
   if (b->n_items) {
     // small units k_pairs_fast handed on (a site with too many "other" reads) and pair-less units; exits at once
     // when there is nothing
@@ -990,7 +875,7 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     k_pairs_generic<0><<<grid, kThreads, 0, bstream(b)>>>(P);
     ++ctx->launches;
   }
-  if (timing) CU(ctx, cudaEventRecord(b->ev[1], bstream(b)));
+  if (timing) CU(ctx, cudaEventRecord(b->ev[1].get(), bstream(b)));
   CU(ctx, cudaGetLastError());
   b->ran = true;
   b->last_mode = mode;
@@ -1010,11 +895,11 @@ static int fill_scalars(lgmi_batch* b, lgmi_result* out) {
   float ms = 0.f;
   const bool timing = b->last_timed;
   if (timing) {
-    CU(ctx, cudaEventElapsedTime(&ms, b->ev[0], b->ev[1]));
+    CU(ctx, cudaEventElapsedTime(&ms, b->ev[0].get(), b->ev[1].get()));
     out->kernel_ms = ms;
-    CU(ctx, cudaEventElapsedTime(&ms, b->ev[2], b->ev[3]));
+    CU(ctx, cudaEventElapsedTime(&ms, b->ev[2].get(), b->ev[3].get()));
     out->pairs_kernel_ms = ms;
-    CU(ctx, cudaEventElapsedTime(&ms, b->ev[4], b->ev[5]));
+    CU(ctx, cudaEventElapsedTime(&ms, b->ev[4].get(), b->ev[5].get()));
     out->dense_kernel_ms = ms;
   }
   if (!b->dense_plans.empty()) {
@@ -1029,7 +914,7 @@ static int fill_scalars(lgmi_batch* b, lgmi_result* out) {
       out->n_dense_four += nine ? 0u : 1u;
     }
     if (timing) {
-      CU(ctx, cudaEventElapsedTime(&ms, b->ev[6], b->ev[7]));
+      CU(ctx, cudaEventElapsedTime(&ms, b->ev[6].get(), b->ev[7].get()));
       out->gram_kernel_ms = ms;
       const DensePlan& pl = b->dense_plans.back();
       out->gram_macs = modes[pl.unit] ? pl.list9.macs : pl.list4.macs;
@@ -1068,23 +953,10 @@ extern "C" int lgmi_batch_download(lgmi_batch_t* b, lgmi_result* out) {
   CU(ctx, cudaStreamSynchronize(bstream(b)));
   const uint64_t nrec = b->h_header->n_records;
   if (nrec > b->rec_cap) return fail(ctx, LGMI_ERR_STATE, "record count %llu exceeds capacity", (unsigned long long)nrec);
-  if (nrec > b->h_rec_cap) {
-    if (b->h_records) ctx->host_pool.release(b->h_records);
-    b->h_records = nullptr;
-    b->h_rec_cap = 0;
-    const uint64_t cap = std::max<uint64_t>(nrec + nrec / 8, 1024);
-    CU(ctx, pool_host_alloc(ctx, &b->h_records, cap * sizeof(lgmi_pair_rec)));
-    b->h_rec_cap = cap;
-  }
+  const uint64_t cap = std::max<uint64_t>(nrec + nrec / 8, 1024);  // (the stream is idle: synchronised above)
+  if (nrec > b->h_records.size()) CU(ctx, b->h_records.alloc(ctx->host_pool, cap));
   const bool want_counts = (b->last_mode & LGMI_MODE_EMIT_COUNTS) != 0u;
-  if (want_counts && nrec > b->h_counts_cap) {
-    if (b->h_counts) ctx->host_pool.release(b->h_counts);
-    b->h_counts = nullptr;
-    b->h_counts_cap = 0;
-    const uint64_t cap = std::max<uint64_t>(nrec + nrec / 8, 1024);
-    CU(ctx, pool_host_alloc(ctx, &b->h_counts, cap * 9ull * sizeof(uint32_t)));
-    b->h_counts_cap = cap;
-  }
+  if (want_counts && nrec * 9ull > b->h_counts.size()) CU(ctx, b->h_counts.alloc(ctx->host_pool, cap * 9ull));
   if (nrec) {
     CU(ctx, cudaMemcpyAsync(b->h_records, b->d_records, nrec * sizeof(lgmi_pair_rec), cudaMemcpyDeviceToHost, bstream(b)));
     if (want_counts)
@@ -1094,10 +966,10 @@ extern "C" int lgmi_batch_download(lgmi_batch_t* b, lgmi_result* out) {
   int rc = fill_scalars(b, out);
   if (rc) return rc;
   out->records = b->h_records;
-  out->counts = want_counts ? b->h_counts : nullptr;
+  out->counts = want_counts ? b->h_counts.get() : nullptr;
   out->site_mean = b->h_site_mean;
   out->site_cnt = b->h_site_cnt;
-  out->unit_rec_off = reinterpret_cast<const uint64_t*>(b->h_unit_rec_off);
+  out->unit_rec_off = reinterpret_cast<const uint64_t*>(b->h_unit_rec_off.get());
   return LGMI_OK;
 }
 
@@ -1166,7 +1038,7 @@ extern "C" int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* si
   CU(ctx, cudaSetDevice(ctx->device));
   int rc = ensure_scratch(ctx, bytes);
   if (rc) return rc;
-  char* scratch = static_cast<char*>(ctx->d_scratch);
+  char* scratch = ctx->d_scratch.get();
   uint64_t at = 0;
   for (uint32_t p = 0; p < n_pieces; ++p) {
     const lgmi_batch* b = batches[p];
@@ -1225,38 +1097,38 @@ static StepForm step_form(uint32_t mode, uint32_t max_sites) {
 }
 
 struct lgmi_pipeline {
-  lgmi_ctx* ctx = nullptr;
+  explicit lgmi_pipeline(lgmi_ctx* c) : ctx(c) {}
+  ~lgmi_pipeline();
+  lgmi_ctx* const ctx;
   uint32_t n_units = 0;
   uint64_t plane_words = 0, n_sites = 0, n_candidates = 0;
   struct Chunk {
-    lgmi_batch* b = nullptr;
     uint32_t unit0 = 0, n_units = 0;
     uint64_t plane0 = 0, site0 = 0;
-    cudaEvent_t done = nullptr;     // the group's kernels have finished
-    cudaEvent_t landed = nullptr;   // the group's input is in device memory
-    uint32_t* d_packed = nullptr;   // two-plane input staging (lgmi_pipeline_step_packed)
-    unsigned long long* d_tight_off = nullptr;  // LGMI_MODE_TIGHT_INPUT: first word of each unit, relative to the group
+    Event done;     // the group's kernels have finished
+    Event landed;   // the group's input is in device memory
+    PoolBuf<uint32_t> d_packed;   // two-plane input staging (lgmi_pipeline_step_packed)
+    PoolBuf<unsigned long long> d_tight_off;  // LGMI_MODE_TIGHT_INPUT: first word of each unit, relative to the group
     uint64_t tight0 = 0, tight_words = 0;       // the group's slice of the tight two-plane input
-    double* d_rec_mi = nullptr;     // split output (LGMI_MODE_SPLIT_RECORDS)
-    uint32_t* d_rec_ij = nullptr;
+    PoolBuf<double> d_rec_mi;     // split output (LGMI_MODE_SPLIT_RECORDS)
+    PoolBuf<uint32_t> d_rec_ij;
     uint64_t base = 0;              // first row of the group in the merged output of the current step
+    // declared last, so destroyed first: ~lgmi_batch synchronises the group's stream, whose kernels read and write
+    // the buffers above
+    std::unique_ptr<lgmi_batch> b;
   };
   std::vector<Chunk> chunks;
   // one stream per copy direction: copies of a direction run one after the other anyway, and a stream that
   // copies both ways can land on one engine with another stream's uploads in front of its downloads
-  cudaStream_t h2d = nullptr, d2h = nullptr;
-  lgmi_pair_rec* h_records = nullptr;
-  uint64_t h_rec_cap = 0;
-  uint32_t* h_counts = nullptr;
-  uint64_t h_counts_cap = 0;
-  double* h_rec_mi = nullptr;
-  uint64_t h_rec_mi_cap = 0;
-  uint32_t* h_rec_ij = nullptr;   // (2-byte entries under LGMI_MODE_COMPACT_OUTPUT when every unit has <= 256 sites)
-  uint64_t h_rec_ij_cap = 0;
+  Stream h2d, d2h;
+  PoolBuf<lgmi_pair_rec> h_records;
+  PoolBuf<uint32_t> h_counts;     // 9 per row
+  PoolBuf<double> h_rec_mi;
+  PoolBuf<uint32_t> h_rec_ij;   // (2-byte entries under LGMI_MODE_COMPACT_OUTPUT when every unit has <= 256 sites)
   uint32_t max_sites = 0;
-  double* h_site_mean = nullptr;
-  uint32_t* h_site_cnt = nullptr;
-  unsigned long long* h_unit_rec_off = nullptr;
+  PoolBuf<double> h_site_mean;
+  PoolBuf<uint32_t> h_site_cnt;
+  PoolBuf<unsigned long long> h_unit_rec_off;
   // a step between lgmi_pipeline_begin* and lgmi_pipeline_finish
   bool in_flight = false;   // begun, not finished
   bool collected = false;   // ... and its downloads queued (lgmi_pipeline_collect)
@@ -1264,37 +1136,15 @@ struct lgmi_pipeline {
   uint64_t pend_rows = 0;
 };
 
-extern "C" void lgmi_pipeline_destroy(lgmi_pipeline_t* p) {
-  if (!p) return;
-  lgmi_ctx* ctx = p->ctx;
-  if (p->ctx) cudaSetDevice(p->ctx->device);
-  // copies into the pinned output arrays must have landed before the arrays go back to the cache
-  if (p->d2h) cudaStreamSynchronize(p->d2h);
-  if (p->h2d) cudaStreamSynchronize(p->h2d);
-  for (lgmi_pipeline::Chunk& c : p->chunks) {
-    if (c.b) {
-      cudaStream_t st = c.b->own_stream;
-      lgmi_batch_destroy(c.b);
-      if (st) cudaStreamDestroy(st);
-    }
-    if (c.done) cudaEventDestroy(c.done);
-    if (c.landed) cudaEventDestroy(c.landed);
-    ctx->dev_pool.release(c.d_packed);
-    ctx->dev_pool.release(c.d_tight_off);
-    ctx->dev_pool.release(c.d_rec_mi);
-    ctx->dev_pool.release(c.d_rec_ij);
-  }
-  if (p->h2d) cudaStreamDestroy(p->h2d);
-  if (p->d2h) cudaStreamDestroy(p->d2h);
-  ctx->host_pool.release(p->h_rec_mi);
-  ctx->host_pool.release(p->h_rec_ij);
-  ctx->host_pool.release(p->h_records);
-  ctx->host_pool.release(p->h_counts);
-  ctx->host_pool.release(p->h_site_mean);
-  ctx->host_pool.release(p->h_site_cnt);
-  ctx->host_pool.release(p->h_unit_rec_off);
-  delete p;
+lgmi_pipeline::~lgmi_pipeline() {
+  cudaSetDevice(ctx->device);
+  // copies into the pinned output arrays and out of the groups' buffers must have landed before they go back to the
+  // cache
+  if (d2h) cudaStreamSynchronize(d2h.get());
+  if (h2d) cudaStreamSynchronize(h2d.get());
 }
+
+extern "C" void lgmi_pipeline_destroy(lgmi_pipeline_t* p) { delete p; }
 
 extern "C" int lgmi_pipeline_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_units, uint64_t plane_words,
                                     uint64_t n_sites, uint32_t n_chunks, lgmi_pipeline_t** out) {
@@ -1306,9 +1156,8 @@ extern "C" int lgmi_pipeline_create(lgmi_t* ctx, const lgmi_unit_desc* units, ui
   CU(ctx, cudaSetDevice(ctx->device));
 
   // every failure from here on releases what the pipeline holds so far
-  std::unique_ptr<lgmi_pipeline, void (*)(lgmi_pipeline*)> p(new (std::nothrow) lgmi_pipeline(), lgmi_pipeline_destroy);
+  std::unique_ptr<lgmi_pipeline> p(new (std::nothrow) lgmi_pipeline(ctx));
   if (!p) return fail(ctx, LGMI_ERR_NOMEM, "lgmi_pipeline_create: out of host memory");
-  p->ctx = ctx;
   p->n_units = n_units;
   p->plane_words = plane_words;
   p->n_sites = n_sites;
@@ -1317,7 +1166,9 @@ extern "C" int lgmi_pipeline_create(lgmi_t* ctx, const lgmi_unit_desc* units, ui
   for (const GroupPlan& g : plan.groups) {
     p->chunks.emplace_back();
     lgmi_pipeline::Chunk& c = p->chunks.back();
-    if (const int rc = lgmi_batch_create(ctx, g.units.data(), g.n_units, g.plane_words, g.n_sites, &c.b)) return rc;
+    lgmi_batch* b = nullptr;
+    if (const int rc = lgmi_batch_create(ctx, g.units.data(), g.n_units, g.plane_words, g.n_sites, &b)) return rc;
+    c.b.reset(b);
     c.b->unit_base = g.unit0;  // records carry the unit's index in the whole batch
     c.unit0 = g.unit0;
     c.n_units = g.n_units;
@@ -1327,35 +1178,31 @@ extern "C" int lgmi_pipeline_create(lgmi_t* ctx, const lgmi_unit_desc* units, ui
     c.tight_words = g.tight_words;
     if (g.n_units) {
       const size_t bytes = g.tight_off.size() * sizeof(unsigned long long);
-      CU(ctx, pool_malloc(ctx, &c.d_tight_off, bytes));
+      CU(ctx, c.d_tight_off.alloc(ctx->dev_pool, g.tight_off.size()));
       CU(ctx, cudaMemcpy(c.d_tight_off, g.tight_off.data(), bytes, cudaMemcpyHostToDevice));
     }
-    CU(ctx, cudaStreamCreateWithFlags(&c.b->own_stream, cudaStreamNonBlocking));
-    CU(ctx, cudaEventCreateWithFlags(&c.done, cudaEventDisableTiming));
-    CU(ctx, cudaEventCreateWithFlags(&c.landed, cudaEventDisableTiming));
+    CU(ctx, create(c.b->own_stream));
+    CU(ctx, create(c.done, cudaEventDisableTiming));
+    CU(ctx, create(c.landed, cudaEventDisableTiming));
   }
-  CU(ctx, cudaStreamCreateWithFlags(&p->h2d, cudaStreamNonBlocking));
-  CU(ctx, cudaStreamCreateWithFlags(&p->d2h, cudaStreamNonBlocking));
-  CU(ctx, pool_host_alloc(ctx, &p->h_site_mean, std::max<uint64_t>(1, n_sites) * sizeof(double)));
-  CU(ctx, pool_host_alloc(ctx, &p->h_site_cnt, std::max<uint64_t>(1, n_sites) * sizeof(uint32_t)));
-  CU(ctx, pool_host_alloc(ctx, &p->h_unit_rec_off, ((size_t)n_units + 1) * sizeof(unsigned long long)));
+  CU(ctx, create(p->h2d));
+  CU(ctx, create(p->d2h));
+  CU(ctx, p->h_site_mean.alloc(ctx->host_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, p->h_site_cnt.alloc(ctx->host_pool, std::max<uint64_t>(1, n_sites)));
+  CU(ctx, p->h_unit_rec_off.alloc(ctx->host_pool, (size_t)n_units + 1));
   *out = p.release();
   return LGMI_OK;
 }
 
-// grows a pinned output array, keeping what has already landed in it
+// grows a pinned output array of rows of `width` elements to `need` rows, keeping the `keep` rows that have already
+// landed in it
 template <class T>
-static int grow_pinned(lgmi_pipeline* p, T*& buf, uint64_t& cap, uint64_t need, uint64_t keep, size_t elem) {
-  if (need <= cap) return LGMI_OK;
+static int grow_pinned(lgmi_pipeline* p, PoolBuf<T>& buf, uint64_t need, uint64_t keep, size_t width = 1) {
+  if (need * width <= buf.size()) return LGMI_OK;
   lgmi_ctx* ctx = p->ctx;
-  CU(ctx, cudaStreamSynchronize(p->d2h));  // copies into the old array
-  const uint64_t new_cap = std::max<uint64_t>(need + need / 4, 1024);
-  T* fresh = nullptr;
-  CU(ctx, pool_host_alloc(ctx, &fresh, new_cap * elem));
-  if (keep) memcpy(fresh, buf, keep * elem);
-  if (buf) ctx->host_pool.release(buf);
-  buf = fresh;
-  cap = new_cap;
+  CU(ctx, cudaStreamSynchronize(p->d2h.get()));  // copies into the old array
+  const uint64_t rows = std::max<uint64_t>(need + need / 4, 1024);
+  CU(ctx, buf.alloc(ctx->host_pool, rows * width, keep * width));
   return LGMI_OK;
 }
 
@@ -1373,26 +1220,27 @@ static int pipeline_begin(lgmi_pipeline* p, const uint32_t* planes, bool packed,
   if (f.tight && !packed) return fail(ctx, LGMI_ERR_ARG, "LGMI_MODE_TIGHT_INPUT is a form of the two-plane input (lgmi_pipeline_step_packed)");
   p->form = f;
   for (lgmi_pipeline::Chunk& c : p->chunks) {
-    lgmi_batch* b = c.b;
-    cudaStream_t st = b->own_stream;
+    lgmi_batch* b = c.b.get();
+    cudaStream_t st = b->own_stream.get();
     // input on the upload stream, in group order; the group's own stream picks up when it has landed
-    if (b->n_sites) CU(ctx, cudaMemcpyAsync(b->d_flags, site_flags + c.site0, b->n_sites, cudaMemcpyHostToDevice, p->h2d));
+    if (b->n_sites)
+      CU(ctx, cudaMemcpyAsync(b->d_flags, site_flags + c.site0, b->n_sites, cudaMemcpyHostToDevice, p->h2d.get()));
     const uint64_t words2 = b->plane_words / 3u * 2u;           // staging sized for the padded form: either fits
     const uint64_t words_in = f.tight ? c.tight_words : words2;
     if (packed) {  // two planes per site over PCIe, expanded on the device
-      if (!c.d_packed && words2) CU(ctx, pool_malloc(ctx, &c.d_packed, words2 * sizeof(uint32_t)));
+      if (!c.d_packed && words2) CU(ctx, c.d_packed.alloc(ctx->dev_pool, words2));
       if (words_in)
         CU(ctx, cudaMemcpyAsync(c.d_packed, planes + (f.tight ? c.tight0 : c.plane0 / 3u * 2u), words_in * sizeof(uint32_t),
-                                cudaMemcpyHostToDevice, p->h2d));
+                                cudaMemcpyHostToDevice, p->h2d.get()));
     } else if (b->plane_words) {
       CU(ctx, cudaMemcpyAsync(b->d_planes, planes + c.plane0, b->plane_words * sizeof(uint32_t), cudaMemcpyHostToDevice,
-                              p->h2d));
+                              p->h2d.get()));
     }
-    CU(ctx, cudaEventRecord(c.landed, p->h2d));
-    CU(ctx, cudaStreamWaitEvent(st, c.landed, 0));
+    CU(ctx, cudaEventRecord(c.landed.get(), p->h2d.get()));
+    CU(ctx, cudaStreamWaitEvent(st, c.landed.get(), 0));
     if (packed && words2) {
       k_unpack2<<<std::min<uint32_t>(b->n_units, (uint32_t)ctx->num_sms * 16u), 256, 0, st>>>(
-          b->d_units, b->n_units, c.d_packed, b->d_planes, f.tight ? c.d_tight_off : nullptr);
+          b->d_units, b->n_units, c.d_packed, b->d_planes, f.tight ? c.d_tight_off.get() : nullptr);
       ++ctx->launches;
     }
     b->uploaded = true;
@@ -1403,14 +1251,14 @@ static int pipeline_begin(lgmi_pipeline* p, const uint32_t* planes, bool packed,
     if (const int rc = lgmi_batch_run(b, min_common, f.run_mode)) return rc;
     if (f.split) {
       if (!c.d_rec_mi) {
-        CU(ctx, pool_malloc(ctx, &c.d_rec_mi, b->rec_cap * sizeof(double)));
-        CU(ctx, pool_malloc(ctx, &c.d_rec_ij, b->rec_cap * sizeof(uint32_t)));
+        CU(ctx, c.d_rec_mi.alloc(ctx->dev_pool, b->rec_cap));
+        CU(ctx, c.d_rec_ij.alloc(ctx->dev_pool, b->rec_cap));
       }
-      k_split_records<<<(unsigned)ctx->num_sms * 8u, 256, 0, st>>>(b->d_header, b->d_records, c.d_rec_mi, c.d_rec_ij,
-                                                                   f.ij16 ? reinterpret_cast<uint16_t*>(c.d_rec_ij) : nullptr);
+      k_split_records<<<(unsigned)ctx->num_sms * 8u, 256, 0, st>>>(
+          b->d_header, b->d_records, c.d_rec_mi, c.d_rec_ij, f.ij16 ? reinterpret_cast<uint16_t*>(c.d_rec_ij.get()) : nullptr);
       ++ctx->launches;
     }
-    CU(ctx, cudaEventRecord(c.done, st));  // the group's record count is in its (host-resident) header by then
+    CU(ctx, cudaEventRecord(c.done.get(), st));  // the group's record count is in its (host-resident) header by then
   }
   p->in_flight = true;
   return LGMI_OK;
@@ -1432,26 +1280,26 @@ static int pipeline_collect(lgmi_pipeline* p) {
   std::vector<double> t_done, t_issue;
   uint64_t base = 0;
   for (lgmi_pipeline::Chunk& c : p->chunks) {
-    lgmi_batch* b = c.b;
-    CU(ctx, cudaEventSynchronize(c.done));
+    lgmi_batch* b = c.b.get();
+    CU(ctx, cudaEventSynchronize(c.done.get()));
     if (debug) t_done.push_back(since());
     const uint64_t nrec = b->h_header->n_records;
     if (nrec > b->rec_cap) return fail(ctx, LGMI_ERR_STATE, "record count %llu exceeds capacity", (unsigned long long)nrec);
     int rc = LGMI_OK;
     if (f.split) {
-      rc = grow_pinned(p, p->h_rec_mi, p->h_rec_mi_cap, base + nrec, base, sizeof(double));
-      if (!rc) rc = grow_pinned(p, p->h_rec_ij, p->h_rec_ij_cap, base + nrec, base, sizeof(uint32_t));
+      rc = grow_pinned(p, p->h_rec_mi, base + nrec, base);
+      if (!rc) rc = grow_pinned(p, p->h_rec_ij, base + nrec, base);
     } else {
-      rc = grow_pinned(p, p->h_records, p->h_rec_cap, base + nrec, base, sizeof(lgmi_pair_rec));
+      rc = grow_pinned(p, p->h_records, base + nrec, base);
     }
-    if (!rc && f.want_counts) rc = grow_pinned(p, p->h_counts, p->h_counts_cap, base + nrec, base, 9 * sizeof(uint32_t));
+    if (!rc && f.want_counts) rc = grow_pinned(p, p->h_counts, base + nrec, base, 9);
     if (rc) return rc;
-    cudaStream_t st = p->d2h;  // the group is complete (event above): nothing here waits on a kernel
+    cudaStream_t st = p->d2h.get();  // the group is complete (event above): nothing here waits on a kernel
     if (nrec) {
       if (f.split) {
         CU(ctx, cudaMemcpyAsync(p->h_rec_mi + base, c.d_rec_mi, nrec * sizeof(double), cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaMemcpyAsync(reinterpret_cast<char*>(p->h_rec_ij) + base * ij_bytes, c.d_rec_ij, nrec * ij_bytes,
-                                cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaMemcpyAsync(reinterpret_cast<char*>(p->h_rec_ij.get()) + base * ij_bytes, c.d_rec_ij,
+                                nrec * ij_bytes, cudaMemcpyDeviceToHost, st));
       } else {
         CU(ctx, cudaMemcpyAsync(p->h_records + base, b->d_records, nrec * sizeof(lgmi_pair_rec), cudaMemcpyDeviceToHost, st));
       }
@@ -1493,7 +1341,7 @@ static int pipeline_finish(lgmi_pipeline* p, lgmi_result* out) {
   p->in_flight = p->collected = false;
   const StepForm& f = p->form;
   const uint64_t base = p->pend_rows;
-  CU(ctx, cudaStreamSynchronize(p->d2h));
+  CU(ctx, cudaStreamSynchronize(p->d2h.get()));
   for (lgmi_pipeline::Chunk& c : p->chunks) {
     for (uint32_t u = 0; u < c.n_units; ++u) p->h_unit_rec_off[c.unit0 + u] = c.base + c.b->h_unit_rec_off[u];
   }
@@ -1502,18 +1350,18 @@ static int pipeline_finish(lgmi_pipeline* p, lgmi_result* out) {
   out->n_candidates = p->n_candidates;
   out->n_evaluated = 0;
   out->n_records = base;
-  out->records = f.split ? nullptr : p->h_records;
-  out->rec_mi = f.split ? p->h_rec_mi : nullptr;
-  out->rec_ij = f.split ? p->h_rec_ij : nullptr;
+  out->records = f.split ? nullptr : p->h_records.get();
+  out->rec_mi = f.split ? p->h_rec_mi.get() : nullptr;
+  out->rec_ij = f.split ? p->h_rec_ij.get() : nullptr;
   out->rec_ij_bytes = f.split ? (uint32_t)f.ij_bytes() : 0u;
-  out->counts = f.want_counts ? p->h_counts : nullptr;
+  out->counts = f.want_counts ? p->h_counts.get() : nullptr;
   out->n_sites = p->n_sites;
   out->site_mean = p->h_site_mean;
-  out->site_cnt = f.compact ? nullptr : p->h_site_cnt;
-  out->unit_rec_off = reinterpret_cast<const uint64_t*>(p->h_unit_rec_off);
+  out->site_cnt = f.compact ? nullptr : p->h_site_cnt.get();
+  out->unit_rec_off = reinterpret_cast<const uint64_t*>(p->h_unit_rec_off.get());
   for (lgmi_pipeline::Chunk& c : p->chunks) {
     lgmi_result r;
-    int rc = fill_scalars(c.b, &r);
+    int rc = fill_scalars(c.b.get(), &r);
     if (rc) return rc;
     out->n_evaluated += r.n_evaluated;
     out->kernel_ms += r.kernel_ms;
@@ -1558,8 +1406,7 @@ extern "C" int lgmi_submit(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_
                            uint64_t plane_words, const uint8_t* site_flags, uint64_t n_sites, int min_common,
                            uint32_t mode) {
   if (!ctx) return LGMI_ERR_ARG;
-  if (ctx->oneshot) lgmi_batch_destroy(ctx->oneshot);
-  ctx->oneshot = nullptr;
+  lgmi_batch_destroy(ctx->oneshot);
   lgmi_batch* b = nullptr;
   int rc = lgmi_batch_create(ctx, units, n_units, plane_words, n_sites, &b);
   if (rc) return rc;
@@ -1588,7 +1435,7 @@ extern "C" int lgmi_site_mean_csr(lgmi_t* ctx, const uint64_t* offsets, const do
   const size_t out_bytes = n_sites * sizeof(double);
   int rc = ensure_scratch(ctx, off_bytes + val_bytes + out_bytes + 64);
   if (rc) return rc;
-  char* p = static_cast<char*>(ctx->d_scratch);
+  char* p = ctx->d_scratch.get();
   unsigned long long* d_off = reinterpret_cast<unsigned long long*>(p);
   double* d_val = reinterpret_cast<double*>(p + off_bytes);
   double* d_out = reinterpret_cast<double*>(p + off_bytes + val_bytes);
@@ -1624,7 +1471,7 @@ extern "C" int lgmi_ecdf(lgmi_t* ctx, const double* mean, const uint8_t* site_fl
   const size_t a_tmp = align_up(a_cnt + 8, 256);
   int rc = ensure_scratch(ctx, a_tmp + sort_bytes);
   if (rc) return rc;
-  char* p = static_cast<char*>(ctx->d_scratch);
+  char* p = ctx->d_scratch.get();
   double* d_mean = reinterpret_cast<double*>(p + a_mean);
   double* d_keys = reinterpret_cast<double*>(p + a_keys);
   double* d_sorted = reinterpret_cast<double*>(p + a_sorted);
@@ -1662,7 +1509,7 @@ static int ecdf_sort(lgmi_ctx* ctx, const double* x, uint64_t n, size_t extra_by
   const size_t a_extra = align_up(a_tmp + sort_bytes, 256);
   int rc = ensure_scratch(ctx, a_extra + extra_bytes);
   if (rc) return rc;
-  char* p = static_cast<char*>(ctx->d_scratch);
+  char* p = ctx->d_scratch.get();
   double* d_x = reinterpret_cast<double*>(p + a_x);
   *d_sorted = reinterpret_cast<double*>(p + a_sorted);
   *d_nan = reinterpret_cast<unsigned long long*>(p + a_nan);
