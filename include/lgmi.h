@@ -288,6 +288,55 @@ LGMI_API int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site
                               lgmi_batch_t* const* batches, const uint32_t* unit_in_batch, double* mean_out,
                               uint32_t* cnt_out);
 
+/* ----- split units over processes (one process per GPU) -------------------- *
+ * The same pieces with their batches in other processes: a piece is exported *
+ * as plain bytes (CUDA IPC handles of the batch's plane and dense-MI blocks   *
+ * and of an interprocess event), sent by any means, and imported by the       *
+ * plane copy and the per-site pass below.  Offsets count from the base of     *
+ * each block (a whole device allocation).                                     *
+ *                                                                             *
+ * Lifetime: an exporting batch must stay alive until every process that      *
+ * imported from it has destroyed its importing batch or has returned from     *
+ * lgmi_split_means_ipc (a barrier between the processes).                     */
+typedef struct {
+  uint8_t plane_mem[64];  /* cudaIpcMemHandle_t of the batch's plane block     */
+  uint8_t dense_mem[64];  /* cudaIpcMemHandle_t of its dense-MI block          */
+  uint8_t event[64];      /* cudaIpcEventHandle_t of its interprocess event,  *
+                           * recorded behind all the batch had queued          */
+  uint64_t plane_word;    /* the piece's first plane word                      */
+  uint64_t plane_words;   /* words of the piece's own rows (3 * W * rows)      */
+  uint64_t dense_off;     /* first double of the piece's MI slice              */
+  uint64_t dense_pairs;   /* length of that slice: the piece's pairs           */
+  uint64_t batch_id;      /* the batch, within the exporting process           */
+  uint32_t unit;          /* the piece's unit index in its batch               */
+  uint32_t n_sites;       /* sites of the piece's suffix unit                  */
+  uint32_t row_limit;     /* its row limit (0: not a piece)                    */
+  uint32_t ran;           /* 1 if the batch had been run when this was filled  */
+  int32_t pid;            /* exporting process                                 */
+  char pci_bus_id[36];    /* the source device, cudaDeviceGetPCIBusId form     */
+} lgmi_piece_ipc;         /* 288 bytes                                         */
+
+/* Fills *out for unit `unit` of b (created with a row limit for it) after    *
+ * recording b's interprocess event on b's stream, behind everything queued    *
+ * so far (the upload, or the run).                                            */
+LGMI_API int lgmi_piece_export(lgmi_batch_t* b, uint32_t unit, lgmi_piece_ipc* out);
+/* lgmi_batch_copy_planes from a piece exported by another process: n_words   *
+ * plane words of its batch from src_word (within the piece's own rows) to     *
+ * dst_word of dst, queued on dst's stream behind the piece's event.  The      *
+ * source device is found by PCI bus id and must be visible to this process;   *
+ * two processes on one device copy device to device.  The mappings opened     *
+ * belong to dst (closed by lgmi_batch_destroy; reused by later copies).  A    *
+ * piece exported by this process is LGMI_ERR_ARG: use lgmi_batch_copy_planes. */
+LGMI_API int lgmi_batch_copy_planes_ipc(lgmi_batch_t* dst, uint64_t dst_word, const lgmi_piece_ipc* src,
+                                        uint64_t src_word, uint64_t n_words);
+/* lgmi_split_means with pieces in any process, exported after their run      *
+ * (else LGMI_ERR_STATE; LGMI_ERR_ARG if they do not make up the unit).  A     *
+ * slice from another process is copied behind its piece's event; the          *
+ * mappings opened for that are closed before the call returns.  The same     *
+ * bits as lgmi_split_means.                                                   */
+LGMI_API int lgmi_split_means_ipc(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site_flags, uint32_t n_pieces,
+                                  const lgmi_piece_ipc* pieces, double* mean_out, uint32_t* cnt_out);
+
 /* ----- pipelined step over HOST buffers ------------------------------------ *
  * Same result as upload + run + download of one batch (mismatch.py:387-404    *
  * for every unit), but the units are cut into n_chunks consecutive groups of  *

@@ -45,6 +45,7 @@ EXPORTS = (
     "lgmi_batch_create", "lgmi_batch_destroy", "lgmi_batch_upload", "lgmi_batch_run",
     "lgmi_batch_download", "lgmi_batch_sync", "lgmi_batch_device_ptrs",
     "lgmi_batch_create_rows", "lgmi_batch_upload_rows", "lgmi_batch_copy_planes", "lgmi_split_means",
+    "lgmi_piece_export", "lgmi_batch_copy_planes_ipc", "lgmi_split_means_ipc",
     "lgmi_batch_algorithmic_bytes", "lgmi_pipeline_create", "lgmi_pipeline_step", "lgmi_pipeline_step_packed",
     "lgmi_pipeline_begin", "lgmi_pipeline_begin_packed", "lgmi_pipeline_collect", "lgmi_pipeline_finish",
     "lgmi_pipeline_destroy",
@@ -75,6 +76,26 @@ class Result(C.Structure):
         ("rec_mi", C.c_void_p),
         ("rec_ij", C.c_void_p),
         ("n_dense_four", C.c_uint32),
+    ]
+
+
+class PieceIpc(C.Structure):
+    """lgmi_piece_ipc: one piece of a split unit as another process imports it (plain bytes, 288 of them)."""
+    _fields_ = [
+        ("plane_mem", C.c_uint8 * 64),
+        ("dense_mem", C.c_uint8 * 64),
+        ("event", C.c_uint8 * 64),
+        ("plane_word", C.c_uint64),
+        ("plane_words", C.c_uint64),
+        ("dense_off", C.c_uint64),
+        ("dense_pairs", C.c_uint64),
+        ("batch_id", C.c_uint64),
+        ("unit", C.c_uint32),
+        ("n_sites", C.c_uint32),
+        ("row_limit", C.c_uint32),
+        ("ran", C.c_uint32),
+        ("pid", C.c_int32),
+        ("pci_bus_id", C.c_char * 36),
     ]
 
 
@@ -123,6 +144,9 @@ def load():
         "lgmi_batch_upload_rows": (i32, [vp, vp, u64, u64, vp]),
         "lgmi_batch_copy_planes": (i32, [vp, u64, vp, u64, u64]),
         "lgmi_split_means": (i32, [vp, u32, vp, u32, vp, vp, vp, vp]),
+        "lgmi_piece_export": (i32, [vp, u32, C.POINTER(PieceIpc)]),
+        "lgmi_batch_copy_planes_ipc": (i32, [vp, u64, C.POINTER(PieceIpc), u64, u64]),
+        "lgmi_split_means_ipc": (i32, [vp, u32, vp, u32, vp, vp, vp]),
         "lgmi_pipeline_create": (i32, [vp, vp, u32, u64, u64, u32, pvp]),
         "lgmi_pipeline_step": (i32, [vp, vp, vp, i32, u32, C.POINTER(Result)]),
         "lgmi_pipeline_step_packed": (i32, [vp, vp, vp, i32, u32, C.POINTER(Result)]),

@@ -252,6 +252,21 @@ class Batch:
         check(self._lib.lgmi_batch_copy_planes(self.handle, int(dst_word), src.handle, int(src_word), int(n_words)),
               self.ctx.handle)
 
+    def export_piece(self, k) -> bytes:
+        """Piece k of this batch as the bytes another process imports (lgmi_piece_export: CUDA IPC handles of the
+        batch's blocks and of an event recorded behind everything queued so far, i.e. the upload or the run).  The
+        batch must outlive every importer's use of them."""
+        out = _lib.PieceIpc()
+        check(self._lib.lgmi_piece_export(self.handle, int(k), C.byref(out)), self.ctx.handle)
+        return bytes(out)
+
+    def copy_planes_from_ipc(self, dst_word, piece: bytes, src_word, n_words):
+        """copy_planes_from with the source a piece exported by another process (export_piece's bytes): n_words
+        plane words of its batch from src_word, behind its event (lgmi_batch_copy_planes_ipc)."""
+        src = _lib.PieceIpc.from_buffer_copy(piece)
+        check(self._lib.lgmi_batch_copy_planes_ipc(self.handle, int(dst_word), C.byref(src), int(src_word),
+                                                   int(n_words)), self.ctx.handle)
+
     def run(self, min_common, mode=MODE_ALL_PAIRS):
         check(self._lib.lgmi_batch_run(self.handle, int(min_common), int(mode)), self.ctx.handle)
 
@@ -414,6 +429,19 @@ def split_means(ctx: Context, site_flags, pieces):
     cnt = np.empty(n, dtype=np.uint32)
     check(ctx._lib.lgmi_split_means(ctx.handle, n, ptr(flags), len(pieces), C.cast(handles, C.c_void_p), ptr(units),
                                     ptr(mean), ptr(cnt)), ctx.handle)
+    return mean, cnt
+
+
+def split_means_ipc(ctx: Context, site_flags, pieces):
+    """split_means over pieces in any process: `pieces` = export_piece bytes of every piece in row order, each
+    exported after its run (lgmi_split_means_ipc).  The same bits as split_means."""
+    flags = np.ascontiguousarray(site_flags, dtype=np.uint8)
+    n = flags.size
+    arr = (_lib.PieceIpc * len(pieces))(*[_lib.PieceIpc.from_buffer_copy(p) for p in pieces])
+    mean = np.empty(n, dtype=np.float64)
+    cnt = np.empty(n, dtype=np.uint32)
+    check(ctx._lib.lgmi_split_means_ipc(ctx.handle, n, ptr(flags), len(pieces), C.cast(arr, C.c_void_p), ptr(mean),
+                                        ptr(cnt)), ctx.handle)
     return mean, cnt
 
 

@@ -16,8 +16,12 @@
 #include <new>
 #include <queue>
 #include <memory>
+#include <mutex>
 #include <string>
+#include <unordered_map>
 #include <vector>
+
+#include <unistd.h>
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
@@ -66,6 +70,64 @@ static cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) {
   p.reset(h);
   return e;
 }
+
+// Blocks and events of other processes' batches (lgmi_piece_ipc), opened here.  Each handle is opened once per owner:
+// a second cudaIpcOpenMemHandle of the same handle fails.  Released when the owner goes: mappings closed on the
+// device they were opened on, events destroyed.  Whatever was queued on them must have finished by then.
+static_assert(sizeof(cudaIpcMemHandle_t) == sizeof(lgmi_piece_ipc{}.plane_mem) &&
+                  sizeof(cudaIpcEventHandle_t) == sizeof(lgmi_piece_ipc{}.event),
+              "lgmi_piece_ipc carries the runtime's IPC handles as plain bytes");
+struct IpcImports {
+  struct Mem {
+    cudaIpcMemHandle_t handle;
+    int device;
+    void* ptr;
+  };
+  struct Ev {
+    cudaIpcEventHandle_t handle;
+    cudaEvent_t ev;
+  };
+  std::vector<Mem> mems;
+  std::vector<Ev> events;
+  IpcImports() = default;
+  IpcImports(const IpcImports&) = delete;
+  IpcImports& operator=(const IpcImports&) = delete;
+  ~IpcImports() {
+    int current = 0;
+    cudaGetDevice(&current);  // (the owner's own members are released on its device after this)
+    for (const Mem& m : mems) {
+      cudaSetDevice(m.device);
+      cudaIpcCloseMemHandle(m.ptr);
+    }
+    for (const Ev& e : events) cudaEventDestroy(e.ev);
+    cudaSetDevice(current);
+  }
+  // the block of `bytes` (a cudaIpcMemHandle_t) mapped into `device`'s address space
+  cudaError_t open_mem(const uint8_t* bytes, int device, void** out) {
+    for (const Mem& m : mems)
+      if (m.device == device && !memcmp(&m.handle, bytes, sizeof m.handle)) return *out = m.ptr, cudaSuccess;
+    Mem m{{}, device, nullptr};
+    memcpy(&m.handle, bytes, sizeof m.handle);
+    cudaError_t e = cudaSetDevice(device);
+    if (e == cudaSuccess) e = cudaIpcOpenMemHandle(&m.ptr, m.handle, cudaIpcMemLazyEnablePeerAccess);
+    if (e != cudaSuccess) return e;
+    mems.push_back(m);
+    *out = m.ptr;
+    return cudaSuccess;
+  }
+  // the event of `bytes` (a cudaIpcEventHandle_t), opened with the current device
+  cudaError_t open_event(const uint8_t* bytes, cudaEvent_t* out) {
+    for (const Ev& e : events)
+      if (!memcmp(&e.handle, bytes, sizeof e.handle)) return *out = e.ev, cudaSuccess;
+    Ev v{{}, nullptr};
+    memcpy(&v.handle, bytes, sizeof v.handle);
+    const cudaError_t e = cudaIpcOpenEventHandle(&v.ev, v.handle);
+    if (e != cudaSuccess) return e;
+    events.push_back(v);
+    *out = v.ev;
+    return cudaSuccess;
+  }
+};
 
 // The raw allocations behind the context's pools.  An exhausted device or host returns cudaErrorMemoryAllocation,
 // which CU reports as LGMI_ERR_NOMEM; the runtime also keeps it as the thread's last error, cleared here so that a
@@ -196,7 +258,18 @@ struct lgmi_batch {
   std::vector<uint32_t> h_row_limit;
   std::vector<uint64_t> h_dense_off;
   Event copy_ev;  // lgmi_batch_copy_planes from this batch: what its stream has queued so far
+  // lgmi_piece_export: the interprocess event other processes' copies wait on, and the batch's id in this process
+  // (0: never exported)
+  Event ipc_ev;
+  uint64_t export_id = 0;
+  IpcImports imports;  // lgmi_batch_copy_planes_ipc into this batch: the other processes' blocks and events it opened
 };
+
+// Batches that have exported a piece, by id: lgmi_split_means_ipc finds a piece of this process here.  Guarded by a
+// mutex because batches on different contexts may be created and destroyed from different threads (DevicePool).
+static std::mutex g_export_mu;
+static std::unordered_map<uint64_t, lgmi_batch*> g_exported;
+static uint64_t g_export_ids = 0;
 
 // --------------------------------------------------------------------------- helpers
 static inline cudaStream_t bstream(const lgmi_batch* b) { return b->own_stream ? b->own_stream.get() : b->ctx->stream; }
@@ -376,6 +449,10 @@ extern "C" int lgmi_set_dense_threshold(lgmi_t* ctx, uint32_t min_sites, uint32_
 lgmi_batch::~lgmi_batch() {
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(bstream(this));  // nothing in flight touches a block when it goes back to the cache
+  if (export_id) {
+    std::lock_guard<std::mutex> lock(g_export_mu);
+    g_exported.erase(export_id);
+  }
 }
 
 extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
@@ -555,6 +632,15 @@ extern "C" int lgmi_batch_upload_rows(lgmi_batch_t* b, const uint32_t* planes, u
   return LGMI_OK;
 }
 
+// Direct peer copies from sdev to the current device ddev where the devices allow them; without peer access the
+// runtime stages them through the host.
+static void enable_peer(int ddev, int sdev) {
+  if (sdev == ddev) return;
+  int can = 0;
+  if (cudaDeviceCanAccessPeer(&can, ddev, sdev) == cudaSuccess && can && cudaDeviceEnablePeerAccess(sdev, 0) != cudaSuccess)
+    cudaGetLastError();  // (cudaErrorPeerAccessAlreadyEnabled, or no peer access: the copy works either way)
+}
+
 extern "C" int lgmi_batch_copy_planes(lgmi_batch_t* dst, uint64_t dst_word, const lgmi_batch_t* src, uint64_t src_word,
                                       uint64_t n_words) {
   if (!dst || !src) return LGMI_ERR_ARG;
@@ -571,16 +657,93 @@ extern "C" int lgmi_batch_copy_planes(lgmi_batch_t* dst, uint64_t dst_word, cons
   if (!s->copy_ev) CU(ctx, create(s->copy_ev, cudaEventDisableTiming));
   CU(ctx, cudaEventRecord(s->copy_ev.get(), bstream(s)));
   CU(ctx, cudaSetDevice(ddev));
-  if (sdev != ddev) {
-    // direct peer copies where the devices allow them; without peer access the runtime stages through the host
-    int can = 0;
-    if (cudaDeviceCanAccessPeer(&can, ddev, sdev) == cudaSuccess && can &&
-        cudaDeviceEnablePeerAccess(sdev, 0) != cudaSuccess)
-      cudaGetLastError();  // (cudaErrorPeerAccessAlreadyEnabled, or no peer access: the copy works either way)
-  }
+  enable_peer(ddev, sdev);
   CU(ctx, cudaStreamWaitEvent(bstream(dst), s->copy_ev.get(), 0));
   CU(ctx, cudaMemcpyPeerAsync(dst->d_planes + dst_word, ddev, s->d_planes + src_word, sdev, n_words * sizeof(uint32_t),
                               bstream(dst)));
+  dst->uploaded = true;
+  return LGMI_OK;
+}
+
+// The device of this process that an exported piece lives on.
+static int piece_device(lgmi_ctx* ctx, const char* fn, const lgmi_piece_ipc* p, int* dev) {
+  if (!memchr(p->pci_bus_id, 0, sizeof p->pci_bus_id))
+    return fail(ctx, LGMI_ERR_ARG, "%s: the piece's PCI bus id is not a string", fn);
+  if (cudaDeviceGetByPCIBusId(dev, p->pci_bus_id) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ctx, LGMI_ERR_ARG, "%s: the piece's device (PCI bus id %s) is not visible to this process", fn,
+                p->pci_bus_id);
+  }
+  return LGMI_OK;
+}
+
+extern "C" int lgmi_piece_export(lgmi_batch_t* b, uint32_t unit, lgmi_piece_ipc* out) {
+  if (!b || !out) return LGMI_ERR_ARG;
+  lgmi_ctx* ctx = b->ctx;
+  if (unit >= b->n_units || b->h_row_limit.empty() || !b->h_row_limit[unit])
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_piece_export: unit %u is not a unit with a row limit", unit);
+  CU(ctx, cudaSetDevice(ctx->device));
+  if (!b->ipc_ev) CU(ctx, create(b->ipc_ev, cudaEventInterprocess | cudaEventDisableTiming));
+  if (!b->export_id) {
+    std::lock_guard<std::mutex> lock(g_export_mu);
+    b->export_id = ++g_export_ids;
+    g_exported[b->export_id] = b;
+  }
+  // behind everything the batch's stream has queued: its upload, or its run
+  CU(ctx, cudaEventRecord(b->ipc_ev.get(), bstream(b)));
+  lgmi_piece_ipc p;
+  memset(&p, 0, sizeof p);
+  // A handle covers one whole allocation and the importer maps it at its base.  The pool hands out whole cudaMalloc
+  // blocks (MemPool::alloc returns the raw allocation), so a PoolBuf's pointer is that base and offsets count from it.
+  cudaIpcMemHandle_t mh;
+  CU(ctx, cudaIpcGetMemHandle(&mh, b->d_planes.get()));
+  memcpy(p.plane_mem, &mh, sizeof mh);
+  CU(ctx, cudaIpcGetMemHandle(&mh, b->d_dense.get()));
+  memcpy(p.dense_mem, &mh, sizeof mh);
+  cudaIpcEventHandle_t eh;
+  CU(ctx, cudaIpcGetEventHandle(&eh, b->ipc_ev.get()));
+  memcpy(p.event, &eh, sizeof eh);
+  const lgmi_unit_desc& u = b->h_units[unit];
+  p.plane_word = u.plane_off;
+  p.plane_words = 3ull * u.row_words * b->h_row_limit[unit];
+  p.dense_off = b->h_dense_off[unit];
+  p.dense_pairs = piece_pairs(b->h_row_limit[unit], u.n_sites);
+  p.batch_id = b->export_id;
+  p.unit = unit;
+  p.n_sites = u.n_sites;
+  p.row_limit = b->h_row_limit[unit];
+  p.ran = b->ran ? 1u : 0u;
+  p.pid = (int32_t)getpid();
+  CU(ctx, cudaDeviceGetPCIBusId(p.pci_bus_id, (int)sizeof p.pci_bus_id, ctx->device));
+  *out = p;
+  return LGMI_OK;
+}
+
+extern "C" int lgmi_batch_copy_planes_ipc(lgmi_batch_t* dst, uint64_t dst_word, const lgmi_piece_ipc* src,
+                                          uint64_t src_word, uint64_t n_words) {
+  if (!dst || !src) return LGMI_ERR_ARG;
+  lgmi_ctx* ctx = dst->ctx;
+  if (src->pid == (int32_t)getpid())
+    return fail(ctx, LGMI_ERR_ARG,
+                "lgmi_batch_copy_planes_ipc: the piece was exported by this process; copy from its batch with "
+                "lgmi_batch_copy_planes");
+  if (dst_word > dst->plane_words || n_words > dst->plane_words - dst_word || src_word < src->plane_word ||
+      src_word - src->plane_word > src->plane_words || n_words > src->plane_words - (src_word - src->plane_word))
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_batch_copy_planes_ipc: %llu words from %llu to %llu out of range",
+                (unsigned long long)n_words, (unsigned long long)src_word, (unsigned long long)dst_word);
+  if (!n_words) return LGMI_OK;
+  int sdev = 0;
+  if (const int rc = piece_device(ctx, "lgmi_batch_copy_planes_ipc", src, &sdev)) return rc;
+  const int ddev = ctx->device;
+  void* base = nullptr;
+  cudaEvent_t ev = nullptr;
+  CU(ctx, dst->imports.open_mem(src->plane_mem, sdev, &base));  // (leaves sdev current: the event is opened there)
+  CU(ctx, dst->imports.open_event(src->event, &ev));
+  CU(ctx, cudaSetDevice(ddev));
+  enable_peer(ddev, sdev);
+  CU(ctx, cudaStreamWaitEvent(bstream(dst), ev, 0));
+  CU(ctx, cudaMemcpyPeerAsync(dst->d_planes + dst_word, ddev, static_cast<const uint32_t*>(base) + src_word, sdev,
+                              n_words * sizeof(uint32_t), bstream(dst)));
   dst->uploaded = true;
   return LGMI_OK;
 }
@@ -997,54 +1160,67 @@ extern "C" int lgmi_batch_algorithmic_bytes(lgmi_batch_t* b, uint64_t* bytes) {
 // --------------------------------------------------------------------------- split units
 // The dense MI slices of a unit's pieces, back to back, are the whole unit's dense MI array (the pieces' pairs are
 // consecutive ranges of its pair order); k_site_mean_dense over that array is the unsplit run's per-site pass.
-extern "C" int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site_flags, uint32_t n_pieces,
-                                lgmi_batch_t* const* batches, const uint32_t* unit_in_batch, double* mean_out,
-                                uint32_t* cnt_out) {
-  if (!ctx || !batches || !unit_in_batch || !n_pieces || (n_sites && (!site_flags || !mean_out || !cnt_out)))
-    return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: NULL argument");
-  const uint32_t S = n_sites;
-  std::vector<uint64_t> slice(n_pieces);
+// One piece as the checks of lgmi_split_means / lgmi_split_means_ipc see it.
+struct SplitPiece {
+  bool present;   // (lgmi_split_means: the batch pointer is not NULL)
+  bool is_piece;  // a unit with a row limit
+  bool ran;
+  uint32_t sites, rows;
+};
+
+// The pieces, in row order, must be the suffixes [row, S) of the unit with row limits that cover its rows; slice[p] is
+// the length of piece p's MI slice.
+static int split_check(lgmi_ctx* ctx, const char* fn, uint32_t S, const std::vector<SplitPiece>& pieces,
+                       std::vector<uint64_t>* slice) {
+  slice->assign(pieces.size(), 0);
   uint64_t row = 0, total = 0;  // piece p: the suffix [row, S) with its row limit
-  for (uint32_t p = 0; p < n_pieces; ++p) {
-    lgmi_batch* b = batches[p];
-    if (!b) return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: piece %u is NULL", p);
-    const uint32_t k = unit_in_batch[p];
-    if (k >= b->n_units || b->h_row_limit.empty() || !b->h_row_limit[k])
-      return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: piece %u is not a unit with a row limit", p);
-    if (!b->ran) return fail(ctx, LGMI_ERR_STATE, "lgmi_split_means: piece %u has not been run", p);
-    const uint32_t Sp = b->h_units[k].n_sites, rows = b->h_row_limit[k];
-    if (row >= S || (uint64_t)Sp != S - row)
-      return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: piece %u (%u sites) is not the suffix of sites [%llu, %u)", p, Sp,
+  for (uint32_t p = 0; p < (uint32_t)pieces.size(); ++p) {
+    const SplitPiece& v = pieces[p];
+    if (!v.present) return fail(ctx, LGMI_ERR_ARG, "%s: piece %u is NULL", fn, p);
+    if (!v.is_piece) return fail(ctx, LGMI_ERR_ARG, "%s: piece %u is not a unit with a row limit", fn, p);
+    if (!v.ran) return fail(ctx, LGMI_ERR_STATE, "%s: piece %u has not been run", fn, p);
+    if (row >= S || (uint64_t)v.sites != S - row)
+      return fail(ctx, LGMI_ERR_ARG, "%s: piece %u (%u sites) is not the suffix of sites [%llu, %u)", fn, p, v.sites,
                   (unsigned long long)row, S);
-    slice[p] = piece_pairs(rows, Sp);
-    total += slice[p];
-    row += rows;
+    (*slice)[p] = piece_pairs(v.rows, v.sites);
+    total += (*slice)[p];
+    row += v.rows;
   }
   const uint64_t np = (uint64_t)S * (S - (S ? 1u : 0u)) / 2;
   if (row != S || total != np)
-    return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: the pieces cover %llu of %llu rows (%llu of %llu pairs)",
+    return fail(ctx, LGMI_ERR_ARG, "%s: the pieces cover %llu of %llu rows (%llu of %llu pairs)", fn,
                 (unsigned long long)row, (unsigned long long)S, (unsigned long long)total, (unsigned long long)np);
-  if (!S) return LGMI_OK;
+  return LGMI_OK;
+}
+
+// Where a piece's MI slice is read from: `src` on `device`, once `after` (if any) has completed.
+struct SliceSource {
+  int device;
+  const double* src;
+  cudaEvent_t after;
+};
+
+// The slices back to back in the context's scratch, then the unsplit run's per-site pass over them (S > 0).
+static int split_gather_means(lgmi_ctx* ctx, uint32_t S, const uint8_t* site_flags, const std::vector<uint64_t>& slice,
+                              const std::vector<SliceSource>& from, double* mean_out, uint32_t* cnt_out) {
+  const uint64_t np = (uint64_t)S * (S - 1u) / 2;
   // scratch: dense [np] | mean [S] | cnt [S] | flags [S] | unit | mean items
   auto up16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
   const uint32_t n_items = (S + (uint32_t)kMeanSites - 1u) / (uint32_t)kMeanSites;
   const size_t o_mean = up16(np * sizeof(double)), o_cnt = o_mean + up16((size_t)S * sizeof(double));
   const size_t o_flags = o_cnt + up16((size_t)S * sizeof(uint32_t)), o_unit = o_flags + up16(S);
   const size_t o_items = o_unit + up16(sizeof(DevUnit)), bytes = o_items + n_items * sizeof(MeanItem);
-  for (uint32_t p = 0; p < n_pieces; ++p) {  // the pieces' kernels have finished (they may run on other devices)
-    CU(ctx, cudaSetDevice(batches[p]->ctx->device));
-    CU(ctx, cudaStreamSynchronize(bstream(batches[p])));
-  }
   CU(ctx, cudaSetDevice(ctx->device));
   int rc = ensure_scratch(ctx, bytes);
   if (rc) return rc;
   char* scratch = ctx->d_scratch.get();
   uint64_t at = 0;
-  for (uint32_t p = 0; p < n_pieces; ++p) {
-    const lgmi_batch* b = batches[p];
-    if (slice[p])
-      CU(ctx, cudaMemcpyPeerAsync(scratch + at * sizeof(double), ctx->device, b->d_dense + b->h_dense_off[unit_in_batch[p]],
-                                  b->ctx->device, slice[p] * sizeof(double), ctx->stream));
+  for (size_t p = 0; p < slice.size(); ++p) {
+    if (slice[p]) {
+      if (from[p].after) CU(ctx, cudaStreamWaitEvent(ctx->stream, from[p].after, 0));
+      CU(ctx, cudaMemcpyPeerAsync(scratch + at * sizeof(double), ctx->device, from[p].src, from[p].device,
+                                  slice[p] * sizeof(double), ctx->stream));
+    }
     at += slice[p];
   }
   DevUnit u{};
@@ -1066,6 +1242,86 @@ extern "C" int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* si
   CU(ctx, cudaMemcpyAsync(cnt_out, scratch + o_cnt, (size_t)S * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
   return LGMI_OK;
+}
+
+extern "C" int lgmi_split_means(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site_flags, uint32_t n_pieces,
+                                lgmi_batch_t* const* batches, const uint32_t* unit_in_batch, double* mean_out,
+                                uint32_t* cnt_out) {
+  if (!ctx || !batches || !unit_in_batch || !n_pieces || (n_sites && (!site_flags || !mean_out || !cnt_out)))
+    return fail(ctx, LGMI_ERR_ARG, "lgmi_split_means: NULL argument");
+  std::vector<SplitPiece> pieces(n_pieces);
+  for (uint32_t p = 0; p < n_pieces; ++p) {
+    const lgmi_batch* b = batches[p];
+    const uint32_t k = unit_in_batch[p];
+    const bool is_piece = b && k < b->n_units && !b->h_row_limit.empty() && b->h_row_limit[k];
+    pieces[p] = SplitPiece{b != nullptr, is_piece, b && b->ran, is_piece ? b->h_units[k].n_sites : 0u,
+                           is_piece ? b->h_row_limit[k] : 0u};
+  }
+  std::vector<uint64_t> slice;
+  if (const int rc = split_check(ctx, "lgmi_split_means", n_sites, pieces, &slice)) return rc;
+  if (!n_sites) return LGMI_OK;
+  std::vector<SliceSource> from(n_pieces);
+  for (uint32_t p = 0; p < n_pieces; ++p) {  // the pieces' kernels have finished (they may run on other devices)
+    const lgmi_batch* b = batches[p];
+    CU(ctx, cudaSetDevice(b->ctx->device));
+    CU(ctx, cudaStreamSynchronize(bstream(b)));
+    from[p] = SliceSource{b->ctx->device, b->d_dense + b->h_dense_off[unit_in_batch[p]], nullptr};
+  }
+  return split_gather_means(ctx, n_sites, site_flags, slice, from, mean_out, cnt_out);
+}
+
+extern "C" int lgmi_split_means_ipc(lgmi_t* ctx, uint32_t n_sites, const uint8_t* site_flags, uint32_t n_pieces,
+                                    const lgmi_piece_ipc* pieces, double* mean_out, uint32_t* cnt_out) {
+  static const char fn[] = "lgmi_split_means_ipc";
+  if (!ctx || !pieces || !n_pieces || (n_sites && (!site_flags || !mean_out || !cnt_out)))
+    return fail(ctx, LGMI_ERR_ARG, "%s: NULL argument", fn);
+  std::vector<SplitPiece> view(n_pieces);
+  for (uint32_t p = 0; p < n_pieces; ++p) {
+    const lgmi_piece_ipc& x = pieces[p];
+    view[p] = SplitPiece{true, x.row_limit != 0u, x.ran != 0u, x.n_sites, x.row_limit};
+  }
+  std::vector<uint64_t> slice;
+  if (const int rc = split_check(ctx, fn, n_sites, view, &slice)) return rc;
+  for (uint32_t p = 0; p < n_pieces; ++p)
+    if (pieces[p].dense_pairs != slice[p])
+      return fail(ctx, LGMI_ERR_ARG, "%s: piece %u carries %llu MI values for %llu pairs", fn, p,
+                  (unsigned long long)pieces[p].dense_pairs, (unsigned long long)slice[p]);
+  if (!n_sites) return LGMI_OK;
+  IpcImports imports;  // closed when this returns, after the guard below has waited for the copies that read them
+  struct Drain {
+    lgmi_ctx* ctx;
+    ~Drain() {
+      cudaSetDevice(ctx->device);
+      cudaStreamSynchronize(ctx->stream);
+    }
+  } drain{ctx};
+  const int32_t self = (int32_t)getpid();
+  std::vector<SliceSource> from(n_pieces);
+  for (uint32_t p = 0; p < n_pieces; ++p) {
+    const lgmi_piece_ipc& x = pieces[p];
+    if (x.pid == self) {  // a batch of this process: read from it, as lgmi_split_means does
+      lgmi_batch* b = nullptr;
+      {
+        std::lock_guard<std::mutex> lock(g_export_mu);
+        const auto it = g_exported.find(x.batch_id);
+        if (it != g_exported.end()) b = it->second;
+      }
+      if (!b || x.unit >= b->n_units || b->h_row_limit.empty() || b->h_row_limit[x.unit] != x.row_limit)
+        return fail(ctx, LGMI_ERR_ARG, "%s: piece %u was exported by this process from a batch that no longer exists", fn, p);
+      CU(ctx, cudaSetDevice(b->ctx->device));
+      CU(ctx, cudaStreamSynchronize(bstream(b)));
+      from[p] = SliceSource{b->ctx->device, b->d_dense + x.dense_off, nullptr};
+    } else {  // another process's batch: through its handles, behind its event
+      int dev = 0;
+      if (const int rc = piece_device(ctx, fn, &x, &dev)) return rc;
+      void* base = nullptr;
+      cudaEvent_t ev = nullptr;
+      CU(ctx, imports.open_mem(x.dense_mem, dev, &base));
+      CU(ctx, imports.open_event(x.event, &ev));
+      from[p] = SliceSource{dev, static_cast<const double*>(base) + x.dense_off, ev};
+    }
+  }
+  return split_gather_means(ctx, n_sites, site_flags, slice, from, mean_out, cnt_out);
 }
 
 // --------------------------------------------------------------------------- pipelined step

@@ -11,7 +11,8 @@ no collective.  A unit whose cost alone exceeds a device's share is split by row
 grid into pieces on several devices (split_plan); its planes cross the host link once, in
 row ranges, and each piece fetches the rows it also needs from the other pieces' devices.
 `shard.py` is the same thing for one PROCESS per GPU (torch.distributed launches:
-bench.py --gpus N); it does not split units."""
+bench.py --gpus N); its local_run splits units the same way, the other processes' pieces reached
+through CUDA IPC handles."""
 from __future__ import annotations
 
 from concurrent.futures import ThreadPoolExecutor
@@ -185,6 +186,32 @@ def plan_pieces(units, n_dev):
     return shards, pieces, splits
 
 
+def piece_batch(ctx, pb: PlaneBatch, pieces):
+    """The batch of `pieces` [(unit, first row, end row)] of pb's units on ctx (api.Batch with row limits): each the
+    suffix unit of sites [a, S) of its unit, back to back, with row limit e - a.  Its planes are left empty: they come
+    from upload_piece_rows and from copies of the other pieces' rows."""
+    desc = np.zeros(len(pieces), dtype=pb.units.dtype)
+    flags = []
+    word = site = 0
+    for q, (u, a, _e) in enumerate(pieces):
+        g = pb.units[u]
+        S, W = int(g['n_sites']), int(g['row_words'])
+        desc[q] = (word, S - a, int(g['n_reads']), W, site)    # the suffix unit of sites [a, S)
+        flags.append(pb.site_flags[int(g['site_off']) + a:int(g['site_off']) + S])
+        word += 3 * (S - a) * W
+        site += S - a
+    # (np.empty: the batch only reads the planes' size; their words come from upload_rows / copies)
+    sub = PlaneBatch(desc, np.empty(word, dtype=np.uint32), np.concatenate(flags))
+    return api.Batch(ctx, sub, row_limit=[e - a for _u, a, e in pieces])
+
+
+def upload_piece_rows(batch, pb: PlaneBatch, pieces):
+    """Uploads each piece's own rows [a, e) of pb's planes (and the flags) to its place in piece_batch's batch."""
+    for q, (u, a, e) in enumerate(pieces):
+        W, base = int(pb.units['row_words'][u]), int(pb.units['plane_off'][u])
+        batch.upload_rows(int(batch.pb.units['plane_off'][q]), pb.planes[base + 3 * a * W:base + 3 * e * W])
+
+
 class DevicePool:
     """Contexts on `devices` (default: every visible GPU), owned by the calling process."""
 
@@ -274,32 +301,15 @@ class DevicePool:
         """One batch of pieces per device (None where there is none), planes in place: each piece's own rows
         uploaded from the host, the rows after them copied from the devices of the later pieces of its unit."""
         n_dev = len(self.devices)
-        batches = [None] * n_dev
+        batches = [piece_batch(self.contexts[k], pb, pieces[k]) if pieces[k] else None for k in range(n_dev)]
         rows_at = {}   # (unit, first row) -> (device, first plane word of the piece there, end row)
         for k in range(n_dev):
-            if not pieces[k]:
-                continue
-            desc = np.zeros(len(pieces[k]), dtype=pb.units.dtype)
-            flags = []
-            word = site = 0
             for q, (u, a, e) in enumerate(pieces[k]):
-                g = pb.units[u]
-                S, W = int(g['n_sites']), int(g['row_words'])
-                desc[q] = (word, S - a, int(g['n_reads']), W, site)    # the suffix unit of sites [a, S)
-                flags.append(pb.site_flags[int(g['site_off']) + a:int(g['site_off']) + S])
-                rows_at[(u, a)] = (k, word, e)
-                word += 3 * (S - a) * W
-                site += S - a
-            # (np.empty: the batch only reads the planes' size; their words come from upload_rows / copies)
-            sub = PlaneBatch(desc, np.empty(word, dtype=np.uint32), np.concatenate(flags))
-            batches[k] = api.Batch(self.contexts[k], sub, row_limit=[e - a for _u, a, e in pieces[k]])
+                rows_at[(u, a)] = (k, int(batches[k].pb.units['plane_off'][q]), e)
         try:
-            def upload(k):   # the host link once: every piece uploads its own rows, one thread per device
-                for q, (u, a, e) in enumerate(pieces[k]):
-                    W, base = int(pb.units['row_words'][u]), int(pb.units['plane_off'][u])
-                    batches[k].upload_rows(int(batches[k].pb.units['plane_off'][q]),
-                                           pb.planes[base + 3 * a * W:base + 3 * e * W])
-            list(self._threads.map(upload, [k for k in range(n_dev) if pieces[k]]))
+            # the host link once: every piece uploads its own rows, one thread per device
+            list(self._threads.map(lambda k: upload_piece_rows(batches[k], pb, pieces[k]),
+                                   [k for k in range(n_dev) if pieces[k]]))
             # then, from this thread, each piece's rows after its own from the pieces that uploaded them: a copy
             # waits on an event recorded behind the upload already queued on the source's stream
             for k in range(n_dev):

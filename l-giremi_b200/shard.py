@@ -5,6 +5,13 @@ cross-unit step is the global ECDF / mip pass (giremi.py:415-429), which needs
 every site's mean MI in one place: per-rank results are gathered to rank 0 and
 put back into the reference's row order (unit -> pair).
 
+local_run also splits a unit too deep for one GPU by rows of its pair grid, as
+multigpu.DevicePool does in one process (multigpu.plan_pieces, the same plan on
+every rank).  A piece reads the plane rows of the later pieces from the other
+processes' devices, and the first piece's owner gathers every piece's MI slice
+for the per-site pass, both through CUDA IPC handles (Batch.export_piece); only
+those handles, a few hundred bytes, travel through object collectives.
+
 torch.distributed is plumbing here (gather of result buffers); it works with
 the "nccl" backend (device tensors) and with "gloo" (host tensors, used by the
 CPU tests)."""
@@ -12,10 +19,13 @@ from __future__ import annotations
 
 import numpy as np
 
-from ._lib import PAIR_REC
+import time
+
+from . import api
+from ._lib import PAIR_REC, PieceIpc
 from .api import partition_lpt, unit_costs
 from .encode import PlaneBatch
-from .multigpu import MergedResult, merge_shards  # noqa: F401  (MergedResult: rank 0's view after the gather)
+from .multigpu import MergedResult, merge_shards, piece_batch, plan_pieces, upload_piece_rows  # noqa: F401
 
 
 def plan(units, world_size):
@@ -80,3 +90,158 @@ def gather_to_rank0(pb_global: PlaneBatch, local_result, local_index, group=None
                       gathered[2][r].view(np.uint32), off, None))
     # ranks hold ascending global indices and emit in (unit, i, j) order: the merge is index bookkeeping
     return merge_shards(pb_global.units, pb_global.n_sites, parts)
+
+
+class LocalRun:
+    """One rank's share of a split-aware step (local_run): `result` (api.StepResult, or None when the rank has no
+    ordinary unit) of its ordinary units `index` (global, ascending); `pieces` [(unit, first row, end row, records,
+    counts | None)] of split units it ran, records numbered as in the piece (i, j from its first row); `means`
+    {unit: (site_mean, site_cnt)} of the split units whose first piece it holds.  Host times in ms: `shard_ms` of
+    the ordinary units, `pieces_ms` of the piece batch from creation to results on the host (copies included),
+    `split_means_ms` of the per-site passes; `piece_kernel_ms` is the piece batch's device time."""
+
+    def __init__(self, result, index, pieces=(), means=None, shard_ms=0.0, pieces_ms=0.0, piece_kernel_ms=None,
+                 split_means_ms=0.0):
+        self.result, self.index = result, np.asarray(index, dtype=np.int64)
+        self.pieces, self.means = list(pieces), dict(means or {})
+        self.shard_ms, self.pieces_ms, self.piece_kernel_ms = shard_ms, pieces_ms, piece_kernel_ms
+        self.split_means_ms = split_means_ms
+
+
+def local_run(pb_global: PlaneBatch, rank, world, min_common, mode, ctx, group=None) -> LocalRun:
+    """The step of `rank`'s share of pb_global on ctx, with deep units split over the ranks (plan_pieces, the same on
+    every rank: nothing is exchanged to plan).  With no unit split it is local_shard + one mi_step_batched and makes
+    no collective call.  Otherwise every rank of `group` must call it with the same arguments but its own rank and
+    context: each builds the batch of its pieces and uploads their own rows, takes the rows after them from the
+    ranks holding the later pieces (CUDA IPC: the handles go through all_gather_object), runs, and the owner of a
+    unit's first piece computes its per-site means from every piece's MI slice.  No rank closes its piece batch
+    before all are done with it (barrier)."""
+    shards, pieces, splits = plan_pieces(pb_global.units, world)
+    index = shards[rank]
+    t0 = time.perf_counter()
+    result = api.mi_step_batched(pb_global.subset(index), min_common, mode, ctx=ctx) if len(index) or not splits \
+        else None
+    run = LocalRun(result, index, shard_ms=1e3 * (time.perf_counter() - t0))
+    if not splits:
+        return run
+    import torch.distributed as dist
+    mine = pieces[rank]
+    t0 = time.perf_counter()
+    batch = piece_batch(ctx, pb_global, mine) if mine else None
+    try:
+        if batch is not None:
+            upload_piece_rows(batch, pb_global, mine)
+        # every piece of every rank: (rank, position in its batch, unit, first row, end row, exported bytes)
+        everyone = _all_pieces(batch, mine, rank, world, group)
+        for q, (u, a, e) in enumerate(mine):
+            W = int(pb_global.units['row_words'][u])
+            dst0 = int(batch.pb.units['plane_off'][q])
+            for k, qs, v, c, ce, piece in everyone:
+                if v != u or c < e:
+                    continue
+                if k == rank:
+                    batch.copy_planes_from(dst0 + 3 * (c - a) * W, batch, int(batch.pb.units['plane_off'][qs]),
+                                           3 * (ce - c) * W)
+                else:
+                    src = PieceIpc.from_buffer_copy(piece)
+                    batch.copy_planes_from_ipc(dst0 + 3 * (c - a) * W, piece, src.plane_word, src.plane_words)
+        if batch is not None:
+            batch.run(min_common, mode)
+            res = batch.download(copy=True)
+            run.piece_kernel_ms = res.kernel_ms
+            run.pieces = [(u, a, e, res.unit_records(q), res.unit_counts(q) if res.counts is not None else None)
+                          for q, (u, a, e) in enumerate(mine)]
+        run.pieces_ms = 1e3 * (time.perf_counter() - t0)
+        everyone = _all_pieces(batch, mine, rank, world, group)         # exported again, after the run
+        t0 = time.perf_counter()
+        for u in splits:
+            row_order = sorted((c, k, piece) for k, _q, v, c, _ce, piece in everyone if v == u)
+            if row_order[0][1] != rank:
+                continue
+            S, off = int(pb_global.units['n_sites'][u]), int(pb_global.units['site_off'][u])
+            run.means[u] = api.split_means_ipc(ctx, pb_global.site_flags[off:off + S], [p for _c, _k, p in row_order])
+        run.split_means_ms = 1e3 * (time.perf_counter() - t0)
+        dist.barrier(group=group)            # every import from this rank's batch is done
+    finally:
+        if batch is not None:
+            batch.close()
+    return run
+
+
+def _all_pieces(batch, mine, rank, world, group):
+    """Every rank's pieces with their export_piece bytes, recorded behind all the batch has queued so far."""
+    import torch.distributed as dist
+    local = [(rank, q, u, a, e, batch.export_piece(q)) for q, (u, a, e) in enumerate(mine)]
+    out = [None] * world
+    dist.all_gather_object(out, local, group=group)
+    return [x for part in out for x in part]
+
+
+def gather_run_to_rank0(pb_global: PlaneBatch, run: LocalRun, group=None, device="cpu"):
+    """gather_to_rank0 for local_run: every rank's ordinary shard (with its 3x3 tables under EMIT_COUNTS), its
+    pieces' records and tables and its split units' means reach rank 0, which merges them (merge_shards with the
+    split units placed) into the result of one process's step over pb_global.  Only rank 0 gets a MergedResult;
+    its split_units maps each split unit to [(rank, first row, end row)] of its pieces."""
+    import torch.distributed as dist
+    rank = dist.get_rank(group)
+    world = dist.get_world_size(group)
+    r = run.result
+    n_local = len(run.index)
+
+    def raw(a, dtype):
+        return np.ascontiguousarray(a, dtype=dtype).view(np.uint8).reshape(-1)
+
+    if r is None:
+        shard = [np.empty(0, PAIR_REC), np.empty(0), np.empty(0, np.uint32), np.zeros(n_local + 1, np.uint64), None]
+    else:
+        shard = [r.records, r.site_mean, r.site_cnt, r.unit_rec_off, r.counts]
+    pieces = run.pieces
+    piece_rec = np.concatenate([p[3] for p in pieces]) if pieces else np.empty(0, PAIR_REC)
+    with_counts = [p for p in pieces if p[4] is not None]
+    piece_cnt = np.concatenate([np.asarray(p[4]).reshape(-1, 9) for p in with_counts]) if with_counts \
+        else np.empty((0, 9), np.uint32)
+    units = sorted(run.means)
+    means = np.concatenate([run.means[u][0] for u in units]) if units else np.empty(0)
+    cnts = np.concatenate([run.means[u][1] for u in units]) if units else np.empty(0, np.uint32)
+    payloads = [raw(shard[0], PAIR_REC), raw(shard[1], np.float64), raw(shard[2], np.uint32),
+                raw(shard[3], np.uint64), raw(run.index, np.int64),
+                raw(shard[4] if shard[4] is not None else np.empty((0, 9)), np.uint32),
+                raw(piece_rec, PAIR_REC), raw(piece_cnt, np.uint32), raw(means, np.float64), raw(cnts, np.uint32)]
+    gathered = [_gather_bytes(p, 0, group, device) for p in payloads]
+    # what the byte buffers hold: per piece (unit, first row, end row, rows, tables shipped); the means' units
+    meta = ([(int(u), int(a), int(e), len(rec), c is not None) for u, a, e, rec, c in pieces],
+            units, shard[4] is not None)
+    metas = [None] * world if rank == 0 else None
+    dist.gather_object(meta, metas, dst=0, group=group)
+    if rank != 0:
+        return None
+    parts, split_pieces, split_means = [], {}, {}
+    for k in range(world):
+        index = gathered[4][k].view(np.int64)
+        if len(index):
+            off = gathered[3][k].view(np.uint64)
+            counts = gathered[5][k].view(np.uint32).reshape(-1, 9) if metas[k][2] else None
+            parts.append((index, gathered[0][k].view(PAIR_REC), gathered[1][k].view(np.float64),
+                          gathered[2][k].view(np.uint32), off, counts))
+        rec, tab = gathered[6][k].view(PAIR_REC), gathered[7][k].view(np.uint32).reshape(-1, 9)
+        at = tab_at = 0
+        for u, a, e, n, has_counts in metas[k][0]:
+            c = None
+            if has_counts:
+                c, tab_at = tab[tab_at:tab_at + n], tab_at + n
+            split_pieces.setdefault(u, []).append((a, e, k, rec[at:at + n], c))
+            at += n
+        mean, cnt = gathered[8][k].view(np.float64), gathered[9][k].view(np.uint32)
+        at = 0
+        for u in metas[k][1]:
+            S = int(pb_global.units['n_sites'][u])
+            split_means[u] = (mean[at:at + S], cnt[at:at + S])
+            at += S
+    split = []
+    for u in sorted(split_pieces):
+        ps = sorted(split_pieces[u], key=lambda p: p[0])
+        split.append((u, [(a, rec, c) for a, _e, _k, rec, c in ps]) + split_means[u])
+    merged = merge_shards(pb_global.units, pb_global.n_sites, parts, split)
+    merged.split_units = {u: [(k, a, e) for a, e, k, _r, _c in sorted(split_pieces[u], key=lambda p: p[0])]
+                          for u in split_pieces}
+    return merged
