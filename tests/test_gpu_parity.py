@@ -19,66 +19,12 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import c_oracle  # noqa: E402
 from fuzz import random_mismatches  # noqa: E402
+from parity import _other_heavy_unit, _synth_unit, check_batch, oracle_unit, signed  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
 synth = importlib.import_module("l-giremi_b200.synth")
 enc = importlib.import_module("l-giremi_b200.encode")
-
-
-def signed(labels):
-    out = labels.astype(np.int16)
-    out[out == 255] = -1
-    return out.astype(np.int8)
-
-
-def oracle_unit(eu, min_common):
-    """Oracle on an EncodedUnit: (i, j, mi, tables, mean, cnt)."""
-    S = eu.n_sites
-    if S < 2:
-        z = np.zeros(0, np.int32)
-        return z, z, np.zeros(0), np.zeros((0, 9), np.int64), np.full(S, np.nan), np.zeros(S, np.int32)
-    i, j, mi, tab = c_oracle.unit_pairs_from_labels(signed(eu.labels), None, min_common)
-    is_het = np.array([t == 'het_snp' for t in eu.types], dtype=np.uint8)
-    mean, cnt = c_oracle.site_means(S, is_het, i, j, mi)
-    return i, j, mi, tab, mean, cnt
-
-
-def check_batch(lg, ctx, eus, min_common, min_exact=0.97):
-    """Runs one batch in ALL_PAIRS|EMIT_COUNTS and HET_ONLY modes and checks
-    every output against the oracle."""
-    pb = lg.pack_units(eus)
-    full = lg.mi_step_batched(pb, min_common, lg.MODE_ALL_PAIRS | lg.MODE_EMIT_COUNTS, ctx=ctx)
-    het = lg.mi_step_batched(pb, min_common, lg.MODE_HET_ONLY, ctx=ctx)
-    skip = lg.mi_step_batched(pb, min_common, lg.MODE_HET_ONLY | lg.MODE_SKIP_NONHET, ctx=ctx)
-    assert full.n_candidates == pb.n_candidates == het.n_candidates
-    assert full.unit_rec_off[0] == 0 and full.unit_rec_off[-1] == full.n_records
-    got_mi, want_mi, got_mean, want_mean = [], [], [], []
-    for u, eu in enumerate(eus):
-        i, j, mi, tab, mean, cnt = oracle_unit(eu, min_common)
-        rec = full.unit_records(u)
-        assert np.all(rec['unit'] == u)
-        assert rec['i'].tolist() == i.tolist() and rec['j'].tolist() == j.tolist(), "pair set of unit %d" % u
-        assert np.array_equal(full.unit_counts(u).astype(np.int64), tab), "3x3 counts of unit %d" % u
-        got_mi.append(rec['mi'])
-        want_mi.append(mi)
-        is_het = np.array([t == 'het_snp' for t in eu.types], dtype=bool)
-        keep = is_het[i] | is_het[j] if len(i) else np.zeros(0, bool)
-        for res in (het, skip):
-            hrec = res.unit_records(u)
-            assert hrec['i'].tolist() == i[keep].tolist() and hrec['j'].tolist() == j[keep].tolist()
-            assert np.array_equal(hrec['mi'], rec['mi'][keep])          # same bits in every mode
-        off = int(pb.units['site_off'][u])
-        for res in (full, het, skip):
-            assert res.site_cnt[off:off + eu.n_sites].tolist() == cnt.tolist()
-            assert np.array_equal(res.site_mean[off:off + eu.n_sites], full.site_mean[off:off + eu.n_sites],
-                                  equal_nan=True)
-        got_mean.append(full.site_mean[off:off + eu.n_sites])
-        want_mean.append(mean)
-    cat = lambda v: np.concatenate(v) if v else np.zeros(0)
-    assert_mi_close(cat(got_mi), cat(want_mi), min_exact, "pair MI")
-    assert_mi_close(cat(got_mean), cat(want_mean), min_exact, "mean MI")
-    return full
 
 
 # --------------------------------------------------------------------------- drop-in functions
@@ -258,10 +204,11 @@ def test_many_sites_multi_item_unit(lg, gpu_ctx):
 def test_mid_units_popcount_and_tensor_paths_agree(lg, gpu_ctx):
     """Mid-depth units (more than 64 sites or 256 reads): k_tile_gram_ws + k_tile_finish (tcgen05, the default) and
     k_tile_mi (popcount, path 0) must give the same records, tables and means bit for bit, and both match the oracle.
-    Shapes straddle the 128-site row blocks, the 48-site column blocks and the 128-read k-blocks."""
+    Shapes straddle the 128-site row blocks, the 48-site column blocks and the 128-read k-blocks; (47, 9000) is the
+    deepest unit below the default dense threshold (48 sites x 8192 reads)."""
     rng = np.random.default_rng(20261031)
     shapes = [(65, 40), (48, 257), (49, 300), (129, 129), (97, 1000), (2, 700), (3, 4097), (257, 70), (200, 385),
-              (145, 128), (64, 9000)]
+              (145, 128), (47, 9000)]
     eus = [_synth_unit(rng, S, R, cov) for (S, R), cov in zip(shapes, [0.5, 0.3, 0.7, 0.5, 0.2, 1.0, 0.6, 0.4, 0.5, 0.9, 0.3])]
     eus.insert(3, enc.EncodedUnit([1, 2, 3], ['het_snp', 'mismatch', 'snp'], eus[0].labels[:3, :30]))   # a small unit between
     pb = lg.pack_units(eus)
@@ -270,6 +217,7 @@ def test_mid_units_popcount_and_tensor_paths_agree(lg, gpu_ctx):
         for path in (2, 0):
             gpu_ctx.set_tile_path(path)
             full = check_batch(lg, gpu_ctx, eus, 6, min_exact=0.9)
+            assert full.n_dense_units == 0
             het = lg.mi_step_batched(pb, 9, lg.MODE_HET_ONLY | lg.MODE_SKIP_NONHET | lg.MODE_EMIT_COUNTS, ctx=gpu_ctx)
             out[path] = (full, het)
     finally:
@@ -281,12 +229,6 @@ def test_mid_units_popcount_and_tensor_paths_agree(lg, gpu_ctx):
 
 
 # --------------------------------------------------------------------------- tensor-core path (K3)
-def _synth_unit(rng, S, R, cov):
-    a, k = synth.draw_alleles(rng, 1, S, R, cov)
-    return enc.EncodedUnit([1000 + 37 * s for s in range(S)],
-                           [("mismatch", "snp", "het_snp")[int(x)] for x in k[0]], synth.labels_from_alleles(a[0]))
-
-
 @pytest.fixture()
 def dense_everything(lg, gpu_ctx):
     """Every unit with a pair goes through k_dense_x + k_gram_i8."""
@@ -313,16 +255,6 @@ def test_dense_path_small_shapes(lg, dense_everything):
     assert popc.n_dense_units == 0
     assert np.array_equal(dense.records, popc.records) and np.array_equal(dense.counts, popc.counts)
     assert np.array_equal(dense.site_mean, popc.site_mean, equal_nan=True)
-
-
-def _other_heavy_unit(rng, S, R, cov, third):
-    """Like _synth_unit with a chosen rate of third alleles (label "other")."""
-    a, k = synth.draw_alleles(rng, 1, S, R, cov)
-    al = a[0]
-    extra = (rng.random(al.shape) < third) & (al != synth.NOCOV)
-    al[extra] = synth.THIRD
-    return enc.EncodedUnit([1000 + 37 * s for s in range(S)],
-                           [("mismatch", "snp", "het_snp")[int(x)] for x in k[0]], synth.labels_from_alleles(al))
 
 
 @pytest.mark.parametrize("blocks", [4, 9])

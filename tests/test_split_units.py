@@ -15,6 +15,8 @@ enc = importlib.import_module("l-giremi_b200.encode")
 mg = importlib.import_module("l-giremi_b200.multigpu")
 synth = importlib.import_module("l-giremi_b200.synth")
 
+from parity import _check_split, _pieces  # noqa: E402
+
 
 def _descs(shapes):
     u = np.zeros(len(shapes), dtype=lg_mod.UNIT_DESC)
@@ -115,48 +117,7 @@ def _unit(rng, S, R, cov, third=0.0):
                            synth.labels_from_alleles(al))
 
 
-def _pieces(pb, bounds, unit=0):
-    """A PlaneBatch whose units are the pieces of pb's unit `unit` (suffix units into the same planes) + row limits."""
-    g = pb.units[unit]
-    W = int(g['row_words'])
-    desc = np.zeros(len(bounds) - 1, dtype=lg_mod.UNIT_DESC)
-    for q, a in enumerate(bounds[:-1]):
-        desc[q] = (int(g['plane_off']) + 3 * a * W, int(g['n_sites']) - a, int(g['n_reads']), W, int(g['site_off']) + a)
-    return enc.PlaneBatch(desc, pb.planes, pb.site_flags), [e - a for a, e in zip(bounds[:-1], bounds[1:])]
-
-
-def _joined(res, bounds):
-    rec = np.concatenate([res.unit_records(q).copy() for q in range(len(bounds) - 1)])
-    shift = np.concatenate([np.full(len(res.unit_records(q)), a) for q, a in enumerate(bounds[:-1])])
-    rec['i'] += shift.astype(np.uint16)
-    rec['j'] += shift.astype(np.uint16)
-    rec['unit'] = 0
-    return rec
-
-
 MODES = [api.MODE_HET_ONLY | api.MODE_SKIP_NONHET, api.MODE_HET_ONLY, api.MODE_ALL_PAIRS | api.MODE_EMIT_COUNTS]
-
-
-def _check_split(lg, ctx, pb, bounds, mode, mc=6):
-    whole = lg.mi_step_batched(pb, mc, mode, ctx=ctx, n_chunks=1)
-    sub, lim = _pieces(pb, bounds)
-    b = lg.Batch(ctx, sub, row_limit=lim)
-    try:
-        b.upload()
-        b.run(mc, mode)
-        got = b.download()
-        mean, cnt = lg.split_means(ctx, pb.site_flags, [(b, q) for q in range(len(lim))])
-    finally:
-        b.close()
-    rec = _joined(got, bounds)
-    assert np.array_equal(rec.view(np.uint8), whole.records.view(np.uint8))      # bit for bit, MI included
-    if mode & api.MODE_EMIT_COUNTS:
-        assert np.array_equal(got.counts, whole.counts)
-    assert got.n_candidates == whole.n_candidates and got.n_evaluated == whole.n_evaluated
-    assert np.isnan(got.site_mean).all() and not got.site_cnt.any()                # a piece's means would be partial
-    assert np.array_equal(mean.view(np.uint64), whole.site_mean.view(np.uint64))
-    assert np.array_equal(cnt, whole.site_cnt)
-    return whole
 
 
 BOUNDS = ([0, 128, 512, None], [0, 256, None], [0, None])
