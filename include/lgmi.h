@@ -415,6 +415,31 @@ LGMI_API int lgmi_ecdf_eval(lgmi_t* ctx, const double* x, uint64_t n, const doub
  * row (giremi.py:424-428), which must not cost a device round trip per row.    */
 LGMI_API int lgmi_ecdf_table(lgmi_t* ctx, const double* x, uint64_t n, double* sorted_out, double* y_out);
 
+/* ----- site x splice-site MI: calculate_site_splice_mi.py:106-125 ---------- *
+ * The reference's second mutual_info_score call site, for the requested       *
+ * (site, allele, splice site) triples only.  Synchronous.                     *
+ *   entries  site s owns entries [entry_off[s], entry_off[s+1]): one per list *
+ *            entry of the site (a read listed twice counts twice), its read   *
+ *            entry_read[p] < n_reads and the index entry_allele[p] of the     *
+ *            allele list it comes from, numbered within the site.  At most   *
+ *            64 distinct alleles per site (index >= 64: UNSUPPORTED).         *
+ *   splices  read r has splice sites splice_id[splice_off[r] ..              *
+ *            splice_off[r+1]), ascending and unique (membership is a set).    *
+ *   triples  tri_site[t] < n_sites, tri_allele[t] (an allele index of the     *
+ *            site), tri_splice[t] (any id; one no read has gives 0.0).        *
+ * Over the N entries of the site: x entries whose read is in the allele's     *
+ * list at the site (by read, :121), y whose read has the splice site (:122),  *
+ * xy both.  table_out (optional, 4 per triple) receives [N-x-y+xy, y-xy,      *
+ * x-xy, xy] (rows "with seq", columns "with splice"), mi_out[t] its MI (:123; *
+ * 0.0 for one class).  LGMI_ERR_ARG for a NULL array, an offset array that   *
+ * does not start at 0 or decreases, an id out of range or splice ids out of   *
+ * order.                                                                      */
+LGMI_API int lgmi_site_splice_mi(lgmi_t* ctx, uint32_t n_sites, const uint64_t* entry_off,
+                                 const uint32_t* entry_read, const uint32_t* entry_allele, uint32_t n_reads,
+                                 const uint64_t* splice_off, const uint32_t* splice_id, uint64_t n_triples,
+                                 const uint32_t* tri_site, const uint32_t* tri_allele, const uint32_t* tri_splice,
+                                 double* mi_out, uint32_t* table_out);
+
 /* ----- host-side native pieces either side of the step (no device needed) --- *
  * One read's short-form cs tag (minimap2 --cs): its substitutions in contig    *
  * coordinates (0-based) with the splice-distance filter applied, and its       *

@@ -50,7 +50,7 @@ EXPORTS = (
     "lgmi_pipeline_begin", "lgmi_pipeline_begin_packed", "lgmi_pipeline_collect", "lgmi_pipeline_finish",
     "lgmi_pipeline_destroy",
     "lgmi_submit", "lgmi_wait", "lgmi_site_mean_csr",
-    "lgmi_ecdf", "lgmi_ecdf_eval", "lgmi_ecdf_table", "lgmi_device_count", "lgmi_cs_scan", "lgmi_encode_unit", "lgmi_unit_cost", "lgmi_partition_lpt",
+    "lgmi_ecdf", "lgmi_ecdf_eval", "lgmi_ecdf_table", "lgmi_site_splice_mi", "lgmi_device_count", "lgmi_cs_scan", "lgmi_encode_unit", "lgmi_unit_cost", "lgmi_partition_lpt",
 )
 
 
@@ -161,6 +161,7 @@ def load():
         "lgmi_ecdf": (i32, [vp, vp, vp, u64, C.c_double, vp, vp]),
         "lgmi_ecdf_eval": (i32, [vp, vp, u64, vp, u64, vp]),
         "lgmi_ecdf_table": (i32, [vp, vp, u64, vp, vp]),
+        "lgmi_site_splice_mi": (i32, [vp, u32, vp, vp, vp, u32, vp, vp, u64, vp, vp, vp, vp, vp]),
         "lgmi_device_count": (i32, []),
         "lgmi_cs_scan": (i32, [C.c_char_p, u64, C.c_int64, i32, u32, vp, vp, vp, C.POINTER(u32), u32, vp, vp,
                                C.POINTER(u32)]),

@@ -20,7 +20,7 @@ from . import _lib
 from ._lib import (MODE_ALL_PAIRS, MODE_COMPACT_OUTPUT, MODE_EMIT_COUNTS, MODE_HET_ONLY, MODE_GRAPH, MODE_SKIP_NONHET,
                    MODE_SPLIT_RECORDS, MODE_TIGHT_INPUT,
                    PAIR_REC, SITE_TYPE_CODE, LgmiError, Result, array_at, check, ptr)
-from .encode import EncodedUnit, PlaneBatch, encode_batch, encode_mismatches, pack_units
+from .encode import PlaneBatch, encode_batch, encode_mismatches, pack_units
 
 
 class Context:
@@ -570,46 +570,117 @@ def mip_and_calls(mean_mi, site_types, threshold=0.05, ctx=None):
 # --------------------------------------------------------------------------- #
 # site x splice-site MI: the reference's second mutual_info_score call site
 # --------------------------------------------------------------------------- #
+class SiteSpliceArrays:
+    """Input of lgmi_site_splice_mi (include/lgmi.h), plus the names its integer ids stand for.
+
+    entries  site k owns entries [entry_off[k], entry_off[k+1]): read entry_read[p], allele index entry_allele[p]
+             (within the site); one per list entry, so a read listed twice is there twice
+    splices  read r has the splice ids splice_id[splice_off[r] .. splice_off[r+1]), ascending and unique
+    triples  (tri_site, tri_allele, tri_splice), one per requested pair, in order
+    names    read_names[r], site_labels[k], allele_names[k][a], splice_labels[id]"""
+
+    def __init__(self, entry_off, entry_read, entry_allele, splice_off, splice_id, tri_site, tri_allele, tri_splice,
+                 read_names, site_labels, allele_names, splice_labels):
+        u32 = lambda a: np.ascontiguousarray(a, dtype=np.uint32)
+        self.entry_off = np.ascontiguousarray(entry_off, dtype=np.uint64)
+        self.entry_read, self.entry_allele = u32(entry_read), u32(entry_allele)
+        self.splice_off = np.ascontiguousarray(splice_off, dtype=np.uint64)
+        self.splice_id = u32(splice_id)
+        self.tri_site, self.tri_allele, self.tri_splice = u32(tri_site), u32(tri_allele), u32(tri_splice)
+        self.read_names, self.site_labels = read_names, site_labels
+        self.allele_names, self.splice_labels = allele_names, splice_labels
+
+    @property
+    def n_sites(self):
+        return self.entry_off.size - 1
+
+    @property
+    def n_reads(self):
+        return self.splice_off.size - 1
+
+
+def read_splice_csr(read, splice, n_reads):
+    """(splice_off, splice_id) of records (read[k], splice[k]): per read its splice ids ascending, each once (the
+    reference's membership test is by set, calculate_site_splice_mi.py:122)."""
+    read = np.asarray(read, dtype=np.int64)
+    splice = np.asarray(splice, dtype=np.int64)
+    n_ids = int(splice.max()) + 1 if splice.size else 1
+    key = np.unique(read * n_ids + splice)
+    off = np.zeros(n_reads + 1, dtype=np.uint64)
+    off[1:] = np.cumsum(np.bincount(key // n_ids, minlength=n_reads))
+    return off, (key % n_ids).astype(np.uint32)
+
+
+def site_splice_mi_arrays(a: SiteSpliceArrays, ctx=None, tables=False):
+    """MI of every triple of `a` in one synchronous device call (lgmi_site_splice_mi); with tables=True also the
+    integer 2x2 tables [N-x-y+xy, y-xy, x-xy, xy] as an (n, 4) uint32 array."""
+    ctx = ctx or get_context()
+    n = a.tri_site.size
+    mi = np.empty(n, dtype=np.float64)
+    table = np.empty((n, 4), dtype=np.uint32) if tables else None
+    check(ctx._lib.lgmi_site_splice_mi(ctx.handle, a.n_sites, ptr(a.entry_off), ptr(a.entry_read),
+                                       ptr(a.entry_allele), a.n_reads, ptr(a.splice_off), ptr(a.splice_id), n,
+                                       ptr(a.tri_site), ptr(a.tri_allele), ptr(a.tri_splice), ptr(mi), ptr(table)),
+          ctx.handle)
+    return (mi, table) if tables else mi
+
+
+def site_splice_arrays(sites, splices, pairs) -> SiteSpliceArrays:
+    """The arrays of `site_splice_mutual_info`'s arguments: names interned once, lists flattened without a Python
+    step per entry.  Only the requested sites and splice sites are kept.  A missing site or allele raises KeyError,
+    as the reference's lookups do (calculate_site_splice_mi.py:116-117)."""
+    import itertools
+
+    import pandas as pd
+    site_labels = list(dict.fromkeys(p[0] for p in pairs))
+    site_of = {label: k for k, label in enumerate(site_labels)}
+    allele_names, lists, list_site, list_allele = [], [], [], []
+    for k, label in enumerate(site_labels):
+        alleles = sites[label]
+        allele_names.append(list(alleles))
+        for a, names in enumerate(alleles.values()):
+            lists.append(names)
+            list_site.append(k)
+            list_allele.append(a)
+    lens = np.fromiter(map(len, lists), dtype=np.int64, count=len(lists))
+    names = np.fromiter(itertools.chain.from_iterable(lists), dtype=object, count=int(lens.sum()))
+    entry_read, read_names = pd.factorize(names, use_na_sentinel=False)
+    entry_off = np.zeros(len(site_labels) + 1, dtype=np.uint64)
+    entry_off[1:] = np.cumsum(np.bincount(np.asarray(list_site, dtype=np.int64), weights=lens,
+                                          minlength=len(site_labels)).astype(np.int64))
+    entry_allele = np.repeat(np.asarray(list_allele, dtype=np.uint32), lens)
+    splice_labels = list(dict.fromkeys(p[2] for p in pairs))
+    slists = [splices.get(label, ()) for label in splice_labels]
+    slens = np.fromiter(map(len, slists), dtype=np.int64, count=len(slists))
+    snames = np.fromiter(itertools.chain.from_iterable(slists), dtype=object, count=int(slens.sum()))
+    sread = pd.Index(read_names).get_indexer(snames)
+    sid = np.repeat(np.arange(len(slists), dtype=np.int64), slens)
+    keep = sread >= 0                                   # reads listed at no requested site cannot count
+    splice_off, splice_id = read_splice_csr(sread[keep], sid[keep], len(read_names))
+    spl_of = {label: k for k, label in enumerate(splice_labels)}
+    allele_of = [{seq: a for a, seq in enumerate(names)} for names in allele_names]
+    tri_site = [site_of[p[0]] for p in pairs]
+    tri_allele = [allele_of[k][p[1]] for k, p in zip(tri_site, pairs)]
+    tri_splice = [spl_of[p[2]] for p in pairs]
+    return SiteSpliceArrays(entry_off, entry_read, entry_allele, splice_off, splice_id, tri_site, tri_allele,
+                            tri_splice, list(read_names), site_labels, allele_names, splice_labels)
+
+
 def site_splice_mutual_info(sites, splices, pairs, ctx=None):
-    """The loop of giremi/script/calculate_site_splice_mi.py:106-125 as ONE submit.
+    """The loop of giremi/script/calculate_site_splice_mi.py:106-125 as ONE device call.
 
     `sites`   {site label: {allele: [read names]}}      (:88-92)
     `splices` {splice label: [read names]}              (:95-102)
     `pairs`   iterable of (site label, allele, splice label)   (rows of the pair table)
 
-    Returns the MI of every pair, in order: over all list entries of the site's reads
-    (a read listed twice counts twice, :117-120), labels "carries the allele" x "has the
-    splice site" by read NAME (:121-122).  Each site becomes one unit whose pseudo-sites
-    are the requested alleles and splice sites; every pseudo-site covers every entry, the
-    "with" reads are its major plane, the others its minor plane, so the kernels' 2x2
-    table is the reference's (0/1 sort like minor/major)."""
+    Returns the MI of every pair, in order: over all list entries of the site (a read listed twice counts twice,
+    :117-120), labels "carries the allele" x "has the splice site" by read NAME (:121-122).  The 2x2 tables are
+    counted on the device from interned read ids for the requested pairs only (lgmi_site_splice_mi); at most 64
+    alleles per site."""
     pairs = [tuple(p) for p in pairs]
-    by_site = {}
-    for k, (site_label, seq, splice_label) in enumerate(pairs):
-        by_site.setdefault(site_label, []).append((k, seq, splice_label))
-    units, lookup = [], []                    # lookup[u] = [(pair index, i, j), ...]
-    for site_label, wanted in by_site.items():
-        alleles = sites[site_label]
-        entries = sorted(name for allele in alleles for name in alleles[allele])
-        seqs = list(dict.fromkeys(seq for _k, seq, _s in wanted))
-        spl = list(dict.fromkeys(s for _k, _seq, s in wanted))
-        members = [set(alleles[seq]) for seq in seqs] + [set(splices.get(s, ())) for s in spl]
-        labels = np.empty((len(members), len(entries)), dtype=np.uint8)
-        for row, names in enumerate(members):
-            labels[row] = [2 if name in names else 1 for name in entries]
-        units.append(EncodedUnit(list(range(len(members))), ['mismatch'] * len(members), labels))
-        lookup.append([(k, seqs.index(seq), len(seqs) + spl.index(s)) for k, seq, s in wanted])
-    out = [0.0] * len(pairs)
-    if not units:
-        return out
-    res = mi_step_batched(pack_units(units), 0, MODE_ALL_PAIRS, ctx=ctx)
-    for u, want in enumerate(lookup):
-        rec = res.unit_records(u)
-        S = units[u].n_sites
-        assert len(rec) == S * (S - 1) // 2   # min_common 0: every pair is there, in (i, j) order
-        for k, i, j in want:
-            out[k] = float(rec['mi'][i * (2 * S - i - 1) // 2 + (j - i - 1)])
-    return out
+    if not pairs:
+        return []
+    return site_splice_mi_arrays(site_splice_arrays(sites, splices, pairs), ctx=ctx).tolist()
 
 
 # --------------------------------------------------------------------------- #

@@ -28,6 +28,7 @@
 
 #include "../../include/lgmi.h"
 #include "lgmi_kernels.cuh"
+#include "lgmi_sitesplice.cuh"
 #include "lgmi_plan.h"
 #include "lgmi_pool.h"
 
@@ -1820,6 +1821,191 @@ extern "C" int lgmi_ecdf_table(lgmi_t* ctx, const double* x, uint64_t n, double*
   CU(ctx, cudaMemcpyAsync(sorted_out, d_sorted, n * 8, cudaMemcpyDeviceToHost, ctx->stream));
   CU(ctx, cudaMemcpyAsync(y_out, d_y, (n + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
+  return LGMI_OK;
+}
+
+// --------------------------------------------------------------------------- site x splice-site MI
+// Host side of lgmi_site_splice_mi: the triples grouped into columns (one per distinct (site, splice) of the
+// triples, ascending splice id within a site), each column's triples, and the work items of k_ss_count.
+namespace {
+struct SsPlan {
+  std::vector<uint32_t> slot_splice, slot_tri_off, tri_order;
+  std::vector<uint8_t> tri_allele;
+  std::vector<SsItem> items;
+  uint64_t max_n = 1;  // entries of the deepest requested site
+};
+}  // namespace
+
+static void ss_plan(uint32_t n_sites, const uint64_t* entry_off, uint64_t n_tri, const uint32_t* tri_site,
+                    const uint32_t* tri_allele, const uint32_t* tri_splice, SsPlan& P) {
+  P.tri_order.resize(n_tri);
+  for (uint64_t t = 0; t < n_tri; ++t) P.tri_order[t] = (uint32_t)t;
+  std::sort(P.tri_order.begin(), P.tri_order.end(), [&](uint32_t a, uint32_t b) {
+    if (tri_site[a] != tri_site[b]) return tri_site[a] < tri_site[b];
+    if (tri_splice[a] != tri_splice[b]) return tri_splice[a] < tri_splice[b];
+    return a < b;
+  });
+  P.tri_allele.resize(n_tri);
+  for (uint64_t t = 0; t < n_tri; ++t) P.tri_allele[t] = (uint8_t)tri_allele[t];
+  for (uint64_t k = 0; k < n_tri;) {  // one site's triples: [k, end)
+    const uint32_t s = tri_site[P.tri_order[k]];
+    const uint32_t slot0 = (uint32_t)P.slot_splice.size();
+    uint32_t rows = 0;
+    uint64_t end = k;
+    for (; end < n_tri && tri_site[P.tri_order[end]] == s; ++end) {
+      const uint32_t t = P.tri_order[end];
+      rows = std::max(rows, tri_allele[t] + 1u);
+      if (end == k || tri_splice[t] != P.slot_splice.back()) {
+        P.slot_splice.push_back(tri_splice[t]);
+        P.slot_tri_off.push_back((uint32_t)end);
+      }
+    }
+    const uint32_t n_slots = (uint32_t)P.slot_splice.size() - slot0;
+    const uint64_t lo = entry_off[s], n = entry_off[s + 1] - lo;
+    P.max_n = std::max(P.max_n, n);
+    for (uint32_t c = 0; c < n_slots; c += kSsTileCols)
+      for (uint64_t e = 0; e < n; e += kSsChunk)
+        P.items.push_back(SsItem{lo + e, (uint32_t)std::min<uint64_t>(kSsChunk, n - e), s, slot0 + c,
+                                 std::min(kSsTileCols, n_slots - c), rows, 0u});
+    k = end;
+  }
+  P.slot_tri_off.push_back((uint32_t)n_tri);
+}
+
+static uint32_t bits_for(uint64_t n) {  // bits of the largest value below n (at least 1)
+  uint32_t b = 1;
+  while (b < 64 && (n - 1) >> b) ++b;
+  return b;
+}
+
+extern "C" int lgmi_site_splice_mi(lgmi_t* ctx, uint32_t n_sites, const uint64_t* entry_off,
+                                   const uint32_t* entry_read, const uint32_t* entry_allele, uint32_t n_reads,
+                                   const uint64_t* splice_off, const uint32_t* splice_id, uint64_t n_triples,
+                                   const uint32_t* tri_site, const uint32_t* tri_allele, const uint32_t* tri_splice,
+                                   double* mi_out, uint32_t* table_out) {
+  static const char* me = "lgmi_site_splice_mi";
+  if (!ctx) return LGMI_ERR_ARG;
+  if (n_triples && (!tri_site || !tri_allele || !tri_splice || !mi_out))
+    return fail(ctx, LGMI_ERR_ARG, "%s: NULL triple or output array", me);
+  if (!entry_off || (n_reads && !splice_off)) return fail(ctx, LGMI_ERR_ARG, "%s: NULL offsets", me);
+  if (n_triples > 0xffffffffull) return fail(ctx, LGMI_ERR_UNSUPPORTED, "%s: more than 2^32-1 triples", me);
+  // the site entry CSR
+  if (entry_off[0] != 0) return fail(ctx, LGMI_ERR_ARG, "%s: entry_off[0] = %llu, not 0", me,
+                                     (unsigned long long)entry_off[0]);
+  for (uint32_t s = 0; s < n_sites; ++s)
+    if (entry_off[s + 1] < entry_off[s]) return fail(ctx, LGMI_ERR_ARG, "%s: entry_off decreases at site %u", me, s);
+  const uint64_t n_entries = entry_off[n_sites];
+  if (n_entries && (!entry_read || !entry_allele)) return fail(ctx, LGMI_ERR_ARG, "%s: NULL entry arrays", me);
+  if (n_entries > 0x7fffffffull)
+    return fail(ctx, LGMI_ERR_UNSUPPORTED, "%s: %llu entries, more than the radix sort takes (2^31-1)", me,
+                (unsigned long long)n_entries);
+  for (uint32_t s = 0; s < n_sites; ++s)
+    for (uint64_t p = entry_off[s]; p < entry_off[s + 1]; ++p) {
+      if (entry_read[p] >= n_reads)
+        return fail(ctx, LGMI_ERR_ARG, "%s: entry %llu names read %u of %u", me, (unsigned long long)p, entry_read[p],
+                    n_reads);
+      if (entry_allele[p] >= kSsMaxAlleles)
+        return fail(ctx, LGMI_ERR_UNSUPPORTED,
+                    "%s: site %u has allele index %u; at most 64 distinct alleles per site (the count pass keeps "
+                    "one bit per allele)", me, s, entry_allele[p]);
+    }
+  // the read splice CSR: ids ascending, each once
+  const uint64_t n_splice = n_reads ? splice_off[n_reads] : 0;
+  if (n_reads && splice_off[0] != 0) return fail(ctx, LGMI_ERR_ARG, "%s: splice_off[0] is not 0", me);
+  if (n_splice && !splice_id) return fail(ctx, LGMI_ERR_ARG, "%s: NULL splice_id", me);
+  for (uint32_t r = 0; r < n_reads; ++r) {
+    if (splice_off[r + 1] < splice_off[r]) return fail(ctx, LGMI_ERR_ARG, "%s: splice_off decreases at read %u", me, r);
+    for (uint64_t k = splice_off[r] + 1; k < splice_off[r + 1]; ++k)
+      if (splice_id[k] <= splice_id[k - 1])
+        return fail(ctx, LGMI_ERR_ARG, "%s: splice ids of read %u are not ascending and unique", me, r);
+  }
+  for (uint64_t t = 0; t < n_triples; ++t) {
+    if (tri_site[t] >= n_sites)
+      return fail(ctx, LGMI_ERR_ARG, "%s: triple %llu names site %u of %u", me, (unsigned long long)t, tri_site[t],
+                  n_sites);
+    if (tri_allele[t] >= kSsMaxAlleles)
+      return fail(ctx, LGMI_ERR_UNSUPPORTED, "%s: triple %llu asks for allele index %u; at most 64 per site", me,
+                  (unsigned long long)t, tri_allele[t]);
+  }
+  if (n_triples == 0) return LGMI_OK;
+  CU(ctx, cudaSetDevice(ctx->device));
+  SsPlan P;
+  ss_plan(n_sites, entry_off, n_triples, tri_site, tri_allele, tri_splice, P);
+  if (const int rc = ensure_lntab(ctx, P.max_n)) return rc;
+
+  const uint32_t read_bits = bits_for(std::max<uint32_t>(n_reads, 1u));
+  const uint32_t key_bits = read_bits + bits_for(std::max<uint32_t>(n_sites, 1u));
+  size_t sort_bytes = 0;
+  CU(ctx, cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const unsigned long long*)nullptr,
+                                          (unsigned long long*)nullptr, (const uint8_t*)nullptr, (uint8_t*)nullptr,
+                                          (int)n_entries, 0, (int)key_bits, ctx->stream));
+  MemPool& pool = ctx->dev_pool;
+  const size_t ne = std::max<uint64_t>(1, n_entries), ns = std::max<uint64_t>(1, n_splice);
+  PoolBuf<unsigned long long> d_entry_off, d_keys, d_keys_sorted, d_splice_off;
+  PoolBuf<uint32_t> d_read, d_allele, d_splice_id, d_slot_splice, d_slot_tri_off, d_tri_order, d_tri_site, d_counts,
+      d_table;
+  PoolBuf<uint8_t> d_vals, d_vals_sorted, d_tri_allele;
+  PoolBuf<char> d_sort_tmp;
+  PoolBuf<SsItem> d_items;
+  PoolBuf<double> d_mi;
+  CU(ctx, d_entry_off.alloc(pool, (size_t)n_sites + 1));
+  CU(ctx, d_keys.alloc(pool, ne));
+  CU(ctx, d_keys_sorted.alloc(pool, ne));
+  CU(ctx, d_splice_off.alloc(pool, (size_t)n_reads + 1));
+  CU(ctx, d_read.alloc(pool, ne));
+  CU(ctx, d_allele.alloc(pool, ne));
+  CU(ctx, d_splice_id.alloc(pool, ns));
+  CU(ctx, d_slot_splice.alloc(pool, P.slot_splice.size()));
+  CU(ctx, d_slot_tri_off.alloc(pool, P.slot_tri_off.size()));
+  CU(ctx, d_tri_order.alloc(pool, n_triples));
+  CU(ctx, d_tri_site.alloc(pool, n_triples));
+  CU(ctx, d_tri_allele.alloc(pool, n_triples));
+  CU(ctx, d_counts.alloc(pool, 3 * n_triples));
+  CU(ctx, d_vals.alloc(pool, ne));
+  CU(ctx, d_vals_sorted.alloc(pool, ne));
+  CU(ctx, d_sort_tmp.alloc(pool, std::max<size_t>(sort_bytes, 16)));
+  CU(ctx, d_items.alloc(pool, std::max<size_t>(1, P.items.size())));
+  CU(ctx, d_mi.alloc(pool, n_triples));
+  if (table_out) CU(ctx, d_table.alloc(pool, 4 * n_triples));
+
+  cudaStream_t st = ctx->stream;
+  auto up = [&](void* dst, const void* src, size_t bytes) {
+    return bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st) : cudaSuccess;
+  };
+  CU(ctx, up(d_entry_off, entry_off, ((size_t)n_sites + 1) * 8));
+  CU(ctx, up(d_read, entry_read, n_entries * 4));
+  CU(ctx, up(d_allele, entry_allele, n_entries * 4));
+  if (n_reads) CU(ctx, up(d_splice_off, splice_off, ((size_t)n_reads + 1) * 8));
+  CU(ctx, up(d_splice_id, splice_id, n_splice * 4));
+  CU(ctx, up(d_slot_splice, P.slot_splice.data(), P.slot_splice.size() * 4));
+  CU(ctx, up(d_slot_tri_off, P.slot_tri_off.data(), P.slot_tri_off.size() * 4));
+  CU(ctx, up(d_tri_order, P.tri_order.data(), n_triples * 4));
+  CU(ctx, up(d_tri_site, tri_site, n_triples * 4));
+  CU(ctx, up(d_tri_allele, P.tri_allele.data(), n_triples));
+  CU(ctx, up(d_items, P.items.data(), P.items.size() * sizeof(SsItem)));
+  CU(ctx, cudaMemsetAsync(d_counts, 0, 3 * n_triples * 4, st));
+  if (n_entries) {
+    const unsigned grid = (unsigned)std::min<uint64_t>((n_entries + 255) / 256, 65536);
+    k_ss_keys<<<grid, 256, 0, st>>>(d_entry_off, n_sites, d_read, d_allele, n_entries, read_bits, d_keys, d_vals);
+    ++ctx->launches;
+    CU(ctx, cub::DeviceRadixSort::SortPairs(d_sort_tmp.get(), sort_bytes, d_keys.get(), d_keys_sorted.get(),
+                                            d_vals.get(), d_vals_sorted.get(), (int)n_entries, 0, (int)key_bits, st));
+    ++ctx->launches;
+  }
+  if (!P.items.empty()) {
+    k_ss_count<<<(unsigned)P.items.size(), kSsThreads, 0, st>>>(
+        d_items, d_keys_sorted, d_vals_sorted, d_entry_off, (1ull << read_bits) - 1ull, d_splice_off, d_splice_id,
+        d_slot_splice, d_slot_tri_off, d_tri_order, d_tri_allele, d_counts);
+    ++ctx->launches;
+  }
+  k_ss_mi<<<(unsigned)((n_triples + 255) / 256), 256, 0, st>>>(d_counts, d_tri_site, d_entry_off, n_triples,
+                                                                ctx->d_lntab.get(), d_mi, table_out ? d_table.get()
+                                                                                                    : nullptr);
+  ++ctx->launches;
+  CU(ctx, cudaGetLastError());
+  CU(ctx, cudaMemcpyAsync(mi_out, d_mi, n_triples * 8, cudaMemcpyDeviceToHost, st));
+  if (table_out) CU(ctx, cudaMemcpyAsync(table_out, d_table, n_triples * 16, cudaMemcpyDeviceToHost, st));
+  CU(ctx, cudaStreamSynchronize(st));
   return LGMI_OK;
 }
 
