@@ -30,12 +30,11 @@ class MergedResult:
     unit that was split to its pieces [(device index, first row, end row)] in row order."""
 
     def __init__(self, records, site_mean, site_cnt, unit_rec_off, n_candidates, counts=None, shard_ms=None,
-                 shard_units=None):
+                 shard_units=None, split_units=None):
         self.records, self.site_mean, self.site_cnt = records, site_mean, site_cnt
         self.unit_rec_off, self.n_candidates, self.counts = unit_rec_off, n_candidates, counts
         self.n_records = len(records)
-        self.shard_ms, self.shard_units = shard_ms, shard_units
-        self.split_units = {}
+        self.shard_ms, self.shard_units, self.split_units = shard_ms, shard_units, split_units or {}
 
     def unit_records(self, unit):
         return self.records[int(self.unit_rec_off[unit]):int(self.unit_rec_off[unit + 1])]
@@ -46,11 +45,19 @@ class MergedResult:
         return self.counts[int(self.unit_rec_off[unit]):int(self.unit_rec_off[unit + 1])]
 
 
-def merge_shards(units, n_sites, parts, split=()) -> MergedResult:
+def place_pieces(pieces, means):
+    """merge_shards' `split` and `split_units` arguments from the split units' pieces `pieces` = [(device, unit,
+    first row, end row, records, counts | None)] in any order and their means {unit: (site_mean, site_cnt)}."""
+    ps, units = sorted(pieces, key=lambda p: (p[1], p[2])), sorted({p[1] for p in pieces})
+    split = [(u, [(a, rec, c) for _k, v, a, _e, rec, c in ps if v == u]) + tuple(means[u]) for u in units]
+    return split, {u: [(k, a, e) for k, v, a, e, _r, _c in ps if v == u] for u in units}
+
+
+def merge_shards(units, n_sites, parts, split=(), split_units=None) -> MergedResult:
     """`parts` = [(global unit indices ascending, records, site_mean, site_cnt, unit_rec_off, counts | None)]
     per shard, each in its own local order -> one result in global order.  `split` = [(global unit,
     [(first row, records, counts | None)] of its pieces in row order, site_mean, site_cnt)] for the units
-    that were split: a piece's i and j count from its first row.  Pure index bookkeeping."""
+    that were split (a piece's i and j count from its first row) and `split_units`, as place_pieces gives them."""
     n_units = len(units)
     site_mean = np.full(n_sites, np.nan)
     site_cnt = np.zeros(n_sites, dtype=np.uint32)
@@ -109,7 +116,8 @@ def merge_shards(units, n_sites, parts, split=()) -> MergedResult:
         records['unit'][dst] = np.repeat(index, n).astype(np.uint32)
         if counts is not None and cnts is not None and len(dst):
             counts[dst] = cnts
-    return MergedResult(records, site_mean, site_cnt, unit_rec_off, int((n_s * (n_s - 1) // 2).sum()), counts)
+    return MergedResult(records, site_mean, site_cnt, unit_rec_off, int((n_s * (n_s - 1) // 2).sum()), counts,
+                        split_units=split_units)
 
 
 SPLIT_ROWS = 128   # piece boundaries fall on multiples of this many rows (lgmi_batch_create_rows)
@@ -186,23 +194,50 @@ def plan_pieces(units, n_dev):
     return shards, pieces, splits
 
 
-def piece_batch(ctx, pb: PlaneBatch, pieces):
-    """The batch of `pieces` [(unit, first row, end row)] of pb's units on ctx (api.Batch with row limits): each the
-    suffix unit of sites [a, S) of its unit, back to back, with row limit e - a.  Its planes are left empty: they come
-    from upload_piece_rows and from copies of the other pieces' rows."""
-    desc = np.zeros(len(pieces), dtype=pb.units.dtype)
-    flags = []
+def piece_units(units, pieces):
+    """The descriptor table of the batch of `pieces` [(unit, first row, end row)] of `units`: each piece the suffix
+    unit of sites [a, S) of its unit, planes and sites back to back."""
+    desc = np.zeros(len(pieces), dtype=units.dtype)
     word = site = 0
     for q, (u, a, _e) in enumerate(pieces):
-        g = pb.units[u]
-        S, W = int(g['n_sites']), int(g['row_words'])
-        desc[q] = (word, S - a, int(g['n_reads']), W, site)    # the suffix unit of sites [a, S)
-        flags.append(pb.site_flags[int(g['site_off']) + a:int(g['site_off']) + S])
+        S, W = int(units['n_sites'][u]), int(units['row_words'][u])
+        desc[q] = (word, S - a, int(units['n_reads'][u]), W, site)
         word += 3 * (S - a) * W
         site += S - a
+    return desc
+
+
+def row_order(pieces, unit):
+    """The pieces of `unit` in plan_pieces' `pieces` as (first row, end row, device, position in its batch), in row
+    order: the first one's device computes the unit's per-site means."""
+    return sorted((a, e, k, q) for k, mine in enumerate(pieces) for q, (u, a, e) in enumerate(mine) if u == unit)
+
+
+def plane_copies(units, pieces):
+    """For each device k, in issue order, the copies [(dst_word, src_device, src_position, src_word, n_words)] that
+    bring each piece of pieces[k] the rows after its own, from the later pieces of its unit, once all own rows are
+    uploaded (upload_piece_rows).  src_word is lgmi_piece_export's plane_word of the source, n_words its plane_words."""
+    off = [piece_units(units, mine)['plane_off'] for mine in pieces]
+    every = [(ks, qs, v, c, ce) for ks, theirs in enumerate(pieces) for qs, (v, c, ce) in enumerate(theirs)]
+    copies = [[] for _ in pieces]
+    for k, q, u, a, e in every:
+        W = int(units['row_words'][u])
+        copies[k] += [(int(off[k][q]) + 3 * (c - a) * W, ks, qs, int(off[ks][qs]), 3 * (ce - c) * W)
+                      for ks, qs, v, c, ce in every if v == u and c >= e]
+    return copies
+
+
+def piece_batch(ctx, pb: PlaneBatch, pieces):
+    """The batch of `pieces` [(unit, first row, end row)] of pb's units on ctx (api.Batch with row limits): each the
+    suffix unit of sites [a, S) of its unit (piece_units), with row limit e - a.  Its planes are left empty: they come
+    from upload_piece_rows and from copies of the other pieces' rows (plane_copies)."""
+    desc = piece_units(pb.units, pieces)
+    off, S = pb.units['site_off'], pb.units['n_sites']
+    flags = np.concatenate([pb.site_flags[int(off[u]) + a:int(off[u]) + int(S[u])] for u, a, _e in pieces])
     # (np.empty: the batch only reads the planes' size; their words come from upload_rows / copies)
-    sub = PlaneBatch(desc, np.empty(word, dtype=np.uint32), np.concatenate(flags))
-    return api.Batch(ctx, sub, row_limit=[e - a for _u, a, e in pieces])
+    words = int((3 * desc['n_sites'].astype(np.int64) * desc['row_words']).sum())
+    return api.Batch(ctx, PlaneBatch(desc, np.empty(words, dtype=np.uint32), flags),
+                     row_limit=[e - a for _u, a, e in pieces])
 
 
 def upload_piece_rows(batch, pb: PlaneBatch, pieces):
@@ -235,12 +270,6 @@ class DevicePool:
             c.close()
         self.contexts = []
 
-    def plan(self, pb: PlaneBatch):
-        """[ascending global unit indices of each device's shard] by LPT on S(S-1)/2 * ceil(R/64), when no unit is
-        split (split_plan); otherwise (shards, pieces, splits) of plan_pieces."""
-        shards, pieces, splits = plan_pieces(pb.units, len(self.devices))
-        return (shards, pieces, splits) if splits else shards
-
     def run(self, pb: PlaneBatch, min_common_reads=5, mode=api.MODE_HET_ONLY):
         """The MI step of `pb` over all devices; same result as api.mi_step_batched on one."""
         n_dev = len(self.devices)
@@ -259,66 +288,50 @@ class DevicePool:
                 b.run(min_common_reads, mode)
             if len(index):
                 res = api.mi_step_batched(pb.subset(index), min_common_reads, mode, ctx=self.contexts[k])
+            mine = []
             if b is not None:
-                b.result = b.download(copy=True)
-                self.last_piece_ms[k] = b.result.kernel_ms
-            return res, 1e3 * (time.perf_counter() - t0)
+                r = b.download(copy=True)
+                self.last_piece_ms[k] = r.kernel_ms
+                mine = [(k, u, a, e, r.unit_records(q), r.unit_counts(q) if r.counts is not None else None)
+                        for q, (u, a, e) in enumerate(pieces[k])]
+            return res, mine, 1e3 * (time.perf_counter() - t0)
 
         try:
             done = list(self._threads.map(work, range(n_dev)))
-            parts = [(shards[k], r.records, r.site_mean, r.site_cnt, r.unit_rec_off, r.counts)
-                     for k, (r, _ms) in enumerate(done) if r is not None]
-            split, where = [], {}
+            means = {}
             t0 = time.perf_counter()
-            for u, bounds in splits.items():
-                # (device, position in its piece batch) of every piece of u, in row order
-                loc = sorted((a, k, q) for k in range(n_dev) for q, (v, a, _e) in enumerate(pieces[k]) if v == u)
-                owner = self.contexts[loc[0][1]]
+            for u in splits:
+                order = row_order(pieces, u)
                 S, off = int(pb.units['n_sites'][u]), int(pb.units['site_off'][u])
-                mean, cnt = api.split_means(owner, pb.site_flags[off:off + S], [(batches[k], q) for _a, k, q in loc])
-                recs = []
-                for a, k, q in loc:
-                    res = batches[k].result
-                    recs.append((a, res.unit_records(q), res.unit_counts(q) if res.counts is not None else None))
-                split.append((u, recs, mean, cnt))
-                where[u] = [(k, a, a + int(batches[k].row_limit[q])) for a, k, q in loc]
+                means[u] = api.split_means(self.contexts[order[0][2]], pb.site_flags[off:off + S],
+                                           [(batches[k], q) for _a, _e, k, q in order])
             self.last_split_means_ms = 1e3 * (time.perf_counter() - t0)
         finally:
             for b in batches:
                 if b is not None:
                     b.close()
-        merged = merge_shards(pb.units, pb.n_sites, parts, split)
-        merged.split_units = where
-        merged.shard_ms = [ms for _r, ms in done]
+        parts = [(shards[k], r.records, r.site_mean, r.site_cnt, r.unit_rec_off, r.counts)
+                 for k, (r, _p, _ms) in enumerate(done) if r is not None]
+        merged = merge_shards(pb.units, pb.n_sites, parts, *place_pieces([p for r in done for p in r[1]], means))
+        merged.shard_ms = [ms for _r, _p, ms in done]
         # units per device; a split unit counts on the device of its first piece, which computes its means
-        owned = [len(shards[k]) for k in range(n_dev)]
-        for u, w in where.items():
-            owned[w[0][0]] += 1
-        merged.shard_units = owned
+        owners = [row_order(pieces, u)[0][2] for u in splits]
+        merged.shard_units = [len(s) + owners.count(k) for k, s in enumerate(shards)]
         return merged
 
     def _piece_batches(self, pb, pieces):
         """One batch of pieces per device (None where there is none), planes in place: each piece's own rows
         uploaded from the host, the rows after them copied from the devices of the later pieces of its unit."""
-        n_dev = len(self.devices)
-        batches = [piece_batch(self.contexts[k], pb, pieces[k]) if pieces[k] else None for k in range(n_dev)]
-        rows_at = {}   # (unit, first row) -> (device, first plane word of the piece there, end row)
-        for k in range(n_dev):
-            for q, (u, a, e) in enumerate(pieces[k]):
-                rows_at[(u, a)] = (k, int(batches[k].pb.units['plane_off'][q]), e)
+        batches = [piece_batch(ctx, pb, mine) if mine else None for ctx, mine in zip(self.contexts, pieces)]
         try:
             # the host link once: every piece uploads its own rows, one thread per device
             list(self._threads.map(lambda k: upload_piece_rows(batches[k], pb, pieces[k]),
-                                   [k for k in range(n_dev) if pieces[k]]))
+                                   [k for k, mine in enumerate(pieces) if mine]))
             # then, from this thread, each piece's rows after its own from the pieces that uploaded them: a copy
             # waits on an event recorded behind the upload already queued on the source's stream
-            for k in range(n_dev):
-                for q, (u, a, e) in enumerate(pieces[k]):
-                    W = int(pb.units['row_words'][u])
-                    dst0 = int(batches[k].pb.units['plane_off'][q])
-                    for (v, c), (ks, src0, ce) in rows_at.items():
-                        if v == u and c >= e:
-                            batches[k].copy_planes_from(dst0 + 3 * (c - a) * W, batches[ks], src0, 3 * (ce - c) * W)
+            for k, copies in enumerate(plane_copies(pb.units, pieces)):
+                for dst, ks, _qs, src, n in copies:
+                    batches[k].copy_planes_from(dst, batches[ks], src, n)
         except BaseException:
             for b in batches:
                 if b is not None:

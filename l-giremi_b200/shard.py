@@ -22,10 +22,11 @@ import numpy as np
 import time
 
 from . import api
-from ._lib import PAIR_REC, PieceIpc
+from ._lib import PAIR_REC
 from .api import partition_lpt, unit_costs
 from .encode import PlaneBatch
-from .multigpu import MergedResult, merge_shards, piece_batch, plan_pieces, upload_piece_rows  # noqa: F401
+from .multigpu import (MergedResult, merge_shards, piece_batch, place_pieces, plane_copies,  # noqa: F401
+                       plan_pieces, row_order, upload_piece_rows)
 
 
 def plan(units, world_size):
@@ -131,20 +132,12 @@ def local_run(pb_global: PlaneBatch, rank, world, min_common, mode, ctx, group=N
     try:
         if batch is not None:
             upload_piece_rows(batch, pb_global, mine)
-        # every piece of every rank: (rank, position in its batch, unit, first row, end row, exported bytes)
-        everyone = _all_pieces(batch, mine, rank, world, group)
-        for q, (u, a, e) in enumerate(mine):
-            W = int(pb_global.units['row_words'][u])
-            dst0 = int(batch.pb.units['plane_off'][q])
-            for k, qs, v, c, ce, piece in everyone:
-                if v != u or c < e:
-                    continue
-                if k == rank:
-                    batch.copy_planes_from(dst0 + 3 * (c - a) * W, batch, int(batch.pb.units['plane_off'][qs]),
-                                           3 * (ce - c) * W)
-                else:
-                    src = PieceIpc.from_buffer_copy(piece)
-                    batch.copy_planes_from_ipc(dst0 + 3 * (c - a) * W, piece, src.plane_word, src.plane_words)
+        exported = _export_pieces(batch, mine, world, group)
+        for dst, k, q, src, n in plane_copies(pb_global.units, pieces)[rank]:
+            if k == rank:
+                batch.copy_planes_from(dst, batch, src, n)
+            else:
+                batch.copy_planes_from_ipc(dst, exported[k][q], src, n)
         if batch is not None:
             batch.run(min_common, mode)
             res = batch.download(copy=True)
@@ -152,14 +145,15 @@ def local_run(pb_global: PlaneBatch, rank, world, min_common, mode, ctx, group=N
             run.pieces = [(u, a, e, res.unit_records(q), res.unit_counts(q) if res.counts is not None else None)
                           for q, (u, a, e) in enumerate(mine)]
         run.pieces_ms = 1e3 * (time.perf_counter() - t0)
-        everyone = _all_pieces(batch, mine, rank, world, group)         # exported again, after the run
+        exported = _export_pieces(batch, mine, world, group)         # again, after the run
         t0 = time.perf_counter()
         for u in splits:
-            row_order = sorted((c, k, piece) for k, _q, v, c, _ce, piece in everyone if v == u)
-            if row_order[0][1] != rank:
+            order = row_order(pieces, u)
+            if order[0][2] != rank:
                 continue
             S, off = int(pb_global.units['n_sites'][u]), int(pb_global.units['site_off'][u])
-            run.means[u] = api.split_means_ipc(ctx, pb_global.site_flags[off:off + S], [p for _c, _k, p in row_order])
+            run.means[u] = api.split_means_ipc(ctx, pb_global.site_flags[off:off + S],
+                                               [exported[k][q] for _a, _e, k, q in order])
         run.split_means_ms = 1e3 * (time.perf_counter() - t0)
         dist.barrier(group=group)            # every import from this rank's batch is done
     finally:
@@ -168,13 +162,12 @@ def local_run(pb_global: PlaneBatch, rank, world, min_common, mode, ctx, group=N
     return run
 
 
-def _all_pieces(batch, mine, rank, world, group):
-    """Every rank's pieces with their export_piece bytes, recorded behind all the batch has queued so far."""
+def _export_pieces(batch, mine, world, group):
+    """export_piece bytes of every rank's pieces [rank][position], each behind all its batch has queued so far."""
     import torch.distributed as dist
-    local = [(rank, q, u, a, e, batch.export_piece(q)) for q, (u, a, e) in enumerate(mine)]
     out = [None] * world
-    dist.all_gather_object(out, local, group=group)
-    return [x for part in out for x in part]
+    dist.all_gather_object(out, [batch.export_piece(q) for q in range(len(mine))], group=group)
+    return out
 
 
 def gather_run_to_rank0(pb_global: PlaneBatch, run: LocalRun, group=None, device="cpu"):
@@ -215,7 +208,7 @@ def gather_run_to_rank0(pb_global: PlaneBatch, run: LocalRun, group=None, device
     dist.gather_object(meta, metas, dst=0, group=group)
     if rank != 0:
         return None
-    parts, split_pieces, split_means = [], {}, {}
+    parts, split_pieces, split_means = [], [], {}
     for k in range(world):
         index = gathered[4][k].view(np.int64)
         if len(index):
@@ -229,7 +222,7 @@ def gather_run_to_rank0(pb_global: PlaneBatch, run: LocalRun, group=None, device
             c = None
             if has_counts:
                 c, tab_at = tab[tab_at:tab_at + n], tab_at + n
-            split_pieces.setdefault(u, []).append((a, e, k, rec[at:at + n], c))
+            split_pieces.append((k, u, a, e, rec[at:at + n], c))
             at += n
         mean, cnt = gathered[8][k].view(np.float64), gathered[9][k].view(np.uint32)
         at = 0
@@ -237,11 +230,4 @@ def gather_run_to_rank0(pb_global: PlaneBatch, run: LocalRun, group=None, device
             S = int(pb_global.units['n_sites'][u])
             split_means[u] = (mean[at:at + S], cnt[at:at + S])
             at += S
-    split = []
-    for u in sorted(split_pieces):
-        ps = sorted(split_pieces[u], key=lambda p: p[0])
-        split.append((u, [(a, rec, c) for a, _e, _k, rec, c in ps]) + split_means[u])
-    merged = merge_shards(pb_global.units, pb_global.n_sites, parts, split)
-    merged.split_units = {u: [(k, a, e) for a, e, k, _r, _c in sorted(split_pieces[u], key=lambda p: p[0])]
-                          for u in split_pieces}
-    return merged
+    return merge_shards(pb_global.units, pb_global.n_sites, parts, *place_pieces(split_pieces, split_means))

@@ -4,6 +4,7 @@ A piece of rows [a, b) of a unit is the suffix unit of sites [a, S) with row lim
 row order with i and j shifted by a, must be the whole unit's records, and the means gathered over the pieces the
 unsplit run's, bit for bit.  The planner and the merge are host bookkeeping and run without a device."""
 import importlib
+import types
 
 import numpy as np
 import pytest
@@ -105,6 +106,117 @@ def test_merge_shards_places_pieces():
     assert got.counts[2:6, 0].tolist() == [100, 100, 200, 200] and got.counts[6, 0] == 18
     assert np.array_equal(got.site_mean[3:303], mean) and np.array_equal(got.site_cnt[3:303], cnt)
     assert got.site_mean[:3].tolist() == [1.0, 2.0, 3.0] and got.site_mean[303:].tolist() == [4.0, 5.0]
+
+
+def test_place_pieces_given_in_any_order():
+    """Two split units, their pieces from three devices handed over out of row order (place_pieces, then
+    merge_shards): the whole units' records, tables and means, and split_units in row order."""
+    units = _descs([(20, 10), (300, 10), (5, 10), (400, 10)])
+    units['site_off'] = np.concatenate(([0], np.cumsum(units['n_sites'])[:-1]))
+    rng = np.random.default_rng(77)
+    whole = []                      # per unit: records, tables, site means, site counts
+    for u, S in enumerate(units['n_sites'].tolist()):
+        i, j = np.triu_indices(S, 1)
+        keep = rng.random(len(i)) < 0.2
+        rec = np.zeros(int(keep.sum()), dtype=lg_mod.PAIR_REC)
+        rec['unit'], rec['i'], rec['j'], rec['mi'] = u, i[keep], j[keep], rng.random(int(keep.sum()))
+        whole.append((rec, rng.integers(0, 1000, size=(len(rec), 9)).astype(np.uint32),
+                       np.where(rng.random(S) < 0.2, np.nan, rng.random(S)), rng.integers(0, 50, S).astype(np.uint32)))
+    device = {(1, 0): 2, (1, 128): 0, (1, 256): 1, (3, 0): 1, (3, 128): 2}
+    pieces = []
+    for u, a, e in ((1, 0, 128), (1, 128, 256), (1, 256, 300), (3, 0, 128), (3, 128, 400)):
+        rec, tab = whole[u][0], whole[u][1]
+        sel = (rec['i'] >= a) & (rec['i'] < e)
+        r = rec[sel].copy()
+        r['unit'], r['i'], r['j'] = 9, r['i'] - a, r['j'] - a     # numbered as in the piece's batch
+        pieces.append((device[(u, a)], u, a, e, r, tab[sel]))
+    shard = (np.array([0, 2]), np.concatenate([whole[0][0], whole[2][0]]),
+             np.concatenate([whole[0][2], whole[2][2]]), np.concatenate([whole[0][3], whole[2][3]]),
+             np.array([0, len(whole[0][0]), len(whole[0][0]) + len(whole[2][0])], dtype=np.uint64),
+             np.concatenate([whole[0][1], whole[2][1]]))
+    shard[1]['unit'][len(whole[0][0]):] = 1                   # a shard numbers its units from 0
+    got = mg.merge_shards(units, int(units['n_sites'].sum()), [shard],
+                          *mg.place_pieces([pieces[t] for t in (4, 1, 3, 0, 2)], {1: whole[1][2:], 3: whole[3][2:]}))
+    assert np.array_equal(got.records, np.concatenate([w[0] for w in whole]))
+    assert np.array_equal(got.counts, np.concatenate([w[1] for w in whole]))
+    assert np.array_equal(got.site_mean, np.concatenate([w[2] for w in whole]), equal_nan=True)
+    assert np.array_equal(got.site_cnt, np.concatenate([w[3] for w in whole]))
+    assert got.unit_rec_off.tolist() == np.cumsum([0] + [len(w[0]) for w in whole]).tolist()
+    assert got.split_units == {1: [(2, 0, 128), (0, 128, 256), (1, 256, 300)], 3: [(1, 0, 128), (2, 128, 400)]}
+
+
+class _Words:
+    """pb.planes of a plane batch whose word at position p is p, without holding them."""
+
+    def __getitem__(self, s):
+        return np.arange(s.start, s.stop, dtype=np.int64)
+
+
+class _HostPieces:
+    """A device's batch of pieces as numpy words: what upload_piece_rows and the copies write, and how often."""
+
+    def __init__(self, units, pieces):
+        self.pb = types.SimpleNamespace(units=mg.piece_units(units, pieces))
+        n = int((3 * self.pb.units['n_sites'].astype(np.int64) * self.pb.units['row_words']).sum())
+        self.words, self.writes, self.uploaded = np.zeros(n, np.int64), np.zeros(n, np.int64), np.zeros(n, bool)
+
+    def upload_rows(self, word_begin, words):
+        self.words[word_begin:word_begin + len(words)] = words
+        self.writes[word_begin:word_begin + len(words)] += 1
+        self.uploaded[word_begin:word_begin + len(words)] = True
+
+
+def _with_planes(units):
+    words = 3 * units['n_sites'].astype(np.int64) * units['row_words']
+    units['plane_off'] = np.concatenate(([0], np.cumsum(words)[:-1]))
+    return units
+
+
+def _plans():
+    """(units, pieces) of the cfg4 + cfg3 plan at 2, 4 and 8 devices, of two split units, and of two pieces of one
+    unit on one device."""
+    cfg = np.concatenate([_cfg4_descs(), _descs([(2000, 100000)])])
+    plans = [mg.plan_pieces(cfg, n)[1] for n in (2, 4, 8)]
+    cfg['row_words'] = 3               # (after planning: keeps the stand-in planes of the 2 000-site unit small)
+    hand = _with_planes(_descs([(300, 500), (40, 100), (520, 1000)]))
+    return [(_with_planes(cfg), p) for p in plans] + [
+        (hand, [[(2, 256, 520), (0, 0, 128)], [(2, 0, 256)], [(0, 128, 300)]]),
+        (hand, [[(0, 0, 128), (0, 256, 300)], [(0, 128, 256)]])]
+
+
+def test_plane_copies_assemble_every_piece():
+    """Each device's own rows (upload_piece_rows), then plane_copies in order: every piece holds its unit's suffix
+    planes [3aW, 3SW), every word written once, and a copy reads only rows its source uploaded itself."""
+    for units, pieces in _plans():
+        pb = types.SimpleNamespace(units=units, planes=_Words())
+        host = [_HostPieces(units, mine) for mine in pieces]
+        for b, mine in zip(host, pieces):
+            mg.upload_piece_rows(b, pb, mine)
+        for b, copies in zip(host, mg.plane_copies(units, pieces)):
+            for dst, ks, _qs, src, n in copies:
+                assert host[ks].uploaded[src:src + n].all()
+                b.words[dst:dst + n] = host[ks].words[src:src + n]
+                b.writes[dst:dst + n] += 1
+        off, S, W = units['plane_off'].astype(np.int64), units['n_sites'], units['row_words']
+        for b, mine in zip(host, pieces):
+            want = [np.arange(off[u] + 3 * a * W[u], off[u] + 3 * S[u] * W[u]) for u, a, _e in mine]
+            assert np.array_equal(b.words, np.concatenate(want) if want else np.zeros(0, np.int64))
+            assert (b.writes == 1).all()
+        for u in {u for mine in pieces for u, _a, _e in mine}:
+            order = mg.row_order(pieces, u)
+            assert [a for a, _e, _k, _q in order] == [0] + [e for _a, e, _k, _q in order[:-1]]
+            assert order[-1][1] == units['n_sites'][u] and all(pieces[k][q] == (u, a, e) for a, e, k, q in order)
+
+
+def test_plane_copies_read_what_the_export_reports():
+    """src_word is the source piece's plane_off in its device's batch and n_words its own rows' words: the
+    plane_word and plane_words of lgmi_piece_export, which the copies between processes use."""
+    for units, pieces in _plans():
+        for copies in mg.plane_copies(units, pieces):
+            for _dst, ks, qs, src, n in copies:
+                u, a, e = pieces[ks][qs]
+                assert src == mg.piece_units(units, pieces[ks])['plane_off'][qs]
+                assert n == 3 * int(units['row_words'][u]) * (e - a)
 
 
 # --------------------------------------------------------------------------- on the device
