@@ -103,7 +103,11 @@ typedef struct {
 #define LGMI_MODE_SKIP_NONHET 0x4u /* with HET_ONLY: do not evaluate MI of     */
                                    /* pairs without a het partner (dead work   */
                                    /* in the reference, SURVEY Q7); reported   */
-                                   /* separately, never in the headline        */
+                                   /* separately, never in the headline.  Deep */
+                                   /* units with host flags, not pieces, count */
+                                   /* only the het sites' rows on the tensor   */
+                                   /* cores where that issues at most half the */
+                                   /* multiply-adds (lgmi_set_dense_path)      */
 #define LGMI_MODE_SPLIT_RECORDS 0x8u /* lgmi_pipeline_step*: deliver the rows as  */
                                    /* two arrays rec_mi / rec_ij (12 bytes per  */
                                    /* row over PCIe instead of 16) and leave    */
@@ -211,7 +215,13 @@ LGMI_API int lgmi_set_dense_threshold(lgmi_t* ctx, uint32_t min_sites, uint32_t 
  * from the listed reads (k_dense_prep, k_other_fix); otherwise, and always with    *
  * blocks = 9, all nine blocks of {covered, major or minor, major}.  Same integers  *
  * either way; applies to batches created afterwards.  Environment                  *
- * LGMI_DENSE_PATH=4/9 sets the default.                                            */
+ * LGMI_DENSE_PATH=4/9 sets the default.  Independent of the label form, a run in   *
+ * HET_ONLY | SKIP_NONHET on a batch whose flag bytes came from the host computes,  *
+ * for every deep unit that is not a piece, only the blocks of the het sites' rows  *
+ * against all sites (the het-anchored form) where that issues at most half the    *
+ * multiply-accumulates of the pair triangle; dense_macs / gram_macs report the     *
+ * form each run took.  lgmi_batch_device_ptrs drops it: the flags are then the     *
+ * caller's, unknown to the host.                                                   */
 LGMI_API int lgmi_set_dense_path(lgmi_t* ctx, int blocks);
 /* Mid-depth units (more than 64 sites or 256 reads, below the dense threshold)   *
  * have their counts built on the tensor cores in one batched launch              *

@@ -222,6 +222,19 @@ struct lgmi_batch {
   Event fix_fork, fix_join;    // joined before the tables are read)
   PoolBuf<DenseTile> d_tiles;
   uint64_t dense_macs = 0;      // multiply-accumulates the tile lists amount to
+  // the het-anchored form of the deep units (HET_ONLY | SKIP_NONHET), planned from the host flag bytes at upload;
+  // parallel to dense_plans (empty until flags have been seen)
+  std::vector<HetDensePlan> het_plans;
+  std::vector<DenseTile> h_het_tiles; // their tile lists
+  std::vector<uint32_t> h_het_rows;   // per deep unit H_pad entries from het_rows_off: its het sites, ~0 for padding
+  std::vector<uint64_t> het_rows_off;
+  std::vector<uint8_t> h_unit_het;    // per unit: 1 if the het form is taken when the run allows it
+  std::vector<CUtensorMap> het_tmaps; // per deep unit: its X_het for k_gram_i8's A operand
+  PoolBuf<DenseTile> d_het_tiles;
+  PoolBuf<uint32_t> d_het_rows;
+  PoolBuf<uint8_t> d_unit_het;
+  PoolBuf<uint8_t> d_x_het;           // the het sites' X rows of the unit being contracted, H_pad rows per group
+  std::vector<std::pair<uint64_t, uint64_t>> run_macs;  // per deep unit, the last run's four- and nine-block lists' MACs
   // tiled popcount path
   PoolBuf<TileItem> d_tile_items;
   uint32_t n_tile_items = 0;
@@ -462,6 +475,88 @@ extern "C" void lgmi_batch_destroy(lgmi_batch_t* b) {
   delete b;
 }
 
+// k_gram_i8's tensor map of an X of pl's unit at x: [3 * rows][K_pad bytes], K contiguous; box = 128 rows x 128 bytes,
+// 128B swizzle
+static int encode_x_map(lgmi_ctx* ctx, CUtensorMap* map, void* x, const DensePlan& pl, uint32_t rows) {
+  typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  EncodeTiled encode = reinterpret_cast<EncodeTiled>(ctx->encode_tiled);
+  const cuuint64_t dims[2] = {(cuuint64_t)pl.k_blocks * kDenseBK, 3ull * rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)pl.k_blocks * kDenseBK};
+  const cuuint32_t box[2] = {(cuuint32_t)kDenseBK, 128u};
+  const cuuint32_t estr[2] = {1u, 1u};
+  const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, x, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(ctx, LGMI_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for unit %u", (int)r, pl.unit);
+  return LGMI_OK;
+}
+
+// The het-anchored plans of the batch's deep units from the host flag bytes (site_flags: the batch's), and their
+// tables on the device, copied on stream st.  What a captured launch chain holds of them -- which units take the form,
+// their H_pad, the lengths of their tile lists and the buffers' addresses -- is the layout: when it changes, the
+// stream is drained, buffers are sized and tensor maps encoded again, and the graphs are dropped.  With the same
+// layout, new het sites only replace the tables' contents, in stream order.
+static int plan_het(lgmi_batch* b, const uint8_t* site_flags, cudaStream_t st) {
+  if (b->dense_plans.empty()) return LGMI_OK;
+  lgmi_ctx* ctx = b->ctx;
+  const size_t n = b->dense_plans.size();
+  std::vector<HetDensePlan> plans(n);
+  std::vector<DenseTile> tiles;
+  std::vector<uint32_t> rows;
+  std::vector<uint64_t> rows_off(n);
+  std::vector<uint8_t> unit_het(b->n_units, 0);
+  uint64_t x_bytes = 0;
+  for (size_t d = 0; d < n; ++d) {
+    const DensePlan& pl = b->dense_plans[d];
+    const bool piece = !b->h_row_limit.empty() && b->h_row_limit[pl.unit] != 0u;
+    HetDensePlan& h = plans[d];
+    plan_het_dense(pl, site_flags + b->h_units[pl.unit].site_off, piece, (uint32_t)ctx->num_sms, tiles, &h);
+    rows_off[d] = rows.size();
+    rows.insert(rows.end(), h.het.begin(), h.het.end());
+    rows.resize(rows.size() + (h.H_pad - h.H), ~0u);
+    if (h.fewer) {
+      unit_het[pl.unit] = 1;
+      x_bytes = std::max<uint64_t>(x_bytes, 3ull * h.H_pad * pl.k_blocks * kDenseBK);
+    }
+  }
+  auto layout = [](const HetDensePlan& h) {
+    return std::vector<uint64_t>{h.fewer, h.H_pad, h.H != 0u, h.list4.n, h.list4.n_whole, h.list9.n, h.list9.n_whole};
+  };
+  bool same = b->het_plans.size() == n && b->h_unit_het == unit_het && b->d_het_tiles.size() >= std::max<size_t>(1, tiles.size()) &&
+              b->d_het_rows.size() >= std::max<size_t>(1, rows.size()) && b->d_x_het.size() >= std::max<uint64_t>(1, x_bytes);
+  for (size_t d = 0; same && d < n; ++d)
+    same = layout(b->het_plans[d]) == layout(plans[d]) && b->het_rows_off[d] == rows_off[d];
+  if (!same) {
+    CU(ctx, cudaStreamSynchronize(st));
+    CU(ctx, cudaStreamSynchronize(bstream(b)));  // (runs read the tables there; graphs hold their addresses)
+    b->graphs.clear();
+    b->het_plans.clear();  // (nothing is taken while the tables are being replaced)
+    if (b->d_het_tiles.size() < std::max<size_t>(1, tiles.size())) CU(ctx, b->d_het_tiles.alloc(ctx->dev_pool, std::max<size_t>(1, tiles.size())));
+    if (b->d_het_rows.size() < std::max<size_t>(1, rows.size())) CU(ctx, b->d_het_rows.alloc(ctx->dev_pool, std::max<size_t>(1, rows.size())));
+    if (!b->d_unit_het) CU(ctx, b->d_unit_het.alloc(ctx->dev_pool, std::max<uint32_t>(1, b->n_units)));
+    if (b->d_x_het.size() < std::max<uint64_t>(1, x_bytes)) CU(ctx, b->d_x_het.alloc(ctx->dev_pool, std::max<uint64_t>(1, x_bytes)));
+    b->het_tmaps.assign(n, CUtensorMap{});
+    for (size_t d = 0; d < n; ++d)
+      if (plans[d].fewer && plans[d].H)
+        if (const int rc = encode_x_map(ctx, &b->het_tmaps[d], b->d_x_het, b->dense_plans[d], plans[d].H_pad)) return rc;
+  }
+  b->h_het_tiles = std::move(tiles);
+  b->h_het_rows = std::move(rows);
+  b->het_rows_off = std::move(rows_off);
+  b->h_unit_het = std::move(unit_het);
+  if (!b->h_het_tiles.empty())
+    CU(ctx, cudaMemcpyAsync(b->d_het_tiles, b->h_het_tiles.data(), b->h_het_tiles.size() * sizeof(DenseTile),
+                            cudaMemcpyHostToDevice, st));
+  if (!b->h_het_rows.empty())
+    CU(ctx, cudaMemcpyAsync(b->d_het_rows, b->h_het_rows.data(), b->h_het_rows.size() * sizeof(uint32_t),
+                            cudaMemcpyHostToDevice, st));
+  if (b->n_units)
+    CU(ctx, cudaMemcpyAsync(b->d_unit_het, b->h_unit_het.data(), b->n_units, cudaMemcpyHostToDevice, st));
+  b->het_plans = std::move(plans);
+  return LGMI_OK;
+}
+
 // lgmi_batch_create, and with row_limit (non-NULL) lgmi_batch_create_rows (a unit k with row_limit[k] != 0 is a piece
 // of a split unit, plan_batch): the batch's plan, then its buffers and tables on the device and the tensor maps of
 // its deep units.  Nothing is allocated for a batch whose plan fails.
@@ -553,23 +648,9 @@ static int batch_create(lgmi_t* ctx, const lgmi_unit_desc* units, uint32_t n_uni
       CU(ctx, create(b->fix_join, cudaEventDisableTiming));
     }
     CU(ctx, upload(b->d_tiles, plan.dense_tiles, 0));
-    typedef CUresult (*EncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    EncodeTiled encode = reinterpret_cast<EncodeTiled>(ctx->encode_tiled);
     b->tmaps.resize(b->dense_plans.size());
-    for (size_t d = 0; d < b->dense_plans.size(); ++d) {
-      const DensePlan& pl = b->dense_plans[d];
-      // X of this unit: [3 * S_pad rows][K_pad bytes], K contiguous; box = 128 rows x 128 bytes, 128B swizzle
-      const cuuint64_t dims[2] = {(cuuint64_t)pl.k_blocks * kDenseBK, 3ull * pl.S_pad};
-      const cuuint64_t strides[1] = {(cuuint64_t)pl.k_blocks * kDenseBK};
-      const cuuint32_t box[2] = {(cuuint32_t)kDenseBK, 128u};
-      const cuuint32_t estr[2] = {1u, 1u};
-      const CUresult r = encode(&b->tmaps[d], CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, b->d_x, dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) return fail(ctx, LGMI_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for unit %u", (int)r, pl.unit);
-    }
+    for (size_t d = 0; d < b->dense_plans.size(); ++d)
+      if (const int rc = encode_x_map(ctx, &b->tmaps[d], b->d_x, b->dense_plans[d], b->dense_plans[d].S_pad)) return rc;
   }
   b->rec_cap = std::max<uint64_t>(1, b->n_candidates);
   CU(ctx, b->d_records.alloc(ctx->dev_pool, b->rec_cap));
@@ -609,7 +690,7 @@ extern "C" int lgmi_batch_upload(lgmi_batch_t* b, const uint32_t* planes, const 
   b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags) : 0;
   b->het_known = true;
   b->uploaded = true;
-  return LGMI_OK;
+  return plan_het(b, site_flags, bstream(b));
 }
 
 extern "C" int lgmi_batch_upload_rows(lgmi_batch_t* b, const uint32_t* planes, uint64_t word_begin, uint64_t word_end,
@@ -630,7 +711,7 @@ extern "C" int lgmi_batch_upload_rows(lgmi_batch_t* b, const uint32_t* planes, u
   b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags) : 0;
   b->het_known = true;
   b->uploaded = true;
-  return LGMI_OK;
+  return plan_het(b, site_flags, bstream(b));
 }
 
 // Direct peer copies from sdev to the current device ddev where the devices allow them; without peer access the
@@ -751,6 +832,11 @@ extern "C" int lgmi_batch_copy_planes_ipc(lgmi_batch_t* dst, uint64_t dst_word, 
 
 static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing);
 
+// whether deep unit d of the batch takes the het-anchored form in a run of this mode
+static bool het_form(const lgmi_batch* b, size_t d, uint32_t mode) {
+  return d < b->het_plans.size() && take_het_form(b->het_plans[d], mode, b->het_known);
+}
+
 extern "C" int lgmi_batch_run(lgmi_batch_t* b, int min_common, uint32_t mode) {
   if (!b) return LGMI_ERR_ARG;
   lgmi_ctx* ctx = b->ctx;
@@ -761,6 +847,14 @@ extern "C" int lgmi_batch_run(lgmi_batch_t* b, int min_common, uint32_t mode) {
   // LGMI_MODE_GRAPH (and every group of a pipelined step): the whole launch chain as ONE cudaGraphLaunch
   const bool as_graph = (mode & LGMI_MODE_GRAPH) != 0u || (b->own_stream != nullptr && ctx->pipeline_graphs);
   mode &= ~LGMI_MODE_GRAPH;
+  // the tile lists this run takes per deep unit (which of the two label forms is known after the run): what
+  // dense_macs / gram_macs report, whatever is uploaded before the results are read
+  b->run_macs.resize(b->dense_plans.size());
+  for (size_t d = 0; d < b->dense_plans.size(); ++d) {
+    const bool het = het_form(b, d, mode);
+    const DensePlan& pl = b->dense_plans[d];
+    b->run_macs[d] = {het ? b->het_plans[d].list4.macs : pl.list4.macs, het ? b->het_plans[d].list9.macs : pl.list9.macs};
+  }
   // buffers the chain needs exist before anything is launched or captured
   if ((mode & LGMI_MODE_EMIT_COUNTS) && b->d_counts.size() < b->rec_cap * 9ull) {
     CU(ctx, cudaStreamSynchronize(bstream(b)));
@@ -838,6 +932,9 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
   P.unit_rec_off = b->d_unit_rec_off;
   P.gram = b->d_gram;
   P.unit_mode = b->d_unit_mode;
+  P.unit_het = nullptr;
+  for (size_t d = 0; d < b->dense_plans.size(); ++d)
+    if (het_form(b, d, mode)) P.unit_het = b->d_unit_het;
   P.unit_base = b->unit_base;
   P.tile_counts = b->d_tile_counts;
 
@@ -866,13 +963,16 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
     CU(ctx, cudaMemsetAsync(b->d_unit_mode, 0, (size_t)b->n_units * sizeof(uint32_t), bstream(b)));
   for (const DensePlan& pl : b->dense_plans) {
     // K3: bit-planes -> 0/1 bytes -> count matrices on the tensor cores (lgmi_dense.cuh)
-    uint32_t* mode = b->d_unit_mode + pl.unit;
+    const size_t d = &pl - b->dense_plans.data();
+    const HetDensePlan* het = het_form(b, d, mode) ? &b->het_plans[d] : nullptr;
+    const uint32_t* het_rows = het ? b->d_het_rows + b->het_rows_off[d] : nullptr;
+    uint32_t* unit_mode = b->d_unit_mode + pl.unit;
     const uint32_t* planes = b->d_planes + pl.plane_off;
     const uint64_t K_pad = (uint64_t)pl.k_blocks * kDenseBK;
     if (pl.four) {
       CU(ctx, cudaMemsetAsync(b->d_oth_cnt, 0, (size_t)pl.S * sizeof(uint32_t), bstream(b)));
       k_dense_prep<<<dim3((pl.W + 7u) / 8u, pl.S_pad / 256u), 256, 0, bstream(b)>>>(planes, pl.S, pl.W, pl.S_pad, b->d_xt,
-                                                                                   b->d_oth_cnt, b->d_oth_list, pl.oth_cap, mode);
+                                                                                   b->d_oth_cnt, b->d_oth_list, pl.oth_cap, unit_mode);
       ++ctx->launches;
       // the "other" cells need the lists and the transposed planes only: counted on a second stream, beside the
       // X rows and the first tiles of the GEMM; joined below, before the next unit's k_dense_prep reuses the lists and
@@ -883,38 +983,48 @@ static int run_chain(lgmi_batch* b, int min_common, uint32_t mode, bool timing) 
       CU(ctx, cudaEventRecord(b->fix_fork.get(), bstream(b)));
       CU(ctx, cudaStreamWaitEvent(b->fix_stream.get(), b->fix_fork.get(), 0));
       k_other_fix<<<pl.S, kFixThreads, 0, b->fix_stream.get()>>>(b->d_xt, K_pad, pl.S, pl.S_pad, pl.rows, b->d_oth_cnt,
-                                                              b->d_oth_list, pl.oth_cap, b->d_gram + pl.gram_off, mode);
+                                                              b->d_oth_list, pl.oth_cap, b->d_gram + pl.gram_off, unit_mode,
+                                                              het ? b->d_flags + b->h_units[pl.unit].site_off : nullptr);
       ++ctx->launches;
       CU(ctx, cudaEventRecord(b->fix_join.get(), b->fix_stream.get()));
     } else {
-      CU(ctx, cudaMemsetAsync(mode, 1, sizeof(uint32_t), bstream(b)));  // (any non-zero value: nine blocks)
+      CU(ctx, cudaMemsetAsync(unit_mode, 1, sizeof(uint32_t), bstream(b)));  // (any non-zero value: nine blocks)
     }
-    {
+    if (!het || het->H) {  // (X is the B operand; the het form of a unit without het sites has no tiles)
       const uint64_t warps = (uint64_t)pl.S * ((pl.W + 7u) / 8u);
       const unsigned xgrid = (unsigned)std::min<uint64_t>((warps + 7) / 8, (uint64_t)ctx->num_sms * 16u);
-      k_dense_x<<<xgrid, 256, 0, bstream(b)>>>(planes, pl.S, pl.W, pl.S_pad, b->d_x, mode);
+      k_dense_x<<<xgrid, 256, 0, bstream(b)>>>(planes, pl.S, pl.W, pl.S_pad, b->d_x, unit_mode, nullptr);
+      ++ctx->launches;
+    }
+    if (het && het->H) {  // ... and the het sites' rows, packed, the A operand
+      const uint64_t warps = (uint64_t)het->H_pad * ((pl.W + 7u) / 8u);
+      const unsigned xgrid = (unsigned)std::min<uint64_t>((warps + 7) / 8, (uint64_t)ctx->num_sms * 16u);
+      k_dense_x<<<xgrid, 256, 0, bstream(b)>>>(planes, het->H_pad, pl.W, het->H_pad, b->d_x_het, unit_mode, het_rows);
       ++ctx->launches;
     }
     const bool last = &pl == &b->dense_plans.back();
     if (last && timing) CU(ctx, cudaEventRecord(b->ev[6].get(), bstream(b)));
     for (int form = pl.four ? 0 : 1; form < 2; ++form) {  // the launch of the form the unit is not in returns at once
-      const DenseTileList& L = form ? pl.list9 : pl.list4;
+      const DenseTileList& L = het ? (form ? het->list9 : het->list4) : (form ? pl.list9 : pl.list4);
+      if (!L.n) continue;
       DenseParams D;
-      D.tiles = b->d_tiles + L.off;
+      D.tiles = (het ? b->d_het_tiles : b->d_tiles) + L.off;
       D.n_tiles = L.n;
       D.k_blocks = pl.k_blocks;
       D.S_pad = pl.S_pad;
       D.gram = b->d_gram + pl.gram_off;
       D.error = reinterpret_cast<uint32_t*>(&b->d_header->pad);
-      D.mode = mode;
+      D.mode = unit_mode;
       D.nine = (uint32_t)form;
+      D.a_rows = het ? het->H_pad : pl.S_pad;
+      D.rows = het_rows;
       const unsigned ggrid = (unsigned)std::min<uint32_t>(L.n, (uint32_t)ctx->num_sms);
       if (L.n > L.n_whole) {
         k_zero_partial_tiles<<<L.n - L.n_whole, 256, 0, bstream(b)>>>(D.tiles + L.n_whole, L.n - L.n_whole, pl.S_pad, D.gram,
-                                                                     mode, (uint32_t)form);
+                                                                     unit_mode, (uint32_t)form, het_rows);
         ++ctx->launches;
       }
-      k_gram_i8<<<ggrid, kDenseThreads, kDenseSmemBytes, bstream(b)>>>(b->tmaps[&pl - b->dense_plans.data()], D);
+      k_gram_i8<<<ggrid, kDenseThreads, kDenseSmemBytes, bstream(b)>>>(het ? b->het_tmaps[d] : b->tmaps[d], b->tmaps[d], D);
       ++ctx->launches;
     }
     if (last && timing) CU(ctx, cudaEventRecord(b->ev[7].get(), bstream(b)));
@@ -1072,16 +1182,17 @@ static int fill_scalars(lgmi_batch* b, lgmi_result* out) {
     CU(ctx, cudaMemcpy(modes.data(), b->d_unit_mode, (size_t)b->n_units * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     b->dense_macs = 0;
     out->n_dense_four = 0;
-    for (const DensePlan& pl : b->dense_plans) {
+    for (size_t d = 0; d < b->dense_plans.size(); ++d) {
+      const DensePlan& pl = b->dense_plans[d];
       const bool nine = modes[pl.unit] != 0u;
-      b->dense_macs += nine ? pl.list9.macs : pl.list4.macs;
+      const uint64_t macs = nine ? b->run_macs[d].second : b->run_macs[d].first;
+      b->dense_macs += macs;
       out->n_dense_four += nine ? 0u : 1u;
+      if (timing && d + 1 == b->dense_plans.size()) out->gram_macs = macs;
     }
     if (timing) {
       CU(ctx, cudaEventElapsedTime(&ms, b->ev[6].get(), b->ev[7].get()));
       out->gram_kernel_ms = ms;
-      const DensePlan& pl = b->dense_plans.back();
-      out->gram_macs = modes[pl.unit] ? pl.list9.macs : pl.list4.macs;
     }
   }
   out->n_dense_units = (uint32_t)b->dense_plans.size();
@@ -1146,6 +1257,14 @@ extern "C" int lgmi_batch_device_ptrs(lgmi_batch_t* b, void** d_planes, void** d
   if (d_site_mean) *d_site_mean = b->d_site_mean;
   b->uploaded = true;  // a device-resident caller fills the buffers itself
   b->het_known = false;
+  // ... so the flags may change behind the host's back: the het plans and the graphs captured with them go, and runs
+  // keep the all-pairs form
+  if (!b->het_plans.empty()) {
+    CU(b->ctx, cudaSetDevice(b->ctx->device));
+    CU(b->ctx, cudaStreamSynchronize(bstream(b)));
+    b->graphs.clear();
+    b->het_plans.clear();
+  }
   return LGMI_OK;
 }
 
@@ -1504,6 +1623,7 @@ static int pipeline_begin(lgmi_pipeline* p, const uint32_t* planes, bool packed,
     if (f.run_mode & LGMI_MODE_SKIP_NONHET) {
       b->n_het_candidates = b->n_sites ? het_candidates(b->h_units, b->h_row_limit, site_flags + c.site0) : 0;
       b->het_known = true;
+      if (const int rc = plan_het(b, site_flags + c.site0, st)) return rc;
     }
     if (const int rc = lgmi_batch_run(b, min_common, f.run_mode)) return rc;
     if (f.split) {

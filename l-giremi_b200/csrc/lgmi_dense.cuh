@@ -30,6 +30,11 @@
 // k_count / k_pairs_generic then read the tables from the scratch instead of
 // popcounting (DevUnit::gram_off).
 //
+// Het-anchored form (HetDensePlan, HET_ONLY | SKIP_NONHET): k_dense_x also packs the het sites' rows into X_het,
+// k_gram_i8 takes its A operand from there and writes row h of a tile into row het[h], and k_other_fix writes the
+// "other" cells of the het rows on both sides of the diagonal; the readers take a pair whose first site is not het
+// from its second site's row, transposed.
+//
 // Reference semantics: the counts of /root/reference/src/giremi/mutual_information.py:15-40
 // (labels over the common reads), bit-exact.
 #pragma once
@@ -56,6 +61,8 @@ struct DenseParams {
   uint32_t* error;    // set to 1 if a barrier wait ran out (never in a correct run)
   const uint32_t* mode;  // the unit's form this run (0 four blocks, else nine): a launch whose list is of the
   uint32_t nine;         // other form (nine != 0 vs *mode != 0) returns at once
+  uint32_t a_rows;       // rows per group of the A operand: S_pad (X), or H_pad (X_het, the het-anchored form)
+  const uint32_t* rows;  // het-anchored form: the count-matrix row of each A row (~0: a pad row); NULL: the same row
 };
 
 // ------------------------------------------------------------------ expansion
@@ -149,9 +156,12 @@ __global__ void __launch_bounds__(256) k_dense_prep(const uint32_t* __restrict__
 // nine blocks -- X[g][s][r], one byte per read.  A warp takes 256 reads (8 words) of one site at a time: a lane
 // reads the word its 8 reads live in (one sector per plane and warp) and stores 8 bytes per group, so that every
 // warp-wide store is 256 contiguous bytes.  Independent of the lists and the transposed planes: in the
-// four-block form k_other_fix runs beside it on a second stream.
+// four-block form k_other_fix runs beside it on a second stream.  With `sites` (the het-anchored form) it writes
+// X_het instead: row s of each group holds site sites[s], and a row whose entry is ~0 (padding) is zeroed; S is
+// then the number of rows and S_pad the group stride.
 __global__ void __launch_bounds__(256) k_dense_x(const uint32_t* __restrict__ planes, uint32_t S, uint32_t W, uint32_t S_pad,
-                                                 uint8_t* __restrict__ X, const uint32_t* __restrict__ mode) {
+                                                 uint8_t* __restrict__ X, const uint32_t* __restrict__ mode,
+                                                 const uint32_t* __restrict__ sites) {
   const uint32_t nine = *mode;
   const uint32_t lane = threadIdx.x & 31u;
   const uint32_t k = lane >> 2, q4 = lane & 3u;
@@ -162,8 +172,12 @@ __global__ void __launch_bounds__(256) k_dense_x(const uint32_t* __restrict__ pl
   for (uint64_t e = warp0; e < total; e += n_warps) {
     const uint32_t s = (uint32_t)(e / octets), w = (uint32_t)(e - (uint64_t)s * octets) * 8u + k;
     if (w >= W) continue;
-    const uint32_t* row = planes + (size_t)s * 3u * W + w;
-    const uint32_t Cw = __ldg(row + 2u * W), Mw = __ldg(row) & Cw, Pw = (Mw | __ldg(row + W)) & Cw;
+    const uint32_t site = sites ? __ldg(sites + s) : s;
+    uint32_t Cw = 0u, Mw = 0u, Pw = 0u;
+    if (site != ~0u) {
+      const uint32_t* row = planes + (size_t)site * 3u * W + w;
+      Cw = __ldg(row + 2u * W), Mw = __ldg(row) & Cw, Pw = (Mw | __ldg(row + W)) & Cw;
+    }
     uint8_t* x = X + (size_t)s * K_pad + (size_t)w * 32u + q4 * 8u;
     const uint32_t sh = 8u * q4;
     if (nine) {
@@ -189,7 +203,9 @@ __global__ void __launch_bounds__(256) k_dense_x(const uint32_t* __restrict__ pl
 // 0 / 1 / 2 of pair (s, t), t > s, = reads "other" at s and other / minor / major at t; slot 3 / 6 of pair
 // (t, s), t < s, = reads minor / major at t and "other" at s.  rows: the row limit of a piece of a split unit
 // (S otherwise, a multiple of 128 below S): only pairs with a first site below it are read, so a site at or past
-// it counts its partners below the limit and nothing else.
+// it counts its partners below the limit and nothing else.  het (the unit's flag bytes, het-anchored form; else
+// NULL): only the rows of het sites are read, but on both sides of the diagonal -- row s gets slots 0 / 1 / 2 of
+// every partner t when s is het, and row t gets slots 3 / 6 of partner s when t is het.
 constexpr int kFixThreads = 384;  // 12 warps = 3 labels x 2 word halves x 2 read halves
 constexpr uint32_t kFixStride = 65u;  // words of shared memory per partner bit: (bit, word) and (word, bit) walks both hit 32 banks
 
@@ -198,7 +214,8 @@ __device__ __forceinline__ uint32_t fix_spread(uint32_t x, uint32_t q) { return 
 __global__ void __launch_bounds__(kFixThreads, 3) k_other_fix(const uint32_t* __restrict__ xt, uint64_t K_pad, uint32_t S,
                                                            uint32_t S_pad, uint32_t rows, const uint32_t* __restrict__ cnt,
                                                            const uint32_t* __restrict__ list, uint32_t cap,
-                                                           uint32_t* __restrict__ gram, const uint32_t* __restrict__ mode) {
+                                                           uint32_t* __restrict__ gram, const uint32_t* __restrict__ mode,
+                                                           const uint8_t* __restrict__ het) {
   if (*mode) return;
   __shared__ uint32_t acc[3][32u * kFixStride];  // [label][partner bit * 65 + site word of the pass]
   const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
@@ -274,12 +291,14 @@ __global__ void __launch_bounds__(kFixThreads, 3) k_other_fix(const uint32_t* __
       const uint32_t t = w0 * 32u + tl;
       if (t >= S || (s >= rows && t >= rows)) break;
       const uint32_t at = (tl & 31u) * kFixStride + (tl >> 5);
-      if (t > s) {
+      const bool fwd = het ? t != s && (het[s] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP : t > s, bwd = het ? t != s && (het[t] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP : t < s;
+      if (fwd) {
         uint32_t* out = gram + (size_t)s * S_pad + t;
         out[0] = acc[0][at];
         out[plane] = acc[1][at];
         out[2u * plane] = acc[2][at];
-      } else if (t < s) {
+      }
+      if (bwd) {
         uint32_t* out = gram + (size_t)t * S_pad + s;
         out[3u * plane] = acc[1][at];
         out[6u * plane] = acc[2][at];
@@ -378,19 +397,23 @@ __device__ __forceinline__ void tmem_load_32x32(uint32_t taddr, uint32_t (&r)[32
 // kb0 is 0 zeroes its tile, the others skip)
 __global__ void __launch_bounds__(256) k_zero_partial_tiles(const DenseTile* __restrict__ tiles, uint32_t n_tiles,
                                                             uint32_t S_pad, uint32_t* __restrict__ gram,
-                                                            const uint32_t* __restrict__ mode, uint32_t nine) {
+                                                            const uint32_t* __restrict__ mode, uint32_t nine,
+                                                            const uint32_t* __restrict__ rows) {
   if ((*mode != 0u) != (nine != 0u)) return;  // the list of the unit's other form
   const DenseTile tile = tiles[blockIdx.x];
   if (blockIdx.x >= n_tiles || !tile.partial || tile.kb0 != 0) return;
-  uint32_t* base = gram + ((size_t)(tile.a * 3u + tile.b) * S_pad + (size_t)tile.I * kDenseBM) * S_pad + (size_t)tile.J * kDenseBN;
+  uint32_t* base = gram + (size_t)(tile.a * 3u + tile.b) * S_pad * S_pad + (size_t)tile.J * kDenseBN;
   for (uint32_t e = threadIdx.x; e < (uint32_t)kDenseBM * (kDenseBN / 4); e += blockDim.x) {
-    const uint32_t row = e / (kDenseBN / 4), q = e % (kDenseBN / 4);
-    reinterpret_cast<uint4*>(base + (size_t)row * S_pad)[q] = make_uint4(0u, 0u, 0u, 0u);
+    const uint32_t r = tile.I * kDenseBM + e / (kDenseBN / 4), q = e % (kDenseBN / 4);
+    const uint32_t row = rows ? rows[r] : r;  // (het-anchored form: the tile's rows are the het sites' rows)
+    if (row != ~0u) reinterpret_cast<uint4*>(base + (size_t)row * S_pad)[q] = make_uint4(0u, 0u, 0u, 0u);
   }
 }
 
 // ------------------------------------------------------------------ the GEMM
-__global__ void __launch_bounds__(kDenseThreads, 1) k_gram_i8(const __grid_constant__ CUtensorMap tmap,
+// tmap_a: the A operand's rows (X, or X_het in the het-anchored form), tmap: X, the B operand's
+__global__ void __launch_bounds__(kDenseThreads, 1) k_gram_i8(const __grid_constant__ CUtensorMap tmap_a,
+                                                              const __grid_constant__ CUtensorMap tmap,
                                                               const DenseParams P) {
   if ((*P.mode != 0u) != (P.nine != 0u)) return;  // the list of the unit's other form (CTA-uniform, before any barrier)
   extern __shared__ uint8_t dense_smem_raw[];
@@ -406,6 +429,7 @@ __global__ void __launch_bounds__(kDenseThreads, 1) k_gram_i8(const __grid_const
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
 
   if (threadIdx.x == 0) {
+    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap_a) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap) : "memory");
     for (int s = 0; s < kDenseStages; ++s) {
       mbar_init(&full[s], 1);
@@ -431,7 +455,7 @@ __global__ void __launch_bounds__(kDenseThreads, 1) k_gram_i8(const __grid_const
       uint32_t stage = 0, phase = 0;
       for (uint32_t t = blockIdx.x; t < P.n_tiles; t += gridDim.x) {
         const DenseTile tile = P.tiles[t];
-        const int32_t row_a = (int32_t)(tile.a * P.S_pad + tile.I * kDenseBM);
+        const int32_t row_a = (int32_t)(tile.a * P.a_rows + tile.I * kDenseBM);
         const int32_t row_b = (int32_t)(tile.b * P.S_pad + tile.J * kDenseBN);
         for (uint32_t kb = tile.kb0; kb < tile.kb1; ++kb) {
           mbar_wait(&empty[stage], phase ^ 1u, P.error);
@@ -439,7 +463,7 @@ __global__ void __launch_bounds__(kDenseThreads, 1) k_gram_i8(const __grid_const
           uint8_t* sb = sa + kDenseBM * kDenseBK;
           mbar_expect_tx(&full[stage], kDenseStageBytes);
           const int32_t k0 = (int32_t)(kb * kDenseBK);
-          tma_load_2d(sa, &tmap, &full[stage], k0, row_a);
+          tma_load_2d(sa, &tmap_a, &full[stage], k0, row_a);
           tma_load_2d(sb, &tmap, &full[stage], k0, row_b);
           tma_load_2d(sb + 128 * kDenseBK, &tmap, &full[stage], k0, row_b + 128);
           if (++stage == kDenseStages) {
@@ -483,16 +507,18 @@ __global__ void __launch_bounds__(kDenseThreads, 1) k_gram_i8(const __grid_const
       const DenseTile tile = P.tiles[t];
       mbar_wait(acc_full, acc_phase, P.error);
       tc_fence_after();
-      const uint32_t row = tile.I * kDenseBM + q * 32u + lane;
-      uint32_t* out = P.gram + ((size_t)(tile.a * 3u + tile.b) * P.S_pad + row) * P.S_pad + (size_t)tile.J * kDenseBN;
+      const uint32_t a_row = tile.I * kDenseBM + q * 32u + lane;
+      const uint32_t row = P.rows ? __ldg(P.rows + a_row) : a_row;  // (~0: a pad row of X_het, not stored)
+      const bool store = row != ~0u;
+      uint32_t* out = P.gram + ((size_t)(tile.a * 3u + tile.b) * P.S_pad + (store ? row : 0u)) * P.S_pad + (size_t)tile.J * kDenseBN;
 #pragma unroll 1
       for (uint32_t c = 0; c < kDenseBN / 32; ++c) {
         uint32_t r[32];
         tmem_load_32x32(tmem_base + ((q * 32u) << 16) + c * 32u, r);
-        if (tile.partial) {
+        if (store && tile.partial) {
 #pragma unroll
           for (int v = 0; v < 32; ++v) atomicAdd(out + c * 32u + v, r[v]);  // (RED: no return value is used)
-        } else {
+        } else if (store) {
 #pragma unroll
           for (int v = 0; v < 8; ++v)
             reinterpret_cast<uint4*>(out + c * 32u)[v] = make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]);

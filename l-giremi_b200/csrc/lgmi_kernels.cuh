@@ -52,6 +52,8 @@ struct RunParams {
   uint32_t* n_generic;                 // items k_pairs_generic has to process (host count + dense ones)
   const uint32_t* gram;                // count matrices of the tensor-core path (DevUnit::gram_off)
   const uint32_t* unit_mode;           // per unit, tensor-core path: 0 four Gram blocks + "other" cells, else nine blocks
+  const uint8_t* unit_het;             // per unit, tensor-core path: 1 het-anchored count matrices (HetDensePlan); NULL:
+                                       // none this run
   uint32_t* tile_counts;               // EMIT_COUNTS: 3x3 tables of the k_tile_mi units, 9 per dense slot
   uint32_t unit_base;                  // added to the unit field of every record
   const TiledDesc* tiled_desc;         // k_pairs_generic<1>: its items, in item order
@@ -133,14 +135,21 @@ __device__ __forceinline__ bool pair_table(const uint4* __restrict__ ri, const u
 // Slot a * 3 + b of the scratch holds, for row group a of site i and b of site j (0 covered, 1 major or
 // minor, 2 major), |X_a,i & X_b,j|; the sets are nested, so the labels follow by inclusion-exclusion.
 // nine == 0 (four-block form): only slots 4, 5, 7, 8 are Gram blocks; slots 0, 1, 2, 3, 6 hold the cells
-// with an "other" label as k_other_fix counted them.
+// with an "other" label as k_other_fix counted them.  tr (het-anchored form, i not het): the pair is read from row
+// j, slot a * 3 + b from slot b * 3 + a.
 __device__ __forceinline__ uint32_t gram_table(const uint32_t* __restrict__ g, uint32_t S_pad, uint32_t i, uint32_t j,
-                                               uint32_t nine, uint32_t T[9]) {
+                                               uint32_t nine, uint32_t T[9], bool tr = false) {
   const size_t plane = (size_t)S_pad * S_pad;
-  const uint32_t* p = g + (size_t)i * S_pad + j;
+  const uint32_t* p = g + (tr ? (size_t)j * S_pad + i : (size_t)i * S_pad + j);
   uint32_t G[9];
 #pragma unroll
   for (int k = 0; k < 9; ++k) G[k] = __ldg(p + (size_t)k * plane);
+  if (tr) {
+    const uint32_t g1 = G[1], g2 = G[2], g5 = G[5];
+    G[1] = G[3], G[3] = g1;
+    G[2] = G[6], G[6] = g2;
+    G[5] = G[7], G[7] = g5;
+  }
   const uint32_t PP = G[4], PM = G[5], MP = G[7], MM = G[8];
   T[8] = MM;
   T[7] = MP - MM;            // i major, j minor
@@ -179,14 +188,21 @@ __device__ __forceinline__ uint32_t gram_table(const uint32_t* __restrict__ g, u
 // epilogues of lgmi_fast.cuh over full warps of each class; kKind 0: everything else.
 // 2x2 block of a deep unit's table alone (the pairs without an "other" label need nothing else)
 __device__ __forceinline__ void gram_table_2x2(const uint32_t* __restrict__ g, uint32_t S_pad, uint32_t i, uint32_t j,
-                                               uint32_t& mm, uint32_t& mM, uint32_t& Mm, uint32_t& MM) {
+                                               uint32_t& mm, uint32_t& mM, uint32_t& Mm, uint32_t& MM, bool tr = false) {
   const size_t plane = (size_t)S_pad * S_pad;
-  const uint32_t* p = g + (size_t)i * S_pad + j;
-  const uint32_t PP = __ldg(p + 4u * plane), PM = __ldg(p + 5u * plane), MP = __ldg(p + 7u * plane);
+  const uint32_t* p = g + (tr ? (size_t)j * S_pad + i : (size_t)i * S_pad + j);
+  const uint32_t PP = __ldg(p + 4u * plane), G5 = __ldg(p + 5u * plane), G7 = __ldg(p + 7u * plane);
+  const uint32_t PM = tr ? G7 : G5, MP = tr ? G5 : G7;
   MM = __ldg(p + 8u * plane);
   Mm = MP - MM;
   mM = PM - MM;
   mm = PP - MP - PM + MM;
+}
+
+// a deep unit's pair (i, j), i < j, is read transposed from row j when the unit's count matrices are het-anchored
+// (anchored: only the het sites' rows were written) and i is not het
+__device__ __forceinline__ bool gram_tr(bool anchored, const uint8_t* flags, uint32_t i) {
+  return anchored && (flags[i] & LGMI_SITE_TYPE_MASK) != LGMI_SITE_HET_SNP;
 }
 
 template <int kKind>
@@ -196,6 +212,7 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
   __shared__ uint32_t s_ij[kPairsMax];  // (i << 16) | j
   __shared__ uint32_t s_warp[kThreads / 32];
   __shared__ uint16_t s_list[kKind == 2 ? kPairsMax : 1];  // kKind 2: pairs with a 2x2 table from the front, the others from the back
+  __shared__ uint32_t s_tr[kKind == 2 ? kPairsMax / 32 : 1];  // kKind 2: bit pl: pair pl's table is read transposed (gram_tr)
   __shared__ uint32_t s_n2, s_n3;
   const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
   const LnGlobal ln{P.lntab};
@@ -281,6 +298,7 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
       const uint32_t n_slots = (it.pair_cnt + 31u) & ~31u;
       for (uint32_t pl = tid; pl < n_slots; pl += kThreads) {
         uint32_t cls = 0u;  // 0 no MI, 2 -> 2x2 list, 3 -> 3x3 list
+        bool tr = false;
         if (pl < it.pair_cnt) {
           if (pl != tid) lg_pair_advance(i, j, u.S, kThreads);
           s_ij[pl] = (i << 16) | j;
@@ -290,7 +308,8 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
                        ((flags[j] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP);
           if (evaluate) {
             uint32_t T[9];
-            const uint32_t n_common = gram_table(g, u.S_pad, i, j, nine, T);
+            tr = gram_tr(P.unit_het && P.unit_het[it.unit], flags, i);
+            const uint32_t n_common = gram_table(g, u.S_pad, i, j, nine, T, tr);
             if ((int)n_common >= P.min_common)  // strict '<' drops (mutual_information.py:19)
               cls = (T[0] | T[1] | T[2] | T[3] | T[6]) ? 3u : 2u;
           }
@@ -298,6 +317,8 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
         }
         const uint32_t m2 = __ballot_sync(0xffffffffu, cls == 2u);
         const uint32_t m3 = __ballot_sync(0xffffffffu, cls == 3u);
+        const uint32_t mt = __ballot_sync(0xffffffffu, tr);
+        if (lane == 0) s_tr[pl >> 5] = mt;  // (a warp's 32 slots are consecutive pairs)
         uint32_t b2 = 0u, b3 = 0u;
         if (lane == 0) {
           if (m2) b2 = atomicAdd(&s_n2, (uint32_t)__popc(m2));
@@ -320,7 +341,7 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
           if (q < n2) {
             const uint32_t pl = s_list[q], ij = s_ij[pl];
             uint32_t mm, mM, Mm, MM;
-            gram_table_2x2(g, u.S_pad, ij >> 16, ij & 0xffffu, mm, mM, Mm, MM);
+            gram_table_2x2(g, u.S_pad, ij >> 16, ij & 0xffffu, mm, mM, Mm, MM, (s_tr[pl >> 5] >> (pl & 31u)) & 1u);
             s_mi[pl] = small_counts ? mi_2x2(tab, mm, mM, Mm, MM) : lg_mi_from_2x2(mm, mM, Mm, MM, ln);
           }
         } else {
@@ -328,7 +349,7 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
           if (q < n3) {
             const uint32_t pl = s_list[kPairsMax - 1u - q], ij = s_ij[pl];
             uint32_t T[9];
-            gram_table(g, u.S_pad, ij >> 16, ij & 0xffffu, nine, T);
+            gram_table(g, u.S_pad, ij >> 16, ij & 0xffffu, nine, T, (s_tr[pl >> 5] >> (pl & 31u)) & 1u);
             s_mi[pl] = small_counts ? mi_3x3(tab, T) : lg_mi_from_table(T, ln);
           }
         }
@@ -404,7 +425,8 @@ __global__ void __launch_bounds__(kThreads, kKind == 1 ? 4 : (kKind == 2 ? 3 : 2
 #pragma unroll
             for (int k = 0; k < 9; ++k) T[k] = src[k];
           } else if (u.gram_off != kNoGram) {
-            gram_table(P.gram + u.gram_off, u.S_pad, ij >> 16, ij & 0xffffu, P.unit_mode[it.unit], T);
+            gram_table(P.gram + u.gram_off, u.S_pad, ij >> 16, ij & 0xffffu, P.unit_mode[it.unit], T,
+                       kKind == 2 && ((s_tr[pl >> 5] >> (pl & 31u)) & 1u));
           } else {
             const uint4* ri = base + (size_t)(ij >> 16) * 3u * W4;
             const uint4* rj = base + (size_t)(ij & 0xffffu) * 3u * W4;
@@ -753,8 +775,9 @@ __global__ void __launch_bounds__(kThreads) k_count(const RunParams P) {
         }
         uint32_t n;
         if (u.gram_off != kNoGram) {
+          const bool anchored = P.unit_het && P.unit_het[it.unit];
           uint32_t T[9];
-          n = gram_table(P.gram + u.gram_off, u.S_pad, i, j, P.unit_mode[it.unit], T);
+          n = gram_table(P.gram + u.gram_off, u.S_pad, i, j, P.unit_mode[it.unit], T, gram_tr(anchored, flags, i));
         } else {
           n = pair_common(base + (size_t)i * 3u * W4, base + (size_t)j * 3u * W4, W4);
         }

@@ -208,6 +208,35 @@ inline uint64_t het_candidates(const std::vector<lgmi_unit_desc>& units, const s
   return tot;
 }
 
+// One CTA per SM walks a tile list with stride #SMs: a last, partly filled wave leaves SMs idle for a whole tile
+// time, so its tiles (those listed from L.off on) are cut along K into as many parts as fill it (added atomically
+// into zeroed tiles); then the list's length and multiply-accumulates.
+inline void finish_dense_list(uint32_t k_blocks, uint32_t num_sms, std::vector<DenseTile>& tiles, DenseTileList& L) {
+  const uint32_t n = (uint32_t)(tiles.size() - L.off), grid = num_sms;
+  const uint32_t rem = n % grid;
+  uint32_t parts = rem ? std::min<uint32_t>(8u, grid / rem) : 1u;
+  while (parts > 1u && k_blocks < 8u * parts) --parts;  // at least 8 k-blocks (1 024 reads) per part
+  L.n_whole = n;
+  if (parts >= 2u) {
+    L.n_whole = n - rem;
+    std::vector<DenseTile> tail(tiles.end() - rem, tiles.end());
+    tiles.resize(tiles.size() - rem);
+    for (uint32_t q = 0; q < parts; ++q)
+      for (DenseTile t : tail) {
+        t.kb0 = (uint32_t)((uint64_t)k_blocks * q / parts);
+        t.kb1 = (uint32_t)((uint64_t)k_blocks * (q + 1) / parts);
+        t.partial = 1;
+        tiles.push_back(t);
+      }
+  }
+  L.n = (uint32_t)(tiles.size() - L.off);
+  L.macs = 0;
+  for (uint32_t t = 0; t < L.n; ++t) {
+    const DenseTile& dt = tiles[L.off + t];
+    L.macs += (uint64_t)kDenseBM * kDenseBN * (dt.kb1 - dt.kb0) * kDenseBK;
+  }
+}
+
 // k_gram_i8's work items for row groups g0 .. 2 of X against each other: the tiles holding a pair i < j with
 // i < pl.rows, both real sites
 inline void plan_dense_list(const DensePlan& pl, uint32_t g0, uint32_t num_sms, std::vector<DenseTile>& tiles,
@@ -222,30 +251,58 @@ inline void plan_dense_list(const DensePlan& pl, uint32_t g0, uint32_t num_sms, 
           if (J * (uint32_t)kDenseBN >= pl.S || i_min >= j_max) continue;
           tiles.push_back(DenseTile{(uint8_t)a, (uint8_t)bb, (uint16_t)I, (uint16_t)J, 0, 0u, pl.k_blocks});
         }
-  // one CTA per SM walks the list with stride #SMs: a last, partly filled wave leaves SMs idle for a whole
-  // tile time, so its tiles are cut along K into as many parts as fill it (added atomically into zeroed tiles)
-  const uint32_t n = (uint32_t)(tiles.size() - L.off), grid = num_sms;
-  const uint32_t rem = n % grid;
-  uint32_t parts = rem ? std::min<uint32_t>(8u, grid / rem) : 1u;
-  while (parts > 1u && pl.k_blocks < 8u * parts) --parts;  // at least 8 k-blocks (1 024 reads) per part
-  L.n_whole = n;
-  if (parts >= 2u) {
-    L.n_whole = n - rem;
-    std::vector<DenseTile> tail(tiles.end() - rem, tiles.end());
-    tiles.resize(tiles.size() - rem);
-    for (uint32_t q = 0; q < parts; ++q)
-      for (DenseTile t : tail) {
-        t.kb0 = (uint32_t)((uint64_t)pl.k_blocks * q / parts);
-        t.kb1 = (uint32_t)((uint64_t)pl.k_blocks * (q + 1) / parts);
-        t.partial = 1;
-        tiles.push_back(t);
-      }
+  finish_dense_list(pl.k_blocks, num_sms, tiles, L);
+}
+
+// The het-anchored form of a deep unit.  Under HET_ONLY | SKIP_NONHET only the pairs with a het_snp site are
+// evaluated, and the counts those need are the Gram blocks of the het sites' rows against all sites: k_gram_i8 takes
+// the A operand from X_het, the het sites' X rows packed into H_pad rows per group (pad rows zero), and writes row h
+// of a tile into row het[h] of the unit's count matrices.  A pair (i, j), i < j, is read from row i when i is het and
+// from row j, block index transposed, when only j is.
+struct HetDensePlan {
+  std::vector<uint32_t> het;   // the unit's het sites, ascending
+  uint32_t H = 0, H_pad = 0;   // their number, and that rounded up to a whole row block of 128
+  DenseTileList list4, list9;  // het row blocks x column blocks of groups P, M  /  C, P, M (offsets into `tiles`)
+  bool fewer = false;          // not a piece, and the het lists cost at most half the triangle's multiply-accumulates
+};
+
+// The het plan of deep unit pl from its flag bytes (unit_flags[0 .. S)); piece: the unit is a piece of a split unit
+// (row limit != 0), which keeps the all-pairs form.  Appends the tile lists to `tiles`.
+inline void plan_het_dense(const DensePlan& pl, const uint8_t* unit_flags, bool piece, uint32_t num_sms,
+                           std::vector<DenseTile>& tiles, HetDensePlan* out) {
+  HetDensePlan& h = *out;
+  h = HetDensePlan();
+  for (uint32_t s = 0; s < pl.S; ++s)
+    if ((unit_flags[s] & LGMI_SITE_TYPE_MASK) == LGMI_SITE_HET_SNP) h.het.push_back(s);
+  h.H = (uint32_t)h.het.size();
+  h.H_pad = (h.H + (uint32_t)kDenseBM - 1u) / (uint32_t)kDenseBM * (uint32_t)kDenseBM;
+  for (uint32_t g0 = 0; g0 < 2u; ++g0) {
+    if (g0 == 1u && !pl.four) continue;
+    DenseTileList& L = g0 ? h.list4 : h.list9;
+    L.off = tiles.size();
+    for (uint32_t a = g0; a < 3; ++a)
+      for (uint32_t bb = g0; bb < 3; ++bb)
+        for (uint32_t J = 0; J < pl.S_pad / (uint32_t)kDenseBN; ++J)
+          for (uint32_t I = 0; I < h.H_pad / (uint32_t)kDenseBM; ++I) {
+            // some pair (het[r], s), s != het[r], with r in row block I and s in column block J
+            const uint32_t s0 = J * (uint32_t)kDenseBN, r0 = I * (uint32_t)kDenseBM;
+            if (s0 >= pl.S) continue;
+            const uint32_t n_cols = std::min(pl.S - s0, (uint32_t)kDenseBN), n_rows = std::min(h.H - r0, (uint32_t)kDenseBM);
+            if (n_cols == 1u && n_rows == 1u && h.het[r0] == s0) continue;
+            tiles.push_back(DenseTile{(uint8_t)a, (uint8_t)bb, (uint16_t)I, (uint16_t)J, 0, 0u, pl.k_blocks});
+          }
+    finish_dense_list(pl.k_blocks, num_sms, tiles, L);
   }
-  L.n = (uint32_t)(tiles.size() - L.off);
-  for (uint32_t t = 0; t < L.n; ++t) {
-    const DenseTile& dt = tiles[L.off + t];
-    L.macs += (uint64_t)kDenseBM * kDenseBN * (dt.kb1 - dt.kb0) * kDenseBK;
-  }
+  // (at most half: the form adds a pass over the het rows and transposed table reads; on cfg3 it was faster at 0.44
+  // of the triangle's work and slower at 0.89 -- profiles/r4_dense_het_n1_fewer_macs_rule.json)
+  h.fewer = !piece && 2u * h.list9.macs <= pl.list9.macs && (!pl.four || 2u * h.list4.macs <= pl.list4.macs);
+}
+
+// whether a run takes the het form of a unit: only HET_ONLY | SKIP_NONHET evaluates the het pairs alone, and the
+// plan needs the flag bytes on the host (a caller that fills the device buffers itself keeps the all-pairs form)
+inline bool take_het_form(const HetDensePlan& h, uint32_t mode, bool host_flags) {
+  const uint32_t het_modes = LGMI_MODE_HET_ONLY | LGMI_MODE_SKIP_NONHET;
+  return host_flags && (mode & het_modes) == het_modes && h.fewer;
 }
 
 // a deep unit: its nine count matrices come from k_gram_i8
